@@ -33,7 +33,7 @@ extern "C" {
 #define HPD_EXPORT
 #endif
 
-#define HPD_ABI_VERSION 2
+#define HPD_ABI_VERSION 3
 #define HPD_MAX_KPTS 32     /* joints per person (COCO: 17) */
 #define HPD_MAX_PEOPLE 32   /* max_num_people == top-k; the warp-wide Hungarian handles n <= 32 */
 #define HPD_MAX_EMB 2       /* tag embedding dims: 1 (no flip test) or 2 (flip test) */
@@ -97,10 +97,12 @@ typedef struct HpdParams {
 } HpdParams;
 
 /* Device buffers written by the stages.  WPR = (W + 31) / 32 words per image row.
- * Every field is required by hpd_decode; single-stage calls document what they touch. */
+ * Every field but agg_tags / tag_inputs is required by hpd_decode; single-stage calls document what they touch. */
 typedef struct HpdBuffers {
   float* agg_hm;        /* [B,K,H,W]      aggregated heatmaps (results.py:227)                  */
-  float* agg_tags;      /* [B,K,H,W,E]    resized tags, E innermost (results.py:229-230)        */
+  float* agg_tags;      /* [B,K,H,W,E]    resized tags, E innermost (results.py:229-230).  May be NULL: the
+                         * tag stages then interpolate the tags they read from tag_inputs (bit-identical), and
+                         * hpd_aggregate_tags writes the map on demand                                          */
   uint32_t* nms_mask;   /* [B,K,H,WPR]    bit x%32 of word (y, x/32): pixel survives NMS         */
   float* nms_wmax;      /* [B,K,H,WPR]    max of the NMS'd values of the word's pixels           */
   float* hm_wmax;       /* [B,K,H,WPR]    max of the raw aggregated values of the word's pixels  */
@@ -119,6 +121,9 @@ typedef struct HpdBuffers {
   const double* inv_affine; /* [B][6] optional: per-image 2x3 matrix (row major) that maps network-input pixels back
                          * to the raw image, i.e. get_affine_transform(center, scale, 0, (W, H), inverse=True)
                          * (results.py:158-171, base/transforms/utils.py:25-57).  NULL = identity              */
+  HpdScaleInputs tag_inputs; /* read only when agg_tags is NULL: the tag-scale network outputs (tag, and tag_f when
+                         * E == 2; the other maps are ignored) the tag stages interpolate from.  hpd_decode fills it
+                         * from scales[tag_scale] itself; hpd_topk / hpd_adjust_refine need it from the caller */
 } HpdBuffers;
 
 /* Layout of one result record (all offsets in bytes from the start of the image's row; row_bytes % 8 == 0).
@@ -155,8 +160,13 @@ HPD_EXPORT const char* hpd_last_error_string(void);
 HPD_EXPORT int hpd_workspace_bytes(const HpdParams* p, size_t* out_bytes);
 
 /* (a)+(b) fused aggregation + NMS: model.py:85-96, results.py:46-67,225-230, grouping.py:80-83.
- * Reads scales[0..num_scales); writes agg_hm, agg_tags, nms_mask, nms_wmax, hm_wmax, tag_bmin, tag_bmax. */
+ * Reads scales[0..num_scales); writes agg_hm, agg_tags (unless NULL), nms_mask, nms_wmax, hm_wmax, tag_bmin, tag_bmax. */
 HPD_EXPORT int hpd_aggregate_nms(const HpdParams* p, const HpdScaleInputs* scales, const HpdBuffers* buf, void* stream);
+
+/* The tag half of hpd_aggregate_nms alone (results.py:229-230), for callers that decoded with agg_tags == NULL and
+ * want the map after all: reads the tag / tag_f maps of scales[tag_scale]; writes out [B,K,H,W,E], bit-identical to
+ * the agg_tags hpd_aggregate_nms writes. */
+HPD_EXPORT int hpd_aggregate_tags(const HpdParams* p, const HpdScaleInputs* scales, float* out, void* stream);
 
 /* Standalone bilinear resize with torch's CPU arithmetic (BaseKeypointsResult.match_heatmaps_size,
  * resize_heatmaps_list, resize_heatmaps: results.py:46-67).  in: [batch,channels,h,w] view;
@@ -170,7 +180,7 @@ HPD_EXPORT int hpd_resize_bilinear(const HpdMap* in, int batch, int channels, fl
 HPD_EXPORT int hpd_nms(const HpdParams* p, const HpdBuffers* buf, float* nms_out, void* stream);
 
 /* (c) per-joint top-k with torch-CPU (std::partial_sort) tie order: grouping.py:147-170.
- * Reads agg_hm, agg_tags, nms_mask, nms_wmax; writes scores_k, idx_k, coords_k, tags_k. */
+ * Reads agg_hm, agg_tags (or tag_inputs), nms_mask, nms_wmax; writes scores_k, idx_k, coords_k, tags_k. */
 HPD_EXPORT int hpd_topk(const HpdParams* p, const HpdBuffers* buf, void* stream);
 
 /* (d) associative-embedding grouping: grouping.py:85-145 + py_max_match :55-59 + fallback :262-269.
@@ -178,7 +188,8 @@ HPD_EXPORT int hpd_topk(const HpdParams* p, const HpdBuffers* buf, void* stream)
 HPD_EXPORT int hpd_group(const HpdParams* p, const HpdBuffers* buf, void* stream);
 
 /* (e) adjust + person score + refine: grouping.py:172-191, :276, :193-250.
- * Reads agg_hm, agg_tags, hm_wmax, tag_bmin, tag_bmax, idx_k, scores_k, n_person, flags; updates poses in place;
+ * Reads agg_hm, agg_tags (or tag_inputs), hm_wmax, tag_bmin, tag_bmax, idx_k, scores_k, tags_k (refine: the tags at idx_k, as
+ * hpd_topk writes them), n_person, flags; updates poses in place;
  * writes person_scores and, if buf->records is given, the per-image result records (back-projection through
  * buf->inv_affine + COCO layout, results.py:158-201,240-244, bin/eval.py:31-47) in the epilogue of its last kernel. */
 HPD_EXPORT int hpd_adjust_refine(const HpdParams* p, const HpdBuffers* buf, void* workspace, size_t workspace_bytes,
@@ -186,7 +197,9 @@ HPD_EXPORT int hpd_adjust_refine(const HpdParams* p, const HpdBuffers* buf, void
 
 /* Whole path: hpd_aggregate_nms -> hpd_topk -> hpd_group -> hpd_adjust_refine on one stream.
  * If scales == NULL the aggregation is skipped and buf->agg_hm / agg_tags are taken as inputs
- * (the MPPEHeatmapParser.parse entry, grouping.py:252). */
+ * (the MPPEHeatmapParser.parse entry, grouping.py:252).  With scales and agg_tags == NULL the tag stages read
+ * scales[tag_scale] (buf->tag_inputs is ignored); the network outputs must then stay unchanged until the call's
+ * work has run. */
 HPD_EXPORT int hpd_decode(const HpdParams* p, const HpdScaleInputs* scales, const HpdBuffers* buf, void* workspace,
                size_t workspace_bytes, void* stream);
 

@@ -63,11 +63,6 @@ struct AggArgs {
   int half_in;     // inputs are IEEE halves (HPD_F16); the const float* members then point at __half data
 };
 
-// element i of an input plane (generic kernel: the input type is a run-time flag)
-__device__ __forceinline__ float in_elem(const float* base, size_t i, int half_in) {
-  return half_in ? __half2float(reinterpret_cast<const __half*>(base)[i]) : base[i];
-}
-
 // ---------------------------------------------------------------------------------------------
 // NMS on a (TH+4)x(TW+4) tile already in shared memory (pixels outside the image hold -inf).
 // rowM is scratch [OT_R][TW].  Plane pointers are already offset to this (image, joint).
@@ -294,6 +289,7 @@ __global__ void __launch_bounds__(kAggThreads) agg_nms_generic_kernel(const AggA
              a.hmax + plane * H * a.wpr, a.tmin + plane * ((H + 3) / 4) * a.wpr, a.tmax + plane * ((H + 3) / 4) * a.wpr,
              nullptr);
   }
+  if (a.agg_tags == nullptr) return;   // the tag stages interpolate the few tags they read (tag_at)
   __syncthreads();
 
   // tags (results.py:229-230): E source tiles, single resize, E-innermost stores
@@ -415,6 +411,18 @@ __global__ void __launch_bounds__(256) resize_kernel(const float* __restrict__ i
 }
 
 // ---------------------------------------------------------------------------------------------
+// the full-resolution tag map alone (hpd_aggregate_tags): one thread per output pixel, E-innermost stores
+// ---------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) aggregate_tags_kernel(const TagSource s, float* __restrict__ out) {
+  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y, row = blockIdx.z;
+  if (x >= s.W) return;
+  float t[HPD_MAX_EMB];
+  tag_at(s, row / s.K, row % s.K, y, x, t);
+  float* o = out + (((size_t)row * s.H + y) * s.W + x) * s.E;
+  for (int e = 0; e < s.E; ++e) o[e] = t[e];
+}
+
+// ---------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------
 namespace {
@@ -448,12 +456,62 @@ int check_map(const HpdMap& m, const char* name, bool required) {
   return HPD_OK;
 }
 
+// TagSource over the tag-scale inputs (map = NULL)
+int tag_source_from_inputs(const HpdParams* p, const HpdScaleInputs& in, TagSource* s, const char* who) {
+  if (in.tag.ptr == nullptr || in.tag.h <= 0 || in.tag.w <= 0 || (in.tag.dtype != HPD_F32 && in.tag.dtype != HPD_F16)) {
+    set_error("%s: the tag map of the tag scale is missing or malformed", who);
+    return HPD_EINVAL;
+  }
+  if ((p->emb == 2) != (in.tag_f.ptr != nullptr)) {
+    set_error("%s: emb must be 2 iff the flipped-run tag map is given (got emb=%d)", who, p->emb);
+    return HPD_EINVAL;
+  }
+  if (in.tag_f.ptr && (in.tag_f.h != in.tag.h || in.tag_f.w != in.tag.w || in.tag_f.dtype != in.tag.dtype)) {
+    set_error("%s: the flipped-run tag map must have the shape and dtype of the un-flipped one", who);
+    return HPD_EINVAL;
+  }
+  memset(s, 0, sizeof(*s));
+  s->tag = (const float*)in.tag.ptr; s->tag_sb = in.tag.stride_b; s->tag_sc = in.tag.stride_c;
+  s->tag_f = (const float*)in.tag_f.ptr; s->tagf_sb = in.tag_f.stride_b; s->tagf_sc = in.tag_f.stride_c;
+  s->K = p->num_kpts; s->H = p->out_h; s->W = p->out_w; s->E = p->emb;
+  s->th = in.tag.h; s->tw = in.tag.w;
+  s->s_y = (float)s->th / (float)s->H; s->s_x = (float)s->tw / (float)s->W;   // as launch_aggregate_nms computes them
+  s->half_in = in.tag.dtype == HPD_F16;
+  s->tags_preflipped = p->tags_preflipped;
+  for (int k = 0; k < HPD_MAX_KPTS; ++k) s->flip[k] = p->flip_index[k];
+  return HPD_OK;
+}
+
 }  // namespace
 
+int make_tag_source(const HpdParams* p, const HpdBuffers* buf, TagSource* s, const char* who) {
+  if (buf->agg_tags == nullptr) return tag_source_from_inputs(p, buf->tag_inputs, s, who);
+  memset(s, 0, sizeof(*s));
+  s->map = buf->agg_tags;
+  s->K = p->num_kpts; s->H = p->out_h; s->W = p->out_w; s->E = p->emb;
+  return HPD_OK;
+}
+
+int launch_aggregate_tags(const HpdParams* p, const HpdScaleInputs* scales, float* out, cudaStream_t st) {
+  if (!scales || !out) {
+    set_error("hpd_aggregate_tags: scales and out are required");
+    return HPD_EINVAL;
+  }
+  TagSource s;
+  if (int rc = tag_source_from_inputs(p, scales[p->tag_scale], &s, "hpd_aggregate_tags")) return rc;
+  if (p->out_h > 65535) {
+    set_error("hpd_aggregate_tags: out_h must be <= 65535");
+    return HPD_EINVAL;
+  }
+  const dim3 grid((p->out_w + 255) / 256, p->out_h, p->batch * p->num_kpts);
+  aggregate_tags_kernel<<<grid, 256, 0, st>>>(s, out);
+  count_launch();
+  return check_launch("aggregate_tags_kernel");
+}
+
 int launch_aggregate_nms(const HpdParams* p, const HpdScaleInputs* scales, const HpdBuffers* buf, cudaStream_t st) {
-  if (!scales || !buf->agg_hm || !buf->agg_tags || !buf->nms_mask || !buf->nms_wmax || !buf->hm_wmax || !buf->tag_bmin ||
-      !buf->tag_bmax) {
-    set_error("hpd_aggregate_nms: scales, agg_hm, agg_tags, nms_mask, nms_wmax, hm_wmax, tag_bmin, tag_bmax are required");
+  if (!scales || !buf->agg_hm || !buf->nms_mask || !buf->nms_wmax || !buf->hm_wmax || !buf->tag_bmin || !buf->tag_bmax) {
+    set_error("hpd_aggregate_nms: scales, agg_hm, nms_mask, nms_wmax, hm_wmax, tag_bmin, tag_bmax are required");
     return HPD_EINVAL;
   }
   AggArgs a;
@@ -547,10 +605,14 @@ int launch_aggregate_nms(const HpdParams* p, const HpdScaleInputs* scales, const
       const int NW = a.W >= 512 ? 4 : (a.W >= 256 ? 2 : 1);
       const size_t smem = sizeof(float) * x2::smem_floats(NW, a.E);
       const dim3 grid((a.W + 128 * NW - 1) / (128 * NW), (a.H + x2::RB - 1) / x2::RB, a.B * a.K);
+#define HPD_X2_LAUNCH_WT(E_, NW_, T_, WT_)                                                                  \
+  do {                                                                                                      \
+    if (int rc_ = ensure_dynamic_smem((const void*)x2::agg_nms_x2_kernel<E_, NW_, T_, WT_>, smem, "agg_nms_x2_kernel")) return rc_; \
+    x2::agg_nms_x2_kernel<E_, NW_, T_, WT_><<<grid, 32 * NW_, smem, st>>>(a);                               \
+  } while (0)
 #define HPD_X2_LAUNCH_T(E_, NW_, T_)                                                                        \
   do {                                                                                                      \
-    if (int rc_ = ensure_dynamic_smem((const void*)x2::agg_nms_x2_kernel<E_, NW_, T_>, smem, "agg_nms_x2_kernel")) return rc_; \
-    x2::agg_nms_x2_kernel<E_, NW_, T_><<<grid, 32 * NW_, smem, st>>>(a);                                    \
+    if (a.agg_tags) HPD_X2_LAUNCH_WT(E_, NW_, T_, true); else HPD_X2_LAUNCH_WT(E_, NW_, T_, false);         \
   } while (0)
 #define HPD_X2_LAUNCH(E_, NW_)                                                                              \
   do {                                                                                                      \
@@ -560,6 +622,7 @@ int launch_aggregate_nms(const HpdParams* p, const HpdScaleInputs* scales, const
       else          { if (NW == 4) HPD_X2_LAUNCH(2, 4); else if (NW == 2) HPD_X2_LAUNCH(2, 2); else HPD_X2_LAUNCH(2, 1); }
 #undef HPD_X2_LAUNCH
 #undef HPD_X2_LAUNCH_T
+#undef HPD_X2_LAUNCH_WT
       count_launch();
       return check_launch("agg_nms_x2_kernel");
     }

@@ -11,7 +11,9 @@
 //   * phase 0 (tags first): the tag tiles are staged (16-byte loads, one warp per tile row, the flipped
 //     run read mirrored with the permuted joint index) and every lane writes its 4 columns of all rows
 //     with x4 taps and E-innermost 16-byte stores, plus the per-(4 rows x word) bounds of the first tag
-//     component; the tag tiles alias the half-res tile, so shared memory stays at 30 KB (6 CTAs/SM);
+//     component; the tag tiles alias the half-res tile, so shared memory stays at 30 KB (6 CTAs/SM).
+//     Without a tag map to write (WRITE_TAGS = false, the decode's default) only the first component is
+//     staged and only its bounds are derived: the map was two thirds of the kernel's HBM writes;
 //   * phase 1 (all threads): flip-averaged quarter-res / half-res tiles -> smem, tile interiors 16-byte
 //     aligned, two rows per batch so that all loads of a batch are in flight before the first store;
 //   * phase 2 (all threads): stage mean S at half resolution, in place, exact torch arithmetic
@@ -263,8 +265,9 @@ struct NmsColumnWalk {
 // ([E][TR][tc], tile origin column txo, tile row r = quarter-res row y0/4 - 1 + r) to the E-innermost
 // output, for the lane's 4 output columns X0..X0+3 and the RB rows from y0; plus the per (4 rows x 32
 // columns) range of the first tag component (tag_bmin / tag_bmax, the refine prefilter).  Called by the
-// lanes whose columns are inside the image (W % 32 == 0: whole 8-lane word groups).
-template <int E, int RB, int TR>
+// lanes whose columns are inside the image (W % 32 == 0: whole 8-lane word groups).  WRITE = false: only the
+// bounds (sT then needs only component 0); the output map is left alone, as it is when a.agg_tags is NULL.
+template <int E, int RB, int TR, bool WRITE = true>
 __device__ __forceinline__ void tags_x4_band(const AggArgs& a, const float* __restrict__ sT, int tc, int txo, int X0,
                                              int y0, int b, int k, int lane) {
   const int H = a.H, W = a.W;
@@ -283,6 +286,7 @@ __device__ __forceinline__ void tags_x4_band(const AggArgs& a, const float* __re
       const float* t = sT + e * TR * tc + r * tc + tb;
       const float t0 = t[0], t1 = t[1], t2 = t[2];
       if (e == 0) { mn = fminf(fminf(t0, t1), t2); mx = fmaxf(fmaxf(t0, t1), t2); }
+      if (!WRITE) continue;
       const float a0 = x_first ? t1 : t0, b0 = x_first ? t2 : t1;
       h[e][0] = fmaf(wa0, a0, __fmul_rn(wb0, b0));
       h[e][1] = fmaf(wa1, a0, __fmul_rn(wb1, b0));
@@ -292,7 +296,7 @@ __device__ __forceinline__ void tags_x4_band(const AggArgs& a, const float* __re
   };
   float* tg_plane = a.agg_tags + ((size_t)b * a.K + k) * H * W * E;
   auto emit = [&](int y, float wy0, float wy1, const float (&A)[E][4], const float (&Bv)[E][4]) {
-    if (y < y0 || y >= y0 + RB || y >= H) return;
+    if (!WRITE || a.agg_tags == nullptr || y < y0 || y >= y0 + RB || y >= H) return;
     float o[E][4];
 #pragma unroll
     for (int e = 0; e < E; ++e)
@@ -355,7 +359,9 @@ __device__ __forceinline__ void tags_x4_band(const AggArgs& a, const float* __re
   }
 }
 
-template <int E, int NW, typename T>
+// WRITE_TAGS = false (a.agg_tags == NULL): phase 0 stages only the first tag component and derives only its
+// bounds; the tag stages interpolate the few tags they read themselves (tag_at).
+template <int E, int NW, typename T, bool WRITE_TAGS>
 __global__ void __launch_bounds__(32 * NW) agg_nms_x2_kernel(const AggArgs a) {
   extern __shared__ __align__(16) float smem[];
   constexpr int sc = 64 * NW + 8, lc = 32 * NW + 8, tc = 32 * NW + 8;
@@ -388,18 +394,18 @@ __global__ void __launch_bounds__(32 * NW) agg_nms_x2_kernel(const AggArgs a) {
   {
     const T* tg0 = reinterpret_cast<const T*>(a.tag) + (size_t)b * a.tag_sb + (size_t)k * a.tag_sc;
     const bool unflip = !a.tags_preflipped;   // model.py:93: flip(tag_f, W)[:, FLIP]
-    const T* tg1 = (E > 1) ? reinterpret_cast<const T*>(a.tag_f) + (size_t)b * a.tagf_sb + (size_t)(unflip ? kf : k) * a.tagf_sc : nullptr;
+    const T* tg1 = (E > 1 && WRITE_TAGS) ? reinterpret_cast<const T*>(a.tag_f) + (size_t)b * a.tagf_sb + (size_t)(unflip ? kf : k) * a.tagf_sc : nullptr;
     if (a.in_vec_ok) {
       stage_tile<0, TR, tc, NW, true>(sT, tg0, (const T*)nullptr, false, tyo, txo, a.th, a.tw, warp, lane);
-      if (E > 1) stage_tile<1, TR, tc, NW, true>(sT + TR * tc, (const T*)nullptr, tg1, unflip, tyo, txo, a.th, a.tw, warp, lane);
+      if (E > 1 && WRITE_TAGS) stage_tile<1, TR, tc, NW, true>(sT + TR * tc, (const T*)nullptr, tg1, unflip, tyo, txo, a.th, a.tw, warp, lane);
     } else {
       stage_tile<0, TR, tc, NW, false>(sT, tg0, (const T*)nullptr, false, tyo, txo, a.th, a.tw, warp, lane);
-      if (E > 1) stage_tile<1, TR, tc, NW, false>(sT + TR * tc, (const T*)nullptr, tg1, unflip, tyo, txo, a.th, a.tw, warp, lane);
+      if (E > 1 && WRITE_TAGS) stage_tile<1, TR, tc, NW, false>(sT + TR * tc, (const T*)nullptr, tg1, unflip, tyo, txo, a.th, a.tw, warp, lane);
     }
   }
   __syncthreads();
   // ---------------- phase 0b: tags, x4 taps (results.py:229-230) ------------------------------------
-  if (active) tags_x4_band<E, RB, TR>(a, sT, tc, txo, X0, y0, b, k, lane);
+  if (active) tags_x4_band<WRITE_TAGS ? E : 1, RB, TR, WRITE_TAGS>(a, sT, tc, txo, X0, y0, b, k, lane);
   __syncthreads();   // every warp is done with the tag tiles before the half-res tile overwrites them
 
   // ---------------- phase 1: stage the heatmap inputs -------------------------------------------------

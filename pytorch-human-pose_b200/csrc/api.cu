@@ -110,6 +110,14 @@ int hpd_aggregate_nms(const HpdParams* p, const HpdScaleInputs* scales, const Hp
   return launch_aggregate_nms(p, scales, buf, (cudaStream_t)stream);
 }
 
+int hpd_aggregate_tags(const HpdParams* p, const HpdScaleInputs* scales, float* out, void* stream) {
+  g_launches = 0;
+  const HpdBuffers none = {};
+  int rc = validate(p, &none);
+  if (rc) return rc;
+  return launch_aggregate_tags(p, scales, out, (cudaStream_t)stream);
+}
+
 int hpd_nms(const HpdParams* p, const HpdBuffers* buf, float* nms_out, void* stream) {
   g_launches = 0;
   int rc = validate(p, buf);
@@ -195,12 +203,17 @@ int hpd_decode(const HpdParams* p, const HpdScaleInputs* scales, const HpdBuffer
   int rc = validate(p, buf);
   if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
-  if (scales) rc = launch_aggregate_nms(p, scales, buf, st);
-  else rc = launch_nms(p, buf, nullptr, st);
+  HpdBuffers b = *buf;
+  if (scales) {
+    rc = launch_aggregate_nms(p, scales, &b, st);
+    b.tag_inputs = scales[p->tag_scale];   // the tag stages interpolate from these when agg_tags is NULL
+  } else {
+    rc = launch_nms(p, &b, nullptr, st);
+  }
   if (rc) return rc;
-  if ((rc = launch_topk(p, buf, st))) return rc;
-  if ((rc = launch_group(p, buf, st))) return rc;
-  return launch_adjust_refine(p, buf, workspace, workspace_bytes, st);
+  if ((rc = launch_topk(p, &b, st))) return rc;
+  if ((rc = launch_group(p, &b, st))) return rc;
+  return launch_adjust_refine(p, &b, workspace, workspace_bytes, st);
 }
 
 }  // extern "C"

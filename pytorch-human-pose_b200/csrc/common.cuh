@@ -2,6 +2,7 @@
 // fused multiply-adds in the library are the explicit fmaf() calls that reproduce torch's CPU
 // bilinear kernel (SURVEY.md App. A.2).
 #pragma once
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdint.h>
@@ -52,6 +53,59 @@ __device__ __forceinline__ float lerp2(float wx0, float wx1, float hy0, float hy
   const float top = fmaf(wx0, v00, __fmul_rn(wx1, v01));
   const float bot = fmaf(wx0, v10, __fmul_rn(wx1, v11));
   return fmaf(hy0, top, __fmul_rn(hy1, bot));
+}
+
+// element i of an input plane; half_in: the plane holds IEEE halves (HPD_F16), widened exactly
+__device__ __forceinline__ float in_elem(const float* base, size_t i, int half_in) {
+  return half_in ? __half2float(reinterpret_cast<const __half*>(base)[i]) : base[i];
+}
+#endif  // __CUDACC__
+
+// ---- tag values at full resolution (results.py:229-230) -----------------------------------------
+// Where the tag stages read a tag: the full-resolution map agg_tags [B,K,H,W,E] when the caller keeps one,
+// otherwise the tag-scale network outputs, interpolated at the pixel (tag_at).  The map is never read
+// densely (top-k winners, detected joints, refine candidates), so interpolating where it is read saves
+// writing 4*K*H*W*E bytes per image.
+struct TagSource {
+  const float* map;                  // [B,K,H,W,E] or NULL: interpolate from tag / tag_f
+  const float *tag, *tag_f;          // tag-scale maps (tag_f: flipped run, E == 2); __half data if half_in
+  long long tag_sb, tag_sc, tagf_sb, tagf_sc;
+  int K, H, W, E;
+  int th, tw;                        // tag-scale map size
+  float s_y, s_x;                    // th / H, tw / W
+  int half_in, tags_preflipped;
+  int flip[HPD_MAX_KPTS];
+};
+
+#ifdef __CUDACC__
+// The tag vector of output pixel (y, x) of plane (b, k), exactly as the aggregation kernels write it: the
+// generic kernel's taps (axis_tap on both axes, lerp2), the flipped run read at the mirrored column and the
+// flipped joint unless tags_preflipped (model.py:93).  t[e] for e >= E is left alone.
+__device__ __forceinline__ void tag_at(const TagSource& s, int b, int k, int y, int x, float (&t)[HPD_MAX_EMB]) {
+  const Tap tx = axis_tap(s.s_x, x, s.tw, s.W), ty = axis_tap(s.s_y, y, s.th, s.H);
+#pragma unroll
+  for (int e = 0; e < HPD_MAX_EMB; ++e) {
+    if (e >= s.E) break;
+    const bool unflip = (e == 1) && !s.tags_preflipped;
+    const float* p = (e == 0) ? s.tag : s.tag_f;
+    const size_t po = (e == 0) ? (size_t)b * s.tag_sb + (size_t)k * s.tag_sc
+                               : (size_t)b * s.tagf_sb + (size_t)(unflip ? s.flip[k] : k) * s.tagf_sc;
+    const int c0 = unflip ? s.tw - 1 - tx.i0 : tx.i0, c1 = unflip ? s.tw - 1 - tx.i1 : tx.i1;
+    const size_t r0 = po + (size_t)ty.i0 * s.tw, r1 = po + (size_t)ty.i1 * s.tw;
+    t[e] = lerp2(tx.w0, tx.w1, ty.w0, ty.w1, in_elem(p, r0 + c0, s.half_in), in_elem(p, r0 + c1, s.half_in),
+                 in_elem(p, r1 + c0, s.half_in), in_elem(p, r1 + c1, s.half_in));
+  }
+}
+
+// tag vector of pixel idx = y*W + x of plane row = b*K + k: from the map if there is one, else tag_at
+__device__ __forceinline__ void tag_value(const TagSource& s, int row, int idx, float (&t)[HPD_MAX_EMB]) {
+  if (s.map != nullptr) {
+    const float* q = s.map + ((size_t)row * s.H * s.W + idx) * s.E;
+    t[0] = q[0];
+    if (s.E > 1) t[1] = q[1];
+  } else {
+    tag_at(s, row / s.K, row % s.K, idx / s.W, idx % s.W, t);
+  }
 }
 
 // order-preserving float -> signed int map (for redux.sync max)
@@ -123,6 +177,9 @@ __host__ __device__ inline HpdRecordLayout record_layout(int K, int M, int E) {
 
 // ---- per-stage launchers (defined in the stage .cu files) -------------------------------------
 int launch_aggregate_nms(const HpdParams* p, const HpdScaleInputs* scales, const HpdBuffers* buf, cudaStream_t st);
+int launch_aggregate_tags(const HpdParams* p, const HpdScaleInputs* scales, float* out, cudaStream_t st);
+// where the tag stages read tags: buf->agg_tags if set, else buf->tag_inputs (HPD_EINVAL if neither is given)
+int make_tag_source(const HpdParams* p, const HpdBuffers* buf, TagSource* s, const char* who);
 int launch_nms(const HpdParams* p, const HpdBuffers* buf, float* nms_out, cudaStream_t st);
 int launch_topk(const HpdParams* p, const HpdBuffers* buf, cudaStream_t st);
 int launch_group(const HpdParams* p, const HpdBuffers* buf, cudaStream_t st);

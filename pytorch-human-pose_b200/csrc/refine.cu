@@ -77,8 +77,9 @@ __device__ __forceinline__ void quarter_offset(const float* __restrict__ m, int 
 // one warp per person, one block per image.  Coordinates come from the top-k stage inside hpd_decode and are
 // always inside the map; the standalone adjust / refine twins receive caller-supplied coordinates, which are
 // clamped to the map before any read (the Python wrappers reject them where the reference would raise).
-__global__ void __launch_bounds__(32 * HPD_MAX_PEOPLE) adjust_prepare_kernel(const float* __restrict__ agg_hm, const float* __restrict__ agg_tags,
-                                      const int32_t* __restrict__ idx_k, const int32_t* __restrict__ n_person, int K,
+__global__ void __launch_bounds__(32 * HPD_MAX_PEOPLE) adjust_prepare_kernel(const float* __restrict__ agg_hm, const TagSource tags,
+                                      const int32_t* __restrict__ idx_k, const float* __restrict__ tags_k,
+                                      const int32_t* __restrict__ n_person, int K,
                                       int M, int E, int H, int W, int do_adjust, int do_refine,
                                       float* __restrict__ poses, float* __restrict__ person_scores, RefineWs ws) {
   __shared__ float s_score[HPD_MAX_PEOPLE][HPD_MAX_KPTS];
@@ -91,7 +92,6 @@ __global__ void __launch_bounds__(32 * HPD_MAX_PEOPLE) adjust_prepare_kernel(con
   if (threadIdx.x < HPD_MAX_KPTS) s_cnt[threadIdx.x] = 0;
   __syncthreads();
   const float* hm_b = agg_hm + (size_t)b * K * H * W;
-  const float* tg_b = agg_tags + (size_t)b * K * H * W * E;
   float T0 = 0.f, T1 = 0.f;
   bool missing = false;
   if (p < P) {
@@ -113,7 +113,8 @@ __global__ void __launch_bounds__(32 * HPD_MAX_PEOPLE) adjust_prepare_kernel(con
     if (has && do_refine) {
       const int pos = __popc(hmask & ((1u << lane) - 1u));
       const int xi = min(max((int)x, 0), W - 1), yi = min(max((int)y, 0), H - 1);
-      const float* t = tg_b + (((size_t)lane * H + yi) * W + xi) * E;
+      float t[HPD_MAX_EMB];
+      tag_value(tags, b * K + lane, yi * W + xi, t);
       s_tl[p][pos][0] = t[0];
       s_tl[p][pos][1] = (E > 1) ? t[1] : 0.f;
     }
@@ -143,10 +144,10 @@ __global__ void __launch_bounds__(32 * HPD_MAX_PEOPLE) adjust_prepare_kernel(con
     const size_t bk = (size_t)b * K + lane;
     ws.miss_pid[bk * M + slot] = p;
     const float* m = hm_b + (size_t)lane * H * W;
-    const float* t = tg_b + (size_t)lane * H * W * E;
     unsigned long long best = 0ull;
     // eight candidates at a time: their index loads, then their heatmap / tag loads, are all in flight together
-    // (one dependent DRAM round trip per candidate made this loop most of the kernel's 30 us)
+    // (one dependent DRAM round trip per candidate made this loop most of the kernel's 30 us).  The candidates'
+    // tags are the top-k stage's tags_k (the tags at idx_k), not re-read or re-interpolated.
     for (int j0 = 0; j0 < M; j0 += 8) {
       int idx[8];
       float hv[8], t0[8], t1[8];
@@ -156,9 +157,10 @@ __global__ void __launch_bounds__(32 * HPD_MAX_PEOPLE) adjust_prepare_kernel(con
       for (int u = 0; u < 8; ++u) {
         hv[u] = t0[u] = t1[u] = 0.f;
         if (idx[u] >= 0) {
+          const size_t o = (bk * M + j0 + u) * E;
           hv[u] = m[idx[u]];
-          t0[u] = t[(size_t)idx[u] * E];
-          if (E > 1) t1[u] = t[(size_t)idx[u] * E + 1];
+          t0[u] = tags_k[o];
+          if (E > 1) t1[u] = tags_k[o + 1];
         }
       }
 #pragma unroll
@@ -183,8 +185,56 @@ constexpr int kScanWarps = 16;
 // word is pruned by its maximum instead of being climbed flank by flank in index order; the word maxima of
 // sweep 1 are re-read from cache.  (Round 1 ran the sweeps as two launches of 8 CTAs per plane with the bests in
 // global memory: twice the chunk bookkeeping, and an L2 round trip per chunk for the bests.)
+// Tags of the 32 pixels (y, x0 + lane) of one image row word, loaded by the whole warp (lanes right of the image
+// get the last column's).  From the map: one load per lane and component.  Interpolated: the word's pixels share
+// their two source rows and span a few source columns (10 at the x4 tag resolution), so every distinct source value
+// is loaded once, by the lane of its column, and shuffled to the lanes whose taps use it -- instead of four loads per
+// lane and component.  Bit-identical to tag_at.
+__device__ __forceinline__ void word_tags(const TagSource& s, int b, int k, int y, int x0, int lane, float& t0, float& t1) {
+  const int x = min(x0 + lane, s.W - 1);
+  t1 = 0.f;
+  if (s.map != nullptr) {
+    const float* q = s.map + (((size_t)b * s.K + k) * s.H * s.W + (size_t)y * s.W + x) * s.E;
+    t0 = q[0];
+    if (s.E > 1) t1 = q[1];
+    return;
+  }
+  const Tap tx = axis_tap(s.s_x, x, s.tw, s.W), ty = axis_tap(s.s_y, y, s.th, s.H);
+  const int c_lo = __shfl_sync(kFull, tx.i0, 0);
+  const int span = __shfl_sync(kFull, tx.i1, 31) - c_lo + 1;   // taps are monotone in x
+  if (span > 32) {   // a tag map finer than the output: too many distinct taps to share
+    float t[HPD_MAX_EMB];
+    tag_at(s, b, k, y, x, t);
+    t0 = t[0];
+    if (s.E > 1) t1 = t[1];
+    return;
+  }
+  const int j0 = tx.i0 - c_lo, j1 = tx.i1 - c_lo;
+  float out[HPD_MAX_EMB] = {0.f, 0.f};
+#pragma unroll
+  for (int e = 0; e < HPD_MAX_EMB; ++e) {
+    if (e >= s.E) break;
+    const bool unflip = (e == 1) && !s.tags_preflipped;
+    const float* p = (e == 0) ? s.tag : s.tag_f;
+    const size_t po = (e == 0) ? (size_t)b * s.tag_sb + (size_t)k * s.tag_sc
+                               : (size_t)b * s.tagf_sb + (size_t)(unflip ? s.flip[k] : k) * s.tagf_sc;
+    float v0 = 0.f, v1 = 0.f;
+    if (lane < span) {
+      const int c = c_lo + lane;
+      const size_t col = (size_t)(unflip ? s.tw - 1 - c : c);
+      v0 = in_elem(p, po + (size_t)ty.i0 * s.tw + col, s.half_in);
+      v1 = in_elem(p, po + (size_t)ty.i1 * s.tw + col, s.half_in);
+    }
+    const float v00 = __shfl_sync(kFull, v0, j0), v01 = __shfl_sync(kFull, v0, j1);
+    const float v10 = __shfl_sync(kFull, v1, j0), v11 = __shfl_sync(kFull, v1, j1);
+    out[e] = lerp2(tx.w0, tx.w1, ty.w0, ty.w1, v00, v01, v10, v11);
+  }
+  t0 = out[0];
+  t1 = out[1];
+}
+
 __global__ void __launch_bounds__(kScanWarps * 32) refine_scan_kernel(const float* __restrict__ agg_hm,
-                                                                      const float* __restrict__ agg_tags,
+                                                                      const TagSource tags,
                                                                       const float* __restrict__ hmax,
                                                                       const float* __restrict__ tag_bmin,
                                                                       const float* __restrict__ tag_bmax,
@@ -199,7 +249,6 @@ __global__ void __launch_bounds__(kScanWarps * 32) refine_scan_kernel(const floa
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int nwords = H * wpr;
   const float* m = agg_hm + (size_t)bk * H * W;
-  const float* t = agg_tags + (size_t)bk * H * W * E;
   const float* hx = hmax + (size_t)bk * nwords;
   const int HB = (H + 3) >> 2;
   const float* tlo = tag_bmin + (size_t)bk * HB * wpr;
@@ -271,12 +320,9 @@ __global__ void __launch_bounds__(kScanWarps * 32) refine_scan_kernel(const floa
       const int y = w2 / wpr, x0 = (w2 - y * wpr) * 32;
       const bool valid = x0 + lane < W;
       const int idx = y * W + x0 + lane;
-      float pv = 0.f, t0 = 0.f, t1 = 0.f;
-      if (valid) {
-        pv = m[idx];
-        t0 = t[(size_t)idx * E];
-        if (E > 1) t1 = t[(size_t)idx * E + 1];
-      }
+      float pv = 0.f, t0, t1;
+      if (valid) pv = m[idx];
+      word_tags(tags, b, bk - b * K, y, x0, lane, t0, t1);
       bool improved = false;
       while (todo) {
         const int q = __ffs(todo) - 1;
@@ -389,11 +435,14 @@ size_t refine_workspace_bytes(const HpdParams* p) {
 }
 
 int launch_adjust_refine(const HpdParams* p, const HpdBuffers* buf, void* wsp, size_t ws_bytes, cudaStream_t st) {
-  if (!buf->agg_hm || !buf->agg_tags || !buf->hm_wmax || !buf->tag_bmin || !buf->tag_bmax || !buf->idx_k || !buf->scores_k ||
-      !buf->poses || !buf->person_scores || !buf->n_person) {
-    set_error("hpd_adjust_refine: agg_hm, agg_tags, hm_wmax, idx_k, scores_k, poses, person_scores, n_person are required");
+  if (!buf->agg_hm || !buf->hm_wmax || !buf->tag_bmin || !buf->tag_bmax || !buf->idx_k || !buf->scores_k || !buf->poses ||
+      !buf->person_scores || !buf->n_person || (p->do_refine && !buf->tags_k)) {
+    set_error("hpd_adjust_refine: agg_hm, hm_wmax, tag_bmin, tag_bmax, idx_k, scores_k, poses, person_scores, n_person and "
+              "(refine) tags_k are required");
     return HPD_EINVAL;
   }
+  TagSource tags;
+  if (int rc = make_tag_source(p, buf, &tags, "hpd_adjust_refine")) return rc;
   if (!wsp || ws_bytes < refine_workspace_bytes(p)) {
     set_error("hpd_adjust_refine: workspace of %zu bytes required, got %zu", refine_workspace_bytes(p), ws_bytes);
     return HPD_EWORKSPACE;
@@ -405,13 +454,13 @@ int launch_adjust_refine(const HpdParams* p, const HpdBuffers* buf, void* wsp, s
   const int B = p->batch, K = p->num_kpts, M = p->max_people, E = p->emb, H = p->out_h, W = p->out_w;
   const int wpr = (W + 31) / 32;
   RefineWs ws = carve(wsp, B, K, M);
-  adjust_prepare_kernel<<<B, 32 * M, 0, st>>>(buf->agg_hm, buf->agg_tags, buf->idx_k, buf->n_person, K, M, E, H, W,
+  adjust_prepare_kernel<<<B, 32 * M, 0, st>>>(buf->agg_hm, tags, buf->idx_k, buf->tags_k, buf->n_person, K, M, E, H, W,
                                               p->do_adjust, p->do_refine, buf->poses, buf->person_scores, ws);
   count_launch();
   int rc = check_launch("adjust_prepare_kernel");
   if (rc) return rc;
   if (p->do_refine) {
-    refine_scan_kernel<<<B * K, kScanWarps * 32, 0, st>>>(buf->agg_hm, buf->agg_tags, buf->hm_wmax, buf->tag_bmin, buf->tag_bmax,
+    refine_scan_kernel<<<B * K, kScanWarps * 32, 0, st>>>(buf->agg_hm, tags, buf->hm_wmax, buf->tag_bmin, buf->tag_bmax,
                                                           buf->scores_k, K, M, E, H, W, wpr, ws);
     count_launch();
     if ((rc = check_launch("refine_scan_kernel"))) return rc;

@@ -617,7 +617,7 @@ __device__ __forceinline__ void scan_row(Sink& sink, const float* __restrict__ h
 }
 
 __global__ void __launch_bounds__(kTopkWarps * 32, 1) topk_kernel(const float* __restrict__ agg_hm,
-                                                              const float* __restrict__ agg_tags,
+                                                              const TagSource tags,
                                                               const uint32_t* __restrict__ mask,
                                                               const float* __restrict__ wmax, int rows, int H, int W,
                                                               int wpr, int E, int M, int force_exact, int defer_ties,
@@ -722,7 +722,10 @@ __global__ void __launch_bounds__(kTopkWarps * 32, 1) topk_kernel(const float* _
     idx_k[o] = out_i;
     coords_k[o * 2 + 0] = out_i % W;
     coords_k[o * 2 + 1] = out_i / W;
-    for (int e = 0; e < E; ++e) tags_k[o * E + e] = agg_tags[((size_t)row * H * W + out_i) * E + e];
+    float tv[HPD_MAX_EMB];
+    tag_value(tags, row, out_i, tv);
+    tags_k[o * E] = tv[0];
+    if (E > 1) tags_k[o * E + 1] = tv[1];
   }
 }
 
@@ -737,7 +740,7 @@ constexpr int kSplitWarps = 8;
 constexpr int kSegLogCap = 320;
 
 __global__ void __launch_bounds__(kSplitWarps * 32, 1) topk_split_kernel(const float* __restrict__ agg_hm,
-                                                                     const float* __restrict__ agg_tags,
+                                                                     const TagSource tags,
                                                                      const uint32_t* __restrict__ mask,
                                                                      const float* __restrict__ wmax, int H, int W,
                                                                      int wpr, int E, int M, int force_exact,
@@ -817,7 +820,10 @@ __global__ void __launch_bounds__(kSplitWarps * 32, 1) topk_split_kernel(const f
             idx_k[o] = all.si;
             coords_k[o * 2 + 0] = all.si % W;
             coords_k[o * 2 + 1] = all.si / W;
-            for (int e = 0; e < E; ++e) tags_k[o * E + e] = agg_tags[((size_t)row * H * W + all.si) * E + e];
+            float tv[HPD_MAX_EMB];
+            tag_value(tags, row, all.si, tv);
+            tags_k[o * E] = tv[0];
+            if (E > 1) tags_k[o * E + 1] = tv[1];
           }
           if (lane == 0) s_floor_done = 1;
         }
@@ -904,7 +910,10 @@ __global__ void __launch_bounds__(kSplitWarps * 32, 1) topk_split_kernel(const f
     idx_k[o] = out_i;
     coords_k[o * 2 + 0] = out_i % W;
     coords_k[o * 2 + 1] = out_i / W;
-    for (int e = 0; e < E; ++e) tags_k[o * E + e] = agg_tags[((size_t)row * H * W + out_i) * E + e];
+    float tv[HPD_MAX_EMB];
+    tag_value(tags, row, out_i, tv);
+    tags_k[o * E] = tv[0];
+    if (E > 1) tags_k[o * E + 1] = tv[1];
   }
 }
 
@@ -927,7 +936,7 @@ constexpr int kTiedLogCap = 512;
 __constant__ int kSegFrac[kSplitWarps + 1] = {0, 1, 4, 16, 64, 128, 256, 512, 1024};
 
 __global__ void __launch_bounds__(kSplitWarps * 32, 1) topk_tied_rows_kernel(const float* __restrict__ agg_hm,
-                                                                         const float* __restrict__ agg_tags,
+                                                                         const TagSource tags,
                                                                          const uint32_t* __restrict__ mask,
                                                                          const float* __restrict__ wmax, int H, int W,
                                                                          int wpr, int E, int M,
@@ -1062,37 +1071,42 @@ __global__ void __launch_bounds__(kSplitWarps * 32, 1) topk_tied_rows_kernel(con
     idx_k[o] = out_i;
     coords_k[o * 2 + 0] = out_i % W;
     coords_k[o * 2 + 1] = out_i / W;
-    for (int e = 0; e < E; ++e) tags_k[o * E + e] = agg_tags[((size_t)row * H * W + out_i) * E + e];
+    float tv[HPD_MAX_EMB];
+    tag_value(tags, row, out_i, tv);
+    tags_k[o * E] = tv[0];
+    if (E > 1) tags_k[o * E + 1] = tv[1];
   }
 }
 
 }  // namespace
 
 int launch_topk(const HpdParams* p, const HpdBuffers* buf, cudaStream_t st) {
-  if (!buf->agg_hm || !buf->agg_tags || !buf->nms_mask || !buf->nms_wmax || !buf->scores_k || !buf->idx_k ||
-      !buf->coords_k || !buf->tags_k) {
-    set_error("hpd_topk: agg_hm, agg_tags, nms_mask, nms_wmax, scores_k, idx_k, coords_k, tags_k are required");
+  if (!buf->agg_hm || !buf->nms_mask || !buf->nms_wmax || !buf->scores_k || !buf->idx_k || !buf->coords_k ||
+      !buf->tags_k) {
+    set_error("hpd_topk: agg_hm, nms_mask, nms_wmax, scores_k, idx_k, coords_k, tags_k are required");
     return HPD_EINVAL;
   }
+  TagSource tags;
+  if (int rc = make_tag_source(p, buf, &tags, "hpd_topk")) return rc;
   const int rows = p->batch * p->num_kpts;
   const int wpr = (p->out_w + 31) / 32;
   // small batches: kSplitWarps warps per row cut the per-row latency; large ones fill the GPU with one warp per row
   const bool split = rows <= 512 && (long long)p->out_h * wpr >= 128 * kSplitWarps && !(p->force_generic & 2) &&
                      p->batches_in_flight < 8;
   if (split)
-    topk_split_kernel<<<rows, kSplitWarps * 32, 0, st>>>(buf->agg_hm, buf->agg_tags, buf->nms_mask, buf->nms_wmax, p->out_h,
+    topk_split_kernel<<<rows, kSplitWarps * 32, 0, st>>>(buf->agg_hm, tags, buf->nms_mask, buf->nms_wmax, p->out_h,
                                                          p->out_w, wpr, p->emb, p->max_people, p->force_generic & 1,
                                                          buf->scores_k, buf->idx_k, buf->coords_k, buf->tags_k);
   else {
     // force_generic bit 2 (testing): rows with ties stay in topk_kernel's own one-warp exact stream
     const bool defer = !(p->force_generic & 1) && !(p->force_generic & 4) && (long long)p->out_h * wpr >= 128 * kSplitWarps;
     topk_kernel<<<(rows + kTopkWarps - 1) / kTopkWarps, kTopkWarps * 32, 0, st>>>(
-        buf->agg_hm, buf->agg_tags, buf->nms_mask, buf->nms_wmax, rows, p->out_h, p->out_w, wpr, p->emb, p->max_people,
+        buf->agg_hm, tags, buf->nms_mask, buf->nms_wmax, rows, p->out_h, p->out_w, wpr, p->emb, p->max_people,
         p->force_generic & 1, defer ? 1 : 0, buf->scores_k, buf->idx_k, buf->coords_k, buf->tags_k);
     if (defer) {
       count_launch();
       if (int rc = check_launch("topk_kernel")) return rc;
-      topk_tied_rows_kernel<<<rows, kSplitWarps * 32, 0, st>>>(buf->agg_hm, buf->agg_tags, buf->nms_mask, buf->nms_wmax,
+      topk_tied_rows_kernel<<<rows, kSplitWarps * 32, 0, st>>>(buf->agg_hm, tags, buf->nms_mask, buf->nms_wmax,
                                                                p->out_h, p->out_w, wpr, p->emb, p->max_people, buf->scores_k,
                                                                buf->idx_k, buf->coords_k, buf->tags_k);
     }

@@ -10,7 +10,7 @@ HPD_MAX_KPTS = 32
 HPD_MAX_PEOPLE = 32
 HPD_MAX_EMB = 2
 HPD_MAX_SCALES = 4
-HPD_ABI_VERSION = 2
+HPD_ABI_VERSION = 3
 HPD_F32, HPD_F16 = 0, 1
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -20,6 +20,7 @@ EXPORTS = (
     "hpd_abi_version", "hpd_last_error_string", "hpd_workspace_bytes", "hpd_aggregate_nms", "hpd_nms",
     "hpd_topk", "hpd_group", "hpd_adjust_refine", "hpd_decode", "hpd_last_launch_count", "hpd_resize_bilinear",
     "hpd_record_layout", "hpd_multi_scale_size", "hpd_get_affine_transform", "hpd_prepare_input", "hpd_prepare_geometry",
+    "hpd_aggregate_tags",
 )
 
 
@@ -46,7 +47,8 @@ class HpdParams(ctypes.Structure):
 class HpdBuffers(ctypes.Structure):
     _fields_ = [(n, ctypes.c_void_p) for n in (
         "agg_hm", "agg_tags", "nms_mask", "nms_wmax", "hm_wmax", "scores_k", "idx_k", "coords_k", "tags_k",
-        "poses", "person_scores", "n_person", "flags", "tag_bmin", "tag_bmax", "records", "inv_affine")]
+        "poses", "person_scores", "n_person", "flags", "tag_bmin", "tag_bmax", "records", "inv_affine")] + [
+        ("tag_inputs", HpdScaleInputs)]
 
 
 class HpdRecordLayout(ctypes.Structure):
@@ -83,6 +85,7 @@ def lib():
     P, S, B, V = ctypes.POINTER(HpdParams), ctypes.POINTER(HpdScaleInputs), ctypes.POINTER(HpdBuffers), ctypes.c_void_p
     L.hpd_workspace_bytes.argtypes = [P, ctypes.POINTER(ctypes.c_size_t)]
     L.hpd_aggregate_nms.argtypes = [P, S, B, V]
+    L.hpd_aggregate_tags.argtypes = [P, S, V, V]
     L.hpd_nms.argtypes = [P, B, V, V]
     L.hpd_topk.argtypes = [P, B, V]
     L.hpd_group.argtypes = [P, B, V]

@@ -66,7 +66,6 @@ class DecodeResult:
         self.bufs = bufs
         self._generation = getattr(bufs, "generation", 0)   # a later decode into the same buffer set bumps it
         self.agg_hm = bufs.agg_hm          # [B,K,H,W]
-        self.agg_tags = bufs.agg_tags      # [B,K,H,W,E]
         self.poses = bufs.poses            # [B,M,K,3+E]
         self.person_scores = bufs.person_scores
         self.n_person = bufs.n_person
@@ -78,6 +77,16 @@ class DecodeResult:
             raise ops._lib.HpdError("this DecodeResult was overwritten by a later decode into the same buffer set "
                                     "(same shape and slot): read or clone() a result before decoding again, or use "
                                     "distinct slots")
+
+    @property
+    def agg_tags(self) -> torch.Tensor:
+        """The aggregated tags [B,K,H,W,E] (results.py:229-230).  A buffer set without a tag map (the decoder's
+        default) did not write them: the first read computes the map from the network outputs of the decode (the
+        buffer set keeps a reference to them), bit-identical to the one the aggregation would have written.  Those
+        outputs must then be unchanged since the decode, and the result still live."""
+        if self.bufs.tag_map is None:
+            self._check_live()
+        return self.bufs.agg_tags
 
     def packed(self) -> torch.Tensor:
         """The device tensor that holds everything a caller reads after a decode (one row per image):
@@ -113,7 +122,11 @@ def _finish(poses: np.ndarray, scores: np.ndarray, fallback: int):
 
 class BottomUpDecoder:
     def __init__(self, num_kpts: int = 17, max_num_people: int = 30, det_thr: float = 0.05, tag_thr: float = 0.5,
-                 device="cuda:0", adjust: bool = True, refine: bool = True, max_cached_shapes: int = 4):
+                 device="cuda:0", adjust: bool = True, refine: bool = True, max_cached_shapes: int = 4,
+                 keep_tag_map: bool = False):
+        """keep_tag_map=False: the buffer sets hold no full-resolution tag map (the decode reads only a few thousand
+        tags per map and interpolates them where it reads them); DecodeResult.agg_tags computes the map on demand.
+        True: the aggregation writes it, as the reference computes it (4*K*H*W*E bytes per image of writes)."""
         if not torch.cuda.is_available():
             raise ops._lib.HpdError("hpdecode needs a CUDA device (sm_100a); there is no CPU fallback")
         ops._lib.lib()
@@ -123,11 +136,12 @@ class BottomUpDecoder:
         self.device = torch.device(device)
         self._bufs = OrderedDict()
         self.max_cached_shapes = max_cached_shapes
+        self.keep_tag_map = keep_tag_map
 
     def buffers(self, B, H, W, E, slot=0) -> ops.DecodeBuffers:
         """Buffer set for one (shape, slot), kept in a small LRU: bottom-up inference sees many padded
-        (H, W) (resize_align_multi_scale keeps the aspect ratio) and a set is ~80 MB per image at 512-class
-        sizes, so at most ``max_cached_shapes`` distinct shapes stay resident (slots of one shape are evicted
+        (H, W) (resize_align_multi_scale keeps the aspect ratio) and a set is ~20 MB per image at 512 x 512 (~55 MB
+        with the tag map), so at most ``max_cached_shapes`` distinct shapes stay resident (slots of one shape are evicted
         together; an evicted set is freed once the stream work that uses it has run, by the caching allocator)."""
         shape = (B, H, W, E)
         slots = self._bufs.get(shape)
@@ -138,7 +152,8 @@ class BottomUpDecoder:
         else:
             self._bufs.move_to_end(shape)
         if slot not in slots:
-            slots[slot] = ops.DecodeBuffers(B, self.num_kpts, H, W, E, self.max_num_people, self.device)
+            slots[slot] = ops.DecodeBuffers(B, self.num_kpts, H, W, E, self.max_num_people, self.device,
+                                            tags=self.keep_tag_map)
         return slots[slot]
 
     def _set_inv_affine(self, bufs: ops.DecodeBuffers, inv_affine):
@@ -187,7 +202,9 @@ class DecodePipeline:
     aggregation overlaps batch i's tail.  ``submit`` returns the lane's DecodeResult; it stays valid until the lane
     is reused ``depth`` submits later (call ``result.ready.synchronize()`` or ``drain()`` before reading).
     Lifetime contract for the inputs: ``submit`` records their use on the lane's stream (``Tensor.record_stream``),
-    so the caller may drop them as soon as it returns.
+    so the caller may drop them as soon as it returns.  The lanes' buffer sets hold no tag map unless the decoder keeps
+    one: the lane's buffer set then keeps a reference to the inputs (those ``before_agg`` returned, if any), and ``agg_tags``
+    computes the map from them -- so they must be unchanged when ``agg_tags`` is first read.
 
     ``records_ring``: an optional uint8 tensor [depth, B, row_bytes]; lane i's result records are then written
     straight into ``records_ring[i]`` by the decode's last kernel, so consecutive lanes form one contiguous block
@@ -272,6 +289,7 @@ class DecodePipeline:
                 self.graph_replays += 1
             else:
                 self._launch(ln, bufs, params, scales)
+            bufs.note_inputs(scales, params)           # a replay does not pass through run_decode
             if after_tail is not None:
                 after_tail(ln, res)
             ln["ready"].record()

@@ -96,16 +96,22 @@ class DecodeBuffers:
 
     ``records`` [B,row_bytes] uint8 receives one result record per image (HpdRecordLayout) from the epilogue of
     the last kernel; ``inv_affine`` (optional float64 [B,6] on the device) is the per-image matrix the COCO
-    section's coordinates are back-projected with (None = network-input coordinates)."""
+    section's coordinates are back-projected with (None = network-input coordinates).
+
+    ``tags=False`` allocates no full-resolution tag map (``tag_map`` is None, 4*K*H*W*E bytes per image less): the
+    aggregation then writes none and the tag stages interpolate the few tags they read from the network outputs,
+    which ``run_stage`` hands them from its ``scales``.  ``agg_tags`` is then computed on first read from the network
+    outputs of the last decode into the set (``run_aggregate_tags``), which must be unchanged by then."""
 
     def __init__(self, B: int, K: int, H: int, W: int, E: int, M: int, device, agg_hm: Optional[Tensor] = None,
-                 agg_tags: Optional[Tensor] = None):
+                 agg_tags: Optional[Tensor] = None, tags: bool = True):
         self.shape = (B, K, H, W, E, M)
         wpr = (W + 31) // 32
         f32 = dict(device=device, dtype=torch.float32)
         i32 = dict(device=device, dtype=torch.int32)
         self.agg_hm = agg_hm if agg_hm is not None else torch.empty((B, K, H, W), **f32)
-        self.agg_tags = agg_tags if agg_tags is not None else torch.empty((B, K, H, W, E), **f32)
+        self.tag_map = agg_tags if agg_tags is not None else (torch.empty((B, K, H, W, E), **f32) if tags else None)
+        self._tag_inputs = self._tag_lazy = None
         self.nms_mask = torch.empty((B, K, H, wpr), **i32)
         self.nms_wmax = torch.empty((B, K, H, wpr), **f32)
         self.hm_wmax = torch.empty((B, K, H, wpr), **f32)
@@ -132,7 +138,8 @@ class DecodeBuffers:
         self.shape = (B, K, 0, 0, E, M)
         zf = torch.empty((0,), device=dev, dtype=torch.float32)
         zi = torch.empty((0,), device=dev, dtype=torch.int32)
-        self.agg_hm = self.agg_tags = self.nms_wmax = self.hm_wmax = self.tag_bmin = self.tag_bmax = zf
+        self.agg_hm = self.tag_map = self.nms_wmax = self.hm_wmax = self.tag_bmin = self.tag_bmax = zf
+        self._tag_inputs = self._tag_lazy = None
         self.person_scores = zf
         self.nms_mask = self.idx_k = zi
         self.scores_k, self.coords_k, self.tags_k = scores_k, coords_k, tags_k
@@ -143,10 +150,32 @@ class DecodeBuffers:
         self.workspace = None
         return self
 
+    @property
+    def agg_tags(self) -> Optional[Tensor]:
+        """[B,K,H,W,E] aggregated tags: the tag map, or for a set without one the map computed (once per decode, on
+        the current stream, after the decode's stream) from the network outputs of the last decode into the set."""
+        if self.tag_map is not None or self._tag_inputs is None:
+            return self.tag_map
+        if self._tag_lazy is None:
+            scales, params, stream = self._tag_inputs
+            B, K, H, W, E, _ = self.shape
+            dev = self.agg_hm.device
+            torch.cuda.current_stream(dev).wait_stream(stream)
+            self._tag_lazy = run_aggregate_tags(scales, params, torch.empty((B, K, H, W, E), device=dev, dtype=torch.float32))
+        return self._tag_lazy
+
+    def note_inputs(self, scales: Sequence[dict], params: HpdParams):
+        """A decode into this set from these network outputs was enqueued on the current stream (agg_tags)."""
+        if self.tag_map is None:
+            self._tag_inputs = (scales, params, torch.cuda.current_stream(self.agg_hm.device))
+            self._tag_lazy = None
+
     def struct(self) -> HpdBuffers:
         s = HpdBuffers()
         for name, _ in HpdBuffers._fields_:
-            t = getattr(self, name)
+            if name == "tag_inputs":        # not a buffer: run_stage / hpd_decode fill it from the scales
+                continue
+            t = self.tag_map if name == "agg_tags" else getattr(self, name)
             if t is None:
                 continue
             if name == "inv_affine" and (t.dtype != torch.float64 or t.numel() != 6 * self.shape[0] or not t.is_cuda):
@@ -212,6 +241,7 @@ def run_decode(scales: Optional[Sequence[dict]], bufs: DecodeBuffers, params: Hp
     ws = bufs.ensure_workspace(params)
     with torch.cuda.device(dev):
         if scales is not None:
+            bufs.note_inputs(scales, params)
             arr, _keep = _scales_struct(scales)
             rc = L.hpd_decode(ctypes.byref(params), arr, ctypes.byref(bufs.struct()), ws.data_ptr(), ws.numel(),
                               _stream_ptr(dev))
@@ -223,13 +253,34 @@ def run_decode(scales: Optional[Sequence[dict]], bufs: DecodeBuffers, params: Hp
     return bufs
 
 
+def run_aggregate_tags(scales: Sequence[dict], params: HpdParams, out: Tensor):
+    """hpd_aggregate_tags on the current stream: the full-resolution tag map [B,K,H,W,E] of scales[tag_scale] into
+    ``out``, bit-identical to the one hpd_aggregate_nms writes."""
+    B, K, H, W, E = params.batch, params.num_kpts, params.out_h, params.out_w, params.emb
+    if tuple(out.shape) != (B, K, H, W, E) or not out.is_contiguous() or not out.is_cuda or out.dtype != torch.float32:
+        raise _lib.HpdError(f"aggregate_tags: out must be a contiguous CUDA float32 tensor {(B, K, H, W, E)}")
+    L = _lib.lib()
+    with torch.cuda.device(out.device):
+        arr, _keep = _scales_struct(scales)
+        rc = L.hpd_aggregate_tags(ctypes.byref(params), arr, out.data_ptr(), _stream_ptr(out.device))
+    _lib.check(rc, "hpd_aggregate_tags")
+    _count(L)
+    return out
+
+
 def run_stage(stage: str, bufs: DecodeBuffers, params: HpdParams, scales=None, nms_out: Optional[Tensor] = None):
+    """One stage on the current stream.  Buffers without a tag map (``tags=False``) need ``scales`` for the tag
+    stages (topk, adjust_refine): they interpolate from scales[params.tag_scale]."""
     L = _lib.lib()
     dev = bufs.agg_hm.device
     st = _stream_ptr(dev)
     b = bufs.struct()
+    if bufs.tag_map is None and scales is not None and stage in ("topk", "adjust_refine"):
+        tag_arr, _keep_tag = _scales_struct([scales[params.tag_scale]])
+        b.tag_inputs = tag_arr[0]
     with torch.cuda.device(dev):
         if stage == "aggregate_nms":
+            bufs.note_inputs(scales, params)
             arr, _keep = _scales_struct(scales)
             rc = L.hpd_aggregate_nms(ctypes.byref(params), arr, ctypes.byref(b), st)
         elif stage == "nms":
