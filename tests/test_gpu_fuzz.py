@@ -53,6 +53,17 @@ def _case(seed):
 
 @pytest.mark.parametrize("seed", range(60))
 def test_random_configuration_matches_oracle(seed, oracle):
+    _run_seed(seed, oracle, tags=True)
+
+
+@pytest.mark.parametrize("seed", range(60))
+def test_random_configuration_tagless_matches_oracle(seed, oracle):
+    """The same cases through buffer sets without a tag map (the decoder's default): top-k, adjust and refine
+    interpolate their tags (tag_at, word_tags) under random K and random flip involutions."""
+    _run_seed(seed, oracle, tags=False)
+
+
+def _run_seed(seed, oracle, tags):
     from hpdecode import ops
     from hpdecode.decoder import Records
     c = _case(seed)
@@ -66,9 +77,10 @@ def test_random_configuration_matches_oracle(seed, oracle):
         pairs = rng.permutation(K)[: 2 * (K // 2)].reshape(-1, 2)
         for a, b2 in pairs:
             flip_index[a], flip_index[b2] = int(b2), int(a)
-    bufs = ops.DecodeBuffers(B, K, H, W, E, M, "cuda:0")
-    for t in (bufs.agg_hm, bufs.agg_tags, bufs.poses, bufs.person_scores):
-        t.fill_(float("nan"))
+    bufs = ops.DecodeBuffers(B, K, H, W, E, M, "cuda:0", tags=tags)
+    for t in (bufs.agg_hm, bufs.tag_map, bufs.poses, bufs.person_scores):
+        if t is not None:
+            t.fill_(float("nan"))
     bufs.idx_k.fill_(-1)
     p = ops.make_params(B, K, H, W, E, M, c["det"], c["tthr"], flip_index=flip_index)
     if c["mode"] == 1:
@@ -81,7 +93,8 @@ def test_random_configuration_matches_oracle(seed, oracle):
     for b in range(B):
         hm_o, tg_o = oracle.aggregate([{k: v[b] for k, v in c["scale"].items()}], (H, W), flip_index=flip_index)
         assert np.array_equal(_bits(bufs.agg_hm[b].cpu().numpy()), _bits(hm_o)), f"seed {seed} image {b}: heatmaps"
-        assert np.array_equal(_bits(bufs.agg_tags[b].cpu().numpy()), _bits(tg_o)), f"seed {seed} image {b}: tags"
+        if tags:      # a tag-less set computes agg_tags on demand; its decode read none of it
+            assert np.array_equal(_bits(bufs.agg_tags[b].cpu().numpy()), _bits(tg_o)), f"seed {seed} image {b}: tags"
         ref = oracle.parse(hm_o, tg_o, M, c["det"], c["tthr"])
         assert np.array_equal(bufs.idx_k[b].cpu().numpy(), ref["idx_k"]), f"seed {seed} image {b}: top-k indices ({c['mode']})"
         assert np.array_equal(_bits(bufs.scores_k[b].cpu().numpy()), _bits(ref["scores_k"]))

@@ -90,7 +90,17 @@ def test_bilinear_matches_torch_cpu_on_this_host(oracle):
     import torch
     rng = np.random.default_rng(1)
     for (ih, iw, oh, ow) in [(48, 48, 96, 96), (64, 64, 128, 128), (128, 128, 512, 512), (60, 60, 80, 80),
-                             (40, 56, 160, 224), (80, 80, 80, 80), (120, 120, 160, 160)]:
+                             (40, 56, 160, 224), (80, 80, 80, 80), (120, 120, 160, 160),
+                             # the resizes of tests/test_gpu_refine.py: the 256 x 256 scenes, the generic scene
+                             # (184 x 248), the second scale of the two-scale scene, tag maps finer than the output
+                             # (downsampling), the x2 prefilter shapes and the multi-scale prefilter shapes
+                             (128, 128, 256, 256), (64, 64, 256, 256), (46, 62, 92, 124), (92, 124, 184, 248),
+                             (46, 62, 184, 248), (96, 96, 192, 192), (192, 192, 256, 256), (80, 80, 160, 160),
+                             (160, 160, 128, 128), (200, 200, 128, 128), (40, 40, 80, 80), (40, 40, 160, 160),
+                             (40, 64, 80, 128), (80, 128, 160, 256), (40, 64, 160, 256), (48, 128, 96, 256),
+                             (96, 256, 192, 512), (48, 128, 192, 512), (64, 96, 128, 192), (128, 192, 256, 384),
+                             (64, 96, 256, 384), (96, 144, 192, 288), (192, 288, 256, 384), (80, 128, 320, 512),
+                             (160, 256, 320, 512)]:
         x = rng.standard_normal((3, ih, iw)).astype(np.float32)
         t = torch.nn.functional.interpolate(torch.from_numpy(x)[None], size=[oh, ow], mode="bilinear",
                                             align_corners=False)[0].numpy()
