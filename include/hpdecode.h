@@ -33,11 +33,15 @@ extern "C" {
 #define HPD_EXPORT
 #endif
 
-#define HPD_ABI_VERSION 3
+#define HPD_ABI_VERSION 4
 #define HPD_MAX_KPTS 32     /* joints per person (COCO: 17) */
 #define HPD_MAX_PEOPLE 32   /* max_num_people == top-k; the warp-wide Hungarian handles n <= 32 */
 #define HPD_MAX_EMB 2       /* tag embedding dims: 1 (no flip test) or 2 (flip test) */
 #define HPD_MAX_SCALES 4    /* test scales averaged into one heatmap */
+#define HPD_COCO_MAX_IOU_THRS 16    /* COCO keypoint evaluation: OKS thresholds (pycocotools: 10) */
+#define HPD_COCO_MAX_REC_THRS 128   /* recall thresholds (pycocotools: 101) */
+#define HPD_COCO_MAX_AREAS 4        /* area ranges (pycocotools keypoints: all, medium, large) */
+#define HPD_COCO_MAX_PER_IMAGE 1024 /* detections, and ground-truth annotations, per image */
 
 enum {
   HPD_OK = 0,
@@ -153,6 +157,60 @@ typedef struct HpdImage {
   double m[6];          /* the forward 2x3 matrix cv2.warpAffine receives (base/transforms/utils.py:95-96) */
 } HpdImage;
 
+/* ---- COCO keypoint evaluation (pycocotools COCOeval, iouType "keypoints": evaluate + accumulate) ------------
+ * One category (person).  Images are given in ascending image-id order (COCOeval's p.imgIds), so image index order is
+ * the order accumulate concatenates them in.  Everything that decides a result is float64. */
+typedef struct HpdCocoEvalParams {
+  int32_t num_images;   /* I */
+  int32_t num_kpts;     /* K <= HPD_MAX_KPTS */
+  int32_t max_dets;     /* maxDets[-1] <= HPD_MAX_PEOPLE: detections kept per image, by score */
+  int32_t max_gts;      /* G <= HPD_COCO_MAX_PER_IMAGE: ground-truth slots per image in HpdCocoGts */
+  int32_t num_iou_thrs; /* T <= HPD_COCO_MAX_IOU_THRS */
+  int32_t num_rec_thrs; /* R <= HPD_COCO_MAX_REC_THRS */
+  int32_t num_areas;    /* A <= HPD_COCO_MAX_AREAS */
+  int32_t reserved_;
+  double iou_thrs[HPD_COCO_MAX_IOU_THRS];   /* p.iouThrs, as NumPy computed them (np.linspace) */
+  double rec_thrs[HPD_COCO_MAX_REC_THRS];   /* p.recThrs */
+  double area_rng[HPD_COCO_MAX_AREAS][2];   /* p.areaRng: [lo, hi], inclusive */
+  double kpt_vars[HPD_MAX_KPTS];            /* (p.kpt_oks_sigmas * 2) ** 2, as NumPy computed them */
+} HpdCocoEvalParams;
+
+/* Detections, read in place: image i's row starts at base + row_offset[i] bytes (row_offset[i] < 0: the image has no
+ * detections).  A row holds an int32 count n at +off_count and n persons of [x, y, v] * K + score (float64) at
+ * +off_coco, person_stride doubles apart -- the COCO section of decode result records (HpdRecordLayout: off_coco,
+ * off_n_person, coco_stride), or rows packed from result dicts.  Persons are in the order of the results list: score
+ * ties are broken by it.  Counts are read as min(max(n, 0), max_per_row).  Scores must not be NaN. */
+typedef struct HpdCocoDets {
+  const uint8_t* base;
+  const int64_t* row_offset;  /* [I] device */
+  int64_t off_coco;           /* multiple of 8 (base + row_offset[i] must be 8-byte aligned too) */
+  int64_t off_count;          /* multiple of 4 */
+  int32_t person_stride;      /* doubles between persons, >= 3K + 1 */
+  int32_t max_per_row;        /* D <= HPD_COCO_MAX_PER_IMAGE */
+} HpdCocoDets;
+
+/* Ground truth, padded to G = params.max_gts per image, annotations of an image in dataset order. */
+typedef struct HpdCocoGts {
+  const double* kpts;       /* [I][G][K][3] x, y, v */
+  const double* area;       /* [I][G] the annotation's area */
+  const double* bbox;       /* [I][G][4] x, y, w, h */
+  const uint8_t* iscrowd;   /* [I][G] */
+  const uint8_t* ignore;    /* [I][G] iscrowd || num_keypoints == 0 (COCOeval._prepare) */
+  const int32_t* n_gt;      /* [I] annotations of the image (<= G) */
+} HpdCocoGts;
+
+enum { HPD_COCO_ABSENT = 0, HPD_COCO_TP = 1, HPD_COCO_FP = 2, HPD_COCO_IGNORED = 3 };
+
+/* accumulate's arrays for the one category and the one maxDets entry, -1 where no gt is non-ignored (npig == 0). */
+typedef struct HpdCocoEvalOutputs {
+  double* precision;  /* [T][R][A] */
+  double* recall;     /* [T][A] */
+  double* scores;     /* [T][R][A] */
+  double* oks;        /* optional [I][max_dets][G]: computeOks per image (score rank x gt), 0 outside n_dets x n_gt */
+  uint8_t* codes;     /* optional [A][T][I][max_dets]: HPD_COCO_* of each (area, threshold, image, score rank) */
+  int64_t* npig;      /* optional [A]: non-ignored gts per area range */
+} HpdCocoEvalOutputs;
+
 HPD_EXPORT int hpd_abi_version(void);
 HPD_EXPORT const char* hpd_last_error_string(void);
 
@@ -230,6 +288,15 @@ HPD_EXPORT int hpd_prepare_geometry(int n, const int32_t* img_h, const int32_t* 
  * the reference's tensor.  mean / std: 3 floats each (host). */
 HPD_EXPORT int hpd_prepare_input(const HpdImage* images_host, int batch, float* out, int out_h, int out_w,
                                  const float mean[3], const float std_[3], void* stream);
+
+/* Bytes of scratch hpd_coco_eval needs for these params. */
+HPD_EXPORT int hpd_coco_eval_workspace_bytes(const HpdCocoEvalParams* p, size_t* out_bytes);
+
+/* COCOeval(gt, dt, "keypoints").evaluate() + accumulate() (pycocotools cocoeval.py): OKS per image, the greedy
+ * matching of every (area range, threshold), a stable global score order, and the precision / recall / score arrays.
+ * The summary statistics are a mean over these arrays, left to the host (hpdecode.cocoeval). */
+HPD_EXPORT int hpd_coco_eval(const HpdCocoEvalParams* p, const HpdCocoDets* dets, const HpdCocoGts* gts,
+                             const HpdCocoEvalOutputs* outs, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Number of kernel launches the previous call on this thread enqueued (for bench accounting). */
 HPD_EXPORT int hpd_last_launch_count(void);

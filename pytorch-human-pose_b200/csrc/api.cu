@@ -197,6 +197,22 @@ int hpd_prepare_input(const HpdImage* images_host, int batch, float* out, int ou
   return launch_prepare_input(images_host, batch, out, out_h, out_w, mean, std_, (cudaStream_t)stream);
 }
 
+int hpd_coco_eval_workspace_bytes(const HpdCocoEvalParams* p, size_t* out_bytes) {
+  if (!out_bytes) { set_error("NULL argument"); return HPD_EINVAL; }
+  int rc = validate_coco_params(p);
+  if (rc) return rc;
+  *out_bytes = coco_eval_workspace_bytes(p, &rc);
+  return rc;
+}
+
+int hpd_coco_eval(const HpdCocoEvalParams* p, const HpdCocoDets* dets, const HpdCocoGts* gts,
+                  const HpdCocoEvalOutputs* outs, void* workspace, size_t workspace_bytes, void* stream) {
+  g_launches = 0;
+  int rc = validate_coco_params(p);
+  if (rc) return rc;
+  return launch_coco_eval(p, dets, gts, outs, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
 int hpd_decode(const HpdParams* p, const HpdScaleInputs* scales, const HpdBuffers* buf, void* workspace,
                size_t workspace_bytes, void* stream) {
   g_launches = 0;

@@ -191,5 +191,9 @@ int launch_prepare_input(const HpdImage* images, int batch, float* out, int oh, 
 int multi_scale_size(int h, int w, int input_size, double current_scale, double min_scale, int32_t* size_wh,
                      int32_t* center_xy, double* scale_wh);
 int affine_transform_matrix(const double* center, const double* scale, const int32_t* out_wh, int inverse, double* m);
+int validate_coco_params(const HpdCocoEvalParams* p);
+size_t coco_eval_workspace_bytes(const HpdCocoEvalParams* p, int* rc);
+int launch_coco_eval(const HpdCocoEvalParams* p, const HpdCocoDets* dets, const HpdCocoGts* gts,
+                     const HpdCocoEvalOutputs* outs, void* ws, size_t ws_bytes, cudaStream_t st);
 
 }  // namespace hpd

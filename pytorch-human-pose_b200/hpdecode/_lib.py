@@ -10,7 +10,8 @@ HPD_MAX_KPTS = 32
 HPD_MAX_PEOPLE = 32
 HPD_MAX_EMB = 2
 HPD_MAX_SCALES = 4
-HPD_ABI_VERSION = 3
+HPD_ABI_VERSION = 4
+HPD_COCO_MAX_IOU_THRS, HPD_COCO_MAX_REC_THRS, HPD_COCO_MAX_AREAS, HPD_COCO_MAX_PER_IMAGE = 16, 128, 4, 1024
 HPD_F32, HPD_F16 = 0, 1
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -20,7 +21,7 @@ EXPORTS = (
     "hpd_abi_version", "hpd_last_error_string", "hpd_workspace_bytes", "hpd_aggregate_nms", "hpd_nms",
     "hpd_topk", "hpd_group", "hpd_adjust_refine", "hpd_decode", "hpd_last_launch_count", "hpd_resize_bilinear",
     "hpd_record_layout", "hpd_multi_scale_size", "hpd_get_affine_transform", "hpd_prepare_input", "hpd_prepare_geometry",
-    "hpd_aggregate_tags",
+    "hpd_aggregate_tags", "hpd_coco_eval_workspace_bytes", "hpd_coco_eval",
 )
 
 
@@ -62,6 +63,26 @@ class HpdImage(ctypes.Structure):
                 ("m", ctypes.c_double * 6)]
 
 
+class HpdCocoEvalParams(ctypes.Structure):
+    _fields_ = [(n, ctypes.c_int32) for n in ("num_images", "num_kpts", "max_dets", "max_gts", "num_iou_thrs",
+                                              "num_rec_thrs", "num_areas", "reserved_")] + [
+        ("iou_thrs", ctypes.c_double * HPD_COCO_MAX_IOU_THRS), ("rec_thrs", ctypes.c_double * HPD_COCO_MAX_REC_THRS),
+        ("area_rng", (ctypes.c_double * 2) * HPD_COCO_MAX_AREAS), ("kpt_vars", ctypes.c_double * HPD_MAX_KPTS)]
+
+
+class HpdCocoDets(ctypes.Structure):
+    _fields_ = [("base", ctypes.c_void_p), ("row_offset", ctypes.c_void_p), ("off_coco", ctypes.c_int64),
+                ("off_count", ctypes.c_int64), ("person_stride", ctypes.c_int32), ("max_per_row", ctypes.c_int32)]
+
+
+class HpdCocoGts(ctypes.Structure):
+    _fields_ = [(n, ctypes.c_void_p) for n in ("kpts", "area", "bbox", "iscrowd", "ignore", "n_gt")]
+
+
+class HpdCocoEvalOutputs(ctypes.Structure):
+    _fields_ = [(n, ctypes.c_void_p) for n in ("precision", "recall", "scores", "oks", "codes", "npig")]
+
+
 class HpdError(RuntimeError):
     pass
 
@@ -101,6 +122,10 @@ def lib():
     L.hpd_prepare_geometry.argtypes = [ctypes.c_int, I32P, I32P, ctypes.c_int, ctypes.c_double, ctypes.c_double, I32P, I32P, F64P,
                                        F64P, F64P]
     L.hpd_prepare_input.argtypes = [ctypes.POINTER(HpdImage), ctypes.c_int, V, ctypes.c_int, ctypes.c_int, F32P, F32P, V]
+    CP = ctypes.POINTER(HpdCocoEvalParams)
+    L.hpd_coco_eval_workspace_bytes.argtypes = [CP, ctypes.POINTER(ctypes.c_size_t)]
+    L.hpd_coco_eval.argtypes = [CP, ctypes.POINTER(HpdCocoDets), ctypes.POINTER(HpdCocoGts),
+                                ctypes.POINTER(HpdCocoEvalOutputs), V, ctypes.c_size_t, V]
     for n in EXPORTS:
         if n not in ("hpd_last_error_string",):
             getattr(L, n).restype = ctypes.c_int

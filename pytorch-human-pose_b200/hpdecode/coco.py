@@ -63,3 +63,22 @@ def evaluate_dataset_batched(model, dataset, batch_size: int = 32, limit: Option
         for recs in per_image:          # dataset order, like the reference's loop
             results.extend(recs)
     return results
+
+
+def eval_coco(gt, results, device="cuda:0", verbose: bool = True):
+    """bin/eval.py:52-65 on the device: COCO(gt).loadRes(results) and COCOeval(..., "keypoints") evaluate /
+    accumulate / summarize.  gt: a COCO keypoint annotation dict or the path of its JSON file; results: a list of
+    result dicts or the path of their JSON file.  Prints the summary like pycocotools and returns the
+    CocoEvalResult (``stats`` holds the ten numbers)."""
+    import json
+    from .cocoeval import KeypointEvaluator, KeypointGroundTruth
+    if not isinstance(gt, dict):
+        with open(gt) as f:
+            gt = json.load(f)
+    if not isinstance(results, (list, tuple)):
+        with open(results) as f:
+            results = json.load(f)
+    res = KeypointEvaluator(KeypointGroundTruth.from_coco(gt, device)).evaluate_results(results)
+    if verbose:
+        print("\n".join(res.summary()))
+    return res

@@ -11,6 +11,7 @@ Stage ops mirror the reference methods one to one (paths relative to /root/refer
   hpd::group          MPPEHeatmapParser.match_by_tag grouping.py:85-145 (+ fallback :262-269)
   hpd::adjust_refine  adjust / person score / refine grouping.py:172-191,276,193-250
   hpd::decode         all of the above in one call   (from_preds, results.py:225-238)
+  hpd::coco_eval      pycocotools COCOeval(..., "keypoints").evaluate() + accumulate() (bin/eval.py:52-65)
 """
 import ctypes
 from typing import List, Optional, Sequence
@@ -19,7 +20,8 @@ import torch
 from torch import Tensor
 
 from . import _lib
-from ._lib import HpdBuffers, HpdImage, HpdMap, HpdParams, HpdRecordLayout, HpdScaleInputs
+from ._lib import (HpdBuffers, HpdCocoDets, HpdCocoEvalOutputs, HpdCocoEvalParams, HpdCocoGts, HpdImage, HpdMap,
+                   HpdParams, HpdRecordLayout, HpdScaleInputs)
 
 COCO_FLIP_INDEX = [0, 2, 1, 4, 3, 6, 5, 8, 7, 10, 9, 12, 11, 14, 13, 16, 15]  # transforms.py:11
 JOINTS_ORDER_17 = [0, 1, 2, 3, 4, 5, 6, 11, 12, 7, 8, 9, 10, 13, 14, 15, 16]   # grouping.py:63-65
@@ -299,6 +301,82 @@ def run_stage(stage: str, bufs: DecodeBuffers, params: HpdParams, scales=None, n
     return bufs
 
 
+def coco_eval_params(num_images: int, num_kpts: int, max_dets: int, max_gts: int, iou_thrs: Sequence[float],
+                     rec_thrs: Sequence[float], area_rng: Sequence[float], kpt_vars: Sequence[float]) -> HpdCocoEvalParams:
+    """HpdCocoEvalParams; the thresholds and variances are taken as given (float64, computed by NumPy upstream).
+    area_rng is flat: [lo0, hi0, lo1, hi1, ...]."""
+    p = HpdCocoEvalParams()
+    p.num_images, p.num_kpts, p.max_dets, p.max_gts = num_images, num_kpts, max_dets, max_gts
+    p.num_iou_thrs, p.num_rec_thrs, p.num_areas = len(iou_thrs), len(rec_thrs), len(area_rng) // 2
+    if (len(iou_thrs) > _lib.HPD_COCO_MAX_IOU_THRS or len(rec_thrs) > _lib.HPD_COCO_MAX_REC_THRS
+            or len(area_rng) > 2 * _lib.HPD_COCO_MAX_AREAS or len(area_rng) % 2 or len(kpt_vars) != num_kpts
+            or num_kpts > _lib.HPD_MAX_KPTS):
+        raise _lib.HpdError(f"coco_eval: at most {_lib.HPD_COCO_MAX_IOU_THRS} OKS thresholds, {_lib.HPD_COCO_MAX_REC_THRS} "
+                            f"recall thresholds, {_lib.HPD_COCO_MAX_AREAS} [lo, hi] area ranges and one variance per "
+                            f"joint (<= {_lib.HPD_MAX_KPTS})")
+    for j, v in enumerate(iou_thrs):
+        p.iou_thrs[j] = v
+    for j, v in enumerate(rec_thrs):
+        p.rec_thrs[j] = v
+    for j, v in enumerate(area_rng):
+        p.area_rng[j // 2][j % 2] = v
+    for j, v in enumerate(kpt_vars):
+        p.kpt_vars[j] = v
+    return p
+
+
+def run_coco_eval(params: HpdCocoEvalParams, records: Sequence[Tensor], row_of_image, off_coco: int, off_count: int,
+                  person_stride: int, max_per_row: int, gt: Sequence[Tensor], outs: Sequence[Optional[Tensor]]):
+    """hpd_coco_eval on the current stream.  records: uint8 CUDA tensors [rows, >= row bytes] whose rows are read in
+    place; row_of_image: host int64 [I], the row of image i counted across ``records`` in order (-1: none).
+    gt: (kpts, area, bbox, iscrowd, ignore, n_gt); outs: (precision, recall, scores, oks, codes, npig), the last three
+    optional (None)."""
+    dev = gt[0].device
+    rows = torch.as_tensor(row_of_image, dtype=torch.int64).cpu()
+    if rows.numel() != params.num_images:
+        raise _lib.HpdError("coco_eval: row_of_image needs one entry per image")
+    for t in records:
+        if not t.is_cuda or t.dtype != torch.uint8 or t.dim() != 2 or t.stride(1) != 1 or t.device != dev:
+            raise _lib.HpdError("coco_eval: detection rows must be 2-D uint8 CUDA tensors with packed bytes, on the "
+                                "ground truth's device")
+    if not records:
+        records = [torch.zeros((0, 8), device=dev, dtype=torch.uint8)]
+    base = min(t.data_ptr() for t in records)
+    starts = torch.tensor([0] + [t.shape[0] for t in records], dtype=torch.int64).cumsum(0)
+    if int(rows.max()) >= int(starts[-1]):
+        raise _lib.HpdError("coco_eval: row_of_image points past the last detection row")
+    which = torch.searchsorted(starts[1:], rows, right=True).clamp(max=len(records) - 1)
+    tbase = torch.tensor([t.data_ptr() - base for t in records], dtype=torch.int64)
+    pitch = torch.tensor([t.stride(0) for t in records], dtype=torch.int64)
+    offsets = torch.where(rows >= 0, tbase[which] + (rows - starts[which]) * pitch[which], torch.full_like(rows, -1))
+    offsets = offsets.to(dev)
+    d = HpdCocoDets()
+    d.base, d.row_offset, d.off_coco, d.off_count = base, offsets.data_ptr(), off_coco, off_count
+    d.person_stride, d.max_per_row = person_stride, max_per_row
+    g = HpdCocoGts()
+    for (name, dtype), t in zip((("kpts", torch.float64), ("area", torch.float64), ("bbox", torch.float64),
+                                 ("iscrowd", torch.uint8), ("ignore", torch.uint8), ("n_gt", torch.int32)), gt):
+        if not t.is_cuda or t.dtype != dtype or not t.is_contiguous() or t.device != dev:
+            raise _lib.HpdError(f"coco_eval: gt {name} must be a contiguous CUDA {dtype} tensor")
+        setattr(g, name, t.data_ptr())
+    o = HpdCocoEvalOutputs()
+    for name, t in zip(("precision", "recall", "scores", "oks", "codes", "npig"), outs):
+        if t is not None:
+            if not t.is_cuda or not t.is_contiguous() or t.device != dev:
+                raise _lib.HpdError(f"coco_eval: output {name} must be a contiguous CUDA tensor")
+            setattr(o, name, t.data_ptr())
+    L = _lib.lib()
+    n = ctypes.c_size_t(0)
+    _lib.check(L.hpd_coco_eval_workspace_bytes(ctypes.byref(params), ctypes.byref(n)), "hpd_coco_eval_workspace_bytes")
+    ws = torch.empty((max(n.value, 8),), device=dev, dtype=torch.uint8)
+    with torch.cuda.device(dev):
+        rc = L.hpd_coco_eval(ctypes.byref(params), ctypes.byref(d), ctypes.byref(g), ctypes.byref(o), ws.data_ptr(),
+                             ws.numel(), _stream_ptr(dev))
+    _lib.check(rc, "hpd_coco_eval")
+    _count(L)
+    return outs
+
+
 def _scales_from_lists(hm_lo, hm_hi, tag, hm_lo_f, hm_hi_f, tag_f):
     n = len(hm_lo)
     flip = len(hm_lo_f) > 0
@@ -432,6 +510,44 @@ def prepare_input_op(images: Sequence[Tensor], matrices: Tensor, out_h: int, out
     _lib.check(rc, "hpd_prepare_input")
     _count(L)
     return out
+
+
+@torch.library.custom_op("hpd::coco_eval", mutates_args=())
+def coco_eval_op(records: Sequence[Tensor], row_of_image: Tensor, off_coco: int, off_count: int, person_stride: int,
+                 max_per_row: int, gt_kpts: Tensor, gt_area: Tensor, gt_bbox: Tensor, gt_iscrowd: Tensor,
+                 gt_ignore: Tensor, n_gt: Tensor, iou_thrs: Sequence[float], rec_thrs: Sequence[float],
+                 area_rng: Sequence[float], kpt_vars: Sequence[float], max_dets: int, debug: bool) -> List[Tensor]:
+    """COCOeval(gt, dt, "keypoints").evaluate() + accumulate() for category 1 (pycocotools cocoeval.py):
+    detections read in place from ``records`` (see run_coco_eval), ground truth padded [I,G,...].
+    -> [precision [T,R,A], recall [T,A], scores [T,R,A], oks [I,max_dets,G], codes [A,T,I,max_dets] uint8,
+    npig [A] int64]; the last three are empty unless ``debug``."""
+    I, G, K = gt_kpts.shape[:3]
+    params = coco_eval_params(I, K, max_dets, G, iou_thrs, rec_thrs, area_rng, kpt_vars)
+    T, R, A = params.num_iou_thrs, params.num_rec_thrs, params.num_areas
+    f64 = dict(device=gt_kpts.device, dtype=torch.float64)
+    outs = [torch.empty((T, R, A), **f64), torch.empty((T, A), **f64), torch.empty((T, R, A), **f64)]
+    if debug:
+        outs += [torch.empty((I, max_dets, G), **f64), torch.empty((A, T, I, max_dets), device=gt_kpts.device,
+                 dtype=torch.uint8), torch.empty((A,), device=gt_kpts.device, dtype=torch.int64)]
+    else:
+        outs += [None, None, None]
+    run_coco_eval(params, records, row_of_image, off_coco, off_count, person_stride, max_per_row,
+                  (gt_kpts, gt_area, gt_bbox, gt_iscrowd, gt_ignore, n_gt), outs)
+    return [t if t is not None else gt_kpts.new_empty((0,)) for t in outs]
+
+
+@coco_eval_op.register_fake
+def _(records, row_of_image, off_coco, off_count, person_stride, max_per_row, gt_kpts, gt_area, gt_bbox, gt_iscrowd,
+      gt_ignore, n_gt, iou_thrs, rec_thrs, area_rng, kpt_vars, max_dets, debug):
+    I, G = gt_kpts.shape[:2]
+    T, R, A = len(iou_thrs), len(rec_thrs), len(area_rng) // 2
+    f = lambda *s: gt_kpts.new_empty(s)
+    if debug:
+        tail = [f(I, max_dets, G), gt_kpts.new_empty((A, T, I, max_dets), dtype=torch.uint8),
+                gt_kpts.new_empty((A,), dtype=torch.int64)]
+    else:
+        tail = [f(0), f(0), f(0)]
+    return [f(T, R, A), f(T, A), f(T, R, A)] + tail
 
 
 @prepare_input_op.register_fake

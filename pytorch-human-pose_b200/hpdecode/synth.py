@@ -138,3 +138,100 @@ def crowd(batch: int, size: int = 512, persons: int = 30, flip: bool = True, see
 def image_slice(scales, b: int):
     """Per-image view ([K,h,w] arrays) of a generator's output."""
     return [{k: v[b] for k, v in s.items()} for s in scales]
+
+
+class _Draws:
+    """Consumes U[0,1) float64 values of one seeded hash stream (float32 resolution), block by block."""
+
+    def __init__(self, seed: int, block: int = 1 << 16):
+        self.seed, self.block, self.n = seed, block, 0
+        self.buf, self.pos = np.zeros(0), 0
+
+    def take(self, n: int) -> np.ndarray:
+        if self.pos + n > len(self.buf):
+            self.buf = np.concatenate([self.buf[self.pos:], uniform((max(self.block, n),), self.seed * 7919 + self.n)
+                                       .astype(np.float64)])
+            self.pos, self.n = 0, self.n + 1
+        out = self.buf[self.pos:self.pos + n]
+        self.pos += n
+        return out
+
+    def one(self) -> float:
+        return float(self.take(1)[0])
+
+
+def coco_eval_set(num_images: int, seed: int = 0, num_kpts: int = 17, max_gts: int = 15, dets_per_image: int = 30,
+                  sigmas=None, spread: float = 1.0, crowd_frac: float = 0.05, no_kpt_frac: float = 0.05,
+                  no_gt_frac: float = 0.1, no_det_frac: float = 0.05, score_levels: int = 0):
+    """A seeded COCO keypoint evaluation set: (annotation dict, result list), shaped like val2017 person keypoints.
+
+    Each image has 0..max_gts ground-truth persons (none with probability ``no_gt_frac``) spread over the three area
+    bands (small < 32², medium, large > 96²), some crowd (``crowd_frac``) and some without a labelled joint
+    (``no_kpt_frac``, num_keypoints == 0).  It has ``dets_per_image`` detections (none with probability
+    ``no_det_frac``): most ground-truth persons get one whose joints are the ground truth's moved by up to
+    ``spread`` x 3 OKS standard deviations (so OKS values cover the whole range), some a second, lower-scored one,
+    and the rest are false positives.  ``score_levels`` > 0 rounds scores to that many levels: ties inside and
+    across images.  The result list holds the images in a shuffled order, each image's detections together."""
+    K = num_kpts
+    if sigmas is not None:
+        sig = np.asarray(sigmas, np.float64)
+    elif K == 17:
+        sig = np.array([.26, .25, .25, .35, .35, .79, .79, .72, .72, .62, .62, 1.07, 1.07, .87, .87, .89, .89]) / 10.0
+    else:
+        sig = np.full(K, 0.05)
+    rnd = _Draws(seed)
+    images, anns, per_image = [], [], []
+    image_id = 0
+    for i in range(num_images):
+        image_id += 1 + int(rnd.one() * 3)
+        images.append({"id": image_id, "width": 640, "height": 480})
+        ng = 0 if rnd.one() < no_gt_frac else int(rnd.one() * (max_gts + 1))
+        gts = []
+        for _ in range(ng):
+            band = rnd.one()
+            s = (20.0 if band < 0.3 else 60.0 if band < 0.65 else 160.0) * (0.7 + 0.6 * rnd.one())
+            cx, cy = 40.0 + 560.0 * rnd.one(), 40.0 + 400.0 * rnd.one()
+            u = rnd.take(3 * K)
+            x = cx + (u[:K] - 0.5) * s
+            y = cy + (u[K:2 * K] - 0.5) * s
+            v = np.where(u[2 * K:] > 0.2, 2.0, np.where(u[2 * K:] > 0.1, 1.0, 0.0))
+            if rnd.one() < no_kpt_frac:
+                v[:] = 0.0
+            x, y = np.where(v > 0, x, 0.0), np.where(v > 0, y, 0.0)
+            bbox = [cx - 0.6 * s, cy - 0.6 * s, 1.2 * s, 1.2 * s]
+            area = s * s * (0.5 + 0.4 * rnd.one())
+            kp = np.stack([x, y, v], 1).ravel()
+            ann = {"id": len(anns) + 1, "image_id": image_id, "category_id": 1, "keypoints": kp.tolist(),
+                   "num_keypoints": int(np.count_nonzero(v > 0)), "area": area, "bbox": bbox,
+                   "iscrowd": int(rnd.one() < crowd_frac)}
+            anns.append(ann)
+            gts.append((cx, cy, s, x, y, v, area))
+        dets = []
+        if rnd.one() >= no_det_frac:
+            for cx, cy, s, x, y, v, area in gts:
+                for copy in range(2):
+                    if rnd.one() > (0.85 if copy == 0 else 0.2) or len(dets) >= dets_per_image:
+                        continue
+                    level = 3.0 * spread * rnd.one()
+                    u = rnd.take(2 * K)
+                    sd = sig * 2 * np.sqrt(area) * level
+                    xd = np.where(v > 0, x, cx) + (u[:K] - 0.5) * 2 * sd
+                    yd = np.where(v > 0, y, cy) + (u[K:] - 0.5) * 2 * sd
+                    dets.append((xd, yd, rnd.one() * (0.5 if copy else 1.0)))
+            while len(dets) < dets_per_image:
+                s = 10.0 + 150.0 * rnd.one()
+                cx, cy = 640.0 * rnd.one(), 480.0 * rnd.one()
+                u = rnd.take(2 * K)
+                dets.append((cx + (u[:K] - 0.5) * s, cy + (u[K:] - 0.5) * s, 0.6 * rnd.one()))
+        order = np.argsort(rnd.take(len(dets)), kind="mergesort")
+        recs = []
+        for j in order:
+            xd, yd, score = dets[j]
+            if score_levels:
+                score = round(score * score_levels) / score_levels
+            kp = np.stack([xd, yd, np.ones(K)], 1).ravel()
+            recs.append({"image_id": image_id, "category_id": 1, "keypoints": kp.tolist(), "score": float(score)})
+        per_image.append(recs)
+    results = [r for i in np.argsort(rnd.take(num_images), kind="mergesort") for r in per_image[i]]
+    dataset = {"images": images, "annotations": anns, "categories": [{"id": 1, "name": "person"}]}
+    return dataset, results
