@@ -15,7 +15,8 @@
  *  - Return value: 0 on success, an HPD_E* code otherwise; hpd_last_error_string() gives the
  *    message of the calling thread's last failure.  No C++ exception crosses the ABI.
  *  - Re-entrant: one workspace per in-flight call; safe from one host thread per GPU.
- *  - Inputs must be finite (NaN ordering of torch.topk / MaxPool2d is not reproduced).
+ *  - Inputs must be finite (NaN ordering of torch.topk / MaxPool2d is not reproduced).  hpd_group alone returns on
+ *    any top-k tensors: costs it cannot solve on are guarded and reported in flags bit 1.
  */
 #ifndef HPDECODE_H_
 #define HPDECODE_H_
@@ -33,7 +34,7 @@ extern "C" {
 #define HPD_EXPORT
 #endif
 
-#define HPD_ABI_VERSION 4
+#define HPD_ABI_VERSION 5
 #define HPD_MAX_KPTS 32     /* joints per person (COCO: 17) */
 #define HPD_MAX_PEOPLE 32   /* max_num_people == top-k; the warp-wide Hungarian handles n <= 32 */
 #define HPD_MAX_EMB 2       /* tag embedding dims: 1 (no flip test) or 2 (flip test) */
@@ -117,7 +118,11 @@ typedef struct HpdBuffers {
   float* poses;         /* [B,M,K,3+E]    grouped joints [x,y,score,tag..]; zero-filled rows     */
   float* person_scores; /* [B,M]          grouping.py:276                                        */
   int32_t* n_person;    /* [B]            persons returned (<= M)                                */
-  int32_t* flags;       /* [B]            bit0: empty-scene fallback fired (grouping.py:262-269)  */
+  int32_t* flags;       /* [B]            bit0: empty-scene fallback fired (grouping.py:262-269);
+                         * bit1: grouping guarded a cost the reference's munkres never returns on -- NaN, +-inf or
+                         * |cost| >= 2^63 (from NaN / inf tags or scores, or tags ~1e17 apart) was replaced by 1e10
+                         * (grouping.py:126-128's "cannot match" value), or a solve reached its step-6 cap and left
+                         * that joint's detections unmatched.  Never set on finite inputs of the reference's range. */
   float* tag_bmin;      /* [B,K,HB,WPR]   HB = (H+3)/4: lower / upper bound of the first tag component over     */
   float* tag_bmax;      /* [B,K,HB,WPR]   4 image rows x one 32-pixel word (refine prefilter; -inf/+inf = none) */
   uint8_t* records;     /* [B][row_bytes] optional (NULL = not written): one result record per image, laid out as
@@ -141,7 +146,7 @@ typedef struct HpdBuffers {
  *   poses         f32 [M][K][3+E] grouped joints in network-input pixels (x, y, score, tags), grouping.py:283
  *   person_scores f32 [M]        grouping.py:276
  *   n_person      i32            persons returned
- *   flags         i32            bit 0: empty-scene fallback fired                                              */
+ *   flags         i32            bit 0: empty-scene fallback fired; bit 1: grouping guarded a cost (HpdBuffers)  */
 typedef struct HpdRecordLayout {
   int64_t row_bytes;
   int64_t off_coco, off_poses, off_person_scores, off_n_person, off_flags;
@@ -242,7 +247,7 @@ HPD_EXPORT int hpd_nms(const HpdParams* p, const HpdBuffers* buf, float* nms_out
 HPD_EXPORT int hpd_topk(const HpdParams* p, const HpdBuffers* buf, void* stream);
 
 /* (d) associative-embedding grouping: grouping.py:85-145 + py_max_match :55-59 + fallback :262-269.
- * Reads scores_k, coords_k, tags_k; writes poses, n_person, flags. */
+ * Reads scores_k, coords_k, tags_k; writes poses, n_person, flags.  Returns on every input: see flags bit 1. */
 HPD_EXPORT int hpd_group(const HpdParams* p, const HpdBuffers* buf, void* stream);
 
 /* (e) adjust + person score + refine: grouping.py:172-191, :276, :193-250.

@@ -143,7 +143,7 @@ def match_by_tag(tags_k, coords_k, scores_k, det_thr: float, tag_thr: float, M: 
     nt = ctypes.c_int32(0)
     rc = lib().hpo_match_by_tag(_p(tags_k), _p(coords_k, ctypes.c_int32), _p(scores_k), K, M, E,
                                 ctypes.c_double(det_thr), ctypes.c_double(tag_thr), None, _p(poses),
-                                ctypes.byref(n), ctypes.byref(nt))
+                                ctypes.byref(n), ctypes.byref(nt), None)
     if rc:
         raise ValueError("oracle match_by_tag limits exceeded")
     return poses[: n.value].copy(), nt.value

@@ -126,7 +126,10 @@ struct Munkres {
     int find_in_row(int r, int m) { for (int j = 0; j < n; ++j) if (mark[r][j] == m) return j; return -1; }
     int find_in_col(int c, int m) { for (int i = 0; i < n; ++i) if (mark[i][c] == m) return i; return -1; }
 
-    void run() {
+    // Returns false when the step-6 cap stopped it (see hpo_match_by_tag's cost guard).
+    bool run() {
+        const int cap = n * (n + 1);
+        int n6 = 0;
         std::memset(mark, 0, sizeof(mark));
         clear_covers();
         // step 1
@@ -147,7 +150,7 @@ struct Munkres {
                 for (int i = 0; i < n; ++i)
                     for (int j = 0; j < n; ++j)
                         if (mark[i][j] == 1 && !colc[j]) { colc[j] = true; ++count; }
-                if (count >= n) return;
+                if (count >= n) return true;
                 step = 4;
             } else if (step == 4) {
                 int row = 0, col = 0;
@@ -175,6 +178,7 @@ struct Munkres {
                 for (int i = 0; i < n; ++i) for (int j = 0; j < n; ++j) if (mark[i][j] == 2) mark[i][j] = 0;
                 step = 3;
             } else {  // step 6
+                if (++n6 > cap) return false;
                 double m = 9.223372036854775807e18;  // sys.maxsize
                 for (int i = 0; i < n; ++i) for (int j = 0; j < n; ++j)
                     if (!rowc[i] && !colc[j] && m > at(i, j)) m = at(i, j);
@@ -348,14 +352,17 @@ HPO_API int hpo_munkres(const double* cost, int rows, int cols, int32_t* out_col
 }
 
 // grouping.py:85-145 as a flat-array algorithm.  Output poses [M][K][3+E] f32
-// (zeros for missing joints), *n_person = min(#persons, M), *n_total = #persons.
+// (zeros for missing joints), *n_person = min(#persons, M), *n_total = #persons, *flags (may be
+// NULL) = hpd_group's bit 1: a cost was replaced by the guard below or a solve hit its step-6 cap.
 HPO_API int hpo_match_by_tag(const float* tags_k, const int32_t* coords_k, const float* scores_k,
                              int K, int M, int E, double det_thr, double tag_thr,
-                             const int* joints_order, float* poses, int32_t* n_person, int32_t* n_total) {
+                             const int* joints_order, float* poses, int32_t* n_person, int32_t* n_total,
+                             int32_t* flags) {
     if (K > kMaxKpts || M > kMaxPeople || E > kMaxEmb) return 1;
     static const int kOrder17[17] = {0, 1, 2, 3, 4, 5, 6, 11, 12, 7, 8, 9, 10, 13, 14, 15, 16};
     const int D = 3 + E;
     std::memset(poses, 0, sizeof(float) * (size_t)M * K * D);
+    int fl = 0;
     int P = 0;              // persons tracked (<= M)
     int Ptotal = 0;         // persons created (dict size); only the first M are ever read
     float key[kMaxPeople];
@@ -422,15 +429,21 @@ HPO_API int hpo_match_by_tag(const float* tags_k, const int32_t* coords_k, const
                 }
                 const double dn = std::sqrt(s);
                 dist[(size_t)a * G + p] = dn;
-                C[(size_t)a * n + p] = std::nearbyint(dn) * 100.0 - sc;   // np.round: half to even
+                double c = std::nearbyint(dn) * 100.0 - sc;   // np.round: half to even
+                // Library policy, not the reference's: munkres 1.1.4 never returns on a NaN row, nor
+                // once step 6's sys.maxsize sentinel stops making zeros (costs >= 2^63).  Such costs
+                // become the reference's own "cannot match" value and the image is flagged.
+                if (!(std::fabs(c) < 0x1p63)) { c = 1e10; fl |= 2; }
+                C[(size_t)a * n + p] = c;
             }
             for (int p = G; p < n; ++p) C[(size_t)a * n + p] = 1e10;
         }
         Munkres mk; mk.n = n; mk.C = C.data();
-        mk.run();
+        const bool solved = mk.run();    // with the guard the cap is never reached; if it is, nobody matches
+        if (!solved) fl |= 2;
         for (int a = 0; a < nr; ++a) {
-            const int c = mk.find_in_row(a, 1);
-            if (c < G && dist[(size_t)a * G + c] < tag_thr) {
+            const int c = solved ? mk.find_in_row(a, 1) : -1;
+            if (c >= 0 && c < G && dist[(size_t)a * G + c] < tag_thr) {
                 put_joint(c, k, rows[a]);
                 const float* tg = tags_k + (size_t)(k * M + rows[a]) * E;
                 for (int e = 0; e < E; ++e) taglist[c][ntag[c]][e] = tg[e];
@@ -442,6 +455,7 @@ HPO_API int hpo_match_by_tag(const float* tags_k, const int32_t* coords_k, const
     }
     *n_person = P;
     if (n_total) *n_total = Ptotal;
+    if (flags) *flags = fl;
     return 0;
 }
 
@@ -528,7 +542,7 @@ HPO_API int hpo_parse(const float* hm, const float* tags, int K, int H, int W, i
     if (scores_k_out) std::memcpy(scores_k_out, scores_k.data(), scores_k.size() * 4);
     if (idx_k_out) std::memcpy(idx_k_out, idx_k.data(), idx_k.size() * 4);
     int32_t P = 0, Pt = 0;
-    if (hpo_match_by_tag(tags_k.data(), coords_k.data(), scores_k.data(), K, M, E, det_thr, tag_thr, nullptr, poses, &P, &Pt)) return 1;
+    if (hpo_match_by_tag(tags_k.data(), coords_k.data(), scores_k.data(), K, M, E, det_thr, tag_thr, nullptr, poses, &P, &Pt, nullptr)) return 1;
     *fallback = 0;
     if (P == 0) {
         *fallback = 1;

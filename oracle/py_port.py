@@ -66,7 +66,10 @@ def top_k(hm, tags, M):
     return tags_k.numpy(), coords.numpy().astype(np.int32), scores.numpy(), idx.numpy().astype(np.int32)
 
 
-def match_by_tag(tags_k, coords_k, scores_k, M, det_thr, tag_thr):
+def match_by_tag(tags_k, coords_k, scores_k, M, det_thr, tag_thr, joints_order=None, trace=None):
+    """``joints_order`` replaces grouping.py:63-65's order; ``trace`` (a list) receives one dict per joint step with
+    detections: the selection mask, the person keys and tag lists before the step, the distances and the solver's
+    pairs (tests count the branches their scenes reach from it)."""
     K, _, E = tags_k.shape
     keys = []          # float32 key per person, insertion order
     rows = []          # [K, 3+E] float64 per person
@@ -85,13 +88,17 @@ def match_by_tag(tags_k, coords_k, scores_k, M, det_thr, tag_thr):
         tag_lists.append([tag])
 
     for it in range(K):
-        k = JOINTS_ORDER[it] if K == 17 else it
+        k = joints_order[it] if joints_order is not None else (JOINTS_ORDER[it] if K == 17 else it)
         tags = tags_k[k]
         joints = np.concatenate((coords_k[k], scores_k[k, :, None], tags), 1)
         sel = joints[:, 2] > det_thr
         tags, joints = tags[sel], joints[sel]
         if joints.shape[0] == 0:
             continue
+        step = None if trace is None else dict(k=k, sel=sel, tags=tags, keys=list(keys),
+                                               tag_lists=[list(t) for t in tag_lists[:M]], dist=None, pairs=[])
+        if step is not None:
+            trace.append(step)
         if it == 0 or not keys:
             for tag, joint in zip(tags, joints):
                 seed(k, joint, tag)
@@ -104,7 +111,10 @@ def match_by_tag(tags_k, coords_k, scores_k, M, det_thr, tag_thr):
         n_new = joints.shape[0]
         if n_new > G:
             cost = np.concatenate((cost, np.zeros((n_new, n_new - G)) + 1e10), axis=1)
-        for r, c in Munkres().compute(cost):
+        pairs = Munkres().compute(cost)
+        if step is not None:
+            step.update(dist=saved, pairs=pairs)
+        for r, c in pairs:
             if r < n_new and c < G and saved[r][c] < tag_thr:
                 rows[c][k] = joints[r]
                 tag_lists[c].append(tags[r])

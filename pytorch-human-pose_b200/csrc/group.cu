@@ -22,6 +22,12 @@
 //   * the Hungarian solver replays munkres 1.1.4 step by step: lane r owns matrix row r and a
 //     32-bit mask of its zero entries, so "find the last uncovered zero in cyclic order" is bit
 //     arithmetic; the (C + m) - m update order of step 6 is kept.
+//   * library policy, not the reference's: a cost that is not finite or whose magnitude is >= 2^63
+//     is replaced by 1e10 (grouping.py:126-128's "cannot match" value) before the solver runs, and
+//     flags bit 1 is set.  On such a row munkres 1.1.4 never terminates (a NaN row never gets a
+//     zero; step 6's sys.maxsize sentinel stops making zeros above 2^63).  With finite costs below
+//     2^63 every step 6 makes a zero, so an augmentation needs at most n step-6 calls; the solver
+//     still stops after n (n + 1) of them, sets bit 1 and leaves the step's detections unmatched.
 #include "common.cuh"
 #ifdef HPD_GROUP_PROFILE
 #include <cstdio>
@@ -49,6 +55,7 @@ __device__ long long gp_acc[12];
 constexpr int kGroupWarps = 4;
 constexpr int CW = NP / kGroupWarps;    // matrix columns per warp
 constexpr int TL = HPD_MAX_KPTS * HPD_MAX_EMB + 1;   // odd person stride: lanes hit distinct banks
+constexpr int kSolverCapped = -2;       // munkres_cta's result on every lane when its step-6 cap was reached
 
 struct GroupSmem {
   double C[NP][CS];                     // cost matrix as built (real detections x real persons)
@@ -86,10 +93,12 @@ __device__ __forceinline__ double min4(const double (*pm)[NP], int i) {
 
 // munkres 1.1.4 Munkres.compute on the n x n matrix: rows < nr and columns < G come from sm.C,
 // columns G..n-1 of those rows are 1e10 (grouping.py:126-128), rows nr..n-1 are munkres' zero
-// padding.  Returns the starred column of this lane's row (valid for lane < n).  Called by all
-// four warps; contains __syncthreads().
+// padding.  Returns the starred column of this lane's row (valid for lane < n), or kSolverCapped on
+// every lane after n (n + 1) step-6 calls.  Called by all four warps; contains __syncthreads().
 __device__ int munkres_cta(GroupSmem& sm, int nr, int G, int n, int lane, int w) {
   const unsigned nmask = (n >= 32) ? kFull : ((1u << n) - 1u);
+  const int cap = n * (n + 1);
+  int n6 = 0;
   const int cb = w * CW;
   const double kInf = __longlong_as_double(0x7ff0000000000000ll);
   double c[CW];
@@ -173,7 +182,8 @@ __device__ int munkres_cta(GroupSmem& sm, int nr, int G, int n, int lane, int w)
       if (augment) break;
       GP_BEGIN(t_s6);
       GP_COUNT(10);
-      // step 6
+      // step 6 (the count is uniform over the CTA, so every thread leaves here together)
+      if (++n6 > cap) return kSolverCapped;
       double m = 9.223372036854775807e18;
       if (lane < n && !((rowcov >> lane) & 1u)) {
 #pragma unroll
@@ -240,6 +250,7 @@ __global__ void __launch_bounds__(32 * kGroupWarps) group_kernel(const float* __
   float* out = poses + (size_t)b * M * K * D;
   for (int i = threadIdx.x; i < M * K * D; i += 32 * kGroupWarps) out[i] = 0.f;
 
+  int fl = 0;         // flags[b], uniform
   int P = 0;          // persons stored (<= M), uniform
   int Ptotal = 0;     // persons created, uniform
   float key = 0.f;    // lane p: dict key of person p
@@ -341,6 +352,7 @@ __global__ void __launch_bounds__(32 * kGroupWarps) group_kernel(const float* __
       // cost matrix (grouping.py:116-128): the nr x G real pairs are spread over the four warps,
       // four independent pairs per thread and round (the float64 sqrt chains overlap); the 1e10
       // columns and zero rows are synthesised when the solver loads its registers
+      bool guarded = false;
       {
         constexpr int U = 4;
         const int npairs = nr * G;
@@ -363,15 +375,24 @@ __global__ void __launch_bounds__(32 * kGroupWarps) group_kernel(const float* __
               }
               const double dn = __dsqrt_rn(s);
               sm.D[a][p] = dn;
-              sm.C[a][p] = __dsub_rn(__dmul_rn(rint(dn), 100.0), (double)sc_a);
+              double cst = __dsub_rn(__dmul_rn(rint(dn), 100.0), (double)sc_a);
+              if (!(fabs(cst) < 9.223372036854775808e18)) {   // NaN, +-inf, |cost| >= 2^63
+                cst = 1e10;
+                guarded = true;
+              }
+              sm.C[a][p] = cst;
             }
           }
         }
       }
-      __syncthreads();
+      if (__syncthreads_or(guarded)) fl |= 2;
       GP_END(6, t_cost);
       GP_BEGIN(t_mk);
       star = munkres_cta(sm, nr, G, n, lane, w);
+      if (star == kSolverCapped) {
+        fl |= 2;
+        star = -1;
+      }
       GP_END(7, t_mk);
     }
 
@@ -445,11 +466,10 @@ __global__ void __launch_bounds__(32 * kGroupWarps) group_kernel(const float* __
   }
 #endif
 
-  int fl = 0;
   if (w != 0) return;
   if (Ptotal == 0) {
     // grouping.py:262-269: one pseudo-person from the best candidate of every joint, score := 0.01
-    fl = 1;
+    fl |= 1;
     P = 1;
     for (int k = lane; k < K; k += 32) {
       float* d = out + (size_t)k * D;
