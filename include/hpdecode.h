@@ -9,7 +9,7 @@
  *  - Every pointer is a DEVICE pointer unless the name ends in _host.  The caller owns every
  *    buffer; the library allocates nothing, never synchronises, and enqueues all work on the
  *    given stream (a cudaStream_t passed as void*; NULL = the legacy default stream).
- *  - All maps are float32.  Network outputs are NCHW views with explicit batch / channel
+ *  - All maps the library writes are float32.  Network outputs are float32, float16 or bfloat16 NCHW views with explicit batch / channel
  *    strides in ELEMENTS and contiguous rows (HigherHRNet's hm_lo / tag are channel slices of
  *    one 34-channel tensor: src/keypoints/architectures/higher_hrnet.py:78-79).
  *  - Return value: 0 on success, an HPD_E* code otherwise; hpd_last_error_string() gives the
@@ -34,7 +34,7 @@ extern "C" {
 #define HPD_EXPORT
 #endif
 
-#define HPD_ABI_VERSION 5
+#define HPD_ABI_VERSION 6
 #define HPD_MAX_KPTS 32     /* joints per person (COCO: 17) */
 #define HPD_MAX_PEOPLE 32   /* max_num_people == top-k; the warp-wide Hungarian handles n <= 32 */
 #define HPD_MAX_EMB 2       /* tag embedding dims: 1 (no flip test) or 2 (flip test) */
@@ -53,8 +53,9 @@ enum {
 
 enum {
   HPD_F32 = 0,          /* float32 maps (inference path, model.py:78-111) */
-  HPD_F16 = 1           /* IEEE half maps: the validation-time caller runs the net under autocast
+  HPD_F16 = 1,          /* IEEE half maps: the validation-time caller runs the net under autocast
                          * (module.py:78,100-110); values are widened on load, all arithmetic stays float32 */
+  HPD_BF16 = 2          /* bfloat16 maps (the net under bf16 autocast): widened exactly on load like HPD_F16 */
 };
 
 /* One NCHW tensor view. */
@@ -63,7 +64,7 @@ typedef struct HpdMap {
   int64_t stride_b;   /* elements between images */
   int64_t stride_c;   /* elements between channels; rows are contiguous (stride_y == w) */
   int32_t h, w;
-  int32_t dtype;      /* HPD_F32 or HPD_F16; all maps of one call share it */
+  int32_t dtype;      /* HPD_F32, HPD_F16 or HPD_BF16; all maps of one call share it (hpd_resize_bilinear: HPD_F32) */
   int32_t reserved_;
 } HpdMap;
 

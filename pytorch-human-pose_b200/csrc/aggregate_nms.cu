@@ -17,6 +17,7 @@
 //
 // This file holds the GENERIC kernel (any resize ratios, any number of scales).  It is the
 // correctness anchor; aggregate_nms_x2.cu specialises the standard single-scale x2/x2/x4 case.
+#include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
 #include "common.cuh"
@@ -60,7 +61,7 @@ struct AggArgs {
   int tags_preflipped;
   int in_vec_ok;   // inputs allow 16-byte loads (aligned bases, strides multiples of 4 elements)
   int in_vec_ok_all;   // ... for every scale
-  int half_in;     // inputs are IEEE halves (HPD_F16); the const float* members then point at __half data
+  int dtype;       // HPD_F32 / HPD_F16 / HPD_BF16: the const float* input members point at elements of this type
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -198,8 +199,8 @@ __global__ void __launch_bounds__(kAggThreads) agg_nms_generic_kernel(const AggA
           const int x = lxa + c;
           for (int r = rg; r < nly; r += groups) {
             const int rowo = (lya + r) * S.lw;
-            float v = in_elem(p, po + rowo + x, a.half_in);
-            if (pf) v = __fmul_rn(__fadd_rn(v, in_elem(pf, pfo + rowo + (S.lw - 1 - x), a.half_in)), 0.5f);
+            float v = in_elem(p, po + rowo + x, a.dtype);
+            if (pf) v = __fmul_rn(__fadd_rn(v, in_elem(pf, pfo + rowo + (S.lw - 1 - x), a.dtype)), 0.5f);
             loT[r * a.LO_C + c] = v;
           }
         }
@@ -215,8 +216,8 @@ __global__ void __launch_bounds__(kAggThreads) agg_nms_generic_kernel(const AggA
           const int x = hxa + c;
           for (int r = rg; r < nhy; r += groups) {
             const int rowo = (hya + r) * S.hw;
-            float v = in_elem(p, po + rowo + x, a.half_in);
-            if (pf) v = __fmul_rn(__fadd_rn(v, in_elem(pf, pfo + rowo + (S.hw - 1 - x), a.half_in)), 0.5f);
+            float v = in_elem(p, po + rowo + x, a.dtype);
+            if (pf) v = __fmul_rn(__fadd_rn(v, in_elem(pf, pfo + rowo + (S.hw - 1 - x), a.dtype)), 0.5f);
             hiT[r * a.HI_C + c] = v;
           }
         }
@@ -320,7 +321,7 @@ __global__ void __launch_bounds__(kAggThreads) agg_nms_generic_kernel(const AggA
       for (int i = tid; i < nty * ntx; i += kAggThreads) {
         const int r = i / ntx, c = i % ntx;
         const int y = tya + r, x = txa + c;
-        loT[e * tile_words + r * a.TG_C + c] = in_elem(p, po + (size_t)y * a.tw + (unflip ? a.tw - 1 - x : x), a.half_in);
+        loT[e * tile_words + r * a.TG_C + c] = in_elem(p, po + (size_t)y * a.tw + (unflip ? a.tw - 1 - x : x), a.dtype);
       }
     }
     __syncthreads();
@@ -452,13 +453,14 @@ int check_map(const HpdMap& m, const char* name, bool required) {
     return HPD_OK;
   }
   if (m.h <= 0 || m.w <= 0) { set_error("%s: bad size %dx%d", name, m.h, m.w); return HPD_EINVAL; }
-  if (m.dtype != HPD_F32 && m.dtype != HPD_F16) { set_error("%s: unsupported dtype code %d", name, m.dtype); return HPD_EINVAL; }
+  if (m.dtype != HPD_F32 && m.dtype != HPD_F16 && m.dtype != HPD_BF16) { set_error("%s: unsupported dtype code %d", name, m.dtype); return HPD_EINVAL; }
   return HPD_OK;
 }
 
 // TagSource over the tag-scale inputs (map = NULL)
 int tag_source_from_inputs(const HpdParams* p, const HpdScaleInputs& in, TagSource* s, const char* who) {
-  if (in.tag.ptr == nullptr || in.tag.h <= 0 || in.tag.w <= 0 || (in.tag.dtype != HPD_F32 && in.tag.dtype != HPD_F16)) {
+  if (in.tag.ptr == nullptr || in.tag.h <= 0 || in.tag.w <= 0 || (in.tag.dtype != HPD_F32 && in.tag.dtype != HPD_F16 &&
+                                                                 in.tag.dtype != HPD_BF16)) {
     set_error("%s: the tag map of the tag scale is missing or malformed", who);
     return HPD_EINVAL;
   }
@@ -476,7 +478,7 @@ int tag_source_from_inputs(const HpdParams* p, const HpdScaleInputs& in, TagSour
   s->K = p->num_kpts; s->H = p->out_h; s->W = p->out_w; s->E = p->emb;
   s->th = in.tag.h; s->tw = in.tag.w;
   s->s_y = (float)s->th / (float)s->H; s->s_x = (float)s->tw / (float)s->W;   // as launch_aggregate_nms computes them
-  s->half_in = in.tag.dtype == HPD_F16;
+  s->dtype = in.tag.dtype;
   s->tags_preflipped = p->tags_preflipped;
   for (int k = 0; k < HPD_MAX_KPTS; ++k) s->flip[k] = p->flip_index[k];
   return HPD_OK;
@@ -522,8 +524,8 @@ int launch_aggregate_nms(const HpdParams* p, const HpdScaleInputs* scales, const
   for (int k = 0; k < HPD_MAX_KPTS; ++k) a.flip[k] = p->flip_index[k];
   const bool flip = scales[0].hm_lo_f.ptr != nullptr;
   const int dtype = scales[0].hm_lo.dtype;
-  a.half_in = dtype == HPD_F16;
-  const uintptr_t vec_align = a.half_in ? 8 : 16;    // four elements per vector load
+  a.dtype = dtype;
+  const uintptr_t vec_align = dtype == HPD_F32 ? 16 : 8;    // four elements per vector load
   int LO_R = 1, LO_C = 1, HI_R = 1, HI_C = 1;
   for (int s = 0; s < p->num_scales; ++s) {
     const HpdScaleInputs& in = scales[s];
@@ -616,7 +618,9 @@ int launch_aggregate_nms(const HpdParams* p, const HpdScaleInputs* scales, const
   } while (0)
 #define HPD_X2_LAUNCH(E_, NW_)                                                                              \
   do {                                                                                                      \
-    if (a.half_in) HPD_X2_LAUNCH_T(E_, NW_, __half); else HPD_X2_LAUNCH_T(E_, NW_, float);                  \
+    if (a.dtype == HPD_F16) HPD_X2_LAUNCH_T(E_, NW_, __half);                                                \
+    else if (a.dtype == HPD_BF16) HPD_X2_LAUNCH_T(E_, NW_, __nv_bfloat16);                                  \
+    else HPD_X2_LAUNCH_T(E_, NW_, float);                                                                   \
   } while (0)
       if (a.E == 1) { if (NW == 4) HPD_X2_LAUNCH(1, 4); else if (NW == 2) HPD_X2_LAUNCH(1, 2); else HPD_X2_LAUNCH(1, 1); }
       else          { if (NW == 4) HPD_X2_LAUNCH(2, 4); else if (NW == 2) HPD_X2_LAUNCH(2, 2); else HPD_X2_LAUNCH(2, 1); }
@@ -630,7 +634,7 @@ int launch_aggregate_nms(const HpdParams* p, const HpdScaleInputs* scales, const
   // several scales and / or other hi -> output ratios with the HigherHRNet structure (lo -> hi exactly x2,
   // tags exactly x4) -> column-walking multi-scale kernel (aggregate_nms_ms.cuh)
   {
-    bool ok = !(p->force_generic & 1) && !a.half_in && a.n_scales <= 3 && a.in_vec_ok_all && a.th * 4 == a.H && a.tw * 4 == a.W && a.W % 32 == 0 && a.H % 4 == 0 &&
+    bool ok = !(p->force_generic & 1) && a.n_scales <= 3 && a.in_vec_ok_all && a.th * 4 == a.H && a.tw * 4 == a.W && a.W % 32 == 0 && a.H % 4 == 0 &&
               a.W >= 256 && a.vec_ok;
     for (int s = 0; ok && s < a.n_scales; ++s) {
       const ScaleDev& S = a.sc[s];
@@ -672,18 +676,25 @@ int launch_aggregate_nms(const HpdParams* p, const HpdScaleInputs* scales, const
       const size_t smem = sizeof(float) * (size_t)g.total;
       if (smem <= 200 * 1024) {
         const dim3 grid((a.W + 128 * NW - 1) / (128 * NW), (a.H + ms::RB - 1) / ms::RB, a.B * a.K);
-#define HPD_MS_LAUNCH(E_, NW_, NS_)                                                                              \
+#define HPD_MS_LAUNCH(E_, NW_, NS_, T_)                                                                          \
   do {                                                                                                           \
-    if (int rc_ = ensure_dynamic_smem((const void*)ms::agg_nms_ms_kernel<E_, NW_, NS_>, smem, "agg_nms_ms_kernel")) return rc_; \
-    ms::agg_nms_ms_kernel<E_, NW_, NS_><<<grid, 32 * NW_, smem, st>>>(a, g);                                     \
+    if (int rc_ = ensure_dynamic_smem((const void*)ms::agg_nms_ms_kernel<E_, NW_, NS_, T_>, smem, "agg_nms_ms_kernel")) return rc_; \
+    ms::agg_nms_ms_kernel<E_, NW_, NS_, T_><<<grid, 32 * NW_, smem, st>>>(a, g);                                 \
+  } while (0)
+#define HPD_MS_NS_T(E_, NW_, T_)                                                                                 \
+  do {                                                                                                           \
+    if (a.n_scales == 1) HPD_MS_LAUNCH(E_, NW_, 1, T_); else if (a.n_scales == 2) HPD_MS_LAUNCH(E_, NW_, 2, T_); else HPD_MS_LAUNCH(E_, NW_, 3, T_); \
   } while (0)
 #define HPD_MS_NS(E_, NW_)                                                                                       \
   do {                                                                                                           \
-    if (a.n_scales == 1) HPD_MS_LAUNCH(E_, NW_, 1); else if (a.n_scales == 2) HPD_MS_LAUNCH(E_, NW_, 2); else HPD_MS_LAUNCH(E_, NW_, 3); \
+    if (a.dtype == HPD_F16) HPD_MS_NS_T(E_, NW_, __half);                                                       \
+    else if (a.dtype == HPD_BF16) HPD_MS_NS_T(E_, NW_, __nv_bfloat16);                                         \
+    else HPD_MS_NS_T(E_, NW_, float);                                                                            \
   } while (0)
         if (a.E == 1) { if (NW == 5) HPD_MS_NS(1, 5); else if (NW == 4) HPD_MS_NS(1, 4); else if (NW == 3) HPD_MS_NS(1, 3); else HPD_MS_NS(1, 2); }
         else          { if (NW == 5) HPD_MS_NS(2, 5); else if (NW == 4) HPD_MS_NS(2, 4); else if (NW == 3) HPD_MS_NS(2, 3); else HPD_MS_NS(2, 2); }
 #undef HPD_MS_NS
+#undef HPD_MS_NS_T
 #undef HPD_MS_LAUNCH
         count_launch();
         return check_launch("agg_nms_ms_kernel");

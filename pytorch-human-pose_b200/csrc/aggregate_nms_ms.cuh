@@ -9,7 +9,9 @@
 //     horizontally interpolated S_s rows; the vertical taps of every (scale, output row) come from a small
 //     shared table; the scales are summed sequentially and divided by n like torch.stack(...).mean(0);
 //   * tags come from one scale and must be an exact x4 (as in the reference); NMS, word side arrays and tag
-//     bounds are the x2 kernel's.
+//     bounds are the x2 kernel's;
+//   * input elements are float32, IEEE half or bfloat16 (T); 16-bit values are widened exactly as they are loaded,
+//     shared memory and all arithmetic stay float32.
 // Bit-identical to the generic kernel (tests/test_gpu_stages.py).
 #pragma once
 
@@ -38,27 +40,33 @@ struct Geom {                     // shared-memory layout, computed on the host
   int off_edge, off_tab, total;
 };
 
-// One staged window (a scale's quarter- or half-res rows).  Row r of it is the job "copy nvec 16-byte
-// vectors from p + r*w, flip-averaged with the vectors running backwards from pf + r*w, to
+// One staged window (a scale's quarter- or half-res rows).  Row r of it is the job "copy nvec vectors of four
+// elements from p + r*w, flip-averaged with the vectors running backwards from pf + r*w, to
 // smem[dst + r*stride]".
+template <typename T>
 struct Seg {
-  const float* p;                 // first vector of row 0
-  const float* pf;                // mirrored first vector of row 0 in the flipped run's map, or null
+  const T* p;                     // first vector of row 0
+  const T* pf;                    // mirrored first vector of row 0 in the flipped run's map, or null
   int dst, stride, nvec, w, rows;
 };
 
+// vector q (four elements) of a row, widened to float32: one 16-byte load for float, one 8-byte load for 16-bit types
+__device__ __forceinline__ float4 ld_vec(const float* p, int q) { return __ldg(reinterpret_cast<const float4*>(p) + q); }
+template <typename T>
+__device__ __forceinline__ float4 ld_vec(const T* p, int q) { return x2::In<T>::ld4(p + 4 * q); }
+
 // Stage all windows: the rows of all segments form one job list dealt round-robin to the warps; a warp
-// keeps two rows in flight (all loads of both issued before the first store).  16-byte loads; the flipped
-// operand is read as the mirrored 16 bytes and reversed in registers (model.py:87-90).
-template <int NW, int NSEG>
-__device__ __forceinline__ void stage_segments(float* __restrict__ smem, const Seg* __restrict__ seg, int warp, int lane) {
+// keeps two rows in flight (all loads of both issued before the first store).  Vector loads; the flipped
+// operand is read as the mirrored vector and reversed in registers (model.py:87-90).
+template <int NW, int NSEG, typename T>
+__device__ __forceinline__ void stage_segments(float* __restrict__ smem, const Seg<T>* __restrict__ seg, int warp, int lane) {
   constexpr int MAXIT = 4;
   int start[NSEG + 1];
   start[0] = 0;
 #pragma unroll
   for (int i = 0; i < NSEG; ++i) start[i + 1] = start[i] + seg[i].rows;
   const int njobs = start[NSEG];
-  struct Row { const float* p; const float* pf; float* dst; int nvec; };
+  struct Row { const T* p; const T* pf; float* dst; int nvec; };
   auto locate = [&](int j) {
     Row r{nullptr, nullptr, nullptr, 0};
     if (j < njobs) {
@@ -66,7 +74,7 @@ __device__ __forceinline__ void stage_segments(float* __restrict__ smem, const S
 #pragma unroll
       for (int i = 1; i < NSEG; ++i)
         if (j >= start[i]) { sg = i; first = start[i]; }
-      const Seg& S = seg[sg];
+      const Seg<T>& S = seg[sg];
       const int rr = j - first;
       r.p = S.p + (size_t)rr * S.w;
       r.pf = S.pf ? S.pf + (size_t)rr * S.w : nullptr;
@@ -83,8 +91,8 @@ __device__ __forceinline__ void stage_segments(float* __restrict__ smem, const S
       if (qb + 32 * u >= r.nvec) break;
       const int q = qb + lane + 32 * u;
       if (q < r.nvec) {
-        v[u] = __ldg(reinterpret_cast<const float4*>(r.p) + q);
-        if (r.pf) f[u] = __ldg(reinterpret_cast<const float4*>(r.pf) - q);
+        v[u] = ld_vec(r.p, q);
+        if (r.pf) f[u] = ld_vec(r.pf, -q);
       }
     }
   };
@@ -118,7 +126,7 @@ __device__ __forceinline__ void stage_segments(float* __restrict__ smem, const S
   }
 }
 
-template <int E, int NW, int NS>
+template <int E, int NW, int NS, typename T>
 __global__ void __launch_bounds__(32 * NW, 16 / NW) agg_nms_ms_kernel(const AggArgs a, const Geom g) {
   extern __shared__ __align__(16) float smem[];
   constexpr int tc = 32 * NW + 8;
@@ -150,7 +158,7 @@ __global__ void __launch_bounds__(32 * NW, 16 / NW) agg_nms_ms_kernel(const AggA
   // windows of every scale this CTA needs (hya, hxa, nhy, nhx, lya, lxa) and the staging jobs for them;
   // published by the first barrier of phase 0
   __shared__ int s_win[HPD_MAX_SCALES][6];
-  __shared__ Seg s_seg[2 * HPD_MAX_SCALES];
+  __shared__ Seg<T> s_seg[2 * HPD_MAX_SCALES];
   if (tid < NS) {
     const int s = tid;
     const ScaleDev& S = a.sc[s];
@@ -170,24 +178,26 @@ __global__ void __launch_bounds__(32 * NW, 16 / NW) agg_nms_ms_kernel(const AggA
     tap_x2(min(hxb, S.hw - 1), S.lw, t0, t1, tw0, tw1);
     const int nlx = min(t1 | 3, S.lw - 1) - lxa + 1;
     s_win[s][0] = hya; s_win[s][1] = hxa; s_win[s][2] = nhy; s_win[s][3] = nhx; s_win[s][4] = lya; s_win[s][5] = lxa;
-    Seg& lo = s_seg[2 * s];
-    Seg& hi = s_seg[2 * s + 1];
-    lo.p = S.lo + (size_t)b * S.lo_sb + (size_t)k * S.lo_sc + (size_t)lya * S.lw + lxa;
-    lo.pf = S.lo_f ? S.lo_f + (size_t)b * S.lof_sb + (size_t)kf * S.lof_sc + (size_t)lya * S.lw + (S.lw - 4 - lxa) : nullptr;
+    Seg<T>& lo = s_seg[2 * s];
+    Seg<T>& hi = s_seg[2 * s + 1];
+    lo.p = reinterpret_cast<const T*>(S.lo) + (size_t)b * S.lo_sb + (size_t)k * S.lo_sc + (size_t)lya * S.lw + lxa;
+    lo.pf = S.lo_f ? reinterpret_cast<const T*>(S.lo_f) + (size_t)b * S.lof_sb + (size_t)kf * S.lof_sc + (size_t)lya * S.lw + (S.lw - 4 - lxa)
+                   : nullptr;
     lo.dst = g.off_lo[s]; lo.stride = g.lc[s]; lo.nvec = nlx >> 2; lo.w = S.lw; lo.rows = nly;
-    hi.p = S.hi + (size_t)b * S.hi_sb + (size_t)k * S.hi_sc + (size_t)hya * S.hw + hxa;
-    hi.pf = S.hi_f ? S.hi_f + (size_t)b * S.hif_sb + (size_t)kf * S.hif_sc + (size_t)hya * S.hw + (S.hw - 4 - hxa) : nullptr;
+    hi.p = reinterpret_cast<const T*>(S.hi) + (size_t)b * S.hi_sb + (size_t)k * S.hi_sc + (size_t)hya * S.hw + hxa;
+    hi.pf = S.hi_f ? reinterpret_cast<const T*>(S.hi_f) + (size_t)b * S.hif_sb + (size_t)kf * S.hif_sc + (size_t)hya * S.hw + (S.hw - 4 - hxa)
+                   : nullptr;
     hi.dst = g.off_s[s]; hi.stride = g.hc[s]; hi.nvec = nhx >> 2; hi.w = S.hw; hi.rows = nhy;
   }
 
   // ---------------- phase 0: tags (x4), identical to the x2 kernel ------------------------------------
   {
     const int txo = x0 / 4 - 4, tyo = y0 / 4 - 1;
-    const float* tg0 = a.tag + (size_t)b * a.tag_sb + (size_t)k * a.tag_sc;
+    const T* tg0 = reinterpret_cast<const T*>(a.tag) + (size_t)b * a.tag_sb + (size_t)k * a.tag_sc;
     const bool unflip = !a.tags_preflipped;
-    const float* tg1 = (E > 1) ? a.tag_f + (size_t)b * a.tagf_sb + (size_t)(unflip ? kf : k) * a.tagf_sc : nullptr;
-    x2::stage_tile<0, TR, tc, NW, false>(sT, tg0, (const float*)nullptr, false, tyo, txo, a.th, a.tw, warp, lane);
-    if (E > 1) x2::stage_tile<1, TR, tc, NW, false>(sT + TR * tc, (const float*)nullptr, tg1, unflip, tyo, txo, a.th, a.tw, warp, lane);
+    const T* tg1 = (E > 1) ? reinterpret_cast<const T*>(a.tag_f) + (size_t)b * a.tagf_sb + (size_t)(unflip ? kf : k) * a.tagf_sc : nullptr;
+    x2::stage_tile<0, TR, tc, NW, false, T>(sT, tg0, (const T*)nullptr, false, tyo, txo, a.th, a.tw, warp, lane);
+    if (E > 1) x2::stage_tile<1, TR, tc, NW, false, T>(sT + TR * tc, (const T*)nullptr, tg1, unflip, tyo, txo, a.th, a.tw, warp, lane);
     __syncthreads();
     if (active) x2::tags_x4_band<E, RB, TR>(a, sT, tc, txo, X0, y0, b, k, lane);
     __syncthreads();
@@ -196,7 +206,7 @@ __global__ void __launch_bounds__(32 * NW, 16 / NW) agg_nms_ms_kernel(const AggA
   MSP_MARK(1);
   // ---------------- phase 1: flip-averaged quarter- and half-res windows of every scale -> smem ---------
   // (s_seg / s_win were filled at kernel entry; the barrier that ended phase 0 published them)
-  stage_segments<NW, 2 * NS>(smem, s_seg, warp, lane);
+  stage_segments<NW, 2 * NS, T>(smem, s_seg, warp, lane);
   for (int i = tid; i < NS * NROWS; i += nthr) {     // output row -> S_s rows
     const int s = i / NROWS, t = i - s * NROWS;
     const ScaleDev& S = a.sc[s];

@@ -61,8 +61,9 @@ __device__ __forceinline__ void tap_x2(int o, int I, int& i0, int& i1, float& w0
 // 8 halo columns and for any part right of the map.
 //   MODE 0: dst = p[y][x]      MODE 1: dst = pf[y][mirror ? w-1-x : x]
 //   MODE 2: dst = (p[y][x] + pf[y][w-1-x]) * 0.5   (flip averaging, model.py:90)
-// Input element type: float32 (inference) or IEEE half (the validation-time caller runs the network under fp16
-// autocast, module.py:78).  Halves are widened on load -- exactly -- and everything after is float32 arithmetic.
+// Input element type: float32 (inference), IEEE half (the validation-time caller runs the network under fp16
+// autocast, module.py:78) or bfloat16 (bf16 autocast).  16-bit values are widened on load -- exactly -- and
+// everything after is float32 arithmetic.
 template <typename T> struct In;
 template <> struct In<float> {
   static __device__ __forceinline__ float4 ld4(const float* q) { return __ldg(reinterpret_cast<const float4*>(q)); }
@@ -76,6 +77,16 @@ template <> struct In<__half> {
     return make_float4(a.x, a.y, b.x, b.y);
   }
   static __device__ __forceinline__ float ld1(const __half* q) { return __half2float(__ldg(q)); }
+};
+template <> struct In<__nv_bfloat16> {   // a bfloat16 is the upper 16 bits of the float32 of the same value
+  static __device__ __forceinline__ float4 ld4(const __nv_bfloat16* q) {
+    const uint2 u = __ldg(reinterpret_cast<const uint2*>(q));
+    return make_float4(__uint_as_float(u.x << 16), __uint_as_float(u.x & 0xffff0000u), __uint_as_float(u.y << 16),
+                       __uint_as_float(u.y & 0xffff0000u));
+  }
+  static __device__ __forceinline__ float ld1(const __nv_bfloat16* q) {
+    return __uint_as_float((unsigned)__ldg(reinterpret_cast<const unsigned short*>(q)) << 16);
+  }
 };
 
 template <int MODE>

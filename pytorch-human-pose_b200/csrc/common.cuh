@@ -55,9 +55,12 @@ __device__ __forceinline__ float lerp2(float wx0, float wx1, float hy0, float hy
   return fmaf(hy0, top, __fmul_rn(hy1, bot));
 }
 
-// element i of an input plane; half_in: the plane holds IEEE halves (HPD_F16), widened exactly
-__device__ __forceinline__ float in_elem(const float* base, size_t i, int half_in) {
-  return half_in ? __half2float(reinterpret_cast<const __half*>(base)[i]) : base[i];
+// element i of an input plane of dtype code `dtype` (HPD_F32 / HPD_F16 / HPD_BF16); 16-bit values are widened
+// exactly (a bfloat16 is the upper half of a float32)
+__device__ __forceinline__ float in_elem(const float* base, size_t i, int dtype) {
+  if (dtype == HPD_F32) return base[i];
+  const unsigned short u = reinterpret_cast<const unsigned short*>(base)[i];
+  return dtype == HPD_F16 ? __half2float(__ushort_as_half(u)) : __uint_as_float((unsigned)u << 16);
 }
 #endif  // __CUDACC__
 
@@ -68,12 +71,12 @@ __device__ __forceinline__ float in_elem(const float* base, size_t i, int half_i
 // writing 4*K*H*W*E bytes per image.
 struct TagSource {
   const float* map;                  // [B,K,H,W,E] or NULL: interpolate from tag / tag_f
-  const float *tag, *tag_f;          // tag-scale maps (tag_f: flipped run, E == 2); __half data if half_in
+  const float *tag, *tag_f;          // tag-scale maps (tag_f: flipped run, E == 2); elements of type `dtype`
   long long tag_sb, tag_sc, tagf_sb, tagf_sc;
   int K, H, W, E;
   int th, tw;                        // tag-scale map size
   float s_y, s_x;                    // th / H, tw / W
-  int half_in, tags_preflipped;
+  int dtype, tags_preflipped;        // dtype: HPD_F32 / HPD_F16 / HPD_BF16
   int flip[HPD_MAX_KPTS];
 };
 
@@ -92,8 +95,8 @@ __device__ __forceinline__ void tag_at(const TagSource& s, int b, int k, int y, 
                                : (size_t)b * s.tagf_sb + (size_t)(unflip ? s.flip[k] : k) * s.tagf_sc;
     const int c0 = unflip ? s.tw - 1 - tx.i0 : tx.i0, c1 = unflip ? s.tw - 1 - tx.i1 : tx.i1;
     const size_t r0 = po + (size_t)ty.i0 * s.tw, r1 = po + (size_t)ty.i1 * s.tw;
-    t[e] = lerp2(tx.w0, tx.w1, ty.w0, ty.w1, in_elem(p, r0 + c0, s.half_in), in_elem(p, r0 + c1, s.half_in),
-                 in_elem(p, r1 + c0, s.half_in), in_elem(p, r1 + c1, s.half_in));
+    t[e] = lerp2(tx.w0, tx.w1, ty.w0, ty.w1, in_elem(p, r0 + c0, s.dtype), in_elem(p, r0 + c1, s.dtype),
+                 in_elem(p, r1 + c0, s.dtype), in_elem(p, r1 + c1, s.dtype));
   }
 }
 

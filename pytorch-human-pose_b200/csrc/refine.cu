@@ -222,8 +222,8 @@ __device__ __forceinline__ void word_tags(const TagSource& s, int b, int k, int 
     if (lane < span) {
       const int c = c_lo + lane;
       const size_t col = (size_t)(unflip ? s.tw - 1 - c : c);
-      v0 = in_elem(p, po + (size_t)ty.i0 * s.tw + col, s.half_in);
-      v1 = in_elem(p, po + (size_t)ty.i1 * s.tw + col, s.half_in);
+      v0 = in_elem(p, po + (size_t)ty.i0 * s.tw + col, s.dtype);
+      v1 = in_elem(p, po + (size_t)ty.i1 * s.tw + col, s.dtype);
     }
     const float v00 = __shfl_sync(kFull, v0, j0), v01 = __shfl_sync(kFull, v0, j1);
     const float v10 = __shfl_sync(kFull, v1, j0), v11 = __shfl_sync(kFull, v1, j1);

@@ -10,9 +10,9 @@ HPD_MAX_KPTS = 32
 HPD_MAX_PEOPLE = 32
 HPD_MAX_EMB = 2
 HPD_MAX_SCALES = 4
-HPD_ABI_VERSION = 5
+HPD_ABI_VERSION = 6
 HPD_COCO_MAX_IOU_THRS, HPD_COCO_MAX_REC_THRS, HPD_COCO_MAX_AREAS, HPD_COCO_MAX_PER_IMAGE = 16, 128, 4, 1024
-HPD_F32, HPD_F16 = 0, 1
+HPD_F32, HPD_F16, HPD_BF16 = 0, 1, 2
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libhpdecode.so")

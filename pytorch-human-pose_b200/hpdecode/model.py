@@ -16,6 +16,10 @@ Batched superset: ``predict_batch(raw_images)`` groups images by resized size, r
 and decodes each group in one call.  ``test_scales`` enables real multi-scale inference (the reference has the size
 logic, base/transforms/utils.py:60-97, but only ever calls it with scale 1): heatmaps are averaged over the scales,
 tags come from scale 1.0, everything is projected to the scale-1.0 input frame.
+
+``autocast_dtype`` (torch.bfloat16 or torch.float16) runs every forward -- flipped run and test scales included --
+under ``torch.autocast("cuda", dtype=...)`` and hands the 16-bit outputs to the decoder as they are: the kernels widen
+them exactly on load, so the result is the float32 decode of the up-cast outputs, without a conversion pass.
 """
 from typing import List, Optional, Sequence
 
@@ -38,7 +42,11 @@ class InferenceKeypointsModel:
 
     def __init__(self, net: nn.Module, det_thr: float = 0.05, tag_thr: float = 0.5, use_flip: bool = False,
                  input_size: int = 512, max_num_people: int = 30, device: str = "cuda:0",
-                 ckpt_path: Optional[str] = None, num_kpts: int = 17, test_scales: Sequence[float] = (1.0,)):
+                 ckpt_path: Optional[str] = None, num_kpts: int = 17, test_scales: Sequence[float] = (1.0,),
+                 autocast_dtype: Optional[torch.dtype] = None):
+        if autocast_dtype not in (None, torch.bfloat16, torch.float16):
+            raise ValueError(f"autocast_dtype must be None, torch.bfloat16 or torch.float16 (got {autocast_dtype})")
+        self.autocast_dtype = autocast_dtype
         self.device = device
         self.input_size = input_size
         self.net = net.to(device)
@@ -79,11 +87,26 @@ class InferenceKeypointsModel:
     # -- batched superset -------------------------------------------------------------------------------------------
     @torch.no_grad()
     def _net_outputs(self, x: Tensor) -> dict:
+        if self.autocast_dtype is not None:
+            return self._net_outputs_autocast(x)
         (hm_lo, hm_hi), tag = self.net(x)
         scale = {"hm_lo": hm_lo.float(), "hm_hi": hm_hi.float(), "tag": tag.float()}
         if self.use_flip:   # model.py:85-94, fused into the aggregation kernel
             (fl_lo, fl_hi), fl_tag = self.net(torch.flip(x, [3]))
             scale.update(hm_lo_f=fl_lo.float(), hm_hi_f=fl_hi.float(), tag_f=fl_tag.float())
+        return scale
+
+    def _net_outputs_autocast(self, x: Tensor) -> dict:
+        with torch.autocast("cuda", dtype=self.autocast_dtype):
+            (hm_lo, hm_hi), tag = self.net(x)
+            scale = {"hm_lo": hm_lo, "hm_hi": hm_hi, "tag": tag}
+            if self.use_flip:
+                (fl_lo, fl_hi), fl_tag = self.net(torch.flip(x, [3]))
+                scale.update(hm_lo_f=fl_lo, hm_hi_f=fl_hi, tag_f=fl_tag)
+        # the decoder reads one dtype per call: a net whose head leaves some outputs in float32 under autocast has all
+        # of them up-cast (exact), the usual all-16-bit set goes as it is
+        if len({t.dtype for t in scale.values()}) > 1:
+            scale = {k: v.float() for k, v in scale.items()}
         return scale
 
     @torch.no_grad()

@@ -41,12 +41,16 @@ def _require_cuda(t: Tensor, name: str):
         raise _lib.HpdError(f"{name} must be float32 (got {t.dtype})")
 
 
-def _map(t: Optional[Tensor], name: str, allow_half: bool = False) -> HpdMap:
+# network outputs under fp16 / bf16 autocast (module.py:78): read as they are, widened exactly inside the kernels
+_DTYPE_CODES = {torch.float16: _lib.HPD_F16, torch.bfloat16: _lib.HPD_BF16}
+
+
+def _map(t: Optional[Tensor], name: str, allow_16bit: bool = False) -> HpdMap:
     m = HpdMap()
     if t is None:
         return m
-    if allow_half and t.is_cuda and t.dtype == torch.float16:
-        m.dtype = _lib.HPD_F16      # network outputs under fp16 autocast (module.py:78): widened inside the kernel
+    if allow_16bit and t.is_cuda and t.dtype in _DTYPE_CODES:
+        m.dtype = _DTYPE_CODES[t.dtype]
     else:
         _require_cuda(t, name)
     if t.dim() != 4:
@@ -205,7 +209,7 @@ def _scales_struct(scales: Sequence[dict]):
     for i, s in enumerate(scales):
         for name in ("hm_lo", "hm_hi", "tag", "hm_lo_f", "hm_hi_f", "tag_f"):
             t = s.get(name)
-            setattr(arr[i], name, _map(t, name, allow_half=True))
+            setattr(arr[i], name, _map(t, name, allow_16bit=True))
             keep.append(t)
     return arr, keep
 
@@ -396,12 +400,12 @@ def _scales_from_lists(hm_lo, hm_hi, tag, hm_lo_f, hm_hi_f, tag_f):
 def decode_op(hm_lo: Sequence[Tensor], hm_hi: Sequence[Tensor], tag: Sequence[Tensor], hm_lo_f: Sequence[Tensor],
               hm_hi_f: Sequence[Tensor], tag_f: Sequence[Tensor], out_h: int, out_w: int, max_people: int,
               det_thr: float, tag_thr: float, adjust: bool, refine: bool, tag_scale: int) -> List[Tensor]:
-    """Network outputs (one list entry per test scale) -> [agg_hm, agg_tags, poses, person_scores, n_person,
-    flags, scores_k, idx_k, coords_k, tags_k]."""
+    """Network outputs (one list entry per test scale; float32, or all float16 or all bfloat16) -> [agg_hm, agg_tags,
+    poses, person_scores, n_person, flags, scores_k, idx_k, coords_k, tags_k]."""
     for name, ts in (("hm_lo", hm_lo), ("hm_hi", hm_hi), ("tag", tag), ("hm_lo_f", hm_lo_f), ("hm_hi_f", hm_hi_f),
                      ("tag_f", tag_f)):
         for t in ts:
-            if not (t.is_cuda and t.dtype == torch.float16):
+            if not (t.is_cuda and t.dtype in _DTYPE_CODES):
                 _require_cuda(t, name)
     scales = _scales_from_lists(hm_lo, hm_hi, tag, hm_lo_f, hm_hi_f, tag_f)
     B, K = hm_lo[0].shape[:2]

@@ -59,9 +59,10 @@ def _decode_preaveraged(kpts_heatmaps: List[Tensor], tags_heatmaps: List[Tensor]
     if len(tags_heatmaps) not in (1, 2):
         raise ops._lib.HpdError("1 or 2 tag maps expected")
     dev = _cuda_device(kpts_heatmaps[0])
-    half = all(t.dtype == torch.float16 for t in list(kpts_heatmaps) + list(tags_heatmaps))
-    # fp16 network outputs (validation under autocast, module.py:78) go to the kernel as they are
-    f = lambda t: t.to(dev) if half else t.to(dev, torch.float32)
+    dtypes = {t.dtype for t in list(kpts_heatmaps) + list(tags_heatmaps)}
+    # a uniform set of fp16 or bf16 network outputs (validation under autocast, module.py:78) goes to the kernel as it is
+    same16 = len(dtypes) == 1 and dtypes <= {torch.float16, torch.bfloat16}
+    f = lambda t: t.to(dev) if same16 else t.to(dev, torch.float32)
     scale = {"hm_lo": f(kpts_heatmaps[0]), "hm_hi": f(kpts_heatmaps[1]), "tag": f(tags_heatmaps[0])}
     if len(tags_heatmaps) == 2:
         scale["tag_f"] = f(tags_heatmaps[1])
@@ -155,7 +156,7 @@ class InferenceKeypointsResult(BaseKeypointsResult):
 
 class KeypointsResult(BaseKeypointsResult):
     """results.py:70-124 (validation-time caller): one tag map, E = 1.  The network runs under fp16 autocast there
-    (module.py:78); half inputs are accepted as they are and widened inside the aggregation kernel."""
+    (module.py:78); a uniform set of float16 or bfloat16 inputs is accepted as it is and widened inside the kernels."""
 
     def __init__(self, model_input_image, kpts_heatmaps: List[Tensor], tags_heatmaps: Tensor, limbs,
                  max_num_people: int = 30, det_thr: float = 0.05, tag_thr: float = 0.5):

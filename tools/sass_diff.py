@@ -1,0 +1,50 @@
+"""Compare the SASS of two builds of libhpdecode.so kernel by kernel.
+
+usage: python tools/sass_diff.py OLD.so NEW.so [PATTERN ...]  ->  one line per kernel of OLD whose demangled name
+contains one of the patterns (default: every kernel): "identical", "DIFFERS" or "missing", plus the kernels only NEW has.
+A kernel of NEW that gained a trailing `float` template argument (the element type of the inputs) is compared with the
+OLD kernel without it.  Instruction text and encodings are compared; only the offset comments are dropped.
+Needs only the CUDA toolkit (cuobjdump, c++filt): no GPU.
+"""
+import re
+import subprocess
+import sys
+
+
+def kernels(lib):
+    txt = subprocess.run(["cuobjdump", "-sass", lib], capture_output=True, text=True, check=True).stdout
+    out, cur = {}, None
+    for line in txt.splitlines():
+        m = re.match(r"\s*Function : (\S+)", line)
+        if m:
+            cur = out.setdefault(m.group(1), [])
+            continue
+        if cur is not None and line.strip().startswith("/*"):
+            cur.append(re.sub(r"^\s*/\*[0-9a-f]{4,}\*/", "", line).strip())
+    names = subprocess.run(["c++filt"], input="\n".join(out), capture_output=True, text=True).stdout.splitlines()
+    return {re.sub(r"^void |\(.*\)$", "", n): v for n, v in zip(names, out.values())}
+
+
+def main(old_lib, new_lib, patterns):
+    old, new = kernels(old_lib), kernels(new_lib)
+    alias = {re.sub(r", float>$", ">", n): n for n in new}   # new name without the float element type -> new name
+    seen, rows = set(), []
+    for name in sorted(old):
+        if patterns and not any(p in name for p in patterns):
+            continue
+        twin = name if name in new else alias.get(name)
+        if twin is None:
+            rows.append(("missing", name, "", len(old[name])))
+            continue
+        seen.add(twin)
+        rows.append(("identical" if old[name] == new[twin] else "DIFFERS", name, twin, len(old[name])))
+    for name in sorted(new):
+        if name not in seen and (not patterns or any(p in name for p in patterns)):
+            rows.append(("new", "", name, len(new[name])))
+    for status, o, n, lines in rows:
+        print("%-9s %6d  %s%s" % (status, lines // 2, o or n, "  ->  " + n if o and n and n != o else ""))
+    return 1 if any(r[0] in ("DIFFERS", "missing") for r in rows) else 0
+
+
+if __name__ == "__main__":
+    sys.exit(main(sys.argv[1], sys.argv[2], sys.argv[3:]))
