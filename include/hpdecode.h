@@ -224,12 +224,14 @@ HPD_EXPORT const char* hpd_last_error_string(void);
 HPD_EXPORT int hpd_workspace_bytes(const HpdParams* p, size_t* out_bytes);
 
 /* (a)+(b) fused aggregation + NMS: model.py:85-96, results.py:46-67,225-230, grouping.py:80-83.
- * Reads scales[0..num_scales); writes agg_hm, agg_tags (unless NULL), nms_mask, nms_wmax, hm_wmax, tag_bmin, tag_bmax. */
+ * Reads scales[0..num_scales); writes agg_hm, nms_mask, nms_wmax, hm_wmax, tag_bmin, tag_bmax in one kernel, and
+ * agg_tags unless it is NULL: the tag map is written by a second kernel on the same stream, the one
+ * hpd_aggregate_tags launches (hpd_last_launch_count() is then one higher). */
 HPD_EXPORT int hpd_aggregate_nms(const HpdParams* p, const HpdScaleInputs* scales, const HpdBuffers* buf, void* stream);
 
 /* The tag half of hpd_aggregate_nms alone (results.py:229-230), for callers that decoded with agg_tags == NULL and
- * want the map after all: reads the tag / tag_f maps of scales[tag_scale]; writes out [B,K,H,W,E], bit-identical to
- * the agg_tags hpd_aggregate_nms writes. */
+ * want the map after all: reads the tag / tag_f maps of scales[tag_scale]; writes out [B,K,H,W,E].  It is the one
+ * producer of the map: hpd_aggregate_nms and hpd_decode fill agg_tags with the same kernel. */
 HPD_EXPORT int hpd_aggregate_tags(const HpdParams* p, const HpdScaleInputs* scales, float* out, void* stream);
 
 /* Standalone bilinear resize with torch's CPU arithmetic (BaseKeypointsResult.match_heatmaps_size,
@@ -263,7 +265,8 @@ HPD_EXPORT int hpd_adjust_refine(const HpdParams* p, const HpdBuffers* buf, void
  * If scales == NULL the aggregation is skipped and buf->agg_hm / agg_tags are taken as inputs
  * (the MPPEHeatmapParser.parse entry, grouping.py:252).  With scales and agg_tags == NULL the tag stages read
  * scales[tag_scale] (buf->tag_inputs is ignored); the network outputs must then stay unchanged until the call's
- * work has run. */
+ * work has run.  With scales and a non-NULL agg_tags the map is written as hpd_aggregate_nms writes it (one launch
+ * more) and the tag stages read it. */
 HPD_EXPORT int hpd_decode(const HpdParams* p, const HpdScaleInputs* scales, const HpdBuffers* buf, void* workspace,
                size_t workspace_bytes, void* stream);
 

@@ -1,6 +1,5 @@
 // Stage (a)+(b): fused flip/scale aggregation of the network outputs into full-resolution
-// heatmaps and tag maps, with the 5x5 max-pool NMS evaluated on the same tile while it is still
-// in shared memory.
+// heatmaps, with the 5x5 max-pool NMS evaluated on the same tile while it is still in shared memory.
 //
 // Reference semantics reproduced bit-exactly (paths relative to /root/reference):
 //   model.py:85-96       per stage (pred + flipW(flip_pred)[:, FLIP]) / 2 ; tags kept separate (E = 2)
@@ -15,8 +14,13 @@
 // the survivor bit mask, the maximum NMS'd value (top-k prefilter) and the maximum raw value
 // (refine prefilter); together 3/32 of one map.
 //
+// The full-resolution tag map (results.py:229-230) has one producer, aggregate_tags_kernel (tag_at per
+// pixel).  The decode does not need it: the tag stages interpolate the few tags they read.  When a caller
+// asks for the map, launch_aggregate_nms runs that kernel after the aggregation kernel.
+//
 // This file holds the GENERIC kernel (any resize ratios, any number of scales).  It is the
-// correctness anchor; aggregate_nms_x2.cu specialises the standard single-scale x2/x2/x4 case.
+// correctness anchor; aggregate_nms_x2.cuh specialises the standard single-scale x2/x2/x4 case and
+// aggregate_nms_ms.cuh the multi-scale one.
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
@@ -42,23 +46,20 @@ struct ScaleDev {
 struct AggArgs {
   ScaleDev sc[HPD_MAX_SCALES];
   int n_scales;
-  const float *tag, *tag_f;
-  long long tag_sb, tag_sc, tagf_sb, tagf_sc;
+  const float* tag;   // tag-scale map, first component (the tag bounds)
+  long long tag_sb, tag_sc;
   int th, tw;
-  float s_tag_y, s_tag_x;
-  int B, K, H, W, E, wpr;
+  int B, K, H, W, wpr;
   int flip[HPD_MAX_KPTS];
   float* agg_hm;
-  float* agg_tags;
   uint32_t* mask;
   float* wmax;
   float* hmax;
   float* tmin;     // [B,K,(H+3)/4,wpr] bounds of tag component 0 per 4 rows x word
   float* tmax;
   float* nms_out;  // standalone NMS only
-  int LO_R, LO_C, HI_R, HI_C, TG_R, TG_C;
+  int LO_R, LO_C, HI_R, HI_C;
   int vec_ok;
-  int tags_preflipped;
   int in_vec_ok;   // inputs allow 16-byte loads (aligned bases, strides multiples of 4 elements)
   int in_vec_ok_all;   // ... for every scale
   int dtype;       // HPD_F32 / HPD_F16 / HPD_BF16: the const float* input members point at elements of this type
@@ -126,10 +127,9 @@ __global__ void __launch_bounds__(kAggThreads) agg_nms_generic_kernel(const AggA
   float* outT = smem;                         // [OT_R][OT_C]
   float* rowM = outT + OT_R * OT_C;           // [OT_R][TW]
   float* hiT = rowM + OT_R * TW;              // [HI_R][HI_C]
-  const int lo_words = max(a.LO_R * a.LO_C, a.E * a.TG_R * a.TG_C);
-  float* loT = hiT + a.HI_R * a.HI_C;         // [LO_R][LO_C]  (re-used for the tag tiles)
+  float* loT = hiT + a.HI_R * a.HI_C;         // [LO_R][LO_C]
   // tap tables: index pairs (relative to the source tile origin) and weights
-  int* oc_i0 = (int*)(loT + lo_words);        // out col -> hi tile col        [OT_C]
+  int* oc_i0 = (int*)(loT + a.LO_R * a.LO_C); // out col -> hi tile col        [OT_C]
   int* oc_i1 = oc_i0 + OT_C;
   float* oc_w0 = (float*)(oc_i1 + OT_C);
   float* oc_w1 = oc_w0 + OT_C;
@@ -290,74 +290,6 @@ __global__ void __launch_bounds__(kAggThreads) agg_nms_generic_kernel(const AggA
              a.hmax + plane * H * a.wpr, a.tmin + plane * ((H + 3) / 4) * a.wpr, a.tmax + plane * ((H + 3) / 4) * a.wpr,
              nullptr);
   }
-  if (a.agg_tags == nullptr) return;   // the tag stages interpolate the few tags they read (tag_at)
-  __syncthreads();
-
-  // tags (results.py:229-230): E source tiles, single resize, E-innermost stores
-  {
-    const int txa = axis_tap(a.s_tag_x, x0, a.tw, W).i0, txb = axis_tap(a.s_tag_x, min(x0 + TW, W) - 1, a.tw, W).i1;
-    const int tya = axis_tap(a.s_tag_y, y0, a.th, H).i0, tyb = axis_tap(a.s_tag_y, min(y0 + TH, H) - 1, a.th, H).i1;
-    const int ntx = txb - txa + 1, nty = tyb - tya + 1;
-    for (int i = tid; i < TW; i += kAggThreads) {
-      const int ox = x0 + i;
-      if (ox < W) {
-        const Tap t = axis_tap(a.s_tag_x, ox, a.tw, W);
-        oc_i0[i] = t.i0 - txa; oc_i1[i] = t.i1 - txa; oc_w0[i] = t.w0; oc_w1[i] = t.w1;
-      }
-    }
-    for (int i = tid; i < TH; i += kAggThreads) {
-      const int oy = y0 + i;
-      if (oy < H) {
-        const Tap t = axis_tap(a.s_tag_y, oy, a.th, H);
-        or_i0[i] = t.i0 - tya; or_i1[i] = t.i1 - tya; or_w0[i] = t.w0; or_w1[i] = t.w1;
-      }
-    }
-    const int tile_words = a.TG_R * a.TG_C;
-    for (int e = 0; e < a.E; ++e) {
-      const bool unflip = (e == 1) && !a.tags_preflipped;   // model.py:93: flip(tag_f, W)[:, FLIP]
-      const float* p = (e == 0) ? a.tag : a.tag_f;
-      const size_t po = (e == 0) ? (size_t)b * a.tag_sb + (size_t)k * a.tag_sc
-                                 : (size_t)b * a.tagf_sb + (size_t)(unflip ? kf : k) * a.tagf_sc;
-      for (int i = tid; i < nty * ntx; i += kAggThreads) {
-        const int r = i / ntx, c = i % ntx;
-        const int y = tya + r, x = txa + c;
-        loT[e * tile_words + r * a.TG_C + c] = in_elem(p, po + (size_t)y * a.tw + (unflip ? a.tw - 1 - x : x), a.dtype);
-      }
-    }
-    __syncthreads();
-    float* dst = a.agg_tags + ((size_t)b * a.K + k) * H * W * a.E;
-    for (int i = tid; i < TH * TW / 4; i += kAggThreads) {
-      const int r = i / (TW / 4), c = (i % (TW / 4)) * 4;
-      const int y = y0 + r, x = x0 + c;
-      if (y >= H || x >= W) continue;
-      float v[4][HPD_MAX_EMB];
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        if (x + j < W) {
-          const int c0 = oc_i0[c + j], c1 = oc_i1[c + j];
-          for (int e = 0; e < a.E; ++e) {
-            const float* r0 = loT + e * tile_words + or_i0[r] * a.TG_C;
-            const float* r1 = loT + e * tile_words + or_i1[r] * a.TG_C;
-            v[j][e] = lerp2(oc_w0[c + j], oc_w1[c + j], or_w0[r], or_w1[r], r0[c0], r0[c1], r1[c0], r1[c1]);
-          }
-        } else {
-          for (int e = 0; e < a.E; ++e) v[j][e] = 0.f;
-        }
-      }
-      float* o = dst + ((size_t)y * W + x) * a.E;
-      if (a.vec_ok) {
-        if (a.E == 1) {
-          *reinterpret_cast<float4*>(o) = make_float4(v[0][0], v[1][0], v[2][0], v[3][0]);
-        } else {
-          *reinterpret_cast<float4*>(o) = make_float4(v[0][0], v[0][1], v[1][0], v[1][1]);
-          *reinterpret_cast<float4*>(o + 4) = make_float4(v[2][0], v[2][1], v[3][0], v[3][1]);
-        }
-      } else {
-        for (int j = 0; j < 4 && x + j < W; ++j)
-          for (int e = 0; e < a.E; ++e) o[j * a.E + e] = v[j][e];
-      }
-    }
-  }
 }
 
 }  // namespace hpd
@@ -428,8 +360,8 @@ __global__ void __launch_bounds__(256) aggregate_tags_kernel(const TagSource s, 
 // ---------------------------------------------------------------------------------------------
 namespace {
 
-// Largest source-tile extent any output tile needs along one axis: out span (tile + halo)
-// -> mid extent, -> inner extent when the resize is nested (lo -> hi -> out).
+// Largest source-tile extent any output tile needs along one axis of the nested resize lo -> hi -> out:
+// out span (tile + halo) -> mid (hi) extent -> inner (lo) extent.
 void axis_extents(int out_size, int tile, int halo, int mid_size, float s_mid, int in_size, float s_in, int* mid_ext,
                   int* in_ext) {
   int me = 1, ie = 1;
@@ -438,13 +370,11 @@ void axis_extents(int out_size, int tile, int halo, int mid_size, float s_mid, i
     const int ob = (o0 + tile + halo < out_size ? o0 + tile + halo : out_size) - 1;
     const int ma = axis_tap(s_mid, oa, mid_size, out_size).i0, mb = axis_tap(s_mid, ob, mid_size, out_size).i1;
     me = mb - ma + 1 > me ? mb - ma + 1 : me;
-    if (in_size > 0) {
-      const int ia = axis_tap(s_in, ma, in_size, mid_size).i0, ib = axis_tap(s_in, mb, in_size, mid_size).i1;
-      ie = ib - ia + 1 > ie ? ib - ia + 1 : ie;
-    }
+    const int ia = axis_tap(s_in, ma, in_size, mid_size).i0, ib = axis_tap(s_in, mb, in_size, mid_size).i1;
+    ie = ib - ia + 1 > ie ? ib - ia + 1 : ie;
   }
   *mid_ext = me;
-  if (in_ext) *in_ext = ie;
+  *in_ext = ie;
 }
 
 int check_map(const HpdMap& m, const char* name, bool required) {
@@ -511,7 +441,10 @@ int launch_aggregate_tags(const HpdParams* p, const HpdScaleInputs* scales, floa
   return check_launch("aggregate_tags_kernel");
 }
 
-int launch_aggregate_nms(const HpdParams* p, const HpdScaleInputs* scales, const HpdBuffers* buf, cudaStream_t st) {
+namespace {
+
+// The aggregation + NMS kernel alone: agg_hm, the word side arrays and the tag bounds.
+int launch_aggregation_kernel(const HpdParams* p, const HpdScaleInputs* scales, const HpdBuffers* buf, cudaStream_t st) {
   if (!scales || !buf->agg_hm || !buf->nms_mask || !buf->nms_wmax || !buf->hm_wmax || !buf->tag_bmin || !buf->tag_bmax) {
     set_error("hpd_aggregate_nms: scales, agg_hm, nms_mask, nms_wmax, hm_wmax, tag_bmin, tag_bmax are required");
     return HPD_EINVAL;
@@ -519,7 +452,7 @@ int launch_aggregate_nms(const HpdParams* p, const HpdScaleInputs* scales, const
   AggArgs a;
   memset(&a, 0, sizeof(a));
   a.n_scales = p->num_scales;
-  a.B = p->batch; a.K = p->num_kpts; a.H = p->out_h; a.W = p->out_w; a.E = p->emb;
+  a.B = p->batch; a.K = p->num_kpts; a.H = p->out_h; a.W = p->out_w;
   a.wpr = (p->out_w + 31) / 32;
   for (int k = 0; k < HPD_MAX_KPTS; ++k) a.flip[k] = p->flip_index[k];
   const bool flip = scales[0].hm_lo_f.ptr != nullptr;
@@ -569,18 +502,13 @@ int launch_aggregate_nms(const HpdParams* p, const HpdScaleInputs* scales, const
       return HPD_EINVAL;
     }
     a.tag = (const float*)in.tag.ptr; a.tag_sb = in.tag.stride_b; a.tag_sc = in.tag.stride_c;
-    a.tag_f = (const float*)in.tag_f.ptr; a.tagf_sb = in.tag_f.stride_b; a.tagf_sc = in.tag_f.stride_c;
     a.th = in.tag.h; a.tw = in.tag.w;
-    a.s_tag_y = (float)a.th / (float)a.H; a.s_tag_x = (float)a.tw / (float)a.W;
-    axis_extents(a.W, TW, 0, a.tw, a.s_tag_x, 0, 0.f, &a.TG_C, nullptr);
-    axis_extents(a.H, TH, 0, a.th, a.s_tag_y, 0, 0.f, &a.TG_R, nullptr);
   }
-  a.LO_R = LO_R; a.LO_C = LO_C | 1; a.HI_R = HI_R; a.HI_C = HI_C | 1; a.TG_C |= 1;
-  a.agg_hm = buf->agg_hm; a.agg_tags = buf->agg_tags; a.mask = buf->nms_mask; a.wmax = buf->nms_wmax;
+  a.LO_R = LO_R; a.LO_C = LO_C | 1; a.HI_R = HI_R; a.HI_C = HI_C | 1;
+  a.agg_hm = buf->agg_hm; a.mask = buf->nms_mask; a.wmax = buf->nms_wmax;
   a.hmax = buf->hm_wmax;
   a.tmin = buf->tag_bmin;
   a.tmax = buf->tag_bmax;
-  a.tags_preflipped = p->tags_preflipped;
   {
     auto okp = [vec_align](const float* q, long long sb, long long sc_) { return q == nullptr || ((uintptr_t)q % vec_align == 0 && sb % 4 == 0 && sc_ % 4 == 0); };
     a.in_vec_ok_all = 1;
@@ -590,7 +518,7 @@ int launch_aggregate_nms(const HpdParams* p, const HpdScaleInputs* scales, const
         a.in_vec_ok_all = 0;
     }
   }
-  a.vec_ok = (a.W % 4 == 0) && ((uintptr_t)a.agg_hm % 16 == 0) && ((uintptr_t)a.agg_tags % 16 == 0);
+  a.vec_ok = (a.W % 4 == 0) && ((uintptr_t)a.agg_hm % 16 == 0);
 
   // standard single-scale x2/x2/x4 layout -> specialised kernel (aggregate_nms_x2.cuh)
   {
@@ -602,31 +530,25 @@ int launch_aggregate_nms(const HpdParams* p, const HpdScaleInputs* scales, const
       {
         auto ok = [vec_align](const float* q, long long sb, long long sc_) { return q == nullptr || ((uintptr_t)q % vec_align == 0 && sb % 4 == 0 && sc_ % 4 == 0); };
         a.in_vec_ok = S.lw % 4 == 0 && ok(S.lo, S.lo_sb, S.lo_sc) && ok(S.hi, S.hi_sb, S.hi_sc) && ok(S.lo_f, S.lof_sb, S.lof_sc) &&
-                      ok(S.hi_f, S.hif_sb, S.hif_sc) && ok(a.tag, a.tag_sb, a.tag_sc) && ok(a.tag_f, a.tagf_sb, a.tagf_sc);
+                      ok(S.hi_f, S.hif_sb, S.hif_sc) && ok(a.tag, a.tag_sb, a.tag_sc);
       }
       const int NW = a.W >= 512 ? 4 : (a.W >= 256 ? 2 : 1);
-      const size_t smem = sizeof(float) * x2::smem_floats(NW, a.E);
+      const size_t smem = sizeof(float) * x2::smem_floats(NW);
       const dim3 grid((a.W + 128 * NW - 1) / (128 * NW), (a.H + x2::RB - 1) / x2::RB, a.B * a.K);
-#define HPD_X2_LAUNCH_WT(E_, NW_, T_, WT_)                                                                  \
+#define HPD_X2_LAUNCH(NW_, T_)                                                                              \
   do {                                                                                                      \
-    if (int rc_ = ensure_dynamic_smem((const void*)x2::agg_nms_x2_kernel<E_, NW_, T_, WT_>, smem, "agg_nms_x2_kernel")) return rc_; \
-    x2::agg_nms_x2_kernel<E_, NW_, T_, WT_><<<grid, 32 * NW_, smem, st>>>(a);                               \
+    if (int rc_ = ensure_dynamic_smem((const void*)x2::agg_nms_x2_kernel<NW_, T_>, smem, "agg_nms_x2_kernel")) return rc_; \
+    x2::agg_nms_x2_kernel<NW_, T_><<<grid, 32 * NW_, smem, st>>>(a);                                        \
   } while (0)
-#define HPD_X2_LAUNCH_T(E_, NW_, T_)                                                                        \
+#define HPD_X2_LAUNCH_T(NW_)                                                                                \
   do {                                                                                                      \
-    if (a.agg_tags) HPD_X2_LAUNCH_WT(E_, NW_, T_, true); else HPD_X2_LAUNCH_WT(E_, NW_, T_, false);         \
+    if (a.dtype == HPD_F16) HPD_X2_LAUNCH(NW_, __half);                                                     \
+    else if (a.dtype == HPD_BF16) HPD_X2_LAUNCH(NW_, __nv_bfloat16);                                        \
+    else HPD_X2_LAUNCH(NW_, float);                                                                         \
   } while (0)
-#define HPD_X2_LAUNCH(E_, NW_)                                                                              \
-  do {                                                                                                      \
-    if (a.dtype == HPD_F16) HPD_X2_LAUNCH_T(E_, NW_, __half);                                                \
-    else if (a.dtype == HPD_BF16) HPD_X2_LAUNCH_T(E_, NW_, __nv_bfloat16);                                  \
-    else HPD_X2_LAUNCH_T(E_, NW_, float);                                                                   \
-  } while (0)
-      if (a.E == 1) { if (NW == 4) HPD_X2_LAUNCH(1, 4); else if (NW == 2) HPD_X2_LAUNCH(1, 2); else HPD_X2_LAUNCH(1, 1); }
-      else          { if (NW == 4) HPD_X2_LAUNCH(2, 4); else if (NW == 2) HPD_X2_LAUNCH(2, 2); else HPD_X2_LAUNCH(2, 1); }
-#undef HPD_X2_LAUNCH
+      if (NW == 4) HPD_X2_LAUNCH_T(4); else if (NW == 2) HPD_X2_LAUNCH_T(2); else HPD_X2_LAUNCH_T(1);
 #undef HPD_X2_LAUNCH_T
-#undef HPD_X2_LAUNCH_WT
+#undef HPD_X2_LAUNCH
       count_launch();
       return check_launch("agg_nms_x2_kernel");
     }
@@ -663,7 +585,7 @@ int launch_aggregate_nms(const HpdParams* p, const HpdScaleInputs* scales, const
         g.lr[s] = lr;
         g.lc[s] = (lc + 6 + 3) & ~3;
       }
-      const int tag_words = a.E * ms::TR * (32 * NW + 8);
+      const int tag_words = ms::TR * (32 * NW + 8);
       off = off > tag_words ? off : tag_words;
       off = (off + 3) & ~3;
       for (int s = 0; s < a.n_scales; ++s) {
@@ -676,23 +598,22 @@ int launch_aggregate_nms(const HpdParams* p, const HpdScaleInputs* scales, const
       const size_t smem = sizeof(float) * (size_t)g.total;
       if (smem <= 200 * 1024) {
         const dim3 grid((a.W + 128 * NW - 1) / (128 * NW), (a.H + ms::RB - 1) / ms::RB, a.B * a.K);
-#define HPD_MS_LAUNCH(E_, NW_, NS_, T_)                                                                          \
+#define HPD_MS_LAUNCH(NW_, NS_, T_)                                                                              \
   do {                                                                                                           \
-    if (int rc_ = ensure_dynamic_smem((const void*)ms::agg_nms_ms_kernel<E_, NW_, NS_, T_>, smem, "agg_nms_ms_kernel")) return rc_; \
-    ms::agg_nms_ms_kernel<E_, NW_, NS_, T_><<<grid, 32 * NW_, smem, st>>>(a, g);                                 \
+    if (int rc_ = ensure_dynamic_smem((const void*)ms::agg_nms_ms_kernel<NW_, NS_, T_>, smem, "agg_nms_ms_kernel")) return rc_; \
+    ms::agg_nms_ms_kernel<NW_, NS_, T_><<<grid, 32 * NW_, smem, st>>>(a, g);                                     \
   } while (0)
-#define HPD_MS_NS_T(E_, NW_, T_)                                                                                 \
+#define HPD_MS_NS_T(NW_, T_)                                                                                     \
   do {                                                                                                           \
-    if (a.n_scales == 1) HPD_MS_LAUNCH(E_, NW_, 1, T_); else if (a.n_scales == 2) HPD_MS_LAUNCH(E_, NW_, 2, T_); else HPD_MS_LAUNCH(E_, NW_, 3, T_); \
+    if (a.n_scales == 1) HPD_MS_LAUNCH(NW_, 1, T_); else if (a.n_scales == 2) HPD_MS_LAUNCH(NW_, 2, T_); else HPD_MS_LAUNCH(NW_, 3, T_); \
   } while (0)
-#define HPD_MS_NS(E_, NW_)                                                                                       \
+#define HPD_MS_NS(NW_)                                                                                           \
   do {                                                                                                           \
-    if (a.dtype == HPD_F16) HPD_MS_NS_T(E_, NW_, __half);                                                       \
-    else if (a.dtype == HPD_BF16) HPD_MS_NS_T(E_, NW_, __nv_bfloat16);                                         \
-    else HPD_MS_NS_T(E_, NW_, float);                                                                            \
+    if (a.dtype == HPD_F16) HPD_MS_NS_T(NW_, __half);                                                           \
+    else if (a.dtype == HPD_BF16) HPD_MS_NS_T(NW_, __nv_bfloat16);                                             \
+    else HPD_MS_NS_T(NW_, float);                                                                                \
   } while (0)
-        if (a.E == 1) { if (NW == 5) HPD_MS_NS(1, 5); else if (NW == 4) HPD_MS_NS(1, 4); else if (NW == 3) HPD_MS_NS(1, 3); else HPD_MS_NS(1, 2); }
-        else          { if (NW == 5) HPD_MS_NS(2, 5); else if (NW == 4) HPD_MS_NS(2, 4); else if (NW == 3) HPD_MS_NS(2, 3); else HPD_MS_NS(2, 2); }
+        if (NW == 5) HPD_MS_NS(5); else if (NW == 4) HPD_MS_NS(4); else if (NW == 3) HPD_MS_NS(3); else HPD_MS_NS(2);
 #undef HPD_MS_NS
 #undef HPD_MS_NS_T
 #undef HPD_MS_LAUNCH
@@ -701,9 +622,8 @@ int launch_aggregate_nms(const HpdParams* p, const HpdScaleInputs* scales, const
       }
     }
   }
-  const int lo_words = (a.LO_R * a.LO_C > a.E * a.TG_R * a.TG_C) ? a.LO_R * a.LO_C : a.E * a.TG_R * a.TG_C;
-  const size_t smem = sizeof(float) * ((size_t)OT_R * OT_C + (size_t)OT_R * TW + (size_t)a.HI_R * a.HI_C + lo_words +
-                                       4 * (OT_C + OT_R + a.HI_C + a.HI_R));
+  const size_t smem = sizeof(float) * ((size_t)OT_R * OT_C + (size_t)OT_R * TW + (size_t)a.HI_R * a.HI_C +
+                                       (size_t)a.LO_R * a.LO_C + 4 * (OT_C + OT_R + a.HI_C + a.HI_R));
   if (smem > 227 * 1024) {
     set_error("resize ratios need %zu bytes of shared memory per tile (> 227 KB)", smem);
     return HPD_EINVAL;
@@ -713,6 +633,13 @@ int launch_aggregate_nms(const HpdParams* p, const HpdScaleInputs* scales, const
   agg_nms_generic_kernel<<<grid, kAggThreads, smem, st>>>(a);
   count_launch();
   return check_launch("agg_nms_generic_kernel");
+}
+
+}  // namespace
+
+int launch_aggregate_nms(const HpdParams* p, const HpdScaleInputs* scales, const HpdBuffers* buf, cudaStream_t st) {
+  if (int rc = launch_aggregation_kernel(p, scales, buf, st)) return rc;
+  return buf->agg_tags ? launch_aggregate_tags(p, scales, buf->agg_tags, st) : HPD_OK;
 }
 
 int launch_nms(const HpdParams* p, const HpdBuffers* buf, float* nms_out, cudaStream_t st) {

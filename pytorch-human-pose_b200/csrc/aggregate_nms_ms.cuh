@@ -9,7 +9,7 @@
 //     horizontally interpolated S_s rows; the vertical taps of every (scale, output row) come from a small
 //     shared table; the scales are summed sequentially and divided by n like torch.stack(...).mean(0);
 //   * tags come from one scale and must be an exact x4 (as in the reference); NMS, word side arrays and tag
-//     bounds are the x2 kernel's;
+//     bounds are the x2 kernel's, and like it this kernel writes no tag map;
 //   * input elements are float32, IEEE half or bfloat16 (T); 16-bit values are widened exactly as they are loaded,
 //     shared memory and all arithmetic stay float32.
 // Bit-identical to the generic kernel (tests/test_gpu_stages.py).
@@ -126,12 +126,12 @@ __device__ __forceinline__ void stage_segments(float* __restrict__ smem, const S
   }
 }
 
-template <int E, int NW, int NS, typename T>
+template <int NW, int NS, typename T>
 __global__ void __launch_bounds__(32 * NW, 16 / NW) agg_nms_ms_kernel(const AggArgs a, const Geom g) {
   extern __shared__ __align__(16) float smem[];
   constexpr int tc = 32 * NW + 8;
   constexpr int nthr = 32 * NW;
-  float* sT = smem;                                   // tags alias the S tiles (consumed first)
+  float* sT = smem;                                   // the tag tile aliases the S tiles (consumed first)
   float* sEdge = smem + g.off_edge;
   // out-row -> S_s row taps: [NS][NROWS] x (packed i0 | i1 << 8 | advance << 16, w0, w1); the advance code
   // says how the walk's two cached rows move on: 0 keep both, 1 shift (new i0 = old i1), 2 reload; -1 = the
@@ -190,16 +190,13 @@ __global__ void __launch_bounds__(32 * NW, 16 / NW) agg_nms_ms_kernel(const AggA
     hi.dst = g.off_s[s]; hi.stride = g.hc[s]; hi.nvec = nhx >> 2; hi.w = S.hw; hi.rows = nhy;
   }
 
-  // ---------------- phase 0: tags (x4), identical to the x2 kernel ------------------------------------
+  // ---------------- phase 0: tag bounds (x4), identical to the x2 kernel --------------------------------
   {
     const int txo = x0 / 4 - 4, tyo = y0 / 4 - 1;
     const T* tg0 = reinterpret_cast<const T*>(a.tag) + (size_t)b * a.tag_sb + (size_t)k * a.tag_sc;
-    const bool unflip = !a.tags_preflipped;
-    const T* tg1 = (E > 1) ? reinterpret_cast<const T*>(a.tag_f) + (size_t)b * a.tagf_sb + (size_t)(unflip ? kf : k) * a.tagf_sc : nullptr;
-    x2::stage_tile<0, TR, tc, NW, false, T>(sT, tg0, (const T*)nullptr, false, tyo, txo, a.th, a.tw, warp, lane);
-    if (E > 1) x2::stage_tile<1, TR, tc, NW, false, T>(sT + TR * tc, (const T*)nullptr, tg1, unflip, tyo, txo, a.th, a.tw, warp, lane);
+    x2::stage_tile<false, TR, tc, NW, false, T>(sT, tg0, (const T*)nullptr, tyo, txo, a.th, a.tw, warp, lane);
     __syncthreads();
-    if (active) x2::tags_x4_band<E, RB, TR>(a, sT, tc, txo, X0, y0, b, k, lane);
+    if (active) x2::tag_bounds_x4_band<RB, TR>(a, sT, tc, txo, X0, y0, b, k, lane);
     __syncthreads();
   }
 
@@ -430,7 +427,7 @@ __global__ void __launch_bounds__(32 * NW, 16 / NW) agg_nms_ms_kernel(const AggA
   MSP_MARK(4);
 #ifdef HPD_MS_PROFILE
   if (prof)
-    printf("ms profile (cycles): tags %lld, stage+S tiles %lld, taps+halo %lld, walk %lld\n", pt[1] - pt[0], pt[2] - pt[1],
+    printf("ms profile (cycles): tag bounds %lld, stage+S tiles %lld, taps+halo %lld, walk %lld\n", pt[1] - pt[0], pt[2] - pt[1],
            pt[3] - pt[2], pt[4] - pt[3]);
 #endif
 }

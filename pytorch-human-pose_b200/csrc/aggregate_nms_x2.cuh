@@ -8,12 +8,12 @@
 // Work decomposition (B200: issue-bound otherwise -- the generic kernel spends ~370 instructions
 // per output pixel; this one ~65, which leaves the kernel bound by HBM writes):
 //   * one CTA = a band of RB output rows x (128 * NW) columns of one (image, joint) plane;
-//   * phase 0 (tags first): the tag tiles are staged (16-byte loads, one warp per tile row, the flipped
-//     run read mirrored with the permuted joint index) and every lane writes its 4 columns of all rows
-//     with x4 taps and E-innermost 16-byte stores, plus the per-(4 rows x word) bounds of the first tag
-//     component; the tag tiles alias the half-res tile, so shared memory stays at 30 KB (6 CTAs/SM).
-//     Without a tag map to write (WRITE_TAGS = false, the decode's default) only the first component is
-//     staged and only its bounds are derived: the map was two thirds of the kernel's HBM writes;
+//   * phase 0 (tag bounds): the quarter-res tile of the first tag component is staged (16-byte loads, one
+//     warp per tile row) and every word of the band gets the per-(4 rows x word) range of the tags its
+//     pixels interpolate from (tag_bmin / tag_bmax, the refine prefilter).  The tag tile aliases the
+//     half-res tile, so shared memory stays at 30 KB (6 CTAs/SM).  The full-resolution tag map is not
+//     written here: the tag stages interpolate the few tags they read (tag_at), and aggregate_tags_kernel
+//     writes the map for callers that keep one;
 //   * phase 1 (all threads): flip-averaged quarter-res / half-res tiles -> smem, tile interiors 16-byte
 //     aligned, two rows per batch so that all loads of a batch are in flight before the first store;
 //   * phase 2 (all threads): stage mean S at half resolution, in place, exact torch arithmetic
@@ -35,9 +35,8 @@ constexpr int NROWS = RB + 4;          // output rows walked (band + 2 halo rows
 
 __host__ __device__ inline int SC(int NW) { return 64 * NW + 8; }   // half-res cols: hx0-4 .. (interior 16B aligned)
 __host__ __device__ inline int LC(int NW) { return 32 * NW + 8; }   // quarter-res cols: lx0-4 ..
-__host__ __device__ inline int TC(int NW) { return 32 * NW + 8; }   // quarter-res cols: lx0-4 ..
-__host__ __device__ inline size_t smem_floats(int NW, int E) {
-  (void)E;   // the tag tiles (E * TR * TC <= SR * SC floats) alias the half-res tile
+__host__ __device__ inline size_t smem_floats(int NW) {
+  // the tag tile (TR * LC <= SR * SC floats) aliases the half-res tile
   return (size_t)SR * SC(NW) + (size_t)LR * LC(NW) + (size_t)NW * NROWS * 4 + 4 * SR + 8;
 }
 
@@ -59,8 +58,7 @@ __device__ __forceinline__ void tap_x2(int o, int I, int& i0, int& i1, float& w0
 // batch are in flight before the first is consumed).  VEC: 16-byte loads/stores for the interior
 // (the flipped operand is read as the mirrored 16 bytes and reversed in registers), scalars for the
 // 8 halo columns and for any part right of the map.
-//   MODE 0: dst = p[y][x]      MODE 1: dst = pf[y][mirror ? w-1-x : x]
-//   MODE 2: dst = (p[y][x] + pf[y][w-1-x]) * 0.5   (flip averaging, model.py:90)
+//   AVG = false: dst = p[y][x]      AVG = true: dst = (p[y][x] + pf[y][w-1-x]) * 0.5   (flip averaging, model.py:90)
 // Input element type: float32 (inference), IEEE half (the validation-time caller runs the network under fp16
 // autocast, module.py:78) or bfloat16 (bf16 autocast).  16-bit values are widened on load -- exactly -- and
 // everything after is float32 arithmetic.
@@ -89,18 +87,17 @@ template <> struct In<__nv_bfloat16> {   // a bfloat16 is the upper 16 bits of t
   }
 };
 
-template <int MODE>
+template <bool AVG>
 __device__ __forceinline__ float stage_combine(float v, float f) {
-  return (MODE == 2) ? __fmul_rn(__fadd_rn(v, f), 0.5f) : (MODE == 0 ? v : f);
+  return AVG ? __fmul_rn(__fadd_rn(v, f), 0.5f) : v;
 }
 
-template <int MODE, int ROWS, int COLS, int NW, bool VEC, typename T = float>
+template <bool AVG, int ROWS, int COLS, int NW, bool VEC, typename T = float>
 __device__ __forceinline__ void stage_tile(float* __restrict__ dst, const T* __restrict__ p,
-                                           const T* __restrict__ pf, bool mirror, int yo, int xo, int h, int w,
+                                           const T* __restrict__ pf, int yo, int xo, int h, int w,
                                            int warp, int lane) {
   constexpr int RPB = 2;
   const int xm = w - 1;
-  const bool mir = (MODE == 2) || mirror;
   if (VEC) {
     constexpr int NV = (COLS - 8) / 4, VIT = (NV + 31) / 32;
 #pragma unroll 1
@@ -119,22 +116,18 @@ __device__ __forceinline__ void stage_tile(float* __restrict__ dst, const T* __r
           f[j][u] = v[j][u];
           if (r < ROWS && q < NV) {
             if (x + 3 <= xm) {
-              if (MODE != 1) v[j][u] = In<T>::ld4(p + row + x);
-              if (MODE != 0) {
-                if (mir) {
-                  const float4 t = In<T>::ld4(pf + row + (xm - x - 3));
-                  f[j][u] = make_float4(t.w, t.z, t.y, t.x);
-                } else {
-                  f[j][u] = In<T>::ld4(pf + row + x);
-                }
+              v[j][u] = In<T>::ld4(p + row + x);
+              if (AVG) {
+                const float4 t = In<T>::ld4(pf + row + (xm - x - 3));
+                f[j][u] = make_float4(t.w, t.z, t.y, t.x);
               }
             } else {   // right of the map: replicate the last column
               float tv[4], tf[4];
 #pragma unroll
               for (int c = 0; c < 4; ++c) {
                 const int xc = min(x + c, xm);
-                tv[c] = (MODE != 1) ? In<T>::ld1(p + row + xc) : 0.f;
-                tf[c] = (MODE != 0) ? In<T>::ld1(pf + row + (mir ? xm - xc : xc)) : 0.f;
+                tv[c] = In<T>::ld1(p + row + xc);
+                tf[c] = AVG ? In<T>::ld1(pf + row + (xm - xc)) : 0.f;
               }
               v[j][u] = make_float4(tv[0], tv[1], tv[2], tv[3]);
               f[j][u] = make_float4(tf[0], tf[1], tf[2], tf[3]);
@@ -145,8 +138,8 @@ __device__ __forceinline__ void stage_tile(float* __restrict__ dst, const T* __r
         if (r < ROWS && lane < 8) {
           const int c = (lane < 4) ? lane : COLS - 8 + lane;
           const int x = clampi(xo + c, 0, xm);
-          if (MODE != 1) hv[j] = In<T>::ld1(p + row + x);
-          if (MODE != 0) hf[j] = In<T>::ld1(pf + row + (mir ? xm - x : x));
+          hv[j] = In<T>::ld1(p + row + x);
+          if (AVG) hf[j] = In<T>::ld1(pf + row + (xm - x));
         }
       }
 #pragma unroll
@@ -158,10 +151,10 @@ __device__ __forceinline__ void stage_tile(float* __restrict__ dst, const T* __r
           const int q = lane + 32 * u;
           if (q < NV)
             *reinterpret_cast<float4*>(dst + r * COLS + 4 + 4 * q) =
-                make_float4(stage_combine<MODE>(v[j][u].x, f[j][u].x), stage_combine<MODE>(v[j][u].y, f[j][u].y),
-                            stage_combine<MODE>(v[j][u].z, f[j][u].z), stage_combine<MODE>(v[j][u].w, f[j][u].w));
+                make_float4(stage_combine<AVG>(v[j][u].x, f[j][u].x), stage_combine<AVG>(v[j][u].y, f[j][u].y),
+                            stage_combine<AVG>(v[j][u].z, f[j][u].z), stage_combine<AVG>(v[j][u].w, f[j][u].w));
         }
-        if (lane < 8) dst[r * COLS + ((lane < 4) ? lane : COLS - 8 + lane)] = stage_combine<MODE>(hv[j], hf[j]);
+        if (lane < 8) dst[r * COLS + ((lane < 4) ? lane : COLS - 8 + lane)] = stage_combine<AVG>(hv[j], hf[j]);
       }
     }
   } else {
@@ -179,8 +172,8 @@ __device__ __forceinline__ void stage_tile(float* __restrict__ dst, const T* __r
           v[j][u] = 0.f; f[j][u] = 0.f;
           if (r < ROWS && c < COLS) {
             const int x = clampi(xo + c, 0, xm);
-            if (MODE != 1) v[j][u] = In<T>::ld1(p + row + x);
-            if (MODE != 0) f[j][u] = In<T>::ld1(pf + row + (mir ? xm - x : x));
+            v[j][u] = In<T>::ld1(p + row + x);
+            if (AVG) f[j][u] = In<T>::ld1(pf + row + (xm - x));
           }
         }
       }
@@ -190,7 +183,7 @@ __device__ __forceinline__ void stage_tile(float* __restrict__ dst, const T* __r
 #pragma unroll
         for (int u = 0; u < NIT; ++u) {
           const int c = lane + 32 * u;
-          if (r < ROWS && c < COLS) dst[r * COLS + c] = stage_combine<MODE>(v[j][u], f[j][u]);
+          if (r < ROWS && c < COLS) dst[r * COLS + c] = stage_combine<AVG>(v[j][u], f[j][u]);
         }
       }
     }
@@ -272,80 +265,31 @@ struct NmsColumnWalk {
   }
 };
 
-// Tags of one band: x4 bilinear taps (results.py:229-230) from the staged quarter-res tag tiles sT
-// ([E][TR][tc], tile origin column txo, tile row r = quarter-res row y0/4 - 1 + r) to the E-innermost
-// output, for the lane's 4 output columns X0..X0+3 and the RB rows from y0; plus the per (4 rows x 32
-// columns) range of the first tag component (tag_bmin / tag_bmax, the refine prefilter).  Called by the
-// lanes whose columns are inside the image (W % 32 == 0: whole 8-lane word groups).  WRITE = false: only the
-// bounds (sT then needs only component 0); the output map is left alone, as it is when a.agg_tags is NULL.
-template <int E, int RB, int TR, bool WRITE = true>
-__device__ __forceinline__ void tags_x4_band(const AggArgs& a, const float* __restrict__ sT, int tc, int txo, int X0,
-                                             int y0, int b, int k, int lane) {
-  const int H = a.H, W = a.W;
-  const int q = X0 >> 2;                       // this lane's quarter-res column
-  const int tb = q - 1 - txo;                  // index of T[q-1] in a tile row
-  const bool x_first = (q == 0);
-  // columns 4q+{0,1}: taps (q-1,q) weights (.375,.625),(.125,.875); 4q+{2,3}: (q,q+1) (.875,.125),(.625,.375)
-  const float wa0 = x_first ? 1.f : 0.375f, wb0 = x_first ? 0.f : 0.625f;
-  const float wa1 = x_first ? 1.f : 0.125f, wb1 = x_first ? 0.f : 0.875f;
-  float hA[E][4], hB[E][4];
-  // also returns the range of the sources of the FIRST tag component: every output it contributes to
-  // is a convex combination of them (refine prefilter, tag_bmin / tag_bmax)
-  auto hpass = [&](int r, float (&h)[E][4], float& mn, float& mx) {
-#pragma unroll
-    for (int e = 0; e < E; ++e) {
-      const float* t = sT + e * TR * tc + r * tc + tb;
-      const float t0 = t[0], t1 = t[1], t2 = t[2];
-      if (e == 0) { mn = fminf(fminf(t0, t1), t2); mx = fmaxf(fmaxf(t0, t1), t2); }
-      if (!WRITE) continue;
-      const float a0 = x_first ? t1 : t0, b0 = x_first ? t2 : t1;
-      h[e][0] = fmaf(wa0, a0, __fmul_rn(wb0, b0));
-      h[e][1] = fmaf(wa1, a0, __fmul_rn(wb1, b0));
-      h[e][2] = fmaf(0.875f, t1, __fmul_rn(0.125f, t2));
-      h[e][3] = fmaf(0.625f, t1, __fmul_rn(0.375f, t2));
-    }
+// Tag bounds of one band: per (4 rows x 32 columns) the range of the first tag component's quarter-res
+// sources (tag_bmin / tag_bmax, the refine prefilter).  Every tag of an output pixel is an x4 bilinear
+// combination (results.py:229-230) of the 3 x 3 quarter-res tags around it, so it lies in that range.  sT is
+// the staged tile of the first component ([TR][tc], origin column txo, tile row r = quarter-res row
+// y0/4 - 1 + r); the lane covers output columns X0..X0+3 and the RB rows from y0.  Called by the lanes
+// whose columns are inside the image (W % 32 == 0: whole 8-lane word groups).
+template <int RB, int TR>
+__device__ __forceinline__ void tag_bounds_x4_band(const AggArgs& a, const float* __restrict__ sT, int tc, int txo,
+                                                   int X0, int y0, int b, int k, int lane) {
+  const int H = a.H;
+  const int tb = (X0 >> 2) - 1 - txo;          // index of T[q-1] in a tile row, q = this lane's quarter-res column
+  auto range = [&](int r, float& mn, float& mx) {
+    const float* t = sT + r * tc + tb;
+    const float t0 = t[0], t1 = t[1], t2 = t[2];
+    mn = fminf(fminf(t0, t1), t2); mx = fmaxf(fmaxf(t0, t1), t2);
   };
-  float* tg_plane = a.agg_tags + ((size_t)b * a.K + k) * H * W * E;
-  auto emit = [&](int y, float wy0, float wy1, const float (&A)[E][4], const float (&Bv)[E][4]) {
-    if (!WRITE || a.agg_tags == nullptr || y < y0 || y >= y0 + RB || y >= H) return;
-    float o[E][4];
-#pragma unroll
-    for (int e = 0; e < E; ++e)
-#pragma unroll
-      for (int c = 0; c < 4; ++c) o[e][c] = fmaf(wy0, A[e][c], __fmul_rn(wy1, Bv[e][c]));
-    float* dst = tg_plane + ((size_t)y * W + X0) * E;
-    if (E == 1) {
-      *reinterpret_cast<float4*>(dst) = make_float4(o[0][0], o[0][1], o[0][2], o[0][3]);
-    } else {
-      *reinterpret_cast<float4*>(dst) = make_float4(o[0][0], o[E - 1][0], o[0][1], o[E - 1][1]);
-      *reinterpret_cast<float4*>(dst + 4) = make_float4(o[0][2], o[E - 1][2], o[0][3], o[E - 1][3]);
-    }
-  };
-  // tile rows: r <-> quarter-res row tyo + r = y0/4 - 1 + r.  Rows y0, y0+1 use (i-1, i) with
-  // i = y0/4, i.e. tile rows (0, 1); then each group of 4 rows 4i+2..4i+5 uses rows (i, i+1).
   const unsigned amask = __activemask();      // W % 32 == 0: whole 8-lane word groups are active
   float mnA, mxA, mnB, mxB, mnC, mxC;
-  hpass(0, hA, mnA, mxA);
-  hpass(1, hB, mnB, mxB);
-  if (y0 == 0) {          // first two rows of the image: src clamps to 0 -> taps (row 0, row 1), weights (1, 0)
-    float hC[E][4];
-    hpass(2, hC, mnC, mxC);   // tile row 1 = image row 0, tile row 2 = image row 1
-    emit(0, 1.f, 0.f, hB, hC);
-    emit(1, 1.f, 0.f, hB, hC);
-  } else {
-    emit(y0, 0.375f, 0.625f, hA, hB);
-    emit(y0 + 1, 0.125f, 0.875f, hA, hB);
-  }
+  range(0, mnA, mxA);
+  range(1, mnB, mxB);
   const int HB = (H + 3) >> 2;
   const size_t bbase = (((size_t)b * a.K + k) * HB + (y0 >> 2)) * a.wpr + (X0 >> 5);
 #pragma unroll 1
   for (int g = 0; g < RB / 4; ++g) {
-    // rows y0 + 4g + 2 .. y0 + 4g + 5 : taps (tile row g+1, tile row g+2)
-#pragma unroll
-    for (int e = 0; e < E; ++e)
-#pragma unroll
-      for (int c = 0; c < 4; ++c) hA[e][c] = hB[e][c];
-    hpass(g + 2, hB, mnC, mxC);
+    range(g + 2, mnC, mxC);
     // band of rows y0+4g .. y0+4g+3 reads tile rows g, g+1, g+2: bounds over the 8 lanes of the word
     if (y0 + 4 * g < H) {
       float mn = fminf(fminf(mnA, mnB), mnC), mx = fmaxf(fmaxf(mxA, mxB), mxC);
@@ -360,25 +304,16 @@ __device__ __forceinline__ void tags_x4_band(const AggArgs& a, const float* __re
       }
     }
     mnA = mnB; mxA = mxB; mnB = mnC; mxB = mxC;
-    const int y = y0 + 4 * g + 2;
-    emit(y, 0.875f, 0.125f, hA, hB);
-    emit(y + 1, 0.625f, 0.375f, hA, hB);
-    if (g + 1 < RB / 4) {
-      emit(y + 2, 0.375f, 0.625f, hA, hB);
-      emit(y + 3, 0.125f, 0.875f, hA, hB);
-    }
   }
 }
 
-// WRITE_TAGS = false (a.agg_tags == NULL): phase 0 stages only the first tag component and derives only its
-// bounds; the tag stages interpolate the few tags they read themselves (tag_at).
-template <int E, int NW, typename T, bool WRITE_TAGS>
+template <int NW, typename T>
 __global__ void __launch_bounds__(32 * NW) agg_nms_x2_kernel(const AggArgs a) {
   extern __shared__ __align__(16) float smem[];
   constexpr int sc = 64 * NW + 8, lc = 32 * NW + 8, tc = 32 * NW + 8;
   float* sS = smem;                              // [SR][sc]   hi average, then stage mean S
   float* sL = sS + SR * sc;                      // [LR][lc]   flip-averaged hm_lo
-  float* sT = smem;                              // [E][TR][tc] tags -- aliases sS, consumed (phase 0) before sS is staged
+  float* sT = smem;                              // [TR][tc]   first tag component -- aliases sS, read (phase 0) before sS is staged
   float* sEdge = sL + LR * lc;                   // [NW][NROWS][4] halo-column values per warp
   int* sRowI0 = (int*)(sEdge + NW * NROWS * 4);  // [SR] phase-2 vertical taps (rows of sL)
   int* sRowI1 = sRowI0 + SR;
@@ -395,29 +330,22 @@ __global__ void __launch_bounds__(32 * NW) agg_nms_x2_kernel(const AggArgs a) {
   const int x0 = blockIdx.x * 128 * NW, y0 = blockIdx.y * RB;
   const int hxo = x0 / 2 - 4, hyo = y0 / 2 - 2;     // origins of the half-res tile
   const int lxo = x0 / 4 - 4, lyo = y0 / 4 - 2;     // origins of the quarter-res hm tile
-  const int txo = x0 / 4 - 4, tyo = y0 / 4 - 1;     // origins of the tag tiles
+  const int txo = x0 / 4 - 4, tyo = y0 / 4 - 1;     // origins of the tag tile
 
   const int xw = x0 + 128 * warp;                 // first column of this warp's strip
   const int X0 = xw + 4 * lane;                   // this lane's 4 output columns
   const bool active = X0 < W;
 
-  // ---------------- phase 0a: stage the tag tiles (they alias the half-res tile) ---------------------
+  // ---------------- phase 0a: stage the first tag component (aliases the half-res tile) -------------
   {
     const T* tg0 = reinterpret_cast<const T*>(a.tag) + (size_t)b * a.tag_sb + (size_t)k * a.tag_sc;
-    const bool unflip = !a.tags_preflipped;   // model.py:93: flip(tag_f, W)[:, FLIP]
-    const T* tg1 = (E > 1 && WRITE_TAGS) ? reinterpret_cast<const T*>(a.tag_f) + (size_t)b * a.tagf_sb + (size_t)(unflip ? kf : k) * a.tagf_sc : nullptr;
-    if (a.in_vec_ok) {
-      stage_tile<0, TR, tc, NW, true>(sT, tg0, (const T*)nullptr, false, tyo, txo, a.th, a.tw, warp, lane);
-      if (E > 1 && WRITE_TAGS) stage_tile<1, TR, tc, NW, true>(sT + TR * tc, (const T*)nullptr, tg1, unflip, tyo, txo, a.th, a.tw, warp, lane);
-    } else {
-      stage_tile<0, TR, tc, NW, false>(sT, tg0, (const T*)nullptr, false, tyo, txo, a.th, a.tw, warp, lane);
-      if (E > 1 && WRITE_TAGS) stage_tile<1, TR, tc, NW, false>(sT + TR * tc, (const T*)nullptr, tg1, unflip, tyo, txo, a.th, a.tw, warp, lane);
-    }
+    if (a.in_vec_ok) stage_tile<false, TR, tc, NW, true>(sT, tg0, (const T*)nullptr, tyo, txo, a.th, a.tw, warp, lane);
+    else stage_tile<false, TR, tc, NW, false>(sT, tg0, (const T*)nullptr, tyo, txo, a.th, a.tw, warp, lane);
   }
   __syncthreads();
-  // ---------------- phase 0b: tags, x4 taps (results.py:229-230) ------------------------------------
-  if (active) tags_x4_band<WRITE_TAGS ? E : 1, RB, TR, WRITE_TAGS>(a, sT, tc, txo, X0, y0, b, k, lane);
-  __syncthreads();   // every warp is done with the tag tiles before the half-res tile overwrites them
+  // ---------------- phase 0b: tag bounds (refine prefilter) ------------------------------------------
+  if (active) tag_bounds_x4_band<RB, TR>(a, sT, tc, txo, X0, y0, b, k, lane);
+  __syncthreads();   // every warp is done with the tag tile before the half-res tile overwrites it
 
   // ---------------- phase 1: stage the heatmap inputs -------------------------------------------------
   {
@@ -428,11 +356,11 @@ __global__ void __launch_bounds__(32 * NW) agg_nms_x2_kernel(const AggArgs a) {
 #define HPD_STAGE_ALL(VEC_)                                                                                    \
   do {                                                                                                         \
     if (lof) {                                                                                                 \
-      stage_tile<2, LR, lc, NW, VEC_>(sL, lo, lof, true, lyo, lxo, S.lh, S.lw, warp, lane);                    \
-      stage_tile<2, SR, sc, NW, VEC_>(sS, hi, hif, true, hyo, hxo, S.hh, S.hw, warp, lane);                    \
+      stage_tile<true, LR, lc, NW, VEC_>(sL, lo, lof, lyo, lxo, S.lh, S.lw, warp, lane);                       \
+      stage_tile<true, SR, sc, NW, VEC_>(sS, hi, hif, hyo, hxo, S.hh, S.hw, warp, lane);                       \
     } else {                                                                                                   \
-      stage_tile<0, LR, lc, NW, VEC_>(sL, lo, (const T*)nullptr, false, lyo, lxo, S.lh, S.lw, warp, lane);               \
-      stage_tile<0, SR, sc, NW, VEC_>(sS, hi, (const T*)nullptr, false, hyo, hxo, S.hh, S.hw, warp, lane);               \
+      stage_tile<false, LR, lc, NW, VEC_>(sL, lo, (const T*)nullptr, lyo, lxo, S.lh, S.lw, warp, lane);        \
+      stage_tile<false, SR, sc, NW, VEC_>(sS, hi, (const T*)nullptr, hyo, hxo, S.hh, S.hw, warp, lane);        \
     }                                                                                                          \
   } while (0)
     if (a.in_vec_ok) HPD_STAGE_ALL(true); else HPD_STAGE_ALL(false);

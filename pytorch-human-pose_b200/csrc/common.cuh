@@ -81,9 +81,9 @@ struct TagSource {
 };
 
 #ifdef __CUDACC__
-// The tag vector of output pixel (y, x) of plane (b, k), exactly as the aggregation kernels write it: the
-// generic kernel's taps (axis_tap on both axes, lerp2), the flipped run read at the mirrored column and the
-// flipped joint unless tags_preflipped (model.py:93).  t[e] for e >= E is left alone.
+// The tag vector of output pixel (y, x) of plane (b, k), as aggregate_tags_kernel writes it into the map: bilinear
+// taps on both axes (axis_tap, lerp2), the flipped run read at the mirrored column and the flipped joint unless
+// tags_preflipped (model.py:93).  t[e] for e >= E is left alone.
 __device__ __forceinline__ void tag_at(const TagSource& s, int b, int k, int y, int x, float (&t)[HPD_MAX_EMB]) {
   const Tap tx = axis_tap(s.s_x, x, s.tw, s.W), ty = axis_tap(s.s_y, y, s.th, s.H);
 #pragma unroll

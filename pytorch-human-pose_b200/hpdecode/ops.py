@@ -105,7 +105,7 @@ class DecodeBuffers:
     section's coordinates are back-projected with (None = network-input coordinates).
 
     ``tags=False`` allocates no full-resolution tag map (``tag_map`` is None, 4*K*H*W*E bytes per image less): the
-    aggregation then writes none and the tag stages interpolate the few tags they read from the network outputs,
+    aggregation stage then writes none and the tag stages interpolate the few tags they read from the network outputs,
     which ``run_stage`` hands them from its ``scales``.  ``agg_tags`` is then computed on first read from the network
     outputs of the last decode into the set (``run_aggregate_tags``), which must be unchanged by then."""
 
@@ -261,7 +261,7 @@ def run_decode(scales: Optional[Sequence[dict]], bufs: DecodeBuffers, params: Hp
 
 def run_aggregate_tags(scales: Sequence[dict], params: HpdParams, out: Tensor):
     """hpd_aggregate_tags on the current stream: the full-resolution tag map [B,K,H,W,E] of scales[tag_scale] into
-    ``out``, bit-identical to the one hpd_aggregate_nms writes."""
+    ``out``: the kernel hpd_aggregate_nms runs to fill a tag map."""
     B, K, H, W, E = params.batch, params.num_kpts, params.out_h, params.out_w, params.emb
     if tuple(out.shape) != (B, K, H, W, E) or not out.is_contiguous() or not out.is_cuda or out.dtype != torch.float32:
         raise _lib.HpdError(f"aggregate_tags: out must be a contiguous CUDA float32 tensor {(B, K, H, W, E)}")

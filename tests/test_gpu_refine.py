@@ -712,7 +712,7 @@ def _rand_outputs(lh, lw, E, seed, K=5):
 @pytest.mark.parametrize("E", [1, 2])
 @pytest.mark.parametrize("half", [False, True])
 def test_x2_kernel_bounds_and_word_maxima(lh, lw, E, half):
-    """agg_nms_x2_kernel with and without the tag map (WRITE_TAGS): every tag inside its block's bounds (borders
+    """agg_nms_x2_kernel into buffer sets with and without a tag map: every tag inside its block's bounds (borders
     included), word maxima equal to the oracle's, and the generic kernel's bounds exactly -inf / +inf."""
     s = _rand_outputs(lh, lw, E, seed=lh * 7 + lw + E + 100 * half)
     H, W = 4 * lh, 4 * lw
@@ -788,3 +788,4 @@ def test_tag_map_finer_than_output():
         ops.run_decode(_dev([s]), bufs, p)
         _check(bufs, want, f"tag map 160 -> 128 tags={tags}", M, K, E)
         assert np.array_equal(_bits(bufs.agg_hm[0].cpu().numpy()), _bits(hm))
+        assert np.array_equal(_bits(bufs.agg_tags[0].cpu().numpy()), _bits(tg))

@@ -34,6 +34,14 @@ def _run_aggregate(scales, H, W, E, force_generic, tags_preflipped=False, tag_sc
     return bufs
 
 
+def _assert_tag_map_matches_oracle(bufs, scales, H, W, oracle, tag_scale=0):
+    """Every image's tag map against the oracle's aggregation of the same inputs."""
+    for b in range(bufs.agg_tags.shape[0]):
+        _, tg_o = oracle.aggregate([{k: v[b].cpu().numpy() for k, v in s.items()} for s in scales], (H, W),
+                                   tag_scale=tag_scale)
+        assert np.array_equal(_bits(bufs.agg_tags[b].cpu().numpy()), _bits(tg_o)), f"image {b}: tag map"
+
+
 def _rand_maps(B, lh, lw, flip, seed):
     g = torch.Generator().manual_seed(seed)
     d = {"hm_lo": torch.randn(B, 17, lh, lw, generator=g), "hm_hi": torch.randn(B, 17, 2 * lh, 2 * lw, generator=g),
@@ -46,14 +54,16 @@ def _rand_maps(B, lh, lw, flip, seed):
 
 @pytest.mark.parametrize("lh,lw,flip,B", [(128, 128, True, 2), (128, 128, False, 1), (48, 48, True, 1), (40, 72, True, 1),
                                            (160, 160, True, 1), (64, 176, False, 2), (32, 256, True, 1), (12, 12, True, 1)])
-def test_specialised_kernel_is_bit_identical_to_generic(lh, lw, flip, B):
+def test_specialised_kernel_is_bit_identical_to_generic(lh, lw, flip, B, oracle):
     """aggregate_nms_x2 vs the generic kernel on every output, incl. borders, partial warps (W % 128 != 0),
-    several CTAs per row (W > 512) and tiny maps."""
+    several CTAs per row (W > 512) and tiny maps; the tag map (written by neither: aggregate_tags_kernel) vs the
+    oracle."""
     s = _rand_maps(B, lh, lw, flip, seed=lh * 1000 + lw)
     H, W, E = 4 * lh, 4 * lw, 2 if flip else 1
     fast = _run_aggregate([s], H, W, E, False)
     slow = _run_aggregate([s], H, W, E, True)
-    for name in ("agg_hm", "agg_tags", "nms_mask", "nms_wmax", "hm_wmax"):
+    _assert_tag_map_matches_oracle(fast, [s], H, W, oracle)
+    for name in ("agg_hm", "nms_mask", "nms_wmax", "hm_wmax"):
         a, b = getattr(fast, name).cpu().numpy(), getattr(slow, name).cpu().numpy()
         if name == "nms_wmax":   # prefilter values: the sign of a zero is unspecified
             assert np.array_equal(a, b), f"{name} differs ({lh}x{lw}, flip={flip})"
@@ -272,12 +282,13 @@ def _ms_scales(B, H, W, ratios, flip, seed):
     (128, 256, (0.25, 0.75), 1, True, 1),           # narrowest width the kernel takes (2 warps per CTA)
     (64, 1280, (0.5, 0.75), 0, True, 1),            # two 5-warp CTAs per row band
 ])
-def test_multiscale_kernel_is_bit_identical_to_generic(H, W, ratios, tag_scale, flip, B):
+def test_multiscale_kernel_is_bit_identical_to_generic(H, W, ratios, tag_scale, flip, B, oracle):
     scales = _ms_scales(B, H, W, ratios, flip, seed=H + W)
     E = 2 if flip else 1
     fast = _run_aggregate(scales, H, W, E, False, tag_scale=tag_scale)
     slow = _run_aggregate(scales, H, W, E, True, tag_scale=tag_scale)
-    for name in ("agg_hm", "agg_tags", "nms_mask", "nms_wmax", "hm_wmax"):
+    _assert_tag_map_matches_oracle(fast, scales, H, W, oracle, tag_scale)
+    for name in ("agg_hm", "nms_mask", "nms_wmax", "hm_wmax"):
         a, b = getattr(fast, name).cpu().numpy(), getattr(slow, name).cpu().numpy()
         if name == "nms_wmax":
             assert np.array_equal(a, b), f"{name} differs"

@@ -1,7 +1,7 @@
 """-m gpu: buffer sets without a full-resolution tag map.  The aggregation then writes no agg_tags and the tag stages
 (top-k, adjust, refine) interpolate the tags they read from the network outputs; every output must be bit-identical to
-a decode into a buffer set that holds the map, and the map computed afterwards (hpd_aggregate_tags, the lazy
-DecodeResult.agg_tags) bit-identical to the one the aggregation writes."""
+a decode into a buffer set that holds the map (where the tag stages read the map), the map must equal the oracle's,
+and the map computed afterwards (the lazy DecodeResult.agg_tags) must equal the one the decode wrote."""
 import numpy as np
 import pytest
 import torch
@@ -50,60 +50,63 @@ def _decode_both(scales, H, W, tag_scale=0, force_generic=0, tags_preflipped=Fal
     return out[0], out[1], p
 
 
-def _check_case(scales, H, W, what, **kw):
-    from hpdecode import ops
+def _check_case(scales, H, W, what, oracle, oracle_scales=None, **kw):
+    """oracle_scales: the inputs as the oracle takes them (un-flipped tag_f), if ``scales`` differ from them."""
     tagless, full, p = _decode_both(scales, H, W, **kw)
     _assert_same(tagless, full, what)
-    lazy = ops.run_aggregate_tags(scales, p, torch.empty_like(full.agg_tags))
-    torch.cuda.synchronize()
-    assert np.array_equal(_bits(lazy), _bits(full.agg_tags)), f"{what}: hpd_aggregate_tags differs from agg_tags"
+    ref = oracle_scales if oracle_scales is not None else scales
+    for b in range(p.batch):
+        _, tg_o = oracle.aggregate([{k: v[b].float().cpu().numpy() for k, v in s.items()} for s in ref], (H, W),
+                                   tag_scale=p.tag_scale)
+        assert np.array_equal(_bits(full.agg_tags[b]), np.ascontiguousarray(tg_o, np.float32).view(np.uint32)), \
+            f"{what}: image {b}: tag map vs oracle"
     assert torch.equal(tagless.agg_tags, full.agg_tags), f"{what}: lazy agg_tags of the tag-less set"
     return tagless, full
 
 
-def test_bench_workload_cfg2():
+def test_bench_workload_cfg2(oracle):
     """The flagship batch: HigherHRNet-W32 outputs, 64 x 512^2 + flip (agg_nms_x2_kernel, one warp per top-k row)."""
     from hpdecode import synth_net
     scale = synth_net.network_outputs(64, 512, flip=True, seed=1, C=32, device="cuda:0")
-    tagless, _ = _check_case([scale], 512, 512, "cfg2")
+    tagless, _ = _check_case([scale], 512, 512, "cfg2", oracle)
     assert int(tagless.n_person.sum()) > 0
 
 
-def test_cfg3_three_scales_w48_640():
+def test_cfg3_three_scales_w48_640(oracle):
     """Multi-scale kernel (tags from scale 1.0 of 0.5 / 1.0 / 1.5), W48 640^2 + flip."""
     from hpdecode import synth_net
     S = 640
     ins = [synth_net.network_outputs(2, int(round(S * sc / 64.0)) * 64, flip=True, seed=5, C=48, device="cuda:0", chunk=2)
            for sc in (0.5, 1.0, 1.5)]
-    _check_case(ins, S, S, "cfg3", tag_scale=1)
+    _check_case(ins, S, S, "cfg3", oracle, tag_scale=1)
 
 
 @pytest.mark.parametrize("size,flip", [(256, True), (192, False)])
-def test_half_inputs(size, flip):
+def test_half_inputs(size, flip, oracle):
     scales = _dev(synth.crowd(2, size, persons=10, flip=flip, seed=21), half=True)
-    _check_case(scales, size, size, f"half {size} flip={flip}")
+    _check_case(scales, size, size, f"half {size} flip={flip}", oracle)
 
 
-def test_tags_preflipped():
+def test_tags_preflipped(oracle):
     s = _dev(synth.crowd(2, 256, persons=12, flip=True, seed=23))[0]
     pre = dict(s)
     pre["tag_f"] = torch.flip(s["tag_f"], [3])[:, synth.COCO_FLIP_INDEX].contiguous()
-    a, _ = _check_case([pre], 256, 256, "preflipped", tags_preflipped=True)
-    b, _ = _check_case([s], 256, 256, "not preflipped")
+    a, _ = _check_case([pre], 256, 256, "preflipped", oracle, oracle_scales=[s], tags_preflipped=True)
+    b, _ = _check_case([s], 256, 256, "not preflipped", oracle)
     assert torch.equal(a.tags_k, b.tags_k) and torch.equal(a.records, b.records)
 
 
-def test_single_embedding_without_flip():
-    _check_case(_dev(synth.netlike(2, 256, flip=False, seed=25)), 256, 256, "E=1")
+def test_single_embedding_without_flip(oracle):
+    _check_case(_dev(synth.netlike(2, 256, flip=False, seed=25)), 256, 256, "E=1", oracle)
 
 
 @pytest.mark.parametrize("force_generic", [0, 1, 2, 4])
-def test_generic_kernel_and_topk_variants(force_generic):
+def test_generic_kernel_and_topk_variants(force_generic, oracle):
     """A size no specialised kernel takes (250 x 250 output from 64 x 64 tag maps: not x4, W % 32 != 0), and the
     standard size under force_generic (bit 0: generic aggregation + literal heap top-k; bits 1 / 2: top-k launches)."""
     scales = _dev(synth.crowd(2, 256, persons=10, flip=True, seed=27))
-    _check_case(scales, 250, 250, f"generic 250, force_generic={force_generic}", force_generic=force_generic)
-    _check_case(scales, 256, 256, f"256, force_generic={force_generic}", force_generic=force_generic)
+    _check_case(scales, 250, 250, f"generic 250, force_generic={force_generic}", oracle, force_generic=force_generic)
+    _check_case(scales, 256, 256, f"256, force_generic={force_generic}", oracle, force_generic=force_generic)
 
 
 def test_single_stage_calls():

@@ -3,7 +3,9 @@
 usage: python tools/sass_diff.py OLD.so NEW.so [PATTERN ...]  ->  one line per kernel of OLD whose demangled name
 contains one of the patterns (default: every kernel): "identical", "DIFFERS" or "missing", plus the kernels only NEW has.
 A kernel of NEW that gained a trailing `float` template argument (the element type of the inputs) is compared with the
-OLD kernel without it.  Instruction text and encodings are compared; only the offset comments are dropped.
+OLD kernel without it, and the aggregation kernels that lost their tag-map arguments with the OLD tag-less variants:
+agg_nms_x2_kernel<E, NW, T, false> -> <NW, T>, agg_nms_ms_kernel<E, NW, NS, T> -> <NW, NS, T> (both E of OLD map to
+the one NEW kernel).  Instruction text and encodings are compared; only the offset comments are dropped.
 Needs only the CUDA toolkit (cuobjdump, c++filt): no GPU.
 """
 import re
@@ -25,6 +27,12 @@ def kernels(lib):
     return {re.sub(r"^void |\(.*\)$", "", n): v for n, v in zip(names, out.values())}
 
 
+def without_tag_args(name):
+    """OLD name of a kernel with tag-map template arguments -> its name without them."""
+    name = re.sub(r"(agg_nms_x2_kernel)<\d, (.*), false>$", r"\1<\2>", name)
+    return re.sub(r"(agg_nms_ms_kernel)<\d, (\d, \d, [^,]+)>$", r"\1<\2>", name)
+
+
 def main(old_lib, new_lib, patterns):
     old, new = kernels(old_lib), kernels(new_lib)
     alias = {re.sub(r", float>$", ">", n): n for n in new}   # new name without the float element type -> new name
@@ -32,7 +40,7 @@ def main(old_lib, new_lib, patterns):
     for name in sorted(old):
         if patterns and not any(p in name for p in patterns):
             continue
-        twin = name if name in new else alias.get(name)
+        twin = name if name in new else alias.get(name) or (without_tag_args(name) if without_tag_args(name) in new else None)
         if twin is None:
             rows.append(("missing", name, "", len(old[name])))
             continue
