@@ -298,6 +298,23 @@ HPD_EXPORT int hpd_prepare_geometry(int n, const int32_t* img_h, const int32_t* 
 HPD_EXPORT int hpd_prepare_input(const HpdImage* images_host, int batch, float* out, int out_h, int out_w,
                                  const float mean[3], const float std_[3], void* stream);
 
+/* One output of hpd_prepare_inputs: a test scale's network input [batch,3,out_h,out_w] float32 and, optionally, its
+ * horizontally mirrored copy (the flip-test input, model.py:86), same shape. */
+typedef struct HpdPrepareTarget {
+  float* out;
+  float* out_flipped;   /* NULL = none; must not equal out */
+  int32_t out_h, out_w;
+} HpdPrepareTarget;
+
+/* hpd_prepare_input for every test scale of a batch in one pass: images_host[t*batch + b] is image b with the forward
+ * matrix of target t (the same image pointer for every t, normally).  targets_host[t].out receives exactly what
+ * hpd_prepare_input writes for those descriptors, and out_flipped[b][c][y][out_w-1-x] = out[b][c][y][x] (a second store
+ * of the same value: bit-identical to torch.flip(out, [3]), no extra read).  n_targets <= HPD_MAX_SCALES.  Up to 32
+ * (target, image) pairs go in one launch; larger calls are split (hpd_last_launch_count).  Every argument is checked
+ * before the first launch. */
+HPD_EXPORT int hpd_prepare_inputs(const HpdImage* images_host, int batch, const HpdPrepareTarget* targets_host,
+                                  int n_targets, const float mean[3], const float std_[3], void* stream);
+
 /* Bytes of scratch hpd_coco_eval needs for these params. */
 HPD_EXPORT int hpd_coco_eval_workspace_bytes(const HpdCocoEvalParams* p, size_t* out_bytes);
 

@@ -197,6 +197,12 @@ int hpd_prepare_input(const HpdImage* images_host, int batch, float* out, int ou
   return launch_prepare_input(images_host, batch, out, out_h, out_w, mean, std_, (cudaStream_t)stream);
 }
 
+int hpd_prepare_inputs(const HpdImage* images_host, int batch, const HpdPrepareTarget* targets_host, int n_targets,
+                       const float mean[3], const float std_[3], void* stream) {
+  g_launches = 0;
+  return launch_prepare_inputs(images_host, batch, targets_host, n_targets, mean, std_, (cudaStream_t)stream);
+}
+
 int hpd_coco_eval_workspace_bytes(const HpdCocoEvalParams* p, size_t* out_bytes) {
   if (!out_bytes) { set_error("NULL argument"); return HPD_EINVAL; }
   int rc = validate_coco_params(p);

@@ -191,6 +191,8 @@ size_t refine_workspace_bytes(const HpdParams* p);
 int launch_resize(const HpdMap* in, int batch, int channels, float* out, int oh, int ow, cudaStream_t st);
 int launch_prepare_input(const HpdImage* images, int batch, float* out, int oh, int ow, const float* mean,
                          const float* stdv, cudaStream_t st);
+int launch_prepare_inputs(const HpdImage* images, int batch, const HpdPrepareTarget* targets, int n_targets,
+                          const float* mean, const float* stdv, cudaStream_t st);
 int multi_scale_size(int h, int w, int input_size, double current_scale, double min_scale, int32_t* size_wh,
                      int32_t* center_xy, double* scale_wh);
 int affine_transform_matrix(const double* center, const double* scale, const int32_t* out_wh, int inverse, double* m);

@@ -78,6 +78,19 @@ struct WarpArgs {
   int oh, ow;
 };
 
+// hpd_prepare_inputs: one (target, image) pair per entry, each with its own output size and optional mirrored output
+struct WarpEntry {
+  WarpImage img;
+  float* out;            // [3,oh,ow] of this image at this target
+  float* out_flipped;    // [3,oh,ow] mirrored in x, or nullptr
+  int oh, ow;
+};
+
+struct WarpTargetsArgs {
+  WarpEntry e[kImagesPerLaunch];
+  float mean[3], stdv[3];
+};
+
 __device__ __forceinline__ int cv_round_sat(double v) {   // saturate_cast<int>(double) = cvRound, half to even
   if (v >= 2147483647.0) return 2147483647;
   if (v <= -2147483648.0) return (-2147483647 - 1);
@@ -90,17 +103,19 @@ constexpr int kWarpRows = 16;   // output rows per block
 // depend on the row alone (X0, Y0) or on the column alone (adelta, bdelta): the first are computed once per block row
 // by 16 threads and shared, the second once per thread, so the per-pixel work is integer arithmetic, four 3-byte taps
 // and three table look-ups (the first version redid eight float64 operations per pixel and was issue-bound at 0.43 TB/s).
-__global__ void __launch_bounds__(256) warp_normalise_kernel(const __grid_constant__ WarpArgs a) {
+// Both input kernels run this body, so their outputs agree bit for bit.  kFlip: every value is also stored at column
+// ow-1-x of out_flipped (torch.flip(x, [3]) of the same tensor, without reading it back).
+template <bool kFlip>
+__device__ __forceinline__ void warp_normalise_block(const WarpImage& I, const float* mean, const float* stdv, float* out,
+                                                     float* out_flipped, int oh, int ow) {
   __shared__ float lut[3][256];
   __shared__ int s_x0[kWarpRows], s_y0[kWarpRows];
   constexpr int AB_SCALE = 1 << kAbBits, ROUND_DELTA = AB_SCALE / (1 << kInterBits) / 2;
-  const int n = blockIdx.z;
-  const WarpImage& I = a.img[n];
   const int y_first = blockIdx.y * kWarpRows;
   for (int i = threadIdx.x; i < 768; i += blockDim.x) {
     const int c = i >> 8, v = i & 255;
     // to_tensor: uint8 -> float32, div(255); normalize: sub_(mean).div_(std)
-    lut[c][v] = __fdiv_rn(__fsub_rn(__fdiv_rn((float)v, 255.0f), a.mean[c]), a.stdv[c]);
+    lut[c][v] = __fdiv_rn(__fsub_rn(__fdiv_rn((float)v, 255.0f), mean[c]), stdv[c]);
   }
   if (threadIdx.x < kWarpRows) {
     const double y = (double)(y_first + threadIdx.x);
@@ -109,14 +124,15 @@ __global__ void __launch_bounds__(256) warp_normalise_kernel(const __grid_consta
   }
   __syncthreads();
   const int x = blockIdx.x * blockDim.x + threadIdx.x;
-  if (x >= a.ow) return;
+  if (x >= ow) return;
   const int adelta = cv_round_sat(__dmul_rn(__dmul_rn(I.im[0], (double)x), (double)AB_SCALE));
   const int bdelta = cv_round_sat(__dmul_rn(__dmul_rn(I.im[3], (double)x), (double)AB_SCALE));
-  const size_t plane = (size_t)a.oh * a.ow;
-  float* o = a.out + (size_t)n * 3 * plane + (size_t)y_first * a.ow + x;
-  const int rows = min(kWarpRows, a.oh - y_first);
+  const size_t plane = (size_t)oh * ow;
+  float* o = out + (size_t)y_first * ow + x;
+  float* of = kFlip ? out_flipped + (size_t)y_first * ow + (ow - 1 - x) : nullptr;
+  const int rows = min(kWarpRows, oh - y_first);
 #pragma unroll 4
-  for (int r = 0; r < rows; ++r, o += a.ow) {
+  for (int r = 0; r < rows; ++r, o += ow) {
     const int X = (s_x0[r] + adelta) >> (kAbBits - kInterBits), Y = (s_y0[r] + bdelta) >> (kAbBits - kInterBits);
     const int sx = min(max(X >> kInterBits, -32768), 32767), sy = min(max(Y >> kInterBits, -32768), 32767);
     const int ax = X & 31, ay = Y & 31;
@@ -130,7 +146,9 @@ __global__ void __launch_bounds__(256) warp_normalise_kernel(const __grid_consta
 #pragma unroll
       for (int c = 0; c < 3; ++c) {
         const int acc = (int)r0[c] * w00 + (int)r0[3 + c] * w01 + (int)r1[c] * w10 + (int)r1[3 + c] * w11;
-        o[(size_t)c * plane] = lut[c][(acc + (1 << (kCoefBits - 1))) >> kCoefBits];     // weights sum to 2^15: in 0..255
+        const float v = lut[c][(acc + (1 << (kCoefBits - 1))) >> kCoefBits];     // weights sum to 2^15: in 0..255
+        o[(size_t)c * plane] = v;
+        if (kFlip) of[(size_t)c * plane] = v;
       }
     } else {
 #pragma unroll
@@ -139,10 +157,47 @@ __global__ void __launch_bounds__(256) warp_normalise_kernel(const __grid_consta
         const int v10 = (y1in && x0in) ? r1[c] : 0, v11 = (y1in && x1in) ? r1[3 + c] : 0;
         const int acc = v00 * w00 + v01 * w01 + v10 * w10 + v11 * w11;
         const int px = min(max((acc + (1 << (kCoefBits - 1))) >> kCoefBits, 0), 255);
-        o[(size_t)c * plane] = lut[c][px];
+        const float v = lut[c][px];
+        o[(size_t)c * plane] = v;
+        if (kFlip) of[(size_t)c * plane] = v;
       }
     }
+    if (kFlip) of += ow;
   }
+}
+
+__global__ void __launch_bounds__(256) warp_normalise_kernel(const __grid_constant__ WarpArgs a) {
+  const int n = blockIdx.z;
+  warp_normalise_block<false>(a.img[n], a.mean, a.stdv, a.out + (size_t)n * 3 * a.oh * a.ow, nullptr, a.oh, a.ow);
+}
+
+// Grid (x, y) covers the largest target of the launch; blocks past their own entry's size leave at once.
+__global__ void __launch_bounds__(256) warp_normalise_targets_kernel(const __grid_constant__ WarpTargetsArgs a) {
+  const WarpEntry& e = a.e[blockIdx.z];
+  if ((int)(blockIdx.x * blockDim.x) >= e.ow || (int)blockIdx.y * kWarpRows >= e.oh) return;
+  if (e.out_flipped)
+    warp_normalise_block<true>(e.img, a.mean, a.stdv, e.out, e.out_flipped, e.oh, e.ow);
+  else
+    warp_normalise_block<false>(e.img, a.mean, a.stdv, e.out, nullptr, e.oh, e.ow);
+}
+
+// cv::warpAffine without WARP_INVERSE_MAP inverts M itself, in this order
+void invert_like_warp_affine(const double* m, double* im) {
+  double M[6];
+  memcpy(M, m, sizeof(M));
+  double D = M[0] * M[4] - M[1] * M[3];
+  D = D != 0 ? 1. / D : 0;
+  const double A11 = M[4] * D, A22 = M[0] * D;
+  M[0] = A11; M[1] *= -D;
+  M[3] *= -D; M[4] = A22;
+  const double b1 = -M[0] * M[2] - M[1] * M[5];
+  const double b2 = -M[3] * M[2] - M[4] * M[5];
+  M[2] = b1; M[5] = b2;
+  memcpy(im, M, sizeof(M));
+}
+
+bool bad_image(const HpdImage& im) {
+  return !im.ptr || im.h < 1 || im.w < 1 || im.h > 32767 || im.w > 32767 || im.stride_row < 3LL * im.w;
 }
 
 }  // namespace
@@ -159,23 +214,12 @@ int launch_prepare_input(const HpdImage* images, int batch, float* out, int oh, 
     memset(&a, 0, sizeof(a));
     for (int i = 0; i < n; ++i) {
       const HpdImage& im = images[b0 + i];
-      if (!im.ptr || im.h < 1 || im.w < 1 || im.h > 32767 || im.w > 32767 || im.stride_row < 3LL * im.w) {
+      if (bad_image(im)) {
         set_error("hpd_prepare_input: image %d: bad pointer / size / stride", b0 + i);
         return HPD_EINVAL;
       }
       a.img[i].ptr = im.ptr; a.img[i].stride_row = im.stride_row; a.img[i].h = im.h; a.img[i].w = im.w;
-      // cv::warpAffine without WARP_INVERSE_MAP inverts M itself, in this order
-      double M[6];
-      memcpy(M, im.m, sizeof(M));
-      double D = M[0] * M[4] - M[1] * M[3];
-      D = D != 0 ? 1. / D : 0;
-      const double A11 = M[4] * D, A22 = M[0] * D;
-      M[0] = A11; M[1] *= -D;
-      M[3] *= -D; M[4] = A22;
-      const double b1 = -M[0] * M[2] - M[1] * M[5];
-      const double b2 = -M[3] * M[2] - M[4] * M[5];
-      M[2] = b1; M[5] = b2;
-      memcpy(a.img[i].im, M, sizeof(M));
+      invert_like_warp_affine(im.m, a.img[i].im);
     }
     for (int c = 0; c < 3; ++c) { a.mean[c] = mean[c]; a.stdv[c] = stdv[c]; }
     a.out = out + (size_t)b0 * 3 * oh * ow;
@@ -184,6 +228,60 @@ int launch_prepare_input(const HpdImage* images, int batch, float* out, int oh, 
     warp_normalise_kernel<<<grid, 256, 0, st>>>(a);
     count_launch();
     if (int rc = check_launch("warp_normalise_kernel")) return rc;
+  }
+  return HPD_OK;
+}
+
+int launch_prepare_inputs(const HpdImage* images, int batch, const HpdPrepareTarget* targets, int n_targets,
+                          const float* mean, const float* stdv, cudaStream_t st) {
+  if (!images || !targets || !mean || !stdv || batch < 1 || n_targets < 1 || n_targets > HPD_MAX_SCALES) {
+    set_error("hpd_prepare_inputs: bad arguments (batch >= 1, 1 <= n_targets <= %d, non-NULL arrays)", HPD_MAX_SCALES);
+    return HPD_EINVAL;
+  }
+  // everything is checked before the first launch: a rejected call enqueues nothing
+  for (int t = 0; t < n_targets; ++t) {
+    const HpdPrepareTarget& T = targets[t];
+    if (!T.out || T.out_h < 1 || T.out_w < 1 || T.out_h > 65535 * kWarpRows) {
+      set_error("hpd_prepare_inputs: target %d: bad output pointer / size", t);
+      return HPD_EINVAL;
+    }
+    if (T.out_flipped == T.out) {
+      set_error("hpd_prepare_inputs: target %d: out_flipped must not be out", t);
+      return HPD_EINVAL;
+    }
+    for (int b = 0; b < batch; ++b) {
+      if (bad_image(images[(size_t)t * batch + b])) {
+        set_error("hpd_prepare_inputs: target %d image %d: bad pointer / size / stride", t, b);
+        return HPD_EINVAL;
+      }
+    }
+  }
+  const long long total = (long long)n_targets * batch;
+  for (long long e0 = 0; e0 < total; e0 += kImagesPerLaunch) {
+    const int n = total - e0 < kImagesPerLaunch ? (int)(total - e0) : kImagesPerLaunch;
+    WarpTargetsArgs a;
+    memset(&a, 0, sizeof(a));
+    int max_h = 0, max_w = 0;
+    for (int i = 0; i < n; ++i) {
+      const long long e = e0 + i;          // entry e = image b of target t, images_host's order
+      const int t = (int)(e / batch), b = (int)(e % batch);
+      const HpdImage& im = images[e];
+      const HpdPrepareTarget& T = targets[t];
+      const size_t img_elems = (size_t)3 * T.out_h * T.out_w;
+      WarpEntry& E = a.e[i];
+      E.img.ptr = im.ptr; E.img.stride_row = im.stride_row; E.img.h = im.h; E.img.w = im.w;
+      invert_like_warp_affine(im.m, E.img.im);
+      E.out = T.out + (size_t)b * img_elems;
+      E.out_flipped = T.out_flipped ? T.out_flipped + (size_t)b * img_elems : nullptr;
+      E.oh = T.out_h; E.ow = T.out_w;
+      max_h = max_h > T.out_h ? max_h : T.out_h;
+      max_w = max_w > T.out_w ? max_w : T.out_w;
+    }
+    for (int c = 0; c < 3; ++c) { a.mean[c] = mean[c]; a.stdv[c] = stdv[c]; }
+    const dim3 grid((max_w + 255) / 256, (max_h + kWarpRows - 1) / kWarpRows, n);
+    warp_normalise_targets_kernel<<<grid, 256, 0, st>>>(a);
+    count_launch();
+    if (int rc = check_launch("warp_normalise_targets_kernel")) return rc;
   }
   return HPD_OK;
 }

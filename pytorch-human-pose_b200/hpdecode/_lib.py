@@ -21,7 +21,7 @@ EXPORTS = (
     "hpd_abi_version", "hpd_last_error_string", "hpd_workspace_bytes", "hpd_aggregate_nms", "hpd_nms",
     "hpd_topk", "hpd_group", "hpd_adjust_refine", "hpd_decode", "hpd_last_launch_count", "hpd_resize_bilinear",
     "hpd_record_layout", "hpd_multi_scale_size", "hpd_get_affine_transform", "hpd_prepare_input", "hpd_prepare_geometry",
-    "hpd_aggregate_tags", "hpd_coco_eval_workspace_bytes", "hpd_coco_eval",
+    "hpd_aggregate_tags", "hpd_coco_eval_workspace_bytes", "hpd_coco_eval", "hpd_prepare_inputs",
 )
 
 
@@ -61,6 +61,11 @@ class HpdRecordLayout(ctypes.Structure):
 class HpdImage(ctypes.Structure):
     _fields_ = [("ptr", ctypes.c_void_p), ("stride_row", ctypes.c_int64), ("h", ctypes.c_int32), ("w", ctypes.c_int32),
                 ("m", ctypes.c_double * 6)]
+
+
+class HpdPrepareTarget(ctypes.Structure):
+    _fields_ = [("out", ctypes.c_void_p), ("out_flipped", ctypes.c_void_p), ("out_h", ctypes.c_int32),
+                ("out_w", ctypes.c_int32)]
 
 
 class HpdCocoEvalParams(ctypes.Structure):
@@ -122,6 +127,8 @@ def lib():
     L.hpd_prepare_geometry.argtypes = [ctypes.c_int, I32P, I32P, ctypes.c_int, ctypes.c_double, ctypes.c_double, I32P, I32P, F64P,
                                        F64P, F64P]
     L.hpd_prepare_input.argtypes = [ctypes.POINTER(HpdImage), ctypes.c_int, V, ctypes.c_int, ctypes.c_int, F32P, F32P, V]
+    L.hpd_prepare_inputs.argtypes = [ctypes.POINTER(HpdImage), ctypes.c_int, ctypes.POINTER(HpdPrepareTarget), ctypes.c_int,
+                                     F32P, F32P, V]
     CP = ctypes.POINTER(HpdCocoEvalParams)
     L.hpd_coco_eval_workspace_bytes.argtypes = [CP, ctypes.POINTER(ctypes.c_size_t)]
     L.hpd_coco_eval.argtypes = [CP, ctypes.POINTER(HpdCocoDets), ctypes.POINTER(HpdCocoGts),

@@ -17,11 +17,15 @@ and decodes each group in one call.  ``test_scales`` enables real multi-scale in
 logic, base/transforms/utils.py:60-97, but only ever calls it with scale 1): heatmaps are averaged over the scales,
 tags come from scale 1.0, everything is projected to the scale-1.0 input frame.
 
+``stream(frames)`` is the path for video and directory inference: frames are batched, uploaded through pinned
+staging, prepared at every test scale (flip-test copy included) in one kernel launch, and several batches are kept in
+flight (hpdecode.stream).
+
 ``autocast_dtype`` (torch.bfloat16 or torch.float16) runs every forward -- flipped run and test scales included --
 under ``torch.autocast("cuda", dtype=...)`` and hands the 16-bit outputs to the decoder as they are: the kernels widen
 them exactly on load, so the result is the float32 decode of the up-cast outputs, without a conversion pass.
 """
-from typing import List, Optional, Sequence
+from typing import Iterable, Iterator, List, Optional, Sequence
 
 import numpy as np
 import torch
@@ -86,22 +90,23 @@ class InferenceKeypointsModel:
 
     # -- batched superset -------------------------------------------------------------------------------------------
     @torch.no_grad()
-    def _net_outputs(self, x: Tensor) -> dict:
+    def _net_outputs(self, x: Tensor, x_flipped: Optional[Tensor] = None) -> dict:
+        """x_flipped: torch.flip(x, [3]) when the caller already has it (prepare_inputs writes it with x)."""
         if self.autocast_dtype is not None:
-            return self._net_outputs_autocast(x)
+            return self._net_outputs_autocast(x, x_flipped)
         (hm_lo, hm_hi), tag = self.net(x)
         scale = {"hm_lo": hm_lo.float(), "hm_hi": hm_hi.float(), "tag": tag.float()}
         if self.use_flip:   # model.py:85-94, fused into the aggregation kernel
-            (fl_lo, fl_hi), fl_tag = self.net(torch.flip(x, [3]))
+            (fl_lo, fl_hi), fl_tag = self.net(torch.flip(x, [3]) if x_flipped is None else x_flipped)
             scale.update(hm_lo_f=fl_lo.float(), hm_hi_f=fl_hi.float(), tag_f=fl_tag.float())
         return scale
 
-    def _net_outputs_autocast(self, x: Tensor) -> dict:
+    def _net_outputs_autocast(self, x: Tensor, x_flipped: Optional[Tensor] = None) -> dict:
         with torch.autocast("cuda", dtype=self.autocast_dtype):
             (hm_lo, hm_hi), tag = self.net(x)
             scale = {"hm_lo": hm_lo, "hm_hi": hm_hi, "tag": tag}
             if self.use_flip:
-                (fl_lo, fl_hi), fl_tag = self.net(torch.flip(x, [3]))
+                (fl_lo, fl_hi), fl_tag = self.net(torch.flip(x, [3]) if x_flipped is None else x_flipped)
                 scale.update(hm_lo_f=fl_lo, hm_hi_f=fl_hi, tag_f=fl_tag)
         # the decoder reads one dtype per call: a net whose head leaves some outputs in float32 under autocast has all
         # of them up-cast (exact), the usual all-16-bit set goes as it is
@@ -144,3 +149,15 @@ class InferenceKeypointsModel:
                     rec, j, raw_images[i], annots[i], inverse_transform(x[j]) if keep_maps else None, self.limbs,
                     self.det_thr, self.tag_thr, **maps)
         return results
+
+    def stream(self, frames: Iterable, batch_size: int = 8, depth: int = 4, records: bool = False) -> Iterator:
+        """Frame-stream inference (video, a directory of images): uint8 [h,w,3] frames (host arrays or CUDA tensors)
+        in, one result per frame out, in input order -- an InferenceKeypointsResult (no maps), or the frame's
+        Records with ``records=True``.  Up to ``batch_size`` frames of one size share a batch, ``depth`` batches are
+        in flight (hpdecode.stream.FrameStream); results are yielded as their batches complete."""
+        from .stream import FrameStream
+        fs = FrameStream(self, batch_size, depth, records)
+        for frame in frames:
+            fs.submit([frame])
+            yield from fs.results(wait=False)
+        yield from fs.results()

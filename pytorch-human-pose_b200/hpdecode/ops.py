@@ -11,10 +11,12 @@ Stage ops mirror the reference methods one to one (paths relative to /root/refer
   hpd::group          MPPEHeatmapParser.match_by_tag grouping.py:85-145 (+ fallback :262-269)
   hpd::adjust_refine  adjust / person score / refine grouping.py:172-191,276,193-250
   hpd::decode         all of the above in one call   (from_preds, results.py:225-238)
+  hpd::prepare_input  resize_align_multi_scale + ToTensor + Normalize  utils.py:89-97, model.py:45-50
+  hpd::prepare_inputs the same for every test scale, plus the flip-test input (model.py:86), in one call
   hpd::coco_eval      pycocotools COCOeval(..., "keypoints").evaluate() + accumulate() (bin/eval.py:52-65)
 """
 import ctypes
-from typing import List, Optional, Sequence
+from typing import List, Optional, Sequence, Tuple
 
 import torch
 from torch import Tensor
@@ -514,6 +516,57 @@ def prepare_input_op(images: Sequence[Tensor], matrices: Tensor, out_h: int, out
     _lib.check(rc, "hpd_prepare_input")
     _count(L)
     return out
+
+
+def _image_descriptors(images: Sequence[Tensor], mats, who: str):
+    """HpdImage array: entry e = images[e % len(images)] with the 2x3 matrix mats[e]."""
+    arr = (HpdImage * len(mats))()
+    for i, t in enumerate(images):
+        if not t.is_cuda or t.dtype != torch.uint8 or t.dim() != 3 or t.shape[2] != 3 or t.stride(2) != 1 or t.stride(1) != 3:
+            raise _lib.HpdError("%s: image %d must be a CUDA uint8 [h,w,3] tensor with packed pixels" % (who, i))
+    for e, m in enumerate(mats):
+        t = images[e % len(images)]
+        arr[e].ptr, arr[e].stride_row, arr[e].h, arr[e].w = t.data_ptr(), t.stride(0), t.shape[0], t.shape[1]
+        for j in range(6):
+            arr[e].m[j] = m[j]
+    return arr
+
+
+@torch.library.custom_op("hpd::prepare_inputs", mutates_args=())
+def prepare_inputs_op(images: Sequence[Tensor], matrices: Tensor, sizes_hw: Sequence[int], flip: bool,
+                      mean: Sequence[float], std: Sequence[float]) -> Tuple[List[Tensor], List[Tensor]]:
+    """``prepare_input`` for every test scale of a batch in ONE library call (hpd_prepare_inputs): uint8 [h,w,3] CUDA
+    images; ``matrices``: float64 [T,B,6] on the HOST (the forward matrix of image b at scale t); ``sizes_hw``: the
+    output (h, w) of each scale, flat [h0, w0, h1, w1, ...].  -> (xs, xs_flipped): T tensors [B,3,h_t,w_t] and, with
+    ``flip``, their mirrored copies (torch.flip(x, [3]), bit for bit), else an empty list."""
+    B = len(images)
+    T = len(sizes_hw) // 2
+    if (B == 0 or T == 0 or len(sizes_hw) % 2 or matrices.is_cuda or matrices.dtype != torch.float64
+            or matrices.numel() != 6 * T * B):
+        raise _lib.HpdError("prepare_inputs: need >= 1 image, (h, w) per scale and a host float64 [T,B,6] matrix tensor")
+    dev = images[0].device
+    arr = _image_descriptors(images, matrices.reshape(-1, 6).tolist(), "prepare_inputs")
+    xs = [torch.empty((B, 3, sizes_hw[2 * t], sizes_hw[2 * t + 1]), device=dev, dtype=torch.float32) for t in range(T)]
+    xs_f = [torch.empty_like(x) for x in xs] if flip else []
+    targets = (_lib.HpdPrepareTarget * T)()
+    for t in range(T):
+        targets[t].out, targets[t].out_h, targets[t].out_w = xs[t].data_ptr(), sizes_hw[2 * t], sizes_hw[2 * t + 1]
+        targets[t].out_flipped = xs_f[t].data_ptr() if flip else None
+    mean_c, std_c = (ctypes.c_float * 3)(*mean), (ctypes.c_float * 3)(*std)
+    L = _lib.lib()
+    with torch.cuda.device(dev):
+        rc = L.hpd_prepare_inputs(arr, B, targets, T, mean_c, std_c, _stream_ptr(dev))
+    _lib.check(rc, "hpd_prepare_inputs")
+    _count(L)
+    return xs, xs_f
+
+
+@prepare_inputs_op.register_fake
+def _(images, matrices, sizes_hw, flip, mean, std):
+    B = len(images)
+    xs = [images[0].new_empty((B, 3, sizes_hw[2 * t], sizes_hw[2 * t + 1]), dtype=torch.float32)
+          for t in range(len(sizes_hw) // 2)]
+    return xs, ([torch.empty_like(x) for x in xs] if flip else [])
 
 
 @torch.library.custom_op("hpd::coco_eval", mutates_args=())

@@ -1,0 +1,203 @@
+"""Frame-stream inference: uint8 frames in, one result per frame out, several batches in flight on the device.
+
+The reference's directory and video callers (bin/inference.py:49-114, base/datasets/video.py:142-176) run
+``model(frame)`` once per frame, each call ending in a synchronising device->host copy.  ``FrameStream`` batches the
+frames instead and keeps ``depth`` batches in flight (``DecodePipeline`` lanes); per batch, on the lane's stream:
+
+1. host frames are copied into the lane's pinned staging slot at ``submit`` and uploaded on a stream of their own;
+   an event orders the upload before the lane's work (CUDA frames are read where they are);
+2. ``hpd_prepare_inputs``: the network input of every test scale and, with the flip test, its mirrored copy, in one
+   launch (``prepare_input`` + ``torch.flip`` per scale, bit for bit);
+3. the network, once per scale and run, under the model's autocast setting (``InferenceKeypointsModel._net_outputs``);
+4. the decode with the scale-1.0 inverse matrices, so the records carry raw-frame coordinates;
+5. one device->host copy of the batch's records into the lane's pinned records slot.
+
+A lane and its staging slot are reused only after the host has waited for that lane's records copy (an event, not a
+device synchronise).  A batch closes when it is full or when the frame size changes, so frames of mixed sizes work;
+results come back in submission order either way.  Geometry is computed once per distinct frame size.
+
+The stream decodes into the model decoder's buffer sets (slot = lane): do not call the model's other entry points
+while a stream still has batches in flight (``results()`` drains it).
+"""
+from collections import OrderedDict, deque
+from typing import Iterable, Iterator, List
+
+import numpy as np
+import torch
+
+from . import _lib, geometry, ops
+from .decoder import DecodePipeline, Records
+from .results import InferenceKeypointsResult
+
+
+class FrameStream:
+    """``submit(frames)`` any number of times, then iterate ``results()`` (or the stream itself) for one result per
+    frame in submission order: an InferenceKeypointsResult (no maps, like ``predict_batch``) or, with
+    ``records=True``, the frame's ``Records`` (one row).  Frames are uint8 [h,w,3] NumPy arrays or CUDA tensors."""
+
+    MAX_SIZES = 64    # distinct frame sizes whose geometry is kept
+
+    def __init__(self, model, batch_size: int = 8, depth: int = 4, records: bool = False):
+        if batch_size < 1 or depth < 1:
+            raise ValueError(f"batch_size and depth must be >= 1 (got {batch_size}, {depth})")
+        self.model, self.batch_size, self.depth, self.records = model, int(batch_size), int(depth), records
+        self._open: list = []           # frames of the batch being filled
+        self._open_hw = None
+        self._inflight = deque()        # launched batches, oldest first
+        self._done = deque()            # finished per-frame results not yet handed out
+        self._geom = OrderedDict()      # (h, w) -> geometry of that frame size
+        self.geometry_calls = 0
+        self._init_device()
+
+    # ---- batching -----------------------------------------------------------------------------------------------
+    def submit(self, frames: Iterable):
+        for f in frames:
+            hw = self._frame_hw(f)
+            if self._open and hw != self._open_hw:
+                self._close()                            # one batch is one network input shape
+            if not self._open:
+                while len(self._inflight) >= self.depth:  # the lane this batch takes must have been consumed
+                    self._retire()
+                self._open_hw = hw
+            self._stage(f, len(self._open))
+            self._open.append(f)
+            if len(self._open) == self.batch_size:
+                self._close()
+
+    def results(self, wait: bool = True) -> Iterator:
+        """Finished results in submission order.  wait=True: closes the open batch and waits for everything
+        submitted so far; wait=False: hands out only batches whose records have arrived, without blocking."""
+        if wait and self._open:
+            self._close()
+        while self._inflight and (wait or self._ready(self._inflight[0])):
+            self._retire()
+        while self._done:
+            yield self._done.popleft()
+
+    __iter__ = results
+
+    def _close(self):
+        self._inflight.append(self._launch(self._open, self._open_hw))
+        self._open = []
+
+    def _retire(self):
+        self._done.extend(self._finish(self._inflight.popleft()))
+
+    @staticmethod
+    def _frame_hw(f):
+        if isinstance(f, torch.Tensor):
+            ok = f.is_cuda and f.dtype == torch.uint8 and f.dim() == 3 and f.shape[2] == 3 and f.stride(2) == 1 and f.stride(1) == 3
+        else:
+            ok = isinstance(f, np.ndarray) and f.dtype == np.uint8 and f.ndim == 3 and f.shape[2] == 3
+        if not ok:
+            raise _lib.HpdError("FrameStream: a frame is a uint8 [h,w,3] NumPy array or CUDA tensor (packed pixels)")
+        return int(f.shape[0]), int(f.shape[1])
+
+    def _geometry(self, hw, n):
+        """(sizes_hw per scale, host forward matrices [T,n,6], device scale-1.0 inverse matrices [n,6])."""
+        g = self._geom.get(hw)
+        if g is None:
+            m = self.model
+            sizes_hw, fwd, (_, _, inv) = geometry.multi_scale_geometry([hw], m.input_size, m.test_scales)
+            self.geometry_calls += 1
+            while len(self._geom) >= self.MAX_SIZES:
+                self._geom.popitem(last=False)
+            g = self._geom[hw] = {"sizes_hw": sizes_hw, "fwd": fwd, "inv": inv, "per_n": {}}
+        else:
+            self._geom.move_to_end(hw)
+        per_n = g["per_n"].get(n)
+        if per_n is None:
+            per_n = g["per_n"][n] = (torch.from_numpy(np.repeat(g["fwd"], n, axis=1)),
+                                     torch.from_numpy(np.repeat(g["inv"], n, axis=0)).to(self.device))
+        return (g["sizes_hw"],) + per_n
+
+    # ---- device work ----------------------------------------------------------------------------------------------
+    def _init_device(self):
+        if not torch.cuda.is_available():
+            raise _lib.HpdError("hpdecode needs a CUDA device (sm_100a); there is no CPU fallback")
+        m = self.model
+        self.device = torch.device(m.device)
+        self.pipe = DecodePipeline(m.decoder, self.depth)
+        self._upload = torch.cuda.Stream(device=self.device)
+        self._tag_scale = m.test_scales.index(1.0)
+        K, M, E = m.decoder.num_kpts, m.decoder.max_num_people, 2 if m.use_flip else 1
+        self._rec_shape = (M, K, E)
+        row_bytes = ops.record_layout(K, M, E).row_bytes
+        self._host_rec = torch.empty((self.depth, self.batch_size, row_bytes), dtype=torch.uint8, pin_memory=True)
+        self._pinned: List = [None] * self.depth       # per lane: host frames of the batch, pinned
+        self._staged: List = [None] * self.depth       # per lane: their device copy
+        self._shape_only = {}
+
+    def _stage(self, f, i):
+        lane = self.pipe._next          # the lane the open batch will be submitted on
+        if isinstance(f, torch.Tensor):
+            if f.device != self.device:
+                raise _lib.HpdError(f"FrameStream: frame on {f.device}, model on {self.device}")
+            return
+        h, w = self._open_hw
+        need = self.batch_size * h * w * 3
+        if self._pinned[lane] is None or self._pinned[lane].numel() < need:
+            self._pinned[lane] = torch.empty((need,), dtype=torch.uint8, pin_memory=True)
+            self._staged[lane] = torch.empty((need,), dtype=torch.uint8, device=self.device)
+        np.copyto(self._pinned[lane].numpy()[i * h * w * 3:(i + 1) * h * w * 3].reshape(h, w, 3), f)
+
+    def _placeholders(self, n):
+        """DecodePipeline.submit reads the batch size and the flip test from its ``scales`` argument; the network
+        outputs themselves come from before_agg."""
+        s = self._shape_only.get(n)
+        if s is None:
+            e = torch.empty((n, 0, 0, 0), device=self.device)
+            one = {"hm_lo": e, "hm_hi": e, "tag": e}
+            if self.model.use_flip:
+                one.update(hm_lo_f=e, hm_hi_f=e, tag_f=e)
+            s = self._shape_only[n] = [one] * len(self.model.test_scales)
+        return s
+
+    def _launch(self, frames, hw):
+        m = self.model
+        lane, n, (h, w) = self.pipe._next, len(frames), hw
+        sizes_hw, fwd, inv = self._geometry(hw, n)
+        upload_done = None
+        if any(not isinstance(f, torch.Tensor) for f in frames):
+            self._upload.wait_stream(torch.cuda.current_stream(self.device))   # staging memory may be fresh
+            with torch.cuda.stream(self._upload):
+                nb = n * h * w * 3
+                self._staged[lane][:nb].copy_(self._pinned[lane][:nb], non_blocking=True)
+                upload_done = torch.cuda.Event()
+                upload_done.record()
+        stage = self._staged[lane]
+        imgs = [f if isinstance(f, torch.Tensor) else stage[i * h * w * 3:(i + 1) * h * w * 3].view(h, w, 3)
+                for i, f in enumerate(frames)]
+
+        def before_agg(ln):
+            st = torch.cuda.current_stream(self.device)
+            if upload_done is not None:
+                st.wait_event(upload_done)
+            for f in frames:
+                if isinstance(f, torch.Tensor):
+                    f.record_stream(st)
+            xs, xs_f = torch.ops.hpd.prepare_inputs(imgs, fwd, sizes_hw, m.use_flip, list(geometry.MEAN),
+                                                    list(geometry.STD))
+            return [m._net_outputs(x, xs_f[t] if m.use_flip else None) for t, x in enumerate(xs)]
+
+        def after_tail(ln, res):
+            self._host_rec[lane][:n].copy_(res.records, non_blocking=True)
+
+        ts = self._tag_scale
+        res = self.pipe.submit(self._placeholders(n), (sizes_hw[2 * ts], sizes_hw[2 * ts + 1]), tag_scale=ts,
+                               before_agg=before_agg, after_tail=after_tail, inv_affine=inv)
+        return lane, frames, res        # res keeps the lane's buffer set alive until the batch is retired
+
+    def _ready(self, batch) -> bool:
+        return batch[2].ready.query()
+
+    def _finish(self, batch) -> list:
+        lane, frames, res = batch
+        res.ready.synchronize()
+        raw = self._host_rec[lane][:len(frames)].numpy().copy()
+        M, K, E = self._rec_shape
+        if self.records:
+            return [Records(raw[b:b + 1], M, K, E) for b in range(len(frames))]
+        m, rec = self.model, Records(raw, M, K, E)
+        return [InferenceKeypointsResult.from_records(rec, b, f, None, None, m.limbs, m.det_thr, m.tag_thr)
+                for b, f in enumerate(frames)]
