@@ -75,6 +75,20 @@ typedef struct HpdScaleInputs {
   HpdMap hm_lo_f, hm_hi_f, tag_f;   /* flipped run; ptr == NULL when flip test is off */
 } HpdScaleInputs;
 
+/* Raw network outputs for one test scale, for a head with 1 to HPD_MAX_STAGES heatmap stages (results.py:46-54,226
+ * take them as a list): HRNet with the associative-embedding head and no deconvolution gives one stage at S/4,
+ * HigherHRNet two (S/4, S/2), HigherHRNet with two deconvolution modules three (S/4, S/2, S).  Every stage is flip
+ * averaged, stages 0..n-2 are resized to the last stage's size, and their mean ((U_0 + U_1) + ...) / n is taken
+ * there.  HpdScaleInputs is the two-stage case: {hm = {hm_lo, hm_hi}, num_stages = 2}. */
+#define HPD_MAX_STAGES 4
+typedef struct HpdStageInputs {
+  HpdMap hm[HPD_MAX_STAGES];    /* heatmap stages in the network's order; the mean is taken at hm[num_stages-1]'s size */
+  HpdMap hm_f[HPD_MAX_STAGES];  /* flipped run; ptr NULL when the flip test is off */
+  HpdMap tag, tag_f;            /* as in HpdScaleInputs */
+  int32_t num_stages;           /* 1..HPD_MAX_STAGES */
+  int32_t reserved_;
+} HpdStageInputs;
+
 typedef struct HpdParams {
   int32_t batch;        /* B images per call */
   int32_t num_kpts;     /* K <= HPD_MAX_KPTS */
@@ -229,6 +243,12 @@ HPD_EXPORT int hpd_workspace_bytes(const HpdParams* p, size_t* out_bytes);
  * hpd_aggregate_tags launches (hpd_last_launch_count() is then one higher). */
 HPD_EXPORT int hpd_aggregate_nms(const HpdParams* p, const HpdScaleInputs* scales, const HpdBuffers* buf, void* stream);
 
+/* hpd_aggregate_nms for heads with 1..HPD_MAX_STAGES heatmap stages per scale (HpdStageInputs).  hpd_aggregate_nms is
+ * this call with two stages.  Flipped maps are given for every stage of every scale or for none, each with its stage's
+ * shape; all maps share one dtype.  Everything is checked before the first launch. */
+HPD_EXPORT int hpd_aggregate_nms_stages(const HpdParams* p, const HpdStageInputs* scales, const HpdBuffers* buf,
+                                        void* stream);
+
 /* The tag half of hpd_aggregate_nms alone (results.py:229-230), for callers that decoded with agg_tags == NULL and
  * want the map after all: reads the tag / tag_f maps of scales[tag_scale]; writes out [B,K,H,W,E].  It is the one
  * producer of the map: hpd_aggregate_nms and hpd_decode fill agg_tags with the same kernel. */
@@ -269,6 +289,11 @@ HPD_EXPORT int hpd_adjust_refine(const HpdParams* p, const HpdBuffers* buf, void
  * more) and the tag stages read it. */
 HPD_EXPORT int hpd_decode(const HpdParams* p, const HpdScaleInputs* scales, const HpdBuffers* buf, void* workspace,
                size_t workspace_bytes, void* stream);
+
+/* hpd_decode over HpdStageInputs (1..HPD_MAX_STAGES heatmap stages per scale); hpd_decode is this call with two
+ * stages.  The tag stages read the tag / tag_f maps of scales[tag_scale] as hpd_decode's do. */
+HPD_EXPORT int hpd_decode_stages(const HpdParams* p, const HpdStageInputs* scales, const HpdBuffers* buf, void* workspace,
+                                 size_t workspace_bytes, void* stream);
 
 /* Offsets and size of the per-image result record for these params (num_kpts, max_people, emb). */
 HPD_EXPORT int hpd_record_layout(const HpdParams* p, HpdRecordLayout* out);

@@ -36,11 +36,20 @@ constexpr int OT_R = TH + 2 * HALO, OT_C = TW + 2 * HALO;
 constexpr int kAggThreads = 256;
 
 struct ScaleDev {
-  const float *lo, *hi, *lo_f, *hi_f;
+  const float *lo, *hi, *lo_f, *hi_f;   // first and last heatmap stage (the same map for a single-stage head)
   long long lo_sb, lo_sc, hi_sb, hi_sc, lof_sb, lof_sc, hif_sb, hif_sc;
   int lh, lw, hh, hw;
   float s_lo_y, s_lo_x;  // lo -> hi   ( (float)lh / hh )
   float s_hi_y, s_hi_x;  // hi -> out
+};
+
+// One heatmap stage of one scale (the un-flipped and, with the flip test, the flipped-run map) as the generic kernel
+// reads it.
+struct StageDev {
+  const float *p, *pf;
+  long long sb, sc, fsb, fsc;
+  int h, w;
+  float s_y, s_x;        // this stage -> the last stage
 };
 
 struct AggArgs {
@@ -63,7 +72,19 @@ struct AggArgs {
   int in_vec_ok;   // inputs allow 16-byte loads (aligned bases, strides multiples of 4 elements)
   int in_vec_ok_all;   // ... for every scale
   int dtype;       // HPD_F32 / HPD_F16 / HPD_BF16: the const float* input members point at elements of this type
+  // Heads with other than two heatmap stages (generic kernel only; the specialised kernels read sc[] alone, whose
+  // layout is unchanged): stages per scale, and the stages between the first (sc[].lo) and the last (sc[].hi).
+  int n_stages[HPD_MAX_SCALES];
+  StageDev mid[HPD_MAX_SCALES][HPD_MAX_STAGES - 2];
 };
+
+// Stage i of scale s: sc[s].lo, mid[s][i-1] or sc[s].hi.
+__device__ __forceinline__ StageDev stage_of(const AggArgs& a, int s, int i) {
+  const ScaleDev& S = a.sc[s];
+  if (i == a.n_stages[s] - 1) return StageDev{S.hi, S.hi_f, S.hi_sb, S.hi_sc, S.hif_sb, S.hif_sc, S.hh, S.hw, 1.f, 1.f};
+  if (i == 0) return StageDev{S.lo, S.lo_f, S.lo_sb, S.lo_sc, S.lof_sb, S.lof_sc, S.lh, S.lw, S.s_lo_y, S.s_lo_x};
+  return a.mid[s][i - 1];
+}
 
 // ---------------------------------------------------------------------------------------------
 // NMS on a (TH+4)x(TW+4) tile already in shared memory (pixels outside the image hold -inf).
@@ -155,11 +176,12 @@ __global__ void __launch_bounds__(kAggThreads) agg_nms_generic_kernel(const AggA
 
   for (int s = 0; s < a.n_scales; ++s) {
     const ScaleDev& S = a.sc[s];
+    const int ns = a.n_stages[s];
     const int hxa = axis_tap(S.s_hi_x, oxa, S.hw, W).i0, hxb = axis_tap(S.s_hi_x, oxb, S.hw, W).i1;
     const int hya = axis_tap(S.s_hi_y, oya, S.hh, H).i0, hyb = axis_tap(S.s_hi_y, oyb, S.hh, H).i1;
-    const int lxa = axis_tap(S.s_lo_x, hxa, S.lw, S.hw).i0, lxb = axis_tap(S.s_lo_x, hxb, S.lw, S.hw).i1;
-    const int lya = axis_tap(S.s_lo_y, hya, S.lh, S.hh).i0, lyb = axis_tap(S.s_lo_y, hyb, S.lh, S.hh).i1;
-    const int nhx = hxb - hxa + 1, nhy = hyb - hya + 1, nlx = lxb - lxa + 1, nly = lyb - lya + 1;
+    const int nhx = hxb - hxa + 1, nhy = hyb - hya + 1;
+    const int per = min(nhx, kAggThreads), groups = kAggThreads / per;   // last-stage tile: column-owned passes
+    const int rg = tid / per;
 
     for (int i = tid; i < OT_C; i += kAggThreads) {
       const int ox = x0 - HALO + i;
@@ -179,55 +201,38 @@ __global__ void __launch_bounds__(kAggThreads) agg_nms_generic_kernel(const AggA
         or_i0[i] = -1;
       }
     }
-    for (int i = tid; i < nhx; i += kAggThreads) {
-      const Tap t = axis_tap(S.s_lo_x, hxa + i, S.lw, S.hw);
-      hc_i0[i] = t.i0 - lxa; hc_i1[i] = t.i1 - lxa; hc_w0[i] = t.w0; hc_w1[i] = t.w1;
-    }
-    for (int i = tid; i < nhy; i += kAggThreads) {
-      const Tap t = axis_tap(S.s_lo_y, hya + i, S.lh, S.hh);
-      hr_i0[i] = t.i0 - lya; hr_i1[i] = t.i1 - lya; hr_w0[i] = t.w0; hr_w1[i] = t.w1;
-    }
-    // flip-averaged low-resolution tile (model.py:90)
-    {
-      const size_t po = (size_t)b * S.lo_sb + (size_t)k * S.lo_sc, pfo = (size_t)b * S.lof_sb + (size_t)kf * S.lof_sc;
-      const float* p = S.lo;
-      const float* pf = S.lo_f;
-      const int per = min(nlx, kAggThreads), groups = kAggThreads / per;
-      const int rg = tid / per;
-      if (rg < groups)
-        for (int c = tid % per; c < nlx; c += per) {
-          const int x = lxa + c;
-          for (int r = rg; r < nly; r += groups) {
-            const int rowo = (lya + r) * S.lw;
-            float v = in_elem(p, po + rowo + x, a.dtype);
-            if (pf) v = __fmul_rn(__fadd_rn(v, in_elem(pf, pfo + rowo + (S.lw - 1 - x), a.dtype)), 0.5f);
-            loT[r * a.LO_C + c] = v;
+    // stages 0..ns-2: flip-averaged tile (model.py:90) resized to the last stage (results.py:46-54) and summed
+    // into hiT in stage order (results.py:226: torch.stack(...).mean(0) sums sequentially)
+    for (int si = 0; si + 1 < ns; ++si) {
+      const StageDev St = stage_of(a, s, si);
+      const int lxa = axis_tap(St.s_x, hxa, St.w, S.hw).i0, lxb = axis_tap(St.s_x, hxb, St.w, S.hw).i1;
+      const int lya = axis_tap(St.s_y, hya, St.h, S.hh).i0, lyb = axis_tap(St.s_y, hyb, St.h, S.hh).i1;
+      const int nlx = lxb - lxa + 1, nly = lyb - lya + 1;
+      for (int i = tid; i < nhx; i += kAggThreads) {
+        const Tap t = axis_tap(St.s_x, hxa + i, St.w, S.hw);
+        hc_i0[i] = t.i0 - lxa; hc_i1[i] = t.i1 - lxa; hc_w0[i] = t.w0; hc_w1[i] = t.w1;
+      }
+      for (int i = tid; i < nhy; i += kAggThreads) {
+        const Tap t = axis_tap(St.s_y, hya + i, St.h, S.hh);
+        hr_i0[i] = t.i0 - lya; hr_i1[i] = t.i1 - lya; hr_w0[i] = t.w0; hr_w1[i] = t.w1;
+      }
+      {
+        const size_t po = (size_t)b * St.sb + (size_t)k * St.sc, pfo = (size_t)b * St.fsb + (size_t)kf * St.fsc;
+        const int lper = min(nlx, kAggThreads), lgroups = kAggThreads / lper;
+        const int lrg = tid / lper;
+        if (lrg < lgroups)
+          for (int c = tid % lper; c < nlx; c += lper) {
+            const int x = lxa + c;
+            for (int r = lrg; r < nly; r += lgroups) {
+              const int rowo = (lya + r) * St.w;
+              float v = in_elem(St.p, po + rowo + x, a.dtype);
+              if (St.pf) v = __fmul_rn(__fadd_rn(v, in_elem(St.pf, pfo + rowo + (St.w - 1 - x), a.dtype)), 0.5f);
+              loT[r * a.LO_C + c] = v;
+            }
           }
-        }
-    }
-    {
-      const size_t po = (size_t)b * S.hi_sb + (size_t)k * S.hi_sc, pfo = (size_t)b * S.hif_sb + (size_t)kf * S.hif_sc;
-      const float* p = S.hi;
-      const float* pf = S.hi_f;
-      const int per = min(nhx, kAggThreads), groups = kAggThreads / per;
-      const int rg = tid / per;
-      if (rg < groups)
-        for (int c = tid % per; c < nhx; c += per) {
-          const int x = hxa + c;
-          for (int r = rg; r < nhy; r += groups) {
-            const int rowo = (hya + r) * S.hw;
-            float v = in_elem(p, po + rowo + x, a.dtype);
-            if (pf) v = __fmul_rn(__fadd_rn(v, in_elem(pf, pfo + rowo + (S.hw - 1 - x), a.dtype)), 0.5f);
-            hiT[r * a.HI_C + c] = v;
-          }
-        }
-    }
-    __syncthreads();
-    // stage mean at the high stage's resolution (results.py:225-226), in place.  A thread owns one column
-    // (its taps stay in registers) and strides over the rows.
-    {
-      const int per = min(nhx, kAggThreads), groups = kAggThreads / per;
-      const int rg = tid / per;
+      }
+      __syncthreads();
+      // A thread owns one column (its taps stay in registers) and strides over the rows.
       if (rg < groups)
         for (int c = tid % per; c < nhx; c += per) {
           const int c0 = hc_i0[c], c1 = hc_i1[c];
@@ -236,7 +241,25 @@ __global__ void __launch_bounds__(kAggThreads) agg_nms_generic_kernel(const AggA
             const float* r0 = loT + hr_i0[r] * a.LO_C;
             const float* r1 = loT + hr_i1[r] * a.LO_C;
             const float up = lerp2(cw0, cw1, hr_w0[r], hr_w1[r], r0[c0], r0[c1], r1[c0], r1[c1]);
-            hiT[r * a.HI_C + c] = __fmul_rn(__fadd_rn(up, hiT[r * a.HI_C + c]), 0.5f);
+            hiT[r * a.HI_C + c] = si == 0 ? up : __fadd_rn(hiT[r * a.HI_C + c], up);
+          }
+        }
+      __syncthreads();   // loT and the hc / hr taps are rewritten by the next stage
+    }
+    // last stage, flip-averaged, ends the sum; the stage mean divides by ns (two stages: exactly today's * 0.5)
+    {
+      const StageDev St = stage_of(a, s, ns - 1);
+      const size_t po = (size_t)b * St.sb + (size_t)k * St.sc, pfo = (size_t)b * St.fsb + (size_t)kf * St.fsc;
+      const float nst = (float)ns;
+      if (rg < groups)
+        for (int c = tid % per; c < nhx; c += per) {
+          const int x = hxa + c;
+          for (int r = rg; r < nhy; r += groups) {
+            const int rowo = (hya + r) * St.w;
+            float v = in_elem(St.p, po + rowo + x, a.dtype);
+            if (St.pf) v = __fmul_rn(__fadd_rn(v, in_elem(St.pf, pfo + rowo + (St.w - 1 - x), a.dtype)), 0.5f);
+            if (ns > 1) v = __fdiv_rn(__fadd_rn(hiT[r * a.HI_C + c], v), nst);
+            hiT[r * a.HI_C + c] = v;
           }
         }
     }
@@ -295,6 +318,7 @@ __global__ void __launch_bounds__(kAggThreads) agg_nms_generic_kernel(const AggA
 }  // namespace hpd
 namespace hpd {
 #include "aggregate_nms_x2.cuh"
+#include "aggregate_nms_x4.cuh"
 #include "aggregate_nms_ms.cuh"
 }  // namespace hpd
 namespace hpd {
@@ -443,8 +467,14 @@ int launch_aggregate_tags(const HpdParams* p, const HpdScaleInputs* scales, floa
 
 namespace {
 
+// Name of stage i of an n-stage scale in error messages: two stages are HigherHRNet's hm_lo / hm_hi.
+const char* stage_name(int n, int i) {
+  static const char* any[HPD_MAX_STAGES] = {"hm[0]", "hm[1]", "hm[2]", "hm[3]"};
+  return n == 2 ? (i == 0 ? "hm_lo" : "hm_hi") : any[i];
+}
+
 // The aggregation + NMS kernel alone: agg_hm, the word side arrays and the tag bounds.
-int launch_aggregation_kernel(const HpdParams* p, const HpdScaleInputs* scales, const HpdBuffers* buf, cudaStream_t st) {
+int launch_aggregation_kernel(const HpdParams* p, const HpdStageInputs* scales, const HpdBuffers* buf, cudaStream_t st) {
   if (!scales || !buf->agg_hm || !buf->nms_mask || !buf->nms_wmax || !buf->hm_wmax || !buf->tag_bmin || !buf->tag_bmax) {
     set_error("hpd_aggregate_nms: scales, agg_hm, nms_mask, nms_wmax, hm_wmax, tag_bmin, tag_bmax are required");
     return HPD_EINVAL;
@@ -455,46 +485,73 @@ int launch_aggregation_kernel(const HpdParams* p, const HpdScaleInputs* scales, 
   a.B = p->batch; a.K = p->num_kpts; a.H = p->out_h; a.W = p->out_w;
   a.wpr = (p->out_w + 31) / 32;
   for (int k = 0; k < HPD_MAX_KPTS; ++k) a.flip[k] = p->flip_index[k];
-  const bool flip = scales[0].hm_lo_f.ptr != nullptr;
-  const int dtype = scales[0].hm_lo.dtype;
+  const bool flip = scales[0].hm_f[0].ptr != nullptr;
+  const int dtype = scales[0].hm[0].dtype;
   a.dtype = dtype;
   const uintptr_t vec_align = dtype == HPD_F32 ? 16 : 8;    // four elements per vector load
   int LO_R = 1, LO_C = 1, HI_R = 1, HI_C = 1;
   for (int s = 0; s < p->num_scales; ++s) {
-    const HpdScaleInputs& in = scales[s];
+    const HpdStageInputs& in = scales[s];
+    const int ns = in.num_stages;
+    if (ns < 1 || ns > HPD_MAX_STAGES) {
+      set_error("num_stages must be in [1,%d] (got %d)", HPD_MAX_STAGES, ns);
+      return HPD_EINVAL;
+    }
     int rc;
-    if ((rc = check_map(in.hm_lo, "hm_lo", true)) || (rc = check_map(in.hm_hi, "hm_hi", true))) return rc;
-    for (const HpdMap* m : {&in.hm_lo, &in.hm_hi, &in.tag, &in.hm_lo_f, &in.hm_hi_f, &in.tag_f}) {
-      if (m->ptr != nullptr && m->dtype != dtype) {
-        set_error("all maps of a call must share one dtype");
+    for (int i = 0; i < ns; ++i)
+      if ((rc = check_map(in.hm[i], stage_name(ns, i), true))) return rc;
+    for (int i = 0; i < ns + 2; ++i) {
+      const HpdMap* pair[2] = {i < ns ? &in.hm[i] : (i == ns ? &in.tag : &in.tag_f),
+                               i < ns ? &in.hm_f[i] : (i == ns ? &in.tag : &in.tag_f)};
+      for (const HpdMap* m : pair)
+        if (m->ptr != nullptr && m->dtype != dtype) {
+          set_error("all maps of a call must share one dtype");
+          return HPD_EINVAL;
+        }
+    }
+    for (int i = 0; i < ns; ++i)
+      if (flip != (in.hm_f[i].ptr != nullptr)) {
+        set_error("flip inputs must be given for all stages and scales or for none");
         return HPD_EINVAL;
       }
-    }
-    if (flip != (in.hm_lo_f.ptr != nullptr) || flip != (in.hm_hi_f.ptr != nullptr)) {
-      set_error("flip inputs must be given for all stages and scales or for none");
-      return HPD_EINVAL;
-    }
-    if (flip && (in.hm_lo_f.h != in.hm_lo.h || in.hm_lo_f.w != in.hm_lo.w || in.hm_hi_f.h != in.hm_hi.h ||
-                 in.hm_hi_f.w != in.hm_hi.w)) {
-      set_error("flipped-run maps must have the shapes of the un-flipped run");
-      return HPD_EINVAL;
-    }
+    for (int i = 0; flip && i < ns; ++i)
+      if (in.hm_f[i].h != in.hm[i].h || in.hm_f[i].w != in.hm[i].w) {
+        set_error("flipped-run maps must have the shapes of the un-flipped run");
+        return HPD_EINVAL;
+      }
     ScaleDev& S = a.sc[s];
-    S.lo = (const float*)in.hm_lo.ptr; S.lo_sb = in.hm_lo.stride_b; S.lo_sc = in.hm_lo.stride_c;
-    S.hi = (const float*)in.hm_hi.ptr; S.hi_sb = in.hm_hi.stride_b; S.hi_sc = in.hm_hi.stride_c;
-    S.lo_f = (const float*)in.hm_lo_f.ptr; S.lof_sb = in.hm_lo_f.stride_b; S.lof_sc = in.hm_lo_f.stride_c;
-    S.hi_f = (const float*)in.hm_hi_f.ptr; S.hif_sb = in.hm_hi_f.stride_b; S.hif_sc = in.hm_hi_f.stride_c;
-    S.lh = in.hm_lo.h; S.lw = in.hm_lo.w; S.hh = in.hm_hi.h; S.hw = in.hm_hi.w;
+    const HpdMap &lo = in.hm[0], &hi = in.hm[ns - 1], &lof = in.hm_f[0], &hif = in.hm_f[ns - 1];
+    S.lo = (const float*)lo.ptr; S.lo_sb = lo.stride_b; S.lo_sc = lo.stride_c;
+    S.hi = (const float*)hi.ptr; S.hi_sb = hi.stride_b; S.hi_sc = hi.stride_c;
+    S.lo_f = (const float*)lof.ptr; S.lof_sb = lof.stride_b; S.lof_sc = lof.stride_c;
+    S.hi_f = (const float*)hif.ptr; S.hif_sb = hif.stride_b; S.hif_sc = hif.stride_c;
+    S.lh = lo.h; S.lw = lo.w; S.hh = hi.h; S.hw = hi.w;
     S.s_lo_y = (float)S.lh / (float)S.hh; S.s_lo_x = (float)S.lw / (float)S.hw;
     S.s_hi_y = (float)S.hh / (float)a.H; S.s_hi_x = (float)S.hw / (float)a.W;
-    int me, ie;
-    axis_extents(a.W, TW, HALO, S.hw, S.s_hi_x, S.lw, S.s_lo_x, &me, &ie);
-    HI_C = me > HI_C ? me : HI_C; LO_C = ie > LO_C ? ie : LO_C;
-    axis_extents(a.H, TH, HALO, S.hh, S.s_hi_y, S.lh, S.s_lo_y, &me, &ie);
-    HI_R = me > HI_R ? me : HI_R; LO_R = ie > LO_R ? ie : LO_R;
+    a.n_stages[s] = ns;
+    StageDev st[HPD_MAX_STAGES];
+    for (int i = 0; i < ns; ++i) {
+      StageDev& D = st[i];
+      const HpdMap &m = in.hm[i], &mf = in.hm_f[i];
+      D.p = (const float*)m.ptr; D.sb = m.stride_b; D.sc = m.stride_c;
+      D.pf = (const float*)mf.ptr; D.fsb = mf.stride_b; D.fsc = mf.stride_c;
+      D.h = m.h; D.w = m.w;
+      D.s_y = (float)D.h / (float)S.hh; D.s_x = (float)D.w / (float)S.hw;
+      if (i > 0 && i < ns - 1) a.mid[s][i - 1] = D;
+    }
+    for (int i = 0; i < (ns > 1 ? ns - 1 : 1); ++i) {   // one stage: the last-stage extents only
+      const StageDev& D = st[i];
+      int me, ie;
+      axis_extents(a.W, TW, HALO, S.hw, S.s_hi_x, D.w, D.s_x, &me, &ie);
+      HI_C = me > HI_C ? me : HI_C;
+      if (ns > 1) LO_C = ie > LO_C ? ie : LO_C;
+      axis_extents(a.H, TH, HALO, S.hh, S.s_hi_y, D.h, D.s_y, &me, &ie);
+      HI_R = me > HI_R ? me : HI_R;
+      if (ns > 1) LO_R = ie > LO_R ? ie : LO_R;
+    }
   }
   {
-    const HpdScaleInputs& in = scales[p->tag_scale];
+    const HpdStageInputs& in = scales[p->tag_scale];
     int rc;
     if ((rc = check_map(in.tag, "tag", true))) return rc;
     if ((p->emb == 2) != (in.tag_f.ptr != nullptr)) {
@@ -516,6 +573,10 @@ int launch_aggregation_kernel(const HpdParams* p, const HpdScaleInputs* scales, 
       const ScaleDev& S = a.sc[s];
       if (!(okp(S.lo, S.lo_sb, S.lo_sc) && okp(S.hi, S.hi_sb, S.hi_sc) && okp(S.lo_f, S.lof_sb, S.lof_sc) && okp(S.hi_f, S.hif_sb, S.hif_sc)))
         a.in_vec_ok_all = 0;
+      for (int i = 0; i + 2 < a.n_stages[s]; ++i) {
+        const StageDev& D = a.mid[s][i];
+        if (!(okp(D.p, D.sb, D.sc) && okp(D.pf, D.fsb, D.fsc))) a.in_vec_ok_all = 0;
+      }
     }
   }
   a.vec_ok = (a.W % 4 == 0) && ((uintptr_t)a.agg_hm % 16 == 0);
@@ -523,15 +584,38 @@ int launch_aggregation_kernel(const HpdParams* p, const HpdScaleInputs* scales, 
   // standard single-scale x2/x2/x4 layout -> specialised kernel (aggregate_nms_x2.cuh)
   {
     const ScaleDev& S = a.sc[0];
-    const bool fast = !(p->force_generic & 1) && a.n_scales == 1 && S.hh == 2 * S.lh && S.hw == 2 * S.lw && a.H == 2 * S.hh &&
-                      a.W == 2 * S.hw && a.th == S.lh && a.tw == S.lw && a.W % 32 == 0 && S.lh >= 2 && S.lw >= 2 &&
-                      a.vec_ok;
+    auto ok = [vec_align](const float* q, long long sb, long long sc_) { return q == nullptr || ((uintptr_t)q % vec_align == 0 && sb % 4 == 0 && sc_ % 4 == 0); };
+    const bool fast = !(p->force_generic & 1) && a.n_scales == 1 && a.n_stages[0] == 2 && S.hh == 2 * S.lh && S.hw == 2 * S.lw &&
+                      a.H == 2 * S.hh && a.W == 2 * S.hw && a.th == S.lh && a.tw == S.lw && a.W % 32 == 0 && S.lh >= 2 &&
+                      S.lw >= 2 && a.vec_ok;
+    // single-stage HRNet-AE layout: heatmaps and tags at S/4 -> x4 walk, no half-res stage
+    const bool fast1 = !(p->force_generic & 1) && a.n_scales == 1 && a.n_stages[0] == 1 && a.H == 4 * S.hh && a.W == 4 * S.hw &&
+                       a.th == S.hh && a.tw == S.hw && a.W % 32 == 0 && S.hh >= 2 && S.hw >= 2 && a.vec_ok;
+    if (fast1) {
+      a.in_vec_ok = S.hw % 4 == 0 && ok(S.hi, S.hi_sb, S.hi_sc) && ok(S.hi_f, S.hif_sb, S.hif_sc) && ok(a.tag, a.tag_sb, a.tag_sc);
+      const int NW = a.W >= 512 ? 4 : (a.W >= 256 ? 2 : 1);
+      const size_t smem = sizeof(float) * x4::smem_floats(NW);
+      const dim3 grid((a.W + 128 * NW - 1) / (128 * NW), (a.H + x2::RB - 1) / x2::RB, a.B * a.K);
+#define HPD_X4_LAUNCH(NW_, T_)                                                                              \
+  do {                                                                                                      \
+    if (int rc_ = ensure_dynamic_smem((const void*)x4::agg_nms_x4_kernel<NW_, T_>, smem, "agg_nms_x4_kernel")) return rc_; \
+    x4::agg_nms_x4_kernel<NW_, T_><<<grid, 32 * NW_, smem, st>>>(a);                                        \
+  } while (0)
+#define HPD_X4_LAUNCH_T(NW_)                                                                                \
+  do {                                                                                                      \
+    if (a.dtype == HPD_F16) HPD_X4_LAUNCH(NW_, __half);                                                     \
+    else if (a.dtype == HPD_BF16) HPD_X4_LAUNCH(NW_, __nv_bfloat16);                                        \
+    else HPD_X4_LAUNCH(NW_, float);                                                                         \
+  } while (0)
+      if (NW == 4) HPD_X4_LAUNCH_T(4); else if (NW == 2) HPD_X4_LAUNCH_T(2); else HPD_X4_LAUNCH_T(1);
+#undef HPD_X4_LAUNCH_T
+#undef HPD_X4_LAUNCH
+      count_launch();
+      return check_launch("agg_nms_x4_kernel");
+    }
     if (fast) {
-      {
-        auto ok = [vec_align](const float* q, long long sb, long long sc_) { return q == nullptr || ((uintptr_t)q % vec_align == 0 && sb % 4 == 0 && sc_ % 4 == 0); };
-        a.in_vec_ok = S.lw % 4 == 0 && ok(S.lo, S.lo_sb, S.lo_sc) && ok(S.hi, S.hi_sb, S.hi_sc) && ok(S.lo_f, S.lof_sb, S.lof_sc) &&
-                      ok(S.hi_f, S.hif_sb, S.hif_sc) && ok(a.tag, a.tag_sb, a.tag_sc);
-      }
+      a.in_vec_ok = S.lw % 4 == 0 && ok(S.lo, S.lo_sb, S.lo_sc) && ok(S.hi, S.hi_sb, S.hi_sc) && ok(S.lo_f, S.lof_sb, S.lof_sc) &&
+                    ok(S.hi_f, S.hif_sb, S.hif_sc) && ok(a.tag, a.tag_sb, a.tag_sc);
       const int NW = a.W >= 512 ? 4 : (a.W >= 256 ? 2 : 1);
       const size_t smem = sizeof(float) * x2::smem_floats(NW);
       const dim3 grid((a.W + 128 * NW - 1) / (128 * NW), (a.H + x2::RB - 1) / x2::RB, a.B * a.K);
@@ -560,7 +644,8 @@ int launch_aggregation_kernel(const HpdParams* p, const HpdScaleInputs* scales, 
               a.W >= 256 && a.vec_ok;
     for (int s = 0; ok && s < a.n_scales; ++s) {
       const ScaleDev& S = a.sc[s];
-      ok = S.hh == 2 * S.lh && S.hw == 2 * S.lw && S.lh >= 2 && S.lw >= 4 && S.lw % 4 == 0 && S.hw <= a.W && S.hh <= a.H;
+      ok = a.n_stages[s] == 2 && S.hh == 2 * S.lh && S.hw == 2 * S.lw && S.lh >= 2 && S.lw >= 4 && S.lw % 4 == 0 && S.hw <= a.W &&
+           S.hh <= a.H;
     }
     if (ok) {
       // warps (128-column strips) per CTA: the count in 2..5 that pads the row least, the larger on ties
@@ -637,9 +722,29 @@ int launch_aggregation_kernel(const HpdParams* p, const HpdScaleInputs* scales, 
 
 }  // namespace
 
-int launch_aggregate_nms(const HpdParams* p, const HpdScaleInputs* scales, const HpdBuffers* buf, cudaStream_t st) {
+HpdStageInputs two_stage_inputs(const HpdScaleInputs& s) {
+  HpdStageInputs r;
+  memset(&r, 0, sizeof(r));
+  r.hm[0] = s.hm_lo; r.hm[1] = s.hm_hi; r.hm_f[0] = s.hm_lo_f; r.hm_f[1] = s.hm_hi_f;
+  r.tag = s.tag; r.tag_f = s.tag_f;
+  r.num_stages = 2;
+  return r;
+}
+
+HpdScaleInputs tag_scale_inputs(const HpdStageInputs& s) {
+  HpdScaleInputs r;
+  memset(&r, 0, sizeof(r));
+  r.tag = s.tag; r.tag_f = s.tag_f;
+  return r;
+}
+
+int launch_aggregate_nms(const HpdParams* p, const HpdStageInputs* scales, const HpdBuffers* buf, cudaStream_t st) {
   if (int rc = launch_aggregation_kernel(p, scales, buf, st)) return rc;
-  return buf->agg_tags ? launch_aggregate_tags(p, scales, buf->agg_tags, st) : HPD_OK;
+  if (!buf->agg_tags) return HPD_OK;
+  const HpdScaleInputs tags = tag_scale_inputs(scales[p->tag_scale]);
+  HpdParams q = *p;   // launch_aggregate_tags reads scales[tag_scale]
+  q.tag_scale = 0;
+  return launch_aggregate_tags(&q, &tags, buf->agg_tags, st);
 }
 
 int launch_nms(const HpdParams* p, const HpdBuffers* buf, float* nms_out, cudaStream_t st) {

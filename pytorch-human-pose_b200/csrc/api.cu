@@ -85,6 +85,16 @@ static int validate(const HpdParams* p, const HpdBuffers* buf) {
   return HPD_OK;
 }
 
+// The two-stage HpdScaleInputs of the older entry points as HpdStageInputs (NULL stays NULL); n <= HPD_MAX_SCALES.
+static const HpdStageInputs* as_stages(const HpdScaleInputs* scales, int n, HpdStageInputs* out) {
+  if (!scales) return nullptr;
+  for (int s = 0; s < n; ++s) out[s] = two_stage_inputs(scales[s]);
+  return out;
+}
+
+static int decode_validated(const HpdParams* p, const HpdStageInputs* scales, const HpdBuffers* buf, void* workspace,
+                            size_t workspace_bytes, cudaStream_t st);
+
 }  // namespace hpd
 
 using namespace hpd;
@@ -103,11 +113,19 @@ int hpd_workspace_bytes(const HpdParams* p, size_t* out_bytes) {
   return HPD_OK;
 }
 
-int hpd_aggregate_nms(const HpdParams* p, const HpdScaleInputs* scales, const HpdBuffers* buf, void* stream) {
+int hpd_aggregate_nms_stages(const HpdParams* p, const HpdStageInputs* scales, const HpdBuffers* buf, void* stream) {
   g_launches = 0;
   int rc = validate(p, buf);
   if (rc) return rc;
   return launch_aggregate_nms(p, scales, buf, (cudaStream_t)stream);
+}
+
+int hpd_aggregate_nms(const HpdParams* p, const HpdScaleInputs* scales, const HpdBuffers* buf, void* stream) {
+  g_launches = 0;
+  int rc = validate(p, buf);
+  if (rc) return rc;
+  HpdStageInputs st[HPD_MAX_SCALES];
+  return launch_aggregate_nms(p, as_stages(scales, p->num_scales, st), buf, (cudaStream_t)stream);
 }
 
 int hpd_aggregate_tags(const HpdParams* p, const HpdScaleInputs* scales, float* out, void* stream) {
@@ -224,11 +242,30 @@ int hpd_decode(const HpdParams* p, const HpdScaleInputs* scales, const HpdBuffer
   g_launches = 0;
   int rc = validate(p, buf);
   if (rc) return rc;
-  cudaStream_t st = (cudaStream_t)stream;
+  HpdStageInputs st[HPD_MAX_SCALES];
+  return decode_validated(p, as_stages(scales, p->num_scales, st), buf, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+int hpd_decode_stages(const HpdParams* p, const HpdStageInputs* scales, const HpdBuffers* buf, void* workspace,
+                      size_t workspace_bytes, void* stream) {
+  g_launches = 0;
+  int rc = validate(p, buf);
+  if (rc) return rc;
+  return decode_validated(p, scales, buf, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+}  // extern "C"
+
+namespace hpd {
+
+// hpd_decode / hpd_decode_stages after validate()
+static int decode_validated(const HpdParams* p, const HpdStageInputs* scales, const HpdBuffers* buf, void* workspace,
+                            size_t workspace_bytes, cudaStream_t st) {
+  int rc;
   HpdBuffers b = *buf;
   if (scales) {
     rc = launch_aggregate_nms(p, scales, &b, st);
-    b.tag_inputs = scales[p->tag_scale];   // the tag stages interpolate from these when agg_tags is NULL
+    b.tag_inputs = tag_scale_inputs(scales[p->tag_scale]);   // the tag stages interpolate from these when agg_tags is NULL
   } else {
     rc = launch_nms(p, &b, nullptr, st);
   }
@@ -238,4 +275,4 @@ int hpd_decode(const HpdParams* p, const HpdScaleInputs* scales, const HpdBuffer
   return launch_adjust_refine(p, &b, workspace, workspace_bytes, st);
 }
 
-}  // extern "C"
+}  // namespace hpd

@@ -179,7 +179,9 @@ __host__ __device__ inline HpdRecordLayout record_layout(int K, int M, int E) {
 }
 
 // ---- per-stage launchers (defined in the stage .cu files) -------------------------------------
-int launch_aggregate_nms(const HpdParams* p, const HpdScaleInputs* scales, const HpdBuffers* buf, cudaStream_t st);
+int launch_aggregate_nms(const HpdParams* p, const HpdStageInputs* scales, const HpdBuffers* buf, cudaStream_t st);
+HpdStageInputs two_stage_inputs(const HpdScaleInputs& s);   // {hm = {hm_lo, hm_hi}, num_stages = 2}
+HpdScaleInputs tag_scale_inputs(const HpdStageInputs& s);   // the tag / tag_f maps alone (HpdBuffers.tag_inputs)
 int launch_aggregate_tags(const HpdParams* p, const HpdScaleInputs* scales, float* out, cudaStream_t st);
 // where the tag stages read tags: buf->agg_tags if set, else buf->tag_inputs (HPD_EINVAL if neither is given)
 int make_tag_source(const HpdParams* p, const HpdBuffers* buf, TagSource* s, const char* who);

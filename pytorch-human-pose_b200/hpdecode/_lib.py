@@ -10,6 +10,7 @@ HPD_MAX_KPTS = 32
 HPD_MAX_PEOPLE = 32
 HPD_MAX_EMB = 2
 HPD_MAX_SCALES = 4
+HPD_MAX_STAGES = 4
 HPD_ABI_VERSION = 6
 HPD_COCO_MAX_IOU_THRS, HPD_COCO_MAX_REC_THRS, HPD_COCO_MAX_AREAS, HPD_COCO_MAX_PER_IMAGE = 16, 128, 4, 1024
 HPD_F32, HPD_F16, HPD_BF16 = 0, 1, 2
@@ -22,6 +23,7 @@ EXPORTS = (
     "hpd_topk", "hpd_group", "hpd_adjust_refine", "hpd_decode", "hpd_last_launch_count", "hpd_resize_bilinear",
     "hpd_record_layout", "hpd_multi_scale_size", "hpd_get_affine_transform", "hpd_prepare_input", "hpd_prepare_geometry",
     "hpd_aggregate_tags", "hpd_coco_eval_workspace_bytes", "hpd_coco_eval", "hpd_prepare_inputs",
+    "hpd_aggregate_nms_stages", "hpd_decode_stages",
 )
 
 
@@ -33,6 +35,11 @@ class HpdMap(ctypes.Structure):
 class HpdScaleInputs(ctypes.Structure):
     _fields_ = [("hm_lo", HpdMap), ("hm_hi", HpdMap), ("tag", HpdMap),
                 ("hm_lo_f", HpdMap), ("hm_hi_f", HpdMap), ("tag_f", HpdMap)]
+
+
+class HpdStageInputs(ctypes.Structure):
+    _fields_ = [("hm", HpdMap * HPD_MAX_STAGES), ("hm_f", HpdMap * HPD_MAX_STAGES), ("tag", HpdMap), ("tag_f", HpdMap),
+                ("num_stages", ctypes.c_int32), ("reserved_", ctypes.c_int32)]
 
 
 class HpdParams(ctypes.Structure):
@@ -117,6 +124,9 @@ def lib():
     L.hpd_group.argtypes = [P, B, V]
     L.hpd_adjust_refine.argtypes = [P, B, V, ctypes.c_size_t, V]
     L.hpd_decode.argtypes = [P, S, B, V, ctypes.c_size_t, V]
+    SS = ctypes.POINTER(HpdStageInputs)
+    L.hpd_aggregate_nms_stages.argtypes = [P, SS, B, V]
+    L.hpd_decode_stages.argtypes = [P, SS, B, V, ctypes.c_size_t, V]
     L.hpd_resize_bilinear.argtypes = [ctypes.POINTER(HpdMap), ctypes.c_int, ctypes.c_int, V, ctypes.c_int,
                                       ctypes.c_int, V]
     I32P, F64P, F32P = ctypes.POINTER(ctypes.c_int32), ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_float)

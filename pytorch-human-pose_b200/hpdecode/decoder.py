@@ -166,13 +166,16 @@ class BottomUpDecoder:
     def decode(self, scales: Sequence[dict], out_hw: Tuple[int, int], tag_scale: int = 0,
                tags_preflipped: bool = False, slot: int = 0, inv_affine=None) -> DecodeResult:
         """scales: one dict per test scale with CUDA float32 tensors hm_lo, hm_hi, tag [B,K,h,w] and,
-        for the flip test, hm_lo_f, hm_hi_f, tag_f (raw outputs of the flipped forward).
+        for the flip test, hm_lo_f, hm_hi_f, tag_f (raw outputs of the flipped forward) -- or, for a head with 1 to 4
+        heatmap stages, ``{"hm": [stages], "tag", "hm_f": [stages], "tag_f"}`` (ops.stage_scale).  16-bit outputs
+        (all maps float16 or all bfloat16) are read as they are.
 
         The returned DecodeResult VIEWS the decoder's cached buffer set for this (shape, slot): it is
         overwritten by the next decode of the same shape and slot.  Read it (``to_numpy()``), ``clone()``
         what must outlive that, or pass distinct ``slot`` values for results that are held together."""
         H, W = out_hw
-        B = scales[0]["hm_lo"].shape[0]
+        scales = [ops.stage_scale(s) for s in scales]
+        B = scales[0]["hm"][0].shape[0]
         E = 2 if scales[tag_scale].get("tag_f") is not None else 1
         bufs = self.buffers(B, H, W, E, slot)
         self._set_inv_affine(bufs, inv_affine)     # float64 [B,6]: back-projection of the records' COCO section
@@ -238,7 +241,8 @@ class DecodePipeline:
         ln = self.lanes[self._next]
         self._next = (self._next + 1) % self.depth
         H, W = out_hw
-        B = scales[0]["hm_lo"].shape[0]
+        first = ops.stage_scale(scales[0])["hm"][0]
+        B = first.shape[0]
         E = 2 if scales[tag_scale].get("tag_f") is not None else 1
         d = self.dec
         bufs = d.buffers(B, H, W, E, slot=ln["slot"])
@@ -257,10 +261,10 @@ class DecodePipeline:
         # The inputs were allocated on the caller's stream but are read on the lane's: tell the caching
         # allocator, or a caller that drops them right after submit() (net outputs -> submit -> next forward)
         # could get their memory back while the aggregation kernel is still reading it.
-        for s in scales:
-            for t in s.values():
-                if t is not None and t.is_cuda:
-                    t.record_stream(st)
+        tensors = [t for s in scales for t in ops.scale_tensors(s)]
+        for t in tensors:
+            if t.is_cuda:
+                t.record_stream(st)
         bufs.generation = getattr(bufs, "generation", 0) + 1
         res = DecodeResult(bufs)
         with torch.cuda.stream(st):
@@ -271,7 +275,9 @@ class DecodePipeline:
             if before_agg is not None:
                 scales = before_agg(ln) or scales      # tensors made here belong to the lane's stream already
             if self.use_graphs:
-                key = (tuple(t.data_ptr() for s in scales for t in s.values() if t is not None), B, H, W, tag_scale,
+                if before_agg is not None:
+                    tensors = [t for s in scales for t in ops.scale_tensors(s)]
+                key = (tuple(t.data_ptr() for t in tensors), B, H, W, tag_scale,
                        bufs.records.data_ptr(), 0 if bufs.inv_affine is None else bufs.inv_affine.data_ptr())
                 g = ln["graphs"].get(key)
                 if g is None:

@@ -2,8 +2,9 @@
 
 Same constructor, ``prepare_input(image) -> (x, center, scale)`` and
 ``__call__(raw_image, annot) -> InferenceKeypointsResult`` as the reference, so ``bin/inference.py:57`` and
-``bin/eval.py:28`` run unchanged.  ``net`` is any stock-PyTorch HigherHRNet returning ``([hm_lo, hm_hi], tag)``;
-the convolutions are NOT part of this library.  What differs is where the work happens:
+``bin/eval.py:28`` run unchanged.  ``net`` is any stock-PyTorch network of the HigherHRNet family returning
+``(list_of_stage_heatmaps, tag)`` with 1 to 4 heatmap stages -- ``([hm_lo, hm_hi], tag)`` for HigherHRNet, ``([hm], tag)``
+for HRNet with the associative-embedding head; the convolutions are NOT part of this library.  What differs is where the work happens:
 
 * ``prepare_input``: cv2.warpAffine + ToTensor + Normalize is one device kernel (csrc/input.cu) on the uint8
   image, bit-identical to the reference's tensor;
@@ -38,6 +39,17 @@ from .results import InferenceKeypointsResult, inverse_transform
 # /root/reference/src/keypoints/datasets/coco.py:45-65 (the COCO skeleton: data, used by the plotting consumers)
 COCO_LIMBS = [(9, 7), (7, 5), (5, 3), (3, 1), (1, 0), (0, 2), (1, 2), (2, 4), (4, 6), (6, 8), (8, 10), (5, 6), (5, 11),
               (6, 12), (11, 12), (11, 13), (13, 15), (12, 14), (14, 16)]
+
+
+def _two_stage_dict(s: dict) -> dict:
+    """A two-stage (HigherHRNet) scale in the {hm_lo, hm_hi, tag[, hm_lo_f, hm_hi_f, tag_f]} dict _net_outputs has
+    always returned; other stage counts stay in the stage format."""
+    if len(s["hm"]) != 2:
+        return s
+    out = {"hm_lo": s["hm"][0], "hm_hi": s["hm"][1], "tag": s["tag"]}
+    if s["hm_f"]:
+        out.update(hm_lo_f=s["hm_f"][0], hm_hi_f=s["hm_f"][1], tag_f=s["tag_f"])
+    return out
 
 
 class InferenceKeypointsModel:
@@ -93,25 +105,32 @@ class InferenceKeypointsModel:
     def _net_outputs(self, x: Tensor, x_flipped: Optional[Tensor] = None) -> dict:
         """x_flipped: torch.flip(x, [3]) when the caller already has it (prepare_inputs writes it with x)."""
         if self.autocast_dtype is not None:
-            return self._net_outputs_autocast(x, x_flipped)
-        (hm_lo, hm_hi), tag = self.net(x)
-        scale = {"hm_lo": hm_lo.float(), "hm_hi": hm_hi.float(), "tag": tag.float()}
-        if self.use_flip:   # model.py:85-94, fused into the aggregation kernel
-            (fl_lo, fl_hi), fl_tag = self.net(torch.flip(x, [3]) if x_flipped is None else x_flipped)
-            scale.update(hm_lo_f=fl_lo.float(), hm_hi_f=fl_hi.float(), tag_f=fl_tag.float())
+            return _two_stage_dict(self._net_outputs_autocast(x, x_flipped))
+        return _two_stage_dict(self._scale(x, x_flipped, lambda t: t.float()))
+
+    def _scale(self, x: Tensor, x_flipped: Optional[Tensor], cast) -> dict:
+        """The decoder's scale dict ({"hm": [stages], "tag", "hm_f", "tag_f"}, ops.stage_scale) from the net's
+        ``(stage_heatmaps, tag)`` on x and, with the flip test (model.py:85-94, fused into the aggregation kernel),
+        on the flipped input."""
+        hms, tag = self.net(x)
+        if not 1 <= len(hms) <= 4:
+            raise ValueError(f"the net must return 1 to 4 heatmap stages (got {len(hms)})")
+        scale = {"hm": [cast(h) for h in hms], "tag": cast(tag), "hm_f": [], "tag_f": None}
+        if self.use_flip:
+            fl_hms, fl_tag = self.net(torch.flip(x, [3]) if x_flipped is None else x_flipped)
+            scale.update(hm_f=[cast(h) for h in fl_hms], tag_f=cast(fl_tag))
         return scale
 
     def _net_outputs_autocast(self, x: Tensor, x_flipped: Optional[Tensor] = None) -> dict:
         with torch.autocast("cuda", dtype=self.autocast_dtype):
-            (hm_lo, hm_hi), tag = self.net(x)
-            scale = {"hm_lo": hm_lo, "hm_hi": hm_hi, "tag": tag}
-            if self.use_flip:
-                (fl_lo, fl_hi), fl_tag = self.net(torch.flip(x, [3]) if x_flipped is None else x_flipped)
-                scale.update(hm_lo_f=fl_lo, hm_hi_f=fl_hi, tag_f=fl_tag)
+            scale = self._scale(x, x_flipped, lambda t: t)
         # the decoder reads one dtype per call: a net whose head leaves some outputs in float32 under autocast has all
         # of them up-cast (exact), the usual all-16-bit set goes as it is
-        if len({t.dtype for t in scale.values()}) > 1:
-            scale = {k: v.float() for k, v in scale.items()}
+        tensors = scale["hm"] + scale["hm_f"] + [t for t in (scale["tag"], scale["tag_f"]) if t is not None]
+        if len({t.dtype for t in tensors}) > 1:
+            f = lambda t: None if t is None else t.float()
+            scale = {"hm": [h.float() for h in scale["hm"]], "hm_f": [h.float() for h in scale["hm_f"]],
+                     "tag": f(scale["tag"]), "tag_f": f(scale["tag_f"])}
         return scale
 
     @torch.no_grad()

@@ -11,6 +11,7 @@ Stage ops mirror the reference methods one to one (paths relative to /root/refer
   hpd::group          MPPEHeatmapParser.match_by_tag grouping.py:85-145 (+ fallback :262-269)
   hpd::adjust_refine  adjust / person score / refine grouping.py:172-191,276,193-250
   hpd::decode         all of the above in one call   (from_preds, results.py:225-238)
+  hpd::decode_stages  the same for heads with 1..4 heatmap stages per scale (results.py:46-54,226 take stage lists)
   hpd::prepare_input  resize_align_multi_scale + ToTensor + Normalize  utils.py:89-97, model.py:45-50
   hpd::prepare_inputs the same for every test scale, plus the flip-test input (model.py:86), in one call
   hpd::coco_eval      pycocotools COCOeval(..., "keypoints").evaluate() + accumulate() (bin/eval.py:52-65)
@@ -23,7 +24,7 @@ from torch import Tensor
 
 from . import _lib
 from ._lib import (HpdBuffers, HpdCocoDets, HpdCocoEvalOutputs, HpdCocoEvalParams, HpdCocoGts, HpdImage, HpdMap,
-                   HpdParams, HpdRecordLayout, HpdScaleInputs)
+                   HpdParams, HpdRecordLayout, HpdScaleInputs, HpdStageInputs)
 
 COCO_FLIP_INDEX = [0, 2, 1, 4, 3, 6, 5, 8, 7, 10, 9, 12, 11, 14, 13, 16, 15]  # transforms.py:11
 JOINTS_ORDER_17 = [0, 1, 2, 3, 4, 5, 6, 11, 12, 7, 8, 9, 10, 13, 14, 15, 16]   # grouping.py:63-65
@@ -205,7 +206,49 @@ def _stream_ptr(device) -> int:
     return torch.cuda.current_stream(device).cuda_stream
 
 
+def stage_scale(s: dict) -> dict:
+    """One test scale's network outputs in the library's scale format {"hm": [stages], "hm_f": [stages] or [],
+    "tag", "tag_f"}: heatmap stages in the network's order (1..HPD_MAX_STAGES; the stage mean is taken at the last
+    one's size).  The two-stage HigherHRNet dicts {"hm_lo", "hm_hi", "tag"[, "hm_lo_f", "hm_hi_f", "tag_f"]} are
+    converted; a dict already in this format is returned as it is."""
+    if "hm" in s:
+        return s
+    flip = s.get("hm_lo_f") is not None
+    return {"hm": [s["hm_lo"], s["hm_hi"]], "hm_f": [s["hm_lo_f"], s["hm_hi_f"]] if flip else [],
+            "tag": s.get("tag"), "tag_f": s.get("tag_f")}
+
+
+def scale_tensors(s: dict) -> List[Tensor]:
+    """Every tensor of a scale dict (either format)."""
+    if "hm" not in s:
+        return [t for t in s.values() if t is not None]
+    return [t for t in list(s["hm"]) + list(s.get("hm_f") or []) + [s.get("tag"), s.get("tag_f")] if t is not None]
+
+
+def _stages_struct(scales: Sequence[dict]):
+    arr = (HpdStageInputs * len(scales))()
+    keep = []
+    for i, s in enumerate(scales):
+        s = stage_scale(s)
+        hm, hm_f = list(s["hm"]), list(s.get("hm_f") or [])
+        if not 1 <= len(hm) <= _lib.HPD_MAX_STAGES:
+            raise _lib.HpdError(f"a scale has 1 to {_lib.HPD_MAX_STAGES} heatmap stages (got {len(hm)})")
+        if hm_f and len(hm_f) != len(hm):
+            raise _lib.HpdError(f"flipped-run stages: {len(hm_f)} for {len(hm)} stages")
+        arr[i].num_stages = len(hm)
+        for j, t in enumerate(hm):
+            arr[i].hm[j] = _map(t, f"hm[{j}]", allow_16bit=True)
+        for j, t in enumerate(hm_f):
+            arr[i].hm_f[j] = _map(t, f"hm_f[{j}]", allow_16bit=True)
+        arr[i].tag = _map(s.get("tag"), "tag", allow_16bit=True)
+        arr[i].tag_f = _map(s.get("tag_f"), "tag_f", allow_16bit=True)
+        keep.append(s)
+    return arr, keep
+
+
 def _scales_struct(scales: Sequence[dict]):
+    """HpdScaleInputs of two-stage scale dicts; of the library's scale format only the tag maps are filled (what the
+    tag entry points read)."""
     arr = (HpdScaleInputs * len(scales))()
     keep = []
     for i, s in enumerate(scales):
@@ -250,9 +293,9 @@ def run_decode(scales: Optional[Sequence[dict]], bufs: DecodeBuffers, params: Hp
     with torch.cuda.device(dev):
         if scales is not None:
             bufs.note_inputs(scales, params)
-            arr, _keep = _scales_struct(scales)
-            rc = L.hpd_decode(ctypes.byref(params), arr, ctypes.byref(bufs.struct()), ws.data_ptr(), ws.numel(),
-                              _stream_ptr(dev))
+            arr, _keep = _stages_struct(scales)
+            rc = L.hpd_decode_stages(ctypes.byref(params), arr, ctypes.byref(bufs.struct()), ws.data_ptr(), ws.numel(),
+                                     _stream_ptr(dev))
         else:
             rc = L.hpd_decode(ctypes.byref(params), None, ctypes.byref(bufs.struct()), ws.data_ptr(), ws.numel(),
                               _stream_ptr(dev))
@@ -289,8 +332,8 @@ def run_stage(stage: str, bufs: DecodeBuffers, params: HpdParams, scales=None, n
     with torch.cuda.device(dev):
         if stage == "aggregate_nms":
             bufs.note_inputs(scales, params)
-            arr, _keep = _scales_struct(scales)
-            rc = L.hpd_aggregate_nms(ctypes.byref(params), arr, ctypes.byref(b), st)
+            arr, _keep = _stages_struct(scales)
+            rc = L.hpd_aggregate_nms_stages(ctypes.byref(params), arr, ctypes.byref(b), st)
         elif stage == "nms":
             rc = L.hpd_nms(ctypes.byref(params), ctypes.byref(b), nms_out.data_ptr() if nms_out is not None else None, st)
         elif stage == "topk":
@@ -395,9 +438,56 @@ def _scales_from_lists(hm_lo, hm_hi, tag, hm_lo_f, hm_hi_f, tag_f):
     return out
 
 
+def _decode_scales(scales: Sequence[dict], out_h: int, out_w: int, max_people: int, det_thr: float, tag_thr: float,
+                   adjust: bool, refine: bool, tag_scale: int) -> List[Tensor]:
+    for s in scales:
+        for t in scale_tensors(s):
+            if not (t.is_cuda and t.dtype in _DTYPE_CODES):
+                _require_cuda(t, "network output")
+    first = stage_scale(scales[0])["hm"][0]
+    B, K = first.shape[:2]
+    E = 2 if stage_scale(scales[tag_scale]).get("tag_f") is not None else 1
+    bufs = DecodeBuffers(B, K, out_h, out_w, E, max_people, first.device)
+    params = make_params(B, K, out_h, out_w, E, max_people, det_thr, tag_thr, adjust, refine, len(scales), tag_scale)
+    run_decode(scales, bufs, params)
+    return [bufs.agg_hm, bufs.agg_tags, bufs.poses, bufs.person_scores, bufs.n_person, bufs.flags, bufs.scores_k,
+            bufs.idx_k, bufs.coords_k, bufs.tags_k]
+
+
+def _decode_fake(first: Tensor, out_h: int, out_w: int, max_people: int, E: int) -> List[Tensor]:
+    B, K = first.shape[:2]
+    M = max_people
+    f = lambda *s: first.new_empty(s, dtype=torch.float32)
+    i = lambda *s: first.new_empty(s, dtype=torch.int32)
+    return [f(B, K, out_h, out_w), f(B, K, out_h, out_w, E), f(B, M, K, 3 + E), f(B, M), i(B), i(B), f(B, K, M),
+            i(B, K, M), i(B, K, M, 2), f(B, K, M, E)]
+
+
 # ------------------------------------------------------------------------------------------------
 # torch.library custom ops
 # ------------------------------------------------------------------------------------------------
+@torch.library.custom_op("hpd::decode_stages", mutates_args=())
+def decode_stages_op(hm: Sequence[Tensor], hm_f: Sequence[Tensor], tag: Sequence[Tensor], tag_f: Sequence[Tensor],
+                     num_stages: int, out_h: int, out_w: int, max_people: int, det_thr: float, tag_thr: float,
+                     adjust: bool, refine: bool, tag_scale: int) -> List[Tensor]:
+    """``hpd::decode`` for heads with ``num_stages`` (1..4) heatmap stages per scale.  ``hm``: the stages of every
+    scale, scale-major (scale s, stage i at s * num_stages + i); ``hm_f`` the same for the flipped run, or empty;
+    ``tag`` / ``tag_f``: one entry per scale (``tag_f`` empty without the flip test).  -> [agg_hm, agg_tags, poses,
+    person_scores, n_person, flags, scores_k, idx_k, coords_k, tags_k]."""
+    if num_stages < 1 or len(hm) == 0 or len(hm) % num_stages or (len(hm_f) and len(hm_f) != len(hm)):
+        raise _lib.HpdError("decode_stages: hm (and hm_f) must hold num_stages maps per scale")
+    n = num_stages
+    scales = [{"hm": list(hm[s * n:(s + 1) * n]), "hm_f": list(hm_f[s * n:(s + 1) * n]) if len(hm_f) else [],
+               "tag": tag[s] if s < len(tag) else None, "tag_f": tag_f[s] if s < len(tag_f) else None}
+              for s in range(len(hm) // n)]
+    return _decode_scales(scales, out_h, out_w, max_people, det_thr, tag_thr, adjust, refine, tag_scale)
+
+
+@decode_stages_op.register_fake
+def _(hm, hm_f, tag, tag_f, num_stages, out_h, out_w, max_people, det_thr, tag_thr, adjust, refine, tag_scale):
+    return _decode_fake(hm[0], out_h, out_w, max_people, 2 if len(tag_f) > 0 else 1)
+
+
 @torch.library.custom_op("hpd::decode", mutates_args=())
 def decode_op(hm_lo: Sequence[Tensor], hm_hi: Sequence[Tensor], tag: Sequence[Tensor], hm_lo_f: Sequence[Tensor],
               hm_hi_f: Sequence[Tensor], tag_f: Sequence[Tensor], out_h: int, out_w: int, max_people: int,
@@ -410,13 +500,7 @@ def decode_op(hm_lo: Sequence[Tensor], hm_hi: Sequence[Tensor], tag: Sequence[Te
             if not (t.is_cuda and t.dtype in _DTYPE_CODES):
                 _require_cuda(t, name)
     scales = _scales_from_lists(hm_lo, hm_hi, tag, hm_lo_f, hm_hi_f, tag_f)
-    B, K = hm_lo[0].shape[:2]
-    E = 2 if len(tag_f) > 0 else 1
-    bufs = DecodeBuffers(B, K, out_h, out_w, E, max_people, hm_lo[0].device)
-    params = make_params(B, K, out_h, out_w, E, max_people, det_thr, tag_thr, adjust, refine, len(scales), tag_scale)
-    run_decode(scales, bufs, params)
-    return [bufs.agg_hm, bufs.agg_tags, bufs.poses, bufs.person_scores, bufs.n_person, bufs.flags, bufs.scores_k,
-            bufs.idx_k, bufs.coords_k, bufs.tags_k]
+    return _decode_scales(scales, out_h, out_w, max_people, det_thr, tag_thr, adjust, refine, tag_scale)
 
 
 @torch.library.custom_op("hpd::parse", mutates_args=())
@@ -620,13 +704,7 @@ def _(x, out_h, out_w):
 @decode_op.register_fake
 def _(hm_lo, hm_hi, tag, hm_lo_f, hm_hi_f, tag_f, out_h, out_w, max_people, det_thr, tag_thr, adjust, refine,
       tag_scale):
-    B, K = hm_lo[0].shape[:2]
-    E = 2 if len(tag_f) > 0 else 1
-    M = max_people
-    f = lambda *s: hm_lo[0].new_empty(s)
-    i = lambda *s: hm_lo[0].new_empty(s, dtype=torch.int32)
-    return [f(B, K, out_h, out_w), f(B, K, out_h, out_w, E), f(B, M, K, 3 + E), f(B, M), i(B), i(B), f(B, K, M),
-            i(B, K, M), i(B, K, M, 2), f(B, K, M, E)]
+    return _decode_fake(hm_lo[0], out_h, out_w, max_people, 2 if len(tag_f) > 0 else 1)
 
 
 @parse_op.register_fake

@@ -52,10 +52,12 @@ def _cuda_device(t: Tensor) -> torch.device:
 
 def _decode_preaveraged(kpts_heatmaps: List[Tensor], tags_heatmaps: List[Tensor], img_h: int, img_w: int,
                         max_num_people: int, det_thr: float, tag_thr: float, inv_affine: Optional[np.ndarray] = None):
-    """results.py:225-244 in one device call.  kpts_heatmaps = [stage1, stage2] (flip averaging already applied
-    by the model, model.py:87-90); tags_heatmaps = [tag] or [tag, unflipped flip tag]; inv_affine: float64 [B,6]."""
-    if len(kpts_heatmaps) != 2:
-        raise ops._lib.HpdError("hpdecode handles the two-stage HigherHRNet head (got %d stages)" % len(kpts_heatmaps))
+    """results.py:225-244 in one device call.  kpts_heatmaps = the head's 1..4 stages in the network's order, e.g.
+    [stage1, stage2] for HigherHRNet (flip averaging already applied by the model, model.py:87-90); tags_heatmaps =
+    [tag] or [tag, unflipped flip tag]; inv_affine: float64 [B,6]."""
+    if not 1 <= len(kpts_heatmaps) <= ops._lib.HPD_MAX_STAGES:
+        raise ops._lib.HpdError("hpdecode handles heads with 1 to %d heatmap stages (got %d)"
+                                % (ops._lib.HPD_MAX_STAGES, len(kpts_heatmaps)))
     if len(tags_heatmaps) not in (1, 2):
         raise ops._lib.HpdError("1 or 2 tag maps expected")
     dev = _cuda_device(kpts_heatmaps[0])
@@ -63,10 +65,9 @@ def _decode_preaveraged(kpts_heatmaps: List[Tensor], tags_heatmaps: List[Tensor]
     # a uniform set of fp16 or bf16 network outputs (validation under autocast, module.py:78) goes to the kernel as it is
     same16 = len(dtypes) == 1 and dtypes <= {torch.float16, torch.bfloat16}
     f = lambda t: t.to(dev) if same16 else t.to(dev, torch.float32)
-    scale = {"hm_lo": f(kpts_heatmaps[0]), "hm_hi": f(kpts_heatmaps[1]), "tag": f(tags_heatmaps[0])}
-    if len(tags_heatmaps) == 2:
-        scale["tag_f"] = f(tags_heatmaps[1])
-    B, K = scale["hm_lo"].shape[:2]
+    scale = {"hm": [f(h) for h in kpts_heatmaps], "hm_f": [], "tag": f(tags_heatmaps[0]),
+             "tag_f": f(tags_heatmaps[1]) if len(tags_heatmaps) == 2 else None}
+    B, K = scale["hm"][0].shape[:2]
     E = len(tags_heatmaps)
     bufs = ops.DecodeBuffers(B, K, img_h, img_w, E, max_num_people, dev)
     if inv_affine is not None:

@@ -11,8 +11,10 @@ Architecture (HRNet, Sun et al. 2019; HigherHRNet, Cheng et al. 2020; interface 
 /root/reference/src/keypoints/architectures/higher_hrnet.py:47-81): stem of two stride-2 3x3 convs,
 one bottleneck stage, three multi-resolution stages (1 / 4 / 3 modules of 4 basic blocks per branch,
 widths C, 2C, 4C, 8C) with full fusion, a 1x1 head giving 2K channels at 1/4 resolution (K heatmaps
-+ K tags, returned as channel-slice VIEWS), and one stride-2 transposed-conv head with 4 basic blocks
-giving K heatmaps at 1/2 resolution.  forward(x) -> ([hm_lo, hm_hi], tag).
++ K tags, returned as channel-slice VIEWS), and ``num_deconvs`` stride-2 transposed-conv modules with 4 basic blocks
+each, every one giving K heatmaps at twice the resolution of the previous stage.  forward(x) -> ([hm_lo, hm_hi], tag)
+for the default num_deconvs=1; ([hm], tag) for 0 (HRNet with the associative-embedding head); ([hm_lo, hm_hi, hm_full],
+tag) for 2 (stages at S/4, S/2, S).
 """
 import torch
 from torch import nn
@@ -74,9 +76,12 @@ class _Module(nn.Module):
 
 
 class HigherHRNet(nn.Module):
-    def __init__(self, num_kpts: int = 17, C: int = 32):
+    def __init__(self, num_kpts: int = 17, C: int = 32, num_deconvs: int = 1):
         super().__init__()
+        if num_deconvs not in (0, 1, 2):
+            raise ValueError(f"num_deconvs must be 0, 1 or 2 (got {num_deconvs})")
         self.num_kpts = num_kpts
+        self.num_deconvs = num_deconvs
         self.stem = nn.Sequential(_cbr(3, 64, 3, 2), _cbr(64, 64, 3, 2))
         self.stage1 = nn.Sequential(_Bottleneck(64, 64), *[_Bottleneck(256, 64) for _ in range(3)])
         w = [C, 2 * C, 4 * C, 8 * C]
@@ -93,6 +98,11 @@ class HigherHRNet(nn.Module):
                                     nn.ReLU(inplace=True))
         self.deconv_blocks = nn.Sequential(*[_Basic(C) for _ in range(4)])
         self.final = nn.Conv2d(C, num_kpts, 1)
+        if num_deconvs == 2:   # the second module reads the first one's features and heatmaps
+            self.deconv2 = nn.Sequential(nn.ConvTranspose2d(C + num_kpts, C, 4, 2, 1, bias=False), nn.BatchNorm2d(C),
+                                         nn.ReLU(inplace=True))
+            self.deconv2_blocks = nn.Sequential(*[_Basic(C) for _ in range(4)])
+            self.final2 = nn.Conv2d(C, num_kpts, 1)
 
     def forward(self, x):
         x = self.stage1(self.stem(x))
@@ -107,38 +117,48 @@ class HigherHRNet(nn.Module):
             xs = m(xs)
         feats = xs[0]
         both = self.head(feats)                                   # [B, 2K, S/4, S/4]
-        hm_hi = self.final(self.deconv_blocks(self.deconv(torch.cat((feats, both), 1))))
         K = self.num_kpts
-        return [both[:, :K], hm_hi], both[:, K:]                  # channel-slice views, like the reference
+        if self.num_deconvs == 0:
+            return [both[:, :K]], both[:, K:]
+        f1 = self.deconv_blocks(self.deconv(torch.cat((feats, both), 1)))
+        hm_hi = self.final(f1)
+        if self.num_deconvs == 1:
+            return [both[:, :K], hm_hi], both[:, K:]              # channel-slice views, like the reference
+        hm_full = self.final2(self.deconv2_blocks(self.deconv2(torch.cat((f1, hm_hi), 1))))
+        return [both[:, :K], hm_hi, hm_full], both[:, K:]
 
 
 @torch.no_grad()
 def network_outputs(batch: int, size: int = 512, flip: bool = True, seed: int = 0, C: int = 32, device="cuda:0",
-                    chunk: int = 8, num_kpts: int = 17, image_seed=None):
+                    chunk: int = 8, num_kpts: int = 17, image_seed=None, num_deconvs: int = 1):
     """One scale dict of CUDA tensors [B,K,h,w] produced by a default-init HigherHRNet-W{C} on seeded
     N(0,1) images (torch.manual_seed(seed) -> net -> images, the order SURVEY.md 8(d) fixes).
     ``image_seed`` (default seed + 1) seeds the images separately: several ranks then run ONE network
-    (same ``seed``) on different images."""
+    (same ``seed``) on different images.  ``num_deconvs`` as in HigherHRNet: the default 1 gives the two-stage
+    {hm_lo, hm_hi, tag[, hm_lo_f, hm_hi_f, tag_f]} dict, 0 and 2 the stage format {hm: [...], tag[, hm_f, tag_f]}."""
     torch.manual_seed(seed)
-    net = HigherHRNet(num_kpts, C).eval().to(device)
+    net = HigherHRNet(num_kpts, C, num_deconvs).eval().to(device)
     g = torch.Generator(device="cpu").manual_seed(seed + 1 if image_seed is None else image_seed)
-    out = {k: [] for k in (("hm_lo", "hm_hi", "tag", "hm_lo_f", "hm_hi_f", "tag_f") if flip else ("hm_lo", "hm_hi", "tag"))}
+    n = max(num_deconvs, 0) + 1
+    runs = ("", "_f") if flip else ("",)
+    hms = {r: [[] for _ in range(n)] for r in runs}
+    tags = {r: [] for r in runs}
     for b0 in range(0, batch, chunk):
         x = torch.randn(min(chunk, batch - b0), 3, size, size, generator=g).to(device)
-        (lo, hi), tag = net(x)
-        out["hm_lo"].append(lo)
-        out["hm_hi"].append(hi)
-        out["tag"].append(tag)
-        if flip:
-            (lo, hi), tag = net(torch.flip(x, [3]))
-            out["hm_lo_f"].append(lo)
-            out["hm_hi_f"].append(hi)
-            out["tag_f"].append(tag)
-    # keep hm_lo / tag as channel-slice views of one 2K-channel tensor per batch (strided, like the reference)
+        for r in runs:
+            stages, tag = net(x if r == "" else torch.flip(x, [3]))
+            for i, h in enumerate(stages):
+                hms[r][i].append(h)
+            tags[r].append(tag)
+    # keep the first stage / tag as channel-slice views of one 2K-channel tensor per batch (strided, like the reference)
+    out = {}
+    for r in runs:
+        both = torch.cat([torch.cat((a, t), 1) for a, t in zip(hms[r][0], tags[r])], 0)
+        out["hm" + r] = [both[:, :num_kpts]] + [torch.cat(hs, 0) for hs in hms[r][1:]]
+        out["tag" + r] = both[:, num_kpts:]
+    if num_deconvs != 1:
+        return out if flip else dict(out, hm_f=[], tag_f=None)
     res = {}
-    for suffix in (("", "_f") if flip else ("",)):
-        both = torch.cat([torch.cat((a, t), 1) for a, t in zip(out["hm_lo" + suffix], out["tag" + suffix])], 0)
-        res["hm_lo" + suffix] = both[:, :num_kpts]
-        res["tag" + suffix] = both[:, num_kpts:]
-        res["hm_hi" + suffix] = torch.cat(out["hm_hi" + suffix], 0)
+    for r in runs:
+        res["hm_lo" + r], res["tag" + r], res["hm_hi" + r] = out["hm" + r][0], out["tag" + r], out["hm" + r][1]
     return res
