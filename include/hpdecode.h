@@ -349,6 +349,41 @@ HPD_EXPORT int hpd_coco_eval_workspace_bytes(const HpdCocoEvalParams* p, size_t*
 HPD_EXPORT int hpd_coco_eval(const HpdCocoEvalParams* p, const HpdCocoDets* dets, const HpdCocoGts* gts,
                              const HpdCocoEvalOutputs* outs, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- person tracking across frames (greedy OKS matching, the tracker of mmpose's video demos) ------------------
+ * Frames are result records (HpdRecordLayout for num_kpts, max_people, emb) in time order.  Per frame, its persons
+ * are visited in descending person score (ties: lower index).  Each takes the live track, not yet claimed in this
+ * frame, with the highest OKS against the pose that last matched it (ties: smaller id), if that OKS is > oks_thr;
+ * otherwise it starts a new track (ids 0, 1, ... never reused) if it has >= min_keypoints visible joints, or gets -1.
+ * Tracks started in a frame are not candidates in that frame.  Unclaimed tracks age by one per frame and are dropped
+ * at age max_age.  OKS: over the joints visible in both poses (poses[.][k][2] > 0; none: 0), with the COCO-section
+ * coordinates, s = the mean of the two poses' areas (bounding box of the visible joints; 0 below two) and
+ *   e_k = (dx*dx + dy*dy) / kpt_vars[k] / (s + 2^-52) / 2,  OKS = np.sum(exp(-e)) / |J|   (float64, NumPy's order).
+ * A frame whose flags bit 0 is set (the empty-scene fallback) has no persons.  Person scores must not be NaN. */
+typedef struct HpdTrackParams {
+  int32_t num_kpts;       /* K <= HPD_MAX_KPTS */
+  int32_t max_people;     /* M <= HPD_MAX_PEOPLE: persons per record */
+  int32_t emb;            /* E of the records: 1 or 2 */
+  int32_t max_age;        /* 1..HPD_TRACK_MAX_AGE: a track unclaimed for max_age frames is dropped */
+  int32_t min_keypoints;  /* 0..K visible joints a person needs to start a track */
+  int32_t reserved_;
+  double oks_thr;         /* a match needs OKS > oks_thr (finite) */
+  double kpt_vars[HPD_MAX_KPTS];   /* (2 sigma_k)^2, finite and > 0: cocoeval's kpt_vars for COCO's sigmas */
+} HpdTrackParams;
+#define HPD_TRACK_MAX_AGE 8
+
+/* Bytes of the tracker state for these params (room for max_people * max_age tracks).  The layout is private. */
+HPD_EXPORT int hpd_track_state_bytes(const HpdTrackParams* p, size_t* out_bytes);
+
+/* Drops every track of the state.  clear_ids = 1 also restarts the ids at 0: a new state must be reset so once
+ * before its first hpd_track.  One memset on the stream, no kernel launch. */
+HPD_EXPORT int hpd_track_reset(const HpdTrackParams* p, void* state, size_t state_bytes, int clear_ids, void* stream);
+
+/* Tracks n_frames >= 1 consecutive records (records + f * row_bytes, read in place) in one kernel launch, continuing
+ * from the state and updating it.  track_ids [n_frames][max_people] int32: the id of each person, -1 for persons
+ * that start no track and for slots >= n_person.  Every argument is checked before the launch. */
+HPD_EXPORT int hpd_track(const HpdTrackParams* p, const uint8_t* records, int n_frames, void* state, size_t state_bytes,
+                         int32_t* track_ids, void* stream);
+
 /* Number of kernel launches the previous call on this thread enqueued (for bench accounting). */
 HPD_EXPORT int hpd_last_launch_count(void);
 

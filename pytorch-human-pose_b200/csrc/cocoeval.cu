@@ -101,12 +101,7 @@ __device__ __forceinline__ double oks_pair(const double* xd, const double* yd, c
   const double y0 = __dsub_rn(bb[1], bb[3]), y1 = __dadd_rn(bb[1], __dmul_rn(bb[3], 2.0));
   const double den = __dadd_rn(garea, 0x1p-52);
   const int n = k1 > 0 ? k1 : K;
-  const int n_main = n - n % 8;
-  // r0..r7 are NumPy's eight accumulators, rotated after every term so that r0 always receives the next one;
-  // after a multiple of 8 terms they are back in place
-  double r0 = 0, r1 = 0, r2 = 0, r3 = 0, r4 = 0, r5 = 0, r6 = 0, r7 = 0;
-  double res = -0.0;
-  int c = 0;
+  NpSumF64 acc(n);
   for (int k = 0; k < K; ++k) {
     double dx, dy;
     if (k1 > 0) {
@@ -119,22 +114,9 @@ __device__ __forceinline__ double oks_pair(const double* xd, const double* yd, c
     }
     double e = __dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy));
     e = __ddiv_rn(__ddiv_rn(__ddiv_rn(e, vars[k]), den), 2.0);
-    const double term = exp(-e);
-    if (n < 8) {
-      res = __dadd_rn(res, term);
-    } else if (c < n_main) {
-      const double v = c < 8 ? term : __dadd_rn(r0, term);
-      r0 = r1; r1 = r2; r2 = r3; r3 = r4; r4 = r5; r5 = r6; r6 = r7; r7 = v;
-    } else {
-      if (c == n_main)
-        res = __dadd_rn(__dadd_rn(__dadd_rn(r0, r1), __dadd_rn(r2, r3)), __dadd_rn(__dadd_rn(r4, r5), __dadd_rn(r6, r7)));
-      res = __dadd_rn(res, term);
-    }
-    ++c;
+    acc.add(exp(-e));
   }
-  if (n >= 8 && n_main == n)
-    res = __dadd_rn(__dadd_rn(__dadd_rn(r0, r1), __dadd_rn(r2, r3)), __dadd_rn(__dadd_rn(r4, r5), __dadd_rn(r6, r7)));
-  return __ddiv_rn(__dadd_rn(0.0, res), (double)n);   // the reduction starts from add's identity
+  return __ddiv_rn(acc.sum(), (double)n);
 }
 
 __global__ void __launch_bounds__(kImgThreads) coco_image_kernel(HpdCocoEvalParams p, HpdCocoDets dets, HpdCocoGts gts,

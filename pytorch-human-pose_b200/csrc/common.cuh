@@ -148,6 +148,33 @@ __device__ __forceinline__ float np_sum_pairwise8(const float* a, int n, int str
   return res;
 }
 
+// numpy float64 np.sum of n <= 128 terms fed one at a time in index order (its 128-element block): a plain sum below 8
+// terms, the pairwise-8 unrolled loop from 8 on.  r0..r7 are NumPy's eight accumulators, rotated after every term so
+// that r0 always receives the next one; after a multiple of 8 terms they are back in place.  Exactly n add() calls.
+struct NpSumF64 {
+  double r0 = 0, r1 = 0, r2 = 0, r3 = 0, r4 = 0, r5 = 0, r6 = 0, r7 = 0;
+  double res = -0.0;
+  int c = 0, n, n_main;
+  __device__ __forceinline__ explicit NpSumF64(int n_) : n(n_), n_main(n_ - n_ % 8) {}
+  __device__ __forceinline__ double block8() const {
+    return __dadd_rn(__dadd_rn(__dadd_rn(r0, r1), __dadd_rn(r2, r3)), __dadd_rn(__dadd_rn(r4, r5), __dadd_rn(r6, r7)));
+  }
+  __device__ __forceinline__ void add(double term) {
+    if (n < 8) {
+      res = __dadd_rn(res, term);
+    } else if (c < n_main) {
+      const double v = c < 8 ? term : __dadd_rn(r0, term);
+      r0 = r1; r1 = r2; r2 = r3; r3 = r4; r4 = r5; r5 = r6; r6 = r7; r7 = v;
+    } else {
+      if (c == n_main) res = block8();
+      res = __dadd_rn(res, term);
+    }
+    ++c;
+  }
+  // the reduction starts from add's identity
+  __device__ __forceinline__ double sum() const { return __dadd_rn(0.0, n >= 8 && n_main == n ? block8() : res); }
+};
+
 // np.mean(list of n float32 vectors of E components, axis=0) (grouping.py:114,213):
 // E == 1 reduces a contiguous axis (pairwise-8), E == 2 accumulates row by row (sequential).
 __device__ __forceinline__ void np_mean_vectors(const float* v, int n, int E, int row_stride, float* out) {
@@ -202,5 +229,10 @@ int validate_coco_params(const HpdCocoEvalParams* p);
 size_t coco_eval_workspace_bytes(const HpdCocoEvalParams* p, int* rc);
 int launch_coco_eval(const HpdCocoEvalParams* p, const HpdCocoDets* dets, const HpdCocoGts* gts,
                      const HpdCocoEvalOutputs* outs, void* ws, size_t ws_bytes, cudaStream_t st);
+int validate_track_params(const HpdTrackParams* p, const char* who);
+size_t track_state_bytes(const HpdTrackParams* p);
+int launch_track_reset(const HpdTrackParams* p, void* state, size_t state_bytes, int clear_ids, cudaStream_t st);
+int launch_track(const HpdTrackParams* p, const uint8_t* records, int n_frames, void* state, size_t state_bytes,
+                 int32_t* track_ids, cudaStream_t st);
 
 }  // namespace hpd

@@ -14,6 +14,7 @@ HPD_MAX_STAGES = 4
 HPD_ABI_VERSION = 6
 HPD_COCO_MAX_IOU_THRS, HPD_COCO_MAX_REC_THRS, HPD_COCO_MAX_AREAS, HPD_COCO_MAX_PER_IMAGE = 16, 128, 4, 1024
 HPD_F32, HPD_F16, HPD_BF16 = 0, 1, 2
+HPD_TRACK_MAX_AGE = 8
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libhpdecode.so")
@@ -23,7 +24,7 @@ EXPORTS = (
     "hpd_topk", "hpd_group", "hpd_adjust_refine", "hpd_decode", "hpd_last_launch_count", "hpd_resize_bilinear",
     "hpd_record_layout", "hpd_multi_scale_size", "hpd_get_affine_transform", "hpd_prepare_input", "hpd_prepare_geometry",
     "hpd_aggregate_tags", "hpd_coco_eval_workspace_bytes", "hpd_coco_eval", "hpd_prepare_inputs",
-    "hpd_aggregate_nms_stages", "hpd_decode_stages",
+    "hpd_aggregate_nms_stages", "hpd_decode_stages", "hpd_track_state_bytes", "hpd_track_reset", "hpd_track",
 )
 
 
@@ -95,6 +96,12 @@ class HpdCocoEvalOutputs(ctypes.Structure):
     _fields_ = [(n, ctypes.c_void_p) for n in ("precision", "recall", "scores", "oks", "codes", "npig")]
 
 
+class HpdTrackParams(ctypes.Structure):
+    _fields_ = [(n, ctypes.c_int32) for n in ("num_kpts", "max_people", "emb", "max_age", "min_keypoints",
+                                              "reserved_")] + [
+        ("oks_thr", ctypes.c_double), ("kpt_vars", ctypes.c_double * HPD_MAX_KPTS)]
+
+
 class HpdError(RuntimeError):
     pass
 
@@ -143,6 +150,10 @@ def lib():
     L.hpd_coco_eval_workspace_bytes.argtypes = [CP, ctypes.POINTER(ctypes.c_size_t)]
     L.hpd_coco_eval.argtypes = [CP, ctypes.POINTER(HpdCocoDets), ctypes.POINTER(HpdCocoGts),
                                 ctypes.POINTER(HpdCocoEvalOutputs), V, ctypes.c_size_t, V]
+    TP = ctypes.POINTER(HpdTrackParams)
+    L.hpd_track_state_bytes.argtypes = [TP, ctypes.POINTER(ctypes.c_size_t)]
+    L.hpd_track_reset.argtypes = [TP, V, ctypes.c_size_t, ctypes.c_int, V]
+    L.hpd_track.argtypes = [TP, V, ctypes.c_int, V, ctypes.c_size_t, V, V]
     for n in EXPORTS:
         if n not in ("hpd_last_error_string",):
             getattr(L, n).restype = ctypes.c_int

@@ -20,10 +20,11 @@ from . import ops
 class Records:
     """Host view of the per-image result records written by the decode's last kernel (HpdRecordLayout,
     include/hpdecode.h): ``raw`` is the uint8 [B,row_bytes] array of ONE device->host copy; the fields are
-    zero-copy NumPy views into it."""
+    zero-copy NumPy views into it.  ``track_ids``: optional int32 [B,M] person ids across frames (PoseTracker)."""
 
-    def __init__(self, raw: np.ndarray, M: int, K: int, E: int):
+    def __init__(self, raw: np.ndarray, M: int, K: int, E: int, track_ids: Optional[np.ndarray] = None):
         L = ops.record_layout(K, M, E)
+        self.track_ids = track_ids
         raw = np.ascontiguousarray(raw, np.uint8).reshape(-1, L.row_bytes)
         self.raw, self.M, self.K, self.E = raw, M, K, E
         B, D, C = raw.shape[0], 3 + E, L.coco_stride

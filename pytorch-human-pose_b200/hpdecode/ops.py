@@ -15,6 +15,7 @@ Stage ops mirror the reference methods one to one (paths relative to /root/refer
   hpd::prepare_input  resize_align_multi_scale + ToTensor + Normalize  utils.py:89-97, model.py:45-50
   hpd::prepare_inputs the same for every test scale, plus the flip-test input (model.py:86), in one call
   hpd::coco_eval      pycocotools COCOeval(..., "keypoints").evaluate() + accumulate() (bin/eval.py:52-65)
+  hpd::track          person ids across consecutive frames' result records (greedy OKS tracking; hpdecode.track)
 """
 import ctypes
 from typing import List, Optional, Sequence, Tuple
@@ -24,7 +25,7 @@ from torch import Tensor
 
 from . import _lib
 from ._lib import (HpdBuffers, HpdCocoDets, HpdCocoEvalOutputs, HpdCocoEvalParams, HpdCocoGts, HpdImage, HpdMap,
-                   HpdParams, HpdRecordLayout, HpdScaleInputs, HpdStageInputs)
+                   HpdParams, HpdRecordLayout, HpdScaleInputs, HpdStageInputs, HpdTrackParams)
 
 COCO_FLIP_INDEX = [0, 2, 1, 4, 3, 6, 5, 8, 7, 10, 9, 12, 11, 14, 13, 16, 15]  # transforms.py:11
 JOINTS_ORDER_17 = [0, 1, 2, 3, 4, 5, 6, 11, 12, 7, 8, 9, 10, 13, 14, 15, 16]   # grouping.py:63-65
@@ -426,6 +427,60 @@ def run_coco_eval(params: HpdCocoEvalParams, records: Sequence[Tensor], row_of_i
     return outs
 
 
+def track_params(K: int, M: int, E: int, max_age: int, min_keypoints: int, oks_thr: float,
+                 kpt_vars: Sequence[float]) -> HpdTrackParams:
+    """HpdTrackParams; kpt_vars = (2 sigma)**2 per joint, float64 as NumPy computed them.  The library checks ranges."""
+    if len(kpt_vars) != K or K > _lib.HPD_MAX_KPTS:
+        raise _lib.HpdError(f"track: one variance per joint (got {len(kpt_vars)} for K={K}, K <= {_lib.HPD_MAX_KPTS})")
+    p = HpdTrackParams()
+    p.num_kpts, p.max_people, p.emb, p.max_age, p.min_keypoints = K, M, E, max_age, min_keypoints
+    p.oks_thr = float(oks_thr)
+    for k, v in enumerate(kpt_vars):
+        p.kpt_vars[k] = float(v)
+    return p
+
+
+def track_state_bytes(params: HpdTrackParams) -> int:
+    n = ctypes.c_size_t(0)
+    _lib.check(_lib.lib().hpd_track_state_bytes(ctypes.byref(params), ctypes.byref(n)), "hpd_track_state_bytes")
+    return n.value
+
+
+def _check_state(state: Tensor, device):
+    if not state.is_cuda or state.dtype != torch.uint8 or not state.is_contiguous() or state.device != device:
+        raise _lib.HpdError("track: the state must be a contiguous uint8 CUDA tensor on the records' device")
+
+
+def run_track_reset(params: HpdTrackParams, state: Tensor, clear_ids: bool):
+    """hpd_track_reset on the current stream: drop every track; clear_ids also restarts the ids at 0."""
+    _check_state(state, state.device)
+    with torch.cuda.device(state.device):
+        rc = _lib.lib().hpd_track_reset(ctypes.byref(params), state.data_ptr(), state.numel(), int(clear_ids),
+                                        _stream_ptr(state.device))
+    _lib.check(rc, "hpd_track_reset")
+
+
+def run_track(params: HpdTrackParams, records: Tensor, state: Tensor, out: Tensor) -> Tensor:
+    """hpd_track on the current stream: records uint8 [n, row_bytes] (rows packed, read in place) -> out int32 [n, M]."""
+    row_bytes = record_layout(params.num_kpts, params.max_people, params.emb).row_bytes
+    if (not records.is_cuda or records.dtype != torch.uint8 or records.dim() != 2 or records.shape[1] != row_bytes
+            or records.stride(1) != 1 or (records.shape[0] > 1 and records.stride(0) != row_bytes)):
+        raise _lib.HpdError(f"track: records must be a uint8 CUDA tensor [n, {row_bytes}] with packed rows")
+    _check_state(state, records.device)
+    n, M = records.shape[0], params.max_people
+    if tuple(out.shape) != (n, M) or out.dtype != torch.int32 or not out.is_contiguous() or out.device != records.device:
+        raise _lib.HpdError(f"track: out must be a contiguous int32 tensor {(n, M)} on the records' device")
+    if n == 0:
+        return out
+    L = _lib.lib()
+    with torch.cuda.device(records.device):
+        rc = L.hpd_track(ctypes.byref(params), records.data_ptr(), n, state.data_ptr(), state.numel(), out.data_ptr(),
+                         _stream_ptr(records.device))
+    _lib.check(rc, "hpd_track")
+    _count(L)
+    return out
+
+
 def _scales_from_lists(hm_lo, hm_hi, tag, hm_lo_f, hm_hi_f, tag_f):
     n = len(hm_lo)
     flip = len(hm_lo_f) > 0
@@ -689,6 +744,22 @@ def _(records, row_of_image, off_coco, off_count, person_stride, max_per_row, gt
     else:
         tail = [f(0), f(0), f(0)]
     return [f(T, R, A), f(T, A), f(T, R, A)] + tail
+
+
+@torch.library.custom_op("hpd::track", mutates_args=("state",))
+def track_op(records: Tensor, state: Tensor, num_kpts: int, max_people: int, emb: int, max_age: int,
+             min_keypoints: int, oks_thr: float, kpt_vars: Sequence[float]) -> Tensor:
+    """Person ids of consecutive frames (hpd_track): ``records`` uint8 [n, row_bytes] result records in time order,
+    ``state`` the tracker state (updated in place) -> int32 [n, max_people], -1 for persons without a track and for
+    slots past the frame's persons."""
+    params = track_params(num_kpts, max_people, emb, max_age, min_keypoints, oks_thr, kpt_vars)
+    out = torch.empty((records.shape[0], max_people), device=records.device, dtype=torch.int32)
+    return run_track(params, records, state, out)
+
+
+@track_op.register_fake
+def _(records, state, num_kpts, max_people, emb, max_age, min_keypoints, oks_thr, kpt_vars):
+    return records.new_empty((records.shape[0], max_people), dtype=torch.int32)
 
 
 @prepare_input_op.register_fake

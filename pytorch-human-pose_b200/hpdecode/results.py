@@ -98,6 +98,7 @@ class InferenceKeypointsResult(BaseKeypointsResult):
     limbs: list
     det_thr: float
     tag_thr: float
+    track_ids: Optional[np.ndarray] = None   # int32 [P]: the persons' ids across frames (model.stream(track=True))
 
     @classmethod
     def get_final_kpts_coords(cls, kpts_coords: np.ndarray, center, scale, hm_size) -> np.ndarray:
@@ -147,12 +148,14 @@ class InferenceKeypointsResult(BaseKeypointsResult):
     def from_records(cls, rec: Records, b: int, raw_image, annot, model_input_image, limbs, det_thr, tag_thr,
                      kpts_heatmaps=None, tags_heatmaps=None) -> "InferenceKeypointsResult":
         """Image b of a batch's host records -> the reference's result object (results.py:240-263).  The batched
-        callers pass no maps (they stay on the device); ``from_preds`` passes them like the reference."""
+        callers pass no maps (they stay on the device); ``from_preds`` passes them like the reference.  Records that
+        carry track ids give the image's persons theirs."""
         grouped_joints, obj_scores = rec.image(b)
         return cls(raw_image=raw_image, annot=annot, model_input_image=model_input_image, kpts_heatmaps=kpts_heatmaps,
                    tags_heatmaps=tags_heatmaps, kpts_coords=rec.final_coords(b), kpts_scores=grouped_joints[..., 2],
                    kpts_tags=grouped_joints[..., 3:], obj_scores=obj_scores, limbs=limbs, det_thr=det_thr,
-                   tag_thr=tag_thr)
+                   tag_thr=tag_thr,
+                   track_ids=None if rec.track_ids is None else rec.track_ids[b, :len(obj_scores)].copy())
 
 
 class KeypointsResult(BaseKeypointsResult):

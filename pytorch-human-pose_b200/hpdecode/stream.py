@@ -10,10 +10,13 @@ frames instead and keeps ``depth`` batches in flight (``DecodePipeline`` lanes);
    launch (``prepare_input`` + ``torch.flip`` per scale, bit for bit);
 3. the network, once per scale and run, under the model's autocast setting (``InferenceKeypointsModel._net_outputs``);
 4. the decode with the scale-1.0 inverse matrices, so the records carry raw-frame coordinates;
-5. one device->host copy of the batch's records into the lane's pinned records slot.
+5. one device->host copy of the batch's records into the lane's pinned records slot;
+6. with ``track=True``, on the stream's own tracking stream and in submission order: it waits for the batch's records,
+   runs ``PoseTracker.update`` on them in place (``hpd_track``) and copies the ids into the lane's pinned ids slot.  A
+   change of frame size, which closes a batch, also resets the tracker (ids are not reused).
 
-A lane and its staging slot are reused only after the host has waited for that lane's records copy (an event, not a
-device synchronise).  A batch closes when it is full or when the frame size changes, so frames of mixed sizes work;
+A lane and its staging slot are reused only after the host has waited for that lane's records copy and, when
+tracking, its ids copy (events, not a device synchronise), so a lane's records are tracked before they are overwritten.  A batch closes when it is full or when the frame size changes, so frames of mixed sizes work;
 results come back in submission order either way.  Geometry is computed once per distinct frame size.
 
 The stream decodes into the model decoder's buffer sets (slot = lane): do not call the model's other entry points
@@ -28,19 +31,23 @@ import torch
 from . import _lib, geometry, ops
 from .decoder import DecodePipeline, Records
 from .results import InferenceKeypointsResult
+from .track import PoseTracker
 
 
 class FrameStream:
     """``submit(frames)`` any number of times, then iterate ``results()`` (or the stream itself) for one result per
     frame in submission order: an InferenceKeypointsResult (no maps, like ``predict_batch``) or, with
-    ``records=True``, the frame's ``Records`` (one row).  Frames are uint8 [h,w,3] NumPy arrays or CUDA tensors."""
+    ``records=True``, the frame's ``Records`` (one row).  Frames are uint8 [h,w,3] NumPy arrays or CUDA tensors.
+    ``track=True``: the stream owns a ``PoseTracker`` (``tracker``, default settings) and every result carries its
+    persons' ids across frames (``track_ids``)."""
 
     MAX_SIZES = 64    # distinct frame sizes whose geometry is kept
 
-    def __init__(self, model, batch_size: int = 8, depth: int = 4, records: bool = False):
+    def __init__(self, model, batch_size: int = 8, depth: int = 4, records: bool = False, track: bool = False):
         if batch_size < 1 or depth < 1:
             raise ValueError(f"batch_size and depth must be >= 1 (got {batch_size}, {depth})")
         self.model, self.batch_size, self.depth, self.records = model, int(batch_size), int(depth), records
+        self.track = bool(track)
         self._open: list = []           # frames of the batch being filled
         self._open_hw = None
         self._inflight = deque()        # launched batches, oldest first
@@ -127,6 +134,13 @@ class FrameStream:
         self._pinned: List = [None] * self.depth       # per lane: host frames of the batch, pinned
         self._staged: List = [None] * self.depth       # per lane: their device copy
         self._shape_only = {}
+        self.tracker = None
+        if self.track:
+            self.tracker = PoseTracker(K, M, E, self.device)
+            self._track_stream = torch.cuda.Stream(device=self.device)
+            self._track_stream.wait_stream(torch.cuda.current_stream(self.device))   # the tracker's initial reset
+            self._host_ids = torch.empty((self.depth, self.batch_size, M), dtype=torch.int32, pin_memory=True)
+            self._track_hw = None
 
     def _stage(self, f, i):
         lane = self.pipe._next          # the lane the open batch will be submitted on
@@ -180,24 +194,47 @@ class FrameStream:
                                                     list(geometry.STD))
             return [m._net_outputs(x, xs_f[t] if m.use_flip else None) for t, x in enumerate(xs)]
 
+        written = torch.cuda.Event()
+
         def after_tail(ln, res):
+            written.record()
             self._host_rec[lane][:n].copy_(res.records, non_blocking=True)
 
         ts = self._tag_scale
         res = self.pipe.submit(self._placeholders(n), (sizes_hw[2 * ts], sizes_hw[2 * ts + 1]), tag_scale=ts,
                                before_agg=before_agg, after_tail=after_tail, inv_affine=inv)
-        return lane, frames, res        # res keeps the lane's buffer set alive until the batch is retired
+        tracked = self._track(lane, hw, res, written) if self.track else None
+        return lane, frames, res, tracked     # res keeps the lane's buffer set alive until the batch is retired
+
+    def _track(self, lane, hw, res, written):
+        """Tracks the batch's records on the tracking stream once they are written; -> the event of the ids copy."""
+        st = self._track_stream
+        st.wait_event(written)
+        res.records.record_stream(st)
+        with torch.cuda.stream(st):
+            if self._track_hw is not None and hw != self._track_hw:
+                self.tracker.reset()
+            self._track_hw = hw
+            ids = self.tracker.update(res.records)
+            self._host_ids[lane][:ids.shape[0]].copy_(ids, non_blocking=True)
+            done = torch.cuda.Event()
+            done.record()
+        return done
 
     def _ready(self, batch) -> bool:
-        return batch[2].ready.query()
+        return batch[2].ready.query() and (batch[3] is None or batch[3].query())
 
     def _finish(self, batch) -> list:
-        lane, frames, res = batch
+        lane, frames, res, tracked = batch
         res.ready.synchronize()
         raw = self._host_rec[lane][:len(frames)].numpy().copy()
+        ids = None
+        if tracked is not None:
+            tracked.synchronize()
+            ids = self._host_ids[lane][:len(frames)].numpy().copy()
         M, K, E = self._rec_shape
         if self.records:
-            return [Records(raw[b:b + 1], M, K, E) for b in range(len(frames))]
-        m, rec = self.model, Records(raw, M, K, E)
+            return [Records(raw[b:b + 1], M, K, E, None if ids is None else ids[b:b + 1]) for b in range(len(frames))]
+        m, rec = self.model, Records(raw, M, K, E, ids)
         return [InferenceKeypointsResult.from_records(rec, b, f, None, None, m.limbs, m.det_thr, m.tag_thr)
                 for b, f in enumerate(frames)]
