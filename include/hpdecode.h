@@ -374,8 +374,9 @@ typedef struct HpdTrackParams {
 /* Bytes of the tracker state for these params (room for max_people * max_age tracks).  The layout is private. */
 HPD_EXPORT int hpd_track_state_bytes(const HpdTrackParams* p, size_t* out_bytes);
 
-/* Drops every track of the state.  clear_ids = 1 also restarts the ids at 0: a new state must be reset so once
- * before its first hpd_track.  One memset on the stream, no kernel launch. */
+/* Drops every track of the state (with a smoothing state, their filters too).  clear_ids = 1 also restarts the ids at
+ * 0: a new state must be reset so once before its first hpd_track or hpd_track_smooth.  One memset on the stream, no
+ * kernel launch. */
 HPD_EXPORT int hpd_track_reset(const HpdTrackParams* p, void* state, size_t state_bytes, int clear_ids, void* stream);
 
 /* Tracks n_frames >= 1 consecutive records (records + f * row_bytes, read in place) in one kernel launch, continuing
@@ -383,6 +384,43 @@ HPD_EXPORT int hpd_track_reset(const HpdTrackParams* p, void* state, size_t stat
  * that start no track and for slots >= n_person.  Every argument is checked before the launch. */
 HPD_EXPORT int hpd_track(const HpdTrackParams* p, const uint8_t* records, int n_frames, void* state, size_t state_bytes,
                          int32_t* track_ids, void* stream);
+
+/* ---- smoothing of tracked joints across frames (the 1-Euro filter: Casiez, Roussel, Vogel, CHI 2012) -------------
+ * hpd_track_smooth tracks exactly as hpd_track (same ids; OKS uses the last raw pose) and also filters the COCO-section
+ * coordinates of every tracked person's visible joints, x and y independently, with state per (track, joint) that
+ * lives and dies with the track.  Frames are numbered consecutively across calls, fallback frames included.  For
+ * person p < n_person of frame f with id >= 0 and joint k visible (poses[p][k][2] > 0), with the raw coordinate x:
+ *   the first time joint k of the track is visible:  x^ = x, dx^ = 0, output x, last = f;
+ *   otherwise, with g = f - last >= 1, each step one correctly rounded float64 operation (no FMA), in this order,
+ *   TWO_PI = the float64 2 * pi, products and sums grouped left to right as written:
+ *     te  = (double)g / fps
+ *     rd  = (TWO_PI * d_cutoff) * te;  ad = rd / (rd + 1)
+ *     dx  = (x - x^) / te
+ *     dx^' = ad * dx + (1 - ad) * dx^
+ *     c   = min_cutoff + beta * |dx^'|
+ *     r   = (TWO_PI * c) * te;         a  = r / (r + 1)
+ *     x^' = a * x + (1 - a) * x^
+ *   output x^', store x^', dx^', last = f.
+ * Invisible joints (their state untouched) and persons with id -1 (the empty-scene fallback's pseudo-person included)
+ * are written raw; rows p >= n_person are 0.  A dropped track's filters are gone; a new track starts unseeded. */
+typedef struct HpdSmoothParams {
+  double min_cutoff;   /* Hz, in (0, 1e6] */
+  double beta;         /* speed coefficient, in [0, 1e6] */
+  double d_cutoff;     /* Hz, cutoff of the speed estimate, in (0, 1e6] */
+  double fps;          /* the video's constant frame rate, in [1e-3, 1e6].  Not just > 0: with a subnormal fps,
+                        * te = g / fps overflows to inf and rd / (rd + 1) is inf / inf = NaN.  With these bounds no
+                        * step overflows for coordinates below 1e280 in magnitude. */
+} HpdSmoothParams;
+
+/* Bytes of a smoothing tracker state: the hpd_track state plus the filters of max_people * max_age tracks.  A state is
+ * used with either hpd_track or hpd_track_smooth, never both; hpd_track_reset works on either kind. */
+HPD_EXPORT int hpd_track_smooth_state_bytes(const HpdTrackParams* p, size_t* out_bytes);
+
+/* hpd_track plus smoothing, in one kernel launch: track_ids as hpd_track's, coords [n_frames][max_people][num_kpts][2]
+ * float64 (8-byte aligned).  Every argument is checked before the launch. */
+HPD_EXPORT int hpd_track_smooth(const HpdTrackParams* p, const HpdSmoothParams* sp, const uint8_t* records,
+                                int n_frames, void* state, size_t state_bytes, int32_t* track_ids, double* coords,
+                                void* stream);
 
 /* Number of kernel launches the previous call on this thread enqueued (for bench accounting). */
 HPD_EXPORT int hpd_last_launch_count(void);

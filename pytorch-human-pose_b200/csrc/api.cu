@@ -261,6 +261,23 @@ int hpd_track(const HpdTrackParams* p, const uint8_t* records, int n_frames, voi
   return launch_track(p, records, n_frames, state, state_bytes, track_ids, (cudaStream_t)stream);
 }
 
+int hpd_track_smooth_state_bytes(const HpdTrackParams* p, size_t* out_bytes) {
+  g_launches = 0;
+  int rc = validate_track_params(p, "hpd_track_smooth_state_bytes");
+  if (rc) return rc;
+  if (!out_bytes) { set_error("hpd_track_smooth_state_bytes: out_bytes is NULL"); return HPD_EINVAL; }
+  *out_bytes = track_smooth_state_bytes(p);
+  return HPD_OK;
+}
+
+int hpd_track_smooth(const HpdTrackParams* p, const HpdSmoothParams* sp, const uint8_t* records, int n_frames,
+                     void* state, size_t state_bytes, int32_t* track_ids, double* coords, void* stream) {
+  g_launches = 0;
+  int rc = validate_track_params(p, "hpd_track_smooth");
+  if (rc) return rc;
+  return launch_track_smooth(p, sp, records, n_frames, state, state_bytes, track_ids, coords, (cudaStream_t)stream);
+}
+
 int hpd_decode(const HpdParams* p, const HpdScaleInputs* scales, const HpdBuffers* buf, void* workspace,
                size_t workspace_bytes, void* stream) {
   g_launches = 0;

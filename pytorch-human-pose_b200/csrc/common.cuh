@@ -234,5 +234,8 @@ size_t track_state_bytes(const HpdTrackParams* p);
 int launch_track_reset(const HpdTrackParams* p, void* state, size_t state_bytes, int clear_ids, cudaStream_t st);
 int launch_track(const HpdTrackParams* p, const uint8_t* records, int n_frames, void* state, size_t state_bytes,
                  int32_t* track_ids, cudaStream_t st);
+size_t track_smooth_state_bytes(const HpdTrackParams* p);
+int launch_track_smooth(const HpdTrackParams* p, const HpdSmoothParams* sp, const uint8_t* records, int n_frames,
+                        void* state, size_t state_bytes, int32_t* track_ids, double* coords, cudaStream_t st);
 
 }  // namespace hpd

@@ -13,6 +13,13 @@
 // slot indices, not poses.  Between calls the state holds the live tracks compacted to slots 0..n_live-1.
 //
 // Like hpd_coco_eval, every float64 operation is spelled out and exp() is CUDA's, within 1 ulp of NumPy's.
+//
+// track_kernel<true> (hpd_track_smooth) also runs a One-Euro filter per (track, joint); oracle/smooth_oracle.py states
+// it.  Its state (FilterTable) is too large for shared memory next to the table, so it stays in the state buffer in
+// global memory, indexed by slot, and is touched only for the frame's claimed and new tracks, one thread per (person,
+// joint).  The end-of-call compaction moves tracks to slots 0..n_live-1; the filter region is double-buffered so that
+// it can follow: the call reads and updates buffer `buf` by slot, then copies the live slots in live order to the
+// other buffer and flips `buf`.
 #include <math.h>
 
 #include "common.cuh"
@@ -23,7 +30,8 @@ namespace {
 constexpr int kTrackThreads = 256;
 
 struct TrackHeader {
-  int32_t n_live, next_id, reserved_[2];
+  int32_t n_live, next_id;
+  uint32_t frame, buf;   // hpd_track_smooth only: frames filtered so far (mod 2^32); the filter buffer in use (bit 0)
 };
 
 // Track slots; the same layout in the state (after TrackHeader) and in shared memory.
@@ -44,6 +52,28 @@ __host__ __device__ inline TrackTable carve_table(uint8_t* base, int C, int K) {
   t.vis = reinterpret_cast<uint32_t*>(t.area + C);
   t.id = reinterpret_cast<int32_t*>(t.vis + C);
   t.age = t.id + C;
+  return t;
+}
+
+// One-Euro filter state of the track slots, C x K entries per buffer: the filtered position and speed, the frame the joint
+// was last filtered (so a gap of g frames gives te = g / fps) and whether it was seen since the track began.
+struct FilterTable {
+  double *x, *y, *dx, *dy;   // [C][K]
+  uint32_t *last, *seen;     // [C][K]
+};
+
+__host__ __device__ inline size_t filter_bytes(int C, int K) { return (size_t)C * K * (4 * 8 + 2 * 4); }
+__host__ __device__ inline size_t filter_offset(int C, int K) { return (sizeof(TrackHeader) + table_bytes(C, K) + 7) / 8 * 8; }
+
+__host__ __device__ inline FilterTable carve_filter(uint8_t* base, int C, int K) {
+  FilterTable t;
+  const size_t n = (size_t)C * K;
+  t.x = reinterpret_cast<double*>(base);
+  t.y = t.x + n;
+  t.dx = t.y + n;
+  t.dy = t.dx + n;
+  t.last = reinterpret_cast<uint32_t*>(t.dy + n);
+  t.seen = t.last + n;
   return t;
 }
 
@@ -106,9 +136,28 @@ __device__ __forceinline__ double track_oks(const double* xd, const double* yd, 
   return __ddiv_rn(acc.sum(), (double)n);
 }
 
+constexpr double kTwoPi = 2.0 * 3.141592653589793;   // Python's 2 * math.pi
+
+// One filter step of one coordinate (include/hpdecode.h: hpd_track_smooth), each operation rounded once, no FMA:
+// updates the filtered speed dxh and position xh from the raw x and returns the new position.
+__device__ __forceinline__ double one_euro(double x, double& xh, double& dxh, double te, double ad,
+                                           const HpdSmoothParams& sp) {
+  const double dx = __ddiv_rn(__dsub_rn(x, xh), te);
+  dxh = __dadd_rn(__dmul_rn(ad, dx), __dmul_rn(__dsub_rn(1.0, ad), dxh));
+  const double c = __dadd_rn(sp.min_cutoff, __dmul_rn(sp.beta, fabs(dxh)));
+  const double r = __dmul_rn(__dmul_rn(kTwoPi, c), te);
+  const double a = __ddiv_rn(r, __dadd_rn(r, 1.0));
+  xh = __dadd_rn(__dmul_rn(a, x), __dmul_rn(__dsub_rn(1.0, a), xh));
+  return xh;
+}
+
+// SMOOTH's parameters follow the others, so that track_kernel<false> compiles to the instructions of the untemplated
+// kernel it replaced.
+template <bool SMOOTH>
 __global__ void __launch_bounds__(kTrackThreads) track_kernel(HpdTrackParams p, const uint8_t* __restrict__ records,
                                                               int n_frames, HpdRecordLayout L, uint8_t* state,
-                                                              int32_t* __restrict__ ids) {
+                                                              int32_t* __restrict__ ids, HpdSmoothParams sp,
+                                                              double* __restrict__ coords) {
   extern __shared__ __align__(16) uint8_t smem[];
   __shared__ double s_vars[HPD_MAX_KPTS];
   __shared__ int s_n_live, s_next_id;
@@ -118,6 +167,13 @@ __global__ void __launch_bounds__(kTrackThreads) track_kernel(HpdTrackParams p, 
   carve_smem(smem, M, C, K, &s);
   TrackHeader* hdr = reinterpret_cast<TrackHeader*>(state);
   const TrackTable g = carve_table(state + sizeof(TrackHeader), C, K);
+  uint32_t frame0 = 0, buf = 0;
+  FilterTable fz;
+  if constexpr (SMOOTH) {
+    frame0 = hdr->frame;
+    buf = hdr->buf & 1u;
+    fz = carve_filter(state + filter_offset(C, K) + buf * filter_bytes(C, K), C, K);
+  }
 
   // the state's live tracks are compacted: live position j is slot j
   const int n_live0 = min(max(hdr->n_live, 0), C);
@@ -323,6 +379,47 @@ __global__ void __launch_bounds__(kTrackThreads) track_kernel(HpdTrackParams p, 
         s.t.y[sl * K + i % K] = s.py[i];
       }
     }
+    if constexpr (SMOOTH) {
+      // every row of the frame: tracked persons' visible joints filtered, other persons raw, rows past n_person 0
+      const int n_rec = min(max(*reinterpret_cast<const int32_t*>(r + L.off_n_person), 0), M);
+      const uint32_t fr = frame0 + (uint32_t)f;
+      double* co = coords + (size_t)f * M * K * 2;
+      for (int i = tid; i < M * K; i += kTrackThreads) {
+        const int q = i / K, k = i % K;
+        double x = 0.0, y = 0.0;
+        if (q < n_rec) {
+          x = coco[(size_t)q * L.coco_stride + 3 * k];
+          y = coco[(size_t)q * L.coco_stride + 3 * k + 1];
+        }
+        const int a = q < n ? s.assign[q] : -2;
+        if (a != -2) {   // the person has a track: claimed (a >= 0, the pose update above) or new (slot nslot)
+          const size_t e = (size_t)(a >= 0 ? live[a] : s.nslot[q]) * K + k;
+          const bool vis = (s.pvis[q] >> k) & 1u;
+          if (vis) {
+            double xh = x, yh = y, dxh = 0.0, dyh = 0.0;
+            if (a >= 0 && fz.seen[e]) {
+              xh = fz.x[e];
+              yh = fz.y[e];
+              dxh = fz.dx[e];
+              dyh = fz.dy[e];
+              const double te = __ddiv_rn((double)(fr - fz.last[e]), sp.fps);
+              const double rd = __dmul_rn(__dmul_rn(kTwoPi, sp.d_cutoff), te);
+              const double ad = __ddiv_rn(rd, __dadd_rn(rd, 1.0));
+              x = one_euro(x, xh, dxh, te, ad, sp);
+              y = one_euro(y, yh, dyh, te, ad, sp);
+            }
+            fz.x[e] = xh;
+            fz.y[e] = yh;
+            fz.dx[e] = dxh;
+            fz.dy[e] = dyh;
+            fz.last[e] = fr;
+          }
+          if (vis || a == -1) fz.seen[e] = vis;   // a new track in a reused slot starts unseeded
+        }
+        co[2 * i] = x;
+        co[2 * i + 1] = y;
+      }
+    }
     int32_t* tmp = live;
     live = live2;
     live2 = tmp;
@@ -346,16 +443,36 @@ __global__ void __launch_bounds__(kTrackThreads) track_kernel(HpdTrackParams p, 
     hdr->n_live = n_live;
     hdr->next_id = s_next_id;
   }
+  if constexpr (SMOOTH) {   // the filter follows the compaction into the other buffer
+    const FilterTable to = carve_filter(state + filter_offset(C, K) + (buf ^ 1u) * filter_bytes(C, K), C, K);
+    for (int i = tid; i < n_live * K; i += kTrackThreads) {
+      const size_t e = (size_t)live[i / K] * K + i % K;
+      to.x[i] = fz.x[e];
+      to.y[i] = fz.y[e];
+      to.dx[i] = fz.dx[e];
+      to.dy[i] = fz.dy[e];
+      to.last[i] = fz.last[e];
+      to.seen[i] = fz.seen[e];
+    }
+    if (tid == 0) {
+      hdr->frame = frame0 + (uint32_t)n_frames;
+      hdr->buf = buf ^ 1u;
+    }
+  }
 }
 
 size_t state_bytes_of(const HpdTrackParams* p) {
   return sizeof(TrackHeader) + table_bytes(p->max_people * p->max_age, p->num_kpts);
 }
 
-int check_state(const HpdTrackParams* p, const void* state, size_t state_bytes, const char* who) {
+size_t smooth_state_bytes_of(const HpdTrackParams* p) {
+  const int C = p->max_people * p->max_age, K = p->num_kpts;
+  return filter_offset(C, K) + 2 * filter_bytes(C, K);
+}
+
+int check_state(const void* state, size_t state_bytes, size_t need, const char* who) {
   if (!state) { set_error("%s: state is NULL", who); return HPD_EINVAL; }
   if ((uintptr_t)state % 8) { set_error("%s: state must be 8-byte aligned", who); return HPD_EINVAL; }
-  const size_t need = state_bytes_of(p);
   if (state_bytes < need) {
     set_error("%s: state too small (%zu < %zu bytes)", who, state_bytes, need);
     return HPD_EINVAL;
@@ -394,13 +511,30 @@ int validate_track_params(const HpdTrackParams* p, const char* who) {
   return HPD_OK;
 }
 
+int validate_smooth_params(const HpdSmoothParams* sp, const char* who) {
+  if (!sp) { set_error("%s: smooth params pointer is NULL", who); return HPD_EINVAL; }
+  const struct { const char* name; double v, lo, hi; bool lo_open; } f[] = {
+      {"min_cutoff", sp->min_cutoff, 0.0, 1e6, true}, {"beta", sp->beta, 0.0, 1e6, false},
+      {"d_cutoff", sp->d_cutoff, 0.0, 1e6, true}, {"fps", sp->fps, 1e-3, 1e6, false}};
+  for (const auto& x : f) {
+    if (!(isfinite(x.v) && (x.lo_open ? x.v > x.lo : x.v >= x.lo) && x.v <= x.hi)) {
+      set_error("%s: %s must be finite and in %c%g, %g] (got %g)", who, x.name, x.lo_open ? '(' : '[', x.lo, x.hi, x.v);
+      return HPD_EINVAL;
+    }
+  }
+  return HPD_OK;
+}
+
 size_t track_state_bytes(const HpdTrackParams* p) { return state_bytes_of(p); }
 
+size_t track_smooth_state_bytes(const HpdTrackParams* p) { return smooth_state_bytes_of(p); }
+
 int launch_track_reset(const HpdTrackParams* p, void* state, size_t state_bytes, int clear_ids, cudaStream_t st) {
-  int rc = check_state(p, state, state_bytes, "hpd_track_reset");
+  int rc = check_state(state, state_bytes, state_bytes_of(p), "hpd_track_reset");
   if (rc) return rc;
-  // n_live = 0 drops the tracks; next_id (the header's second word) restarts at 0 only with clear_ids
-  const cudaError_t e = cudaMemsetAsync(state, 0, clear_ids ? 2 * sizeof(int32_t) : sizeof(int32_t), st);
+  // n_live = 0 drops the tracks, and with them their filters; clear_ids zeroes the whole header: next_id restarts at
+  // 0, and a smoothing state's frame counter and buffer bit start from known values
+  const cudaError_t e = cudaMemsetAsync(state, 0, clear_ids ? sizeof(TrackHeader) : sizeof(int32_t), st);
   if (e != cudaSuccess) {
     cudaGetLastError();
     set_error("hpd_track_reset: %s", cudaGetErrorString(e));
@@ -416,15 +550,38 @@ int launch_track(const HpdTrackParams* p, const uint8_t* records, int n_frames, 
   if (n_frames < 1) { set_error("hpd_track: n_frames must be >= 1 (got %d)", n_frames); return HPD_EINVAL; }
   if (!track_ids) { set_error("hpd_track: track_ids is NULL"); return HPD_EINVAL; }
   if ((uintptr_t)track_ids % 4) { set_error("hpd_track: track_ids must be 4-byte aligned"); return HPD_EINVAL; }
-  int rc = check_state(p, state, state_bytes, "hpd_track");
+  int rc = check_state(state, state_bytes, state_bytes_of(p), "hpd_track");
   if (rc) return rc;
   const int C = p->max_people * p->max_age;
   const size_t smem = track_smem_bytes(p->max_people, C, p->num_kpts);
-  if ((rc = ensure_dynamic_smem((const void*)track_kernel, smem, "hpd_track"))) return rc;
-  track_kernel<<<1, kTrackThreads, smem, st>>>(*p, records, n_frames, record_layout(p->num_kpts, p->max_people, p->emb),
-                                               (uint8_t*)state, track_ids);
+  if ((rc = ensure_dynamic_smem((const void*)track_kernel<false>, smem, "hpd_track"))) return rc;
+  track_kernel<false><<<1, kTrackThreads, smem, st>>>(*p, records, n_frames,
+                                                      record_layout(p->num_kpts, p->max_people, p->emb),
+                                                      (uint8_t*)state, track_ids, HpdSmoothParams{}, nullptr);
   count_launch();
   return check_launch("track_kernel");
+}
+
+int launch_track_smooth(const HpdTrackParams* p, const HpdSmoothParams* sp, const uint8_t* records, int n_frames,
+                        void* state, size_t state_bytes, int32_t* track_ids, double* coords, cudaStream_t st) {
+  int rc = validate_smooth_params(sp, "hpd_track_smooth");
+  if (rc) return rc;
+  if (!records) { set_error("hpd_track_smooth: records is NULL"); return HPD_EINVAL; }
+  if ((uintptr_t)records % 8) { set_error("hpd_track_smooth: records must be 8-byte aligned"); return HPD_EINVAL; }
+  if (n_frames < 1) { set_error("hpd_track_smooth: n_frames must be >= 1 (got %d)", n_frames); return HPD_EINVAL; }
+  if (!track_ids) { set_error("hpd_track_smooth: track_ids is NULL"); return HPD_EINVAL; }
+  if ((uintptr_t)track_ids % 4) { set_error("hpd_track_smooth: track_ids must be 4-byte aligned"); return HPD_EINVAL; }
+  if (!coords) { set_error("hpd_track_smooth: coords is NULL"); return HPD_EINVAL; }
+  if ((uintptr_t)coords % 8) { set_error("hpd_track_smooth: coords must be 8-byte aligned"); return HPD_EINVAL; }
+  if ((rc = check_state(state, state_bytes, smooth_state_bytes_of(p), "hpd_track_smooth"))) return rc;
+  const int C = p->max_people * p->max_age;
+  const size_t smem = track_smem_bytes(p->max_people, C, p->num_kpts);
+  if ((rc = ensure_dynamic_smem((const void*)track_kernel<true>, smem, "hpd_track_smooth"))) return rc;
+  track_kernel<true><<<1, kTrackThreads, smem, st>>>(*p, records, n_frames,
+                                                     record_layout(p->num_kpts, p->max_people, p->emb),
+                                                     (uint8_t*)state, track_ids, *sp, coords);
+  count_launch();
+  return check_launch("track_kernel<true>");
 }
 
 }  // namespace hpd

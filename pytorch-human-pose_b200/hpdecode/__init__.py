@@ -12,11 +12,12 @@ from .grouping import MPPEHeatmapParser  # noqa: F401
 from .results import BaseKeypointsResult, InferenceKeypointsResult, KeypointsResult  # noqa: F401
 from .model import InferenceKeypointsModel  # noqa: F401
 from .stream import FrameStream  # noqa: F401
-from .track import PoseTracker  # noqa: F401
+from .track import OneEuro, PoseTracker  # noqa: F401
 from .coco import batch_to_coco, eval_coco, evaluate_dataset_batched, result_to_coco  # noqa: F401
 from .cocoeval import KeypointEvaluator, KeypointGroundTruth  # noqa: F401
 
 __all__ = ["BottomUpDecoder", "DecodePipeline", "DecodeResult", "Records", "MPPEHeatmapParser", "BaseKeypointsResult",
-           "InferenceKeypointsResult", "KeypointsResult", "InferenceKeypointsModel", "FrameStream", "PoseTracker", "batch_to_coco",
+           "InferenceKeypointsResult", "KeypointsResult", "InferenceKeypointsModel", "FrameStream", "PoseTracker",
+           "OneEuro", "batch_to_coco",
            "evaluate_dataset_batched", "result_to_coco", "geometry", "ops", "eval_coco", "KeypointEvaluator",
            "KeypointGroundTruth"]

@@ -25,6 +25,7 @@ EXPORTS = (
     "hpd_record_layout", "hpd_multi_scale_size", "hpd_get_affine_transform", "hpd_prepare_input", "hpd_prepare_geometry",
     "hpd_aggregate_tags", "hpd_coco_eval_workspace_bytes", "hpd_coco_eval", "hpd_prepare_inputs",
     "hpd_aggregate_nms_stages", "hpd_decode_stages", "hpd_track_state_bytes", "hpd_track_reset", "hpd_track",
+    "hpd_track_smooth_state_bytes", "hpd_track_smooth",
 )
 
 
@@ -102,6 +103,10 @@ class HpdTrackParams(ctypes.Structure):
         ("oks_thr", ctypes.c_double), ("kpt_vars", ctypes.c_double * HPD_MAX_KPTS)]
 
 
+class HpdSmoothParams(ctypes.Structure):
+    _fields_ = [(n, ctypes.c_double) for n in ("min_cutoff", "beta", "d_cutoff", "fps")]
+
+
 class HpdError(RuntimeError):
     pass
 
@@ -154,6 +159,8 @@ def lib():
     L.hpd_track_state_bytes.argtypes = [TP, ctypes.POINTER(ctypes.c_size_t)]
     L.hpd_track_reset.argtypes = [TP, V, ctypes.c_size_t, ctypes.c_int, V]
     L.hpd_track.argtypes = [TP, V, ctypes.c_int, V, ctypes.c_size_t, V, V]
+    L.hpd_track_smooth_state_bytes.argtypes = [TP, ctypes.POINTER(ctypes.c_size_t)]
+    L.hpd_track_smooth.argtypes = [TP, ctypes.POINTER(HpdSmoothParams), V, ctypes.c_int, V, ctypes.c_size_t, V, V, V]
     for n in EXPORTS:
         if n not in ("hpd_last_error_string",):
             getattr(L, n).restype = ctypes.c_int

@@ -20,11 +20,14 @@ from . import ops
 class Records:
     """Host view of the per-image result records written by the decode's last kernel (HpdRecordLayout,
     include/hpdecode.h): ``raw`` is the uint8 [B,row_bytes] array of ONE device->host copy; the fields are
-    zero-copy NumPy views into it.  ``track_ids``: optional int32 [B,M] person ids across frames (PoseTracker)."""
+    zero-copy NumPy views into it.  ``track_ids``: optional int32 [B,M] person ids across frames (PoseTracker);
+    ``smoothed_coords``: optional float64 [B,M,K,2] One-Euro-filtered COCO-section coordinates (PoseTracker with
+    smoothing)."""
 
-    def __init__(self, raw: np.ndarray, M: int, K: int, E: int, track_ids: Optional[np.ndarray] = None):
+    def __init__(self, raw: np.ndarray, M: int, K: int, E: int, track_ids: Optional[np.ndarray] = None,
+                 smoothed_coords: Optional[np.ndarray] = None):
         L = ops.record_layout(K, M, E)
-        self.track_ids = track_ids
+        self.track_ids, self.smoothed_coords = track_ids, smoothed_coords
         raw = np.ascontiguousarray(raw, np.uint8).reshape(-1, L.row_bytes)
         self.raw, self.M, self.K, self.E = raw, M, K, E
         B, D, C = raw.shape[0], 3 + E, L.coco_stride
@@ -51,6 +54,12 @@ class Records:
         array, float64 for the empty-scene fallback's pseudo-person."""
         P = int(self.n_person[b])
         xy = self.coco[b, :P, : 3 * self.K].reshape(P, self.K, 3)[..., :2]
+        return xy.copy() if int(self.flags[b]) & 1 else xy.astype(np.float32)
+
+    def smoothed_final_coords(self, b: int) -> np.ndarray:
+        """``final_coords(b)`` with the tracked joints One-Euro filtered (``smoothed_coords``), in the same dtype."""
+        P = int(self.n_person[b])
+        xy = self.smoothed_coords[b, :P]
         return xy.copy() if int(self.flags[b]) & 1 else xy.astype(np.float32)
 
     def coco_records(self, b: int, image_id: int) -> List[dict]:

@@ -16,6 +16,7 @@ Stage ops mirror the reference methods one to one (paths relative to /root/refer
   hpd::prepare_inputs the same for every test scale, plus the flip-test input (model.py:86), in one call
   hpd::coco_eval      pycocotools COCOeval(..., "keypoints").evaluate() + accumulate() (bin/eval.py:52-65)
   hpd::track          person ids across consecutive frames' result records (greedy OKS tracking; hpdecode.track)
+  hpd::track_smooth   the same ids plus the tracked joints' One-Euro-filtered coordinates (hpdecode.track.OneEuro)
 """
 import ctypes
 from typing import List, Optional, Sequence, Tuple
@@ -25,7 +26,7 @@ from torch import Tensor
 
 from . import _lib
 from ._lib import (HpdBuffers, HpdCocoDets, HpdCocoEvalOutputs, HpdCocoEvalParams, HpdCocoGts, HpdImage, HpdMap,
-                   HpdParams, HpdRecordLayout, HpdScaleInputs, HpdStageInputs, HpdTrackParams)
+                   HpdParams, HpdRecordLayout, HpdScaleInputs, HpdSmoothParams, HpdStageInputs, HpdTrackParams)
 
 COCO_FLIP_INDEX = [0, 2, 1, 4, 3, 6, 5, 8, 7, 10, 9, 12, 11, 14, 13, 16, 15]  # transforms.py:11
 JOINTS_ORDER_17 = [0, 1, 2, 3, 4, 5, 6, 11, 12, 7, 8, 9, 10, 13, 14, 15, 16]   # grouping.py:63-65
@@ -460,8 +461,7 @@ def run_track_reset(params: HpdTrackParams, state: Tensor, clear_ids: bool):
     _lib.check(rc, "hpd_track_reset")
 
 
-def run_track(params: HpdTrackParams, records: Tensor, state: Tensor, out: Tensor) -> Tensor:
-    """hpd_track on the current stream: records uint8 [n, row_bytes] (rows packed, read in place) -> out int32 [n, M]."""
+def _check_track_args(params: HpdTrackParams, records: Tensor, state: Tensor, out: Tensor):
     row_bytes = record_layout(params.num_kpts, params.max_people, params.emb).row_bytes
     if (not records.is_cuda or records.dtype != torch.uint8 or records.dim() != 2 or records.shape[1] != row_bytes
             or records.stride(1) != 1 or (records.shape[0] > 1 and records.stride(0) != row_bytes)):
@@ -470,6 +470,12 @@ def run_track(params: HpdTrackParams, records: Tensor, state: Tensor, out: Tenso
     n, M = records.shape[0], params.max_people
     if tuple(out.shape) != (n, M) or out.dtype != torch.int32 or not out.is_contiguous() or out.device != records.device:
         raise _lib.HpdError(f"track: out must be a contiguous int32 tensor {(n, M)} on the records' device")
+
+
+def run_track(params: HpdTrackParams, records: Tensor, state: Tensor, out: Tensor) -> Tensor:
+    """hpd_track on the current stream: records uint8 [n, row_bytes] (rows packed, read in place) -> out int32 [n, M]."""
+    _check_track_args(params, records, state, out)
+    n = records.shape[0]
     if n == 0:
         return out
     L = _lib.lib()
@@ -479,6 +485,41 @@ def run_track(params: HpdTrackParams, records: Tensor, state: Tensor, out: Tenso
     _lib.check(rc, "hpd_track")
     _count(L)
     return out
+
+
+def smooth_params(fps: float, min_cutoff: float, beta: float, d_cutoff: float) -> HpdSmoothParams:
+    """HpdSmoothParams; the library checks ranges."""
+    sp = HpdSmoothParams()
+    sp.min_cutoff, sp.beta, sp.d_cutoff, sp.fps = float(min_cutoff), float(beta), float(d_cutoff), float(fps)
+    return sp
+
+
+def track_smooth_state_bytes(params: HpdTrackParams) -> int:
+    n = ctypes.c_size_t(0)
+    _lib.check(_lib.lib().hpd_track_smooth_state_bytes(ctypes.byref(params), ctypes.byref(n)),
+               "hpd_track_smooth_state_bytes")
+    return n.value
+
+
+def run_track_smooth(params: HpdTrackParams, sparams: HpdSmoothParams, records: Tensor, state: Tensor, out: Tensor,
+                     coords: Tensor) -> Tuple[Tensor, Tensor]:
+    """hpd_track_smooth on the current stream: records uint8 [n, row_bytes] -> out int32 [n, M] and coords float64
+    [n, M, K, 2]."""
+    _check_track_args(params, records, state, out)
+    n, M, K = records.shape[0], params.max_people, params.num_kpts
+    if (tuple(coords.shape) != (n, M, K, 2) or coords.dtype != torch.float64 or not coords.is_contiguous()
+            or coords.device != records.device):
+        raise _lib.HpdError(f"track_smooth: coords must be a contiguous float64 tensor {(n, M, K, 2)} on the records' "
+                            "device")
+    if n == 0:
+        return out, coords
+    L = _lib.lib()
+    with torch.cuda.device(records.device):
+        rc = L.hpd_track_smooth(ctypes.byref(params), ctypes.byref(sparams), records.data_ptr(), n, state.data_ptr(),
+                                state.numel(), out.data_ptr(), coords.data_ptr(), _stream_ptr(records.device))
+    _lib.check(rc, "hpd_track_smooth")
+    _count(L)
+    return out, coords
 
 
 def _scales_from_lists(hm_lo, hm_hi, tag, hm_lo_f, hm_hi_f, tag_f):
@@ -760,6 +801,27 @@ def track_op(records: Tensor, state: Tensor, num_kpts: int, max_people: int, emb
 @track_op.register_fake
 def _(records, state, num_kpts, max_people, emb, max_age, min_keypoints, oks_thr, kpt_vars):
     return records.new_empty((records.shape[0], max_people), dtype=torch.int32)
+
+
+@torch.library.custom_op("hpd::track_smooth", mutates_args=("state",))
+def track_smooth_op(records: Tensor, state: Tensor, num_kpts: int, max_people: int, emb: int, max_age: int,
+                    min_keypoints: int, oks_thr: float, kpt_vars: Sequence[float], fps: float, min_cutoff: float,
+                    beta: float, d_cutoff: float) -> Tuple[Tensor, Tensor]:
+    """hpd::track's ids plus the tracked joints' One-Euro-filtered COCO-section coordinates (hpd_track_smooth):
+    -> (int32 [n, max_people], float64 [n, max_people, num_kpts, 2]); ``state`` is a smoothing tracker state."""
+    params = track_params(num_kpts, max_people, emb, max_age, min_keypoints, oks_thr, kpt_vars)
+    n = records.shape[0]
+    out = torch.empty((n, max_people), device=records.device, dtype=torch.int32)
+    coords = torch.empty((n, max_people, num_kpts, 2), device=records.device, dtype=torch.float64)
+    return run_track_smooth(params, smooth_params(fps, min_cutoff, beta, d_cutoff), records, state, out, coords)
+
+
+@track_smooth_op.register_fake
+def _(records, state, num_kpts, max_people, emb, max_age, min_keypoints, oks_thr, kpt_vars, fps, min_cutoff, beta,
+      d_cutoff):
+    n = records.shape[0]
+    return (records.new_empty((n, max_people), dtype=torch.int32),
+            records.new_empty((n, max_people, num_kpts, 2), dtype=torch.float64))
 
 
 @prepare_input_op.register_fake

@@ -99,6 +99,7 @@ class InferenceKeypointsResult(BaseKeypointsResult):
     det_thr: float
     tag_thr: float
     track_ids: Optional[np.ndarray] = None   # int32 [P]: the persons' ids across frames (model.stream(track=True))
+    smoothed_coords: Optional[np.ndarray] = None   # [P,K,2]: kpts_coords One-Euro filtered (model.stream(smooth=...))
 
     @classmethod
     def get_final_kpts_coords(cls, kpts_coords: np.ndarray, center, scale, hm_size) -> np.ndarray:
@@ -149,13 +150,14 @@ class InferenceKeypointsResult(BaseKeypointsResult):
                      kpts_heatmaps=None, tags_heatmaps=None) -> "InferenceKeypointsResult":
         """Image b of a batch's host records -> the reference's result object (results.py:240-263).  The batched
         callers pass no maps (they stay on the device); ``from_preds`` passes them like the reference.  Records that
-        carry track ids give the image's persons theirs."""
+        carry track ids give the image's persons theirs, and smoothed coordinates, with ``kpts_coords``' dtype."""
         grouped_joints, obj_scores = rec.image(b)
         return cls(raw_image=raw_image, annot=annot, model_input_image=model_input_image, kpts_heatmaps=kpts_heatmaps,
                    tags_heatmaps=tags_heatmaps, kpts_coords=rec.final_coords(b), kpts_scores=grouped_joints[..., 2],
                    kpts_tags=grouped_joints[..., 3:], obj_scores=obj_scores, limbs=limbs, det_thr=det_thr,
                    tag_thr=tag_thr,
-                   track_ids=None if rec.track_ids is None else rec.track_ids[b, :len(obj_scores)].copy())
+                   track_ids=None if rec.track_ids is None else rec.track_ids[b, :len(obj_scores)].copy(),
+                   smoothed_coords=None if rec.smoothed_coords is None else rec.smoothed_final_coords(b))
 
 
 class KeypointsResult(BaseKeypointsResult):

@@ -13,17 +13,19 @@ frames instead and keeps ``depth`` batches in flight (``DecodePipeline`` lanes);
 5. one device->host copy of the batch's records into the lane's pinned records slot;
 6. with ``track=True``, on the stream's own tracking stream and in submission order: it waits for the batch's records,
    runs ``PoseTracker.update`` on them in place (``hpd_track``) and copies the ids into the lane's pinned ids slot.  A
-   change of frame size, which closes a batch, also resets the tracker (ids are not reused).
+   change of frame size, which closes a batch, also resets the tracker (ids are not reused).  With ``smooth``, the
+   tracker also filters the tracked joints (``PoseTracker.update_smoothed``, ``hpd_track_smooth``) and their coordinates
+   go to the lane's pinned coordinates slot in the same way; the size-change reset drops the filters with the tracks.
 
 A lane and its staging slot are reused only after the host has waited for that lane's records copy and, when
-tracking, its ids copy (events, not a device synchronise), so a lane's records are tracked before they are overwritten.  A batch closes when it is full or when the frame size changes, so frames of mixed sizes work;
+tracking, its ids (and coordinates) copy (events, not a device synchronise), so a lane's records are tracked before they are overwritten.  A batch closes when it is full or when the frame size changes, so frames of mixed sizes work;
 results come back in submission order either way.  Geometry is computed once per distinct frame size.
 
 The stream decodes into the model decoder's buffer sets (slot = lane): do not call the model's other entry points
 while a stream still has batches in flight (``results()`` drains it).
 """
 from collections import OrderedDict, deque
-from typing import Iterable, Iterator, List
+from typing import Iterable, Iterator, List, Optional
 
 import numpy as np
 import torch
@@ -31,7 +33,7 @@ import torch
 from . import _lib, geometry, ops
 from .decoder import DecodePipeline, Records
 from .results import InferenceKeypointsResult
-from .track import PoseTracker
+from .track import OneEuro, PoseTracker
 
 
 class FrameStream:
@@ -39,15 +41,21 @@ class FrameStream:
     frame in submission order: an InferenceKeypointsResult (no maps, like ``predict_batch``) or, with
     ``records=True``, the frame's ``Records`` (one row).  Frames are uint8 [h,w,3] NumPy arrays or CUDA tensors.
     ``track=True``: the stream owns a ``PoseTracker`` (``tracker``, default settings) and every result carries its
-    persons' ids across frames (``track_ids``)."""
+    persons' ids across frames (``track_ids``).  ``smooth=OneEuro(fps)`` (needs ``track=True``): the tracker also
+    One-Euro filters the tracked joints, and every result carries ``smoothed_coords``."""
 
     MAX_SIZES = 64    # distinct frame sizes whose geometry is kept
 
-    def __init__(self, model, batch_size: int = 8, depth: int = 4, records: bool = False, track: bool = False):
+    def __init__(self, model, batch_size: int = 8, depth: int = 4, records: bool = False, track: bool = False,
+                 smooth: Optional[OneEuro] = None):
         if batch_size < 1 or depth < 1:
             raise ValueError(f"batch_size and depth must be >= 1 (got {batch_size}, {depth})")
+        if smooth is not None and not track:
+            raise ValueError("smooth needs track=True: the filters follow the tracks")
+        if smooth is not None and not isinstance(smooth, OneEuro):
+            raise TypeError(f"smooth must be a hpdecode.OneEuro or None (got {type(smooth).__name__})")
         self.model, self.batch_size, self.depth, self.records = model, int(batch_size), int(depth), records
-        self.track = bool(track)
+        self.track, self.smooth = bool(track), smooth
         self._open: list = []           # frames of the batch being filled
         self._open_hw = None
         self._inflight = deque()        # launched batches, oldest first
@@ -136,10 +144,13 @@ class FrameStream:
         self._shape_only = {}
         self.tracker = None
         if self.track:
-            self.tracker = PoseTracker(K, M, E, self.device)
+            self.tracker = PoseTracker(K, M, E, self.device, smoothing=self.smooth)
             self._track_stream = torch.cuda.Stream(device=self.device)
             self._track_stream.wait_stream(torch.cuda.current_stream(self.device))   # the tracker's initial reset
             self._host_ids = torch.empty((self.depth, self.batch_size, M), dtype=torch.int32, pin_memory=True)
+            if self.smooth is not None:
+                self._host_xy = torch.empty((self.depth, self.batch_size, M, K, 2), dtype=torch.float64,
+                                            pin_memory=True)
             self._track_hw = None
 
     def _stage(self, f, i):
@@ -207,7 +218,8 @@ class FrameStream:
         return lane, frames, res, tracked     # res keeps the lane's buffer set alive until the batch is retired
 
     def _track(self, lane, hw, res, written):
-        """Tracks the batch's records on the tracking stream once they are written; -> the event of the ids copy."""
+        """Tracks the batch's records on the tracking stream once they are written; -> the event of the ids (and
+        coordinates) copy."""
         st = self._track_stream
         st.wait_event(written)
         res.records.record_stream(st)
@@ -215,7 +227,11 @@ class FrameStream:
             if self._track_hw is not None and hw != self._track_hw:
                 self.tracker.reset()
             self._track_hw = hw
-            ids = self.tracker.update(res.records)
+            if self.smooth is None:
+                ids = self.tracker.update(res.records)
+            else:
+                ids, xy = self.tracker.update_smoothed(res.records)
+                self._host_xy[lane][:xy.shape[0]].copy_(xy, non_blocking=True)
             self._host_ids[lane][:ids.shape[0]].copy_(ids, non_blocking=True)
             done = torch.cuda.Event()
             done.record()
@@ -228,13 +244,16 @@ class FrameStream:
         lane, frames, res, tracked = batch
         res.ready.synchronize()
         raw = self._host_rec[lane][:len(frames)].numpy().copy()
-        ids = None
+        ids = xy = None
         if tracked is not None:
             tracked.synchronize()
             ids = self._host_ids[lane][:len(frames)].numpy().copy()
+            if self.smooth is not None:
+                xy = self._host_xy[lane][:len(frames)].numpy().copy()
         M, K, E = self._rec_shape
         if self.records:
-            return [Records(raw[b:b + 1], M, K, E, None if ids is None else ids[b:b + 1]) for b in range(len(frames))]
-        m, rec = self.model, Records(raw, M, K, E, ids)
+            return [Records(raw[b:b + 1], M, K, E, None if ids is None else ids[b:b + 1],
+                            None if xy is None else xy[b:b + 1]) for b in range(len(frames))]
+        m, rec = self.model, Records(raw, M, K, E, ids, xy)
         return [InferenceKeypointsResult.from_records(rec, b, f, None, None, m.limbs, m.det_thr, m.tag_thr)
                 for b, f in enumerate(frames)]

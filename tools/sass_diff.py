@@ -5,7 +5,8 @@ contains one of the patterns (default: every kernel): "identical", "DIFFERS" or 
 A kernel of NEW that gained a trailing `float` template argument (the element type of the inputs) is compared with the
 OLD kernel without it, and the aggregation kernels that lost their tag-map arguments with the OLD tag-less variants:
 agg_nms_x2_kernel<E, NW, T, false> -> <NW, T>, agg_nms_ms_kernel<E, NW, NS, T> -> <NW, NS, T> (both E of OLD map to
-the one NEW kernel).  Instruction text and encodings are compared; only the offset comments are dropped.
+the one NEW kernel), and track_kernel<false> with the untemplated OLD track_kernel.  Instruction text and encodings
+are compared; only the offset comments and the padding between them are dropped.
 Needs only the CUDA toolkit (cuobjdump, c++filt): no GPU.
 """
 import re
@@ -22,9 +23,23 @@ def kernels(lib):
             cur = out.setdefault(m.group(1), [])
             continue
         if cur is not None and line.strip().startswith("/*"):
-            cur.append(re.sub(r"^\s*/\*[0-9a-f]{4,}\*/", "", line).strip())
+            # cuobjdump pads the encoding comment to a column that depends on the listing: whitespace is not compared
+            cur.append(re.sub(r"\s+", " ", re.sub(r"^\s*/\*[0-9a-f]{4,}\*/", "", line).strip()))
     names = subprocess.run(["c++filt"], input="\n".join(out), capture_output=True, text=True).stdout.splitlines()
-    return {re.sub(r"^void |\(.*\)$", "", n): v for n, v in zip(names, out.values())}
+    return {strip_params(re.sub(r"^void ", "", n)): v for n, v in zip(names, out.values())}
+
+
+def strip_params(name):
+    """Demangled signature -> name: drops the trailing parameter list, whose parentheses balance (a name may hold
+    `(anonymous namespace)`)."""
+    if not name.endswith(")"):
+        return name
+    depth = 0
+    for i in range(len(name) - 1, -1, -1):
+        depth += {")": 1, "(": -1}.get(name[i], 0)
+        if depth == 0:
+            return name[:i]
+    return name
 
 
 def without_tag_args(name):
@@ -36,6 +51,7 @@ def without_tag_args(name):
 def main(old_lib, new_lib, patterns):
     old, new = kernels(old_lib), kernels(new_lib)
     alias = {re.sub(r", float>$", ">", n): n for n in new}   # new name without the float element type -> new name
+    alias.update({n[:-len("<false>")]: n for n in new if n.endswith("track_kernel<false>")})
     seen, rows = set(), []
     for name in sorted(old):
         if patterns and not any(p in name for p in patterns):
