@@ -422,6 +422,64 @@ HPD_EXPORT int hpd_track_smooth(const HpdTrackParams* p, const HpdSmoothParams* 
                                 int n_frames, void* state, size_t state_bytes, int32_t* track_ids, double* coords,
                                 void* stream);
 
+/* ---- drawing decoded poses into frames (skeletons and joints, for video overlays) -------------------------------
+ * For frame f with record R (HpdRecordLayout for num_kpts, max_people, emb), optional ids[f][M] and optional
+ * coords[f][M][K][2]:
+ *  - Persons drawn: none when R's flags bit 0 is set (the empty-scene fallback's pseudo-person is not a person);
+ *    otherwise p < clamp(n_person, 0, M), in ascending p.
+ *  - Joint position: coords[f][p][k] when coords are given, else the COCO-section (x, y) of R (float64, raw-frame
+ *    pixels).  Joint visible: (double)poses[p][k][2] > kpt_thr, and both coordinates finite with |x|, |y| <= 2^20
+ *    (32 times the largest frame side: every product below stays finite).
+ *  - Pixel (c, r) has its centre at X = c, Y = r: cv2.warpAffine's convention, which the input side reproduces, so
+ *    the convention of the records' coordinates.
+ *  - All float64, each step one correctly rounded operation, no FMA, grouped left to right as written.
+ *    Joint disc of radius Rj at (jx, jy): covered iff (X-jx)*(X-jx) + (Y-jy)*(Y-jy) <= Rj*Rj.
+ *    Limb (a, b), both joints visible, h = thickness / 2: ex = bx-ax, ey = by-ay, L2 = ex*ex + ey*ey, px = X-ax,
+ *    py = Y-ay, t = px*ex + py*ey; then
+ *      t <= 0  (a zero-length limb lands here):  covered iff px*px + py*py <= h*h;
+ *      t >= L2:                                   covered iff (X-bx)*(X-bx) + (Y-by)*(Y-by) <= h*h;
+ *      else, with cr = px*ey - py*ex:             covered iff cr*cr <= (h*h)*L2.
+ *  - Paint order: per person p, its limbs in list order, then its joints 0..K-1.  A covered pixel takes the colour
+ *    of the LAST primitive that covers it; uncovered pixels are copied from the input; row padding past 3w bytes of
+ *    the output is not written.  No blending, no anti-aliasing.  thickness 0 draws no limbs, joint_radius 0 no joints.
+ *  - Colours are three bytes in the frame's own channel order.  Without ids limb l takes limb_rgb[l]; with ids a
+ *    person with id >= 0 takes track_rgb[id % num_track_colors] for all its limbs, one with id < 0 untracked_rgb.
+ *    Joints always take joint_rgb. */
+#define HPD_RENDER_MAX_LIMBS 64
+#define HPD_RENDER_MAX_COLORS 32
+typedef struct HpdRenderParams {
+  int32_t num_kpts;       /* K <= HPD_MAX_KPTS */
+  int32_t max_people;     /* M <= HPD_MAX_PEOPLE: persons per record */
+  int32_t emb;            /* E of the records: 1 or 2 */
+  int32_t num_limbs;      /* 0..HPD_RENDER_MAX_LIMBS */
+  int32_t limbs[HPD_RENDER_MAX_LIMBS][2];       /* joint indices in [0, K), distinct within a limb */
+  uint8_t limb_rgb[HPD_RENDER_MAX_LIMBS][3];
+  uint8_t joint_rgb[3];
+  uint8_t untracked_rgb[3];
+  uint8_t reserved0_[2];
+  int32_t num_track_colors;                     /* 1..HPD_RENDER_MAX_COLORS */
+  int32_t reserved1_;
+  uint8_t track_rgb[HPD_RENDER_MAX_COLORS][3];
+  double thickness;       /* limb width in pixels, finite, in [0, 1024] */
+  double joint_radius;    /* finite, in [0, 1024] */
+  double kpt_thr;         /* finite */
+} HpdRenderParams;
+
+/* One frame: uint8 HWC, 3 channels, on the device.  out must not overlap any frame's input or another output. */
+typedef struct HpdRenderFrame {
+  const uint8_t* in;
+  uint8_t* out;
+  int64_t in_stride_row, out_stride_row;   /* bytes between rows, >= 3*w */
+  int32_t h, w;                            /* 1..32767 */
+} HpdRenderFrame;
+
+/* Draws frames_host[f] (descriptors on the host) with the persons of records + f * row_bytes (read in place, 8-byte
+ * aligned), track_ids [n_frames][max_people] int32 (NULL: no ids) and coords [n_frames][max_people][num_kpts][2]
+ * float64 (NULL: the records' COCO section; 8-byte aligned).  Out of place only.  One launch per 32 frames; no
+ * allocation, no workspace.  Every argument is checked before the first launch. */
+HPD_EXPORT int hpd_render_poses(const HpdRenderParams* p, const HpdRenderFrame* frames_host, int n_frames,
+                                const uint8_t* records, const int32_t* track_ids, const double* coords, void* stream);
+
 /* Number of kernel launches the previous call on this thread enqueued (for bench accounting). */
 HPD_EXPORT int hpd_last_launch_count(void);
 

@@ -278,6 +278,12 @@ int hpd_track_smooth(const HpdTrackParams* p, const HpdSmoothParams* sp, const u
   return launch_track_smooth(p, sp, records, n_frames, state, state_bytes, track_ids, coords, (cudaStream_t)stream);
 }
 
+int hpd_render_poses(const HpdRenderParams* p, const HpdRenderFrame* frames_host, int n_frames, const uint8_t* records,
+                     const int32_t* track_ids, const double* coords, void* stream) {
+  g_launches = 0;
+  return launch_render_poses(p, frames_host, n_frames, records, track_ids, coords, (cudaStream_t)stream);
+}
+
 int hpd_decode(const HpdParams* p, const HpdScaleInputs* scales, const HpdBuffers* buf, void* workspace,
                size_t workspace_bytes, void* stream) {
   g_launches = 0;

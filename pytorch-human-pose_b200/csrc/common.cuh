@@ -237,5 +237,7 @@ int launch_track(const HpdTrackParams* p, const uint8_t* records, int n_frames, 
 size_t track_smooth_state_bytes(const HpdTrackParams* p);
 int launch_track_smooth(const HpdTrackParams* p, const HpdSmoothParams* sp, const uint8_t* records, int n_frames,
                         void* state, size_t state_bytes, int32_t* track_ids, double* coords, cudaStream_t st);
+int launch_render_poses(const HpdRenderParams* p, const HpdRenderFrame* frames, int n_frames, const uint8_t* records,
+                        const int32_t* track_ids, const double* coords, cudaStream_t st);
 
 }  // namespace hpd

@@ -13,11 +13,12 @@ from .results import BaseKeypointsResult, InferenceKeypointsResult, KeypointsRes
 from .model import InferenceKeypointsModel  # noqa: F401
 from .stream import FrameStream  # noqa: F401
 from .track import OneEuro, PoseTracker  # noqa: F401
+from .render import PoseRenderer, PoseStyle  # noqa: F401
 from .coco import batch_to_coco, eval_coco, evaluate_dataset_batched, result_to_coco  # noqa: F401
 from .cocoeval import KeypointEvaluator, KeypointGroundTruth  # noqa: F401
 
 __all__ = ["BottomUpDecoder", "DecodePipeline", "DecodeResult", "Records", "MPPEHeatmapParser", "BaseKeypointsResult",
            "InferenceKeypointsResult", "KeypointsResult", "InferenceKeypointsModel", "FrameStream", "PoseTracker",
-           "OneEuro", "batch_to_coco",
+           "OneEuro", "PoseRenderer", "PoseStyle", "batch_to_coco",
            "evaluate_dataset_batched", "result_to_coco", "geometry", "ops", "eval_coco", "KeypointEvaluator",
            "KeypointGroundTruth"]

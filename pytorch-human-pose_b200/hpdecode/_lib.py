@@ -15,6 +15,7 @@ HPD_ABI_VERSION = 6
 HPD_COCO_MAX_IOU_THRS, HPD_COCO_MAX_REC_THRS, HPD_COCO_MAX_AREAS, HPD_COCO_MAX_PER_IMAGE = 16, 128, 4, 1024
 HPD_F32, HPD_F16, HPD_BF16 = 0, 1, 2
 HPD_TRACK_MAX_AGE = 8
+HPD_RENDER_MAX_LIMBS, HPD_RENDER_MAX_COLORS = 64, 32
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libhpdecode.so")
@@ -25,7 +26,7 @@ EXPORTS = (
     "hpd_record_layout", "hpd_multi_scale_size", "hpd_get_affine_transform", "hpd_prepare_input", "hpd_prepare_geometry",
     "hpd_aggregate_tags", "hpd_coco_eval_workspace_bytes", "hpd_coco_eval", "hpd_prepare_inputs",
     "hpd_aggregate_nms_stages", "hpd_decode_stages", "hpd_track_state_bytes", "hpd_track_reset", "hpd_track",
-    "hpd_track_smooth_state_bytes", "hpd_track_smooth",
+    "hpd_track_smooth_state_bytes", "hpd_track_smooth", "hpd_render_poses",
 )
 
 
@@ -107,6 +108,20 @@ class HpdSmoothParams(ctypes.Structure):
     _fields_ = [(n, ctypes.c_double) for n in ("min_cutoff", "beta", "d_cutoff", "fps")]
 
 
+class HpdRenderParams(ctypes.Structure):
+    _fields_ = [(n, ctypes.c_int32) for n in ("num_kpts", "max_people", "emb", "num_limbs")] + [
+        ("limbs", (ctypes.c_int32 * 2) * HPD_RENDER_MAX_LIMBS), ("limb_rgb", (ctypes.c_uint8 * 3) * HPD_RENDER_MAX_LIMBS),
+        ("joint_rgb", ctypes.c_uint8 * 3), ("untracked_rgb", ctypes.c_uint8 * 3), ("reserved0_", ctypes.c_uint8 * 2),
+        ("num_track_colors", ctypes.c_int32), ("reserved1_", ctypes.c_int32),
+        ("track_rgb", (ctypes.c_uint8 * 3) * HPD_RENDER_MAX_COLORS)] + [
+        (n, ctypes.c_double) for n in ("thickness", "joint_radius", "kpt_thr")]
+
+
+class HpdRenderFrame(ctypes.Structure):
+    _fields_ = [("in", ctypes.c_void_p), ("out", ctypes.c_void_p), ("in_stride_row", ctypes.c_int64),
+                ("out_stride_row", ctypes.c_int64), ("h", ctypes.c_int32), ("w", ctypes.c_int32)]
+
+
 class HpdError(RuntimeError):
     pass
 
@@ -161,6 +176,8 @@ def lib():
     L.hpd_track.argtypes = [TP, V, ctypes.c_int, V, ctypes.c_size_t, V, V]
     L.hpd_track_smooth_state_bytes.argtypes = [TP, ctypes.POINTER(ctypes.c_size_t)]
     L.hpd_track_smooth.argtypes = [TP, ctypes.POINTER(HpdSmoothParams), V, ctypes.c_int, V, ctypes.c_size_t, V, V, V]
+    L.hpd_render_poses.argtypes = [ctypes.POINTER(HpdRenderParams), ctypes.POINTER(HpdRenderFrame), ctypes.c_int, V, V, V,
+                                   V]
     for n in EXPORTS:
         if n not in ("hpd_last_error_string",):
             getattr(L, n).restype = ctypes.c_int

@@ -22,12 +22,13 @@ class Records:
     include/hpdecode.h): ``raw`` is the uint8 [B,row_bytes] array of ONE device->host copy; the fields are
     zero-copy NumPy views into it.  ``track_ids``: optional int32 [B,M] person ids across frames (PoseTracker);
     ``smoothed_coords``: optional float64 [B,M,K,2] One-Euro-filtered COCO-section coordinates (PoseTracker with
-    smoothing)."""
+    smoothing); ``rendered``: optional uint8 [B,h,w,3] frames with their persons drawn (PoseRenderer), a NumPy array
+    or a CUDA tensor."""
 
     def __init__(self, raw: np.ndarray, M: int, K: int, E: int, track_ids: Optional[np.ndarray] = None,
-                 smoothed_coords: Optional[np.ndarray] = None):
+                 smoothed_coords: Optional[np.ndarray] = None, rendered=None):
         L = ops.record_layout(K, M, E)
-        self.track_ids, self.smoothed_coords = track_ids, smoothed_coords
+        self.track_ids, self.smoothed_coords, self.rendered = track_ids, smoothed_coords, rendered
         raw = np.ascontiguousarray(raw, np.uint8).reshape(-1, L.row_bytes)
         self.raw, self.M, self.K, self.E = raw, M, K, E
         B, D, C = raw.shape[0], 3 + E, L.coco_stride

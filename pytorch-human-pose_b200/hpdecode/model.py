@@ -170,16 +170,17 @@ class InferenceKeypointsModel:
         return results
 
     def stream(self, frames: Iterable, batch_size: int = 8, depth: int = 4, records: bool = False,
-               track: bool = False, smooth=None) -> Iterator:
+               track: bool = False, smooth=None, render=None) -> Iterator:
         """Frame-stream inference (video, a directory of images): uint8 [h,w,3] frames (host arrays or CUDA tensors)
         in, one result per frame out, in input order -- an InferenceKeypointsResult (no maps), or the frame's
         Records with ``records=True``.  Up to ``batch_size`` frames of one size share a batch, ``depth`` batches are
         in flight (hpdecode.stream.FrameStream); results are yielded as their batches complete.  ``track=True``: the
         results' ``track_ids`` number the persons consistently across frames (hpdecode.track.PoseTracker);
         ``smooth=hpdecode.OneEuro(fps)`` (with ``track=True``) also gives them ``smoothed_coords``, the tracked joints
-        One-Euro filtered."""
+        One-Euro filtered.  ``render=hpdecode.PoseStyle(...)`` gives every result ``rendered``, the frame with its persons
+        drawn on the device (coloured by track with ``track=True``, at the smoothed coordinates with ``smooth``)."""
         from .stream import FrameStream
-        fs = FrameStream(self, batch_size, depth, records, track, smooth)
+        fs = FrameStream(self, batch_size, depth, records, track, smooth, render)
         for frame in frames:
             fs.submit([frame])
             yield from fs.results(wait=False)

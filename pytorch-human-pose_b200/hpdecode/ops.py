@@ -17,6 +17,7 @@ Stage ops mirror the reference methods one to one (paths relative to /root/refer
   hpd::coco_eval      pycocotools COCOeval(..., "keypoints").evaluate() + accumulate() (bin/eval.py:52-65)
   hpd::track          person ids across consecutive frames' result records (greedy OKS tracking; hpdecode.track)
   hpd::track_smooth   the same ids plus the tracked joints' One-Euro-filtered coordinates (hpdecode.track.OneEuro)
+  hpd::render_poses   skeletons and joints drawn into copies of frames from their result records (hpdecode.render)
 """
 import ctypes
 from typing import List, Optional, Sequence, Tuple
@@ -26,7 +27,8 @@ from torch import Tensor
 
 from . import _lib
 from ._lib import (HpdBuffers, HpdCocoDets, HpdCocoEvalOutputs, HpdCocoEvalParams, HpdCocoGts, HpdImage, HpdMap,
-                   HpdParams, HpdRecordLayout, HpdScaleInputs, HpdSmoothParams, HpdStageInputs, HpdTrackParams)
+                   HpdParams, HpdRecordLayout, HpdRenderFrame, HpdRenderParams, HpdScaleInputs, HpdSmoothParams,
+                   HpdStageInputs, HpdTrackParams)
 
 COCO_FLIP_INDEX = [0, 2, 1, 4, 3, 6, 5, 8, 7, 10, 9, 12, 11, 14, 13, 16, 15]  # transforms.py:11
 JOINTS_ORDER_17 = [0, 1, 2, 3, 4, 5, 6, 11, 12, 7, 8, 9, 10, 13, 14, 15, 16]   # grouping.py:63-65
@@ -522,6 +524,74 @@ def run_track_smooth(params: HpdTrackParams, sparams: HpdSmoothParams, records: 
     return out, coords
 
 
+def render_params(K: int, M: int, E: int, limbs: Sequence[int], limb_colors: Sequence[int], joint_color: Sequence[int],
+                  track_colors: Sequence[int], untracked_color: Sequence[int], thickness: float, joint_radius: float,
+                  kpt_thr: float) -> HpdRenderParams:
+    """HpdRenderParams; limbs and colour lists are flat ([a0, b0, a1, b1, ...], [r, g, b, r, g, b, ...]).  The library
+    checks ranges."""
+    L = len(limbs) // 2
+    C = len(track_colors) // 3
+    if (len(limbs) % 2 or L > _lib.HPD_RENDER_MAX_LIMBS or len(limb_colors) != 3 * L or len(track_colors) % 3
+            or C > _lib.HPD_RENDER_MAX_COLORS or len(joint_color) != 3 or len(untracked_color) != 3):
+        raise _lib.HpdError(f"render: up to {_lib.HPD_RENDER_MAX_LIMBS} limbs with one colour each, up to "
+                            f"{_lib.HPD_RENDER_MAX_COLORS} track colours, colours of 3 bytes")
+    p = HpdRenderParams()
+    p.num_kpts, p.max_people, p.emb, p.num_limbs, p.num_track_colors = K, M, E, L, C
+    for l in range(L):
+        p.limbs[l][0], p.limbs[l][1] = limbs[2 * l], limbs[2 * l + 1]
+        for c in range(3):
+            p.limb_rgb[l][c] = limb_colors[3 * l + c]
+    for i in range(C):
+        for c in range(3):
+            p.track_rgb[i][c] = track_colors[3 * i + c]
+    for c in range(3):
+        p.joint_rgb[c], p.untracked_rgb[c] = joint_color[c], untracked_color[c]
+    p.thickness, p.joint_radius, p.kpt_thr = float(thickness), float(joint_radius), float(kpt_thr)
+    return p
+
+
+def _check_frame(t: Tensor, what: str):
+    if not t.is_cuda or t.dtype != torch.uint8 or t.dim() != 3 or t.shape[2] != 3 or t.stride(2) != 1 or t.stride(1) != 3:
+        raise _lib.HpdError(f"render: {what} must be a CUDA uint8 [h,w,3] tensor with packed pixels")
+
+
+def run_render(params: HpdRenderParams, frames: Sequence[Tensor], out: Sequence[Tensor], records: Tensor,
+               track_ids: Optional[Tensor] = None, coords: Optional[Tensor] = None) -> Sequence[Tensor]:
+    """hpd_render_poses on the current stream: frames[i] drawn with the persons of records[i] (uint8 [n, row_bytes],
+    rows packed) into out[i] (same size; any row stride).  track_ids: int32 [n, M]; coords: float64 [n, M, K, 2]."""
+    n, M, K = len(frames), params.max_people, params.num_kpts
+    row_bytes = record_layout(K, M, params.emb).row_bytes
+    if (not records.is_cuda or records.dtype != torch.uint8 or records.dim() != 2 or records.shape != (n, row_bytes)
+            or records.stride(1) != 1 or (n > 1 and records.stride(0) != row_bytes)):
+        raise _lib.HpdError(f"render: records must be a uint8 CUDA tensor [{n}, {row_bytes}] with packed rows")
+    dev = records.device
+    for name, t, dtype, shape in (("track_ids", track_ids, torch.int32, (n, M)),
+                                  ("coords", coords, torch.float64, (n, M, K, 2))):
+        if t is not None and (tuple(t.shape) != shape or t.dtype != dtype or not t.is_contiguous() or t.device != dev):
+            raise _lib.HpdError(f"render: {name} must be a contiguous {dtype} tensor {shape} on the records' device")
+    if len(out) != n:
+        raise _lib.HpdError("render: one output per frame")
+    if n == 0:
+        return out
+    arr = (HpdRenderFrame * n)()
+    for i, (f, o) in enumerate(zip(frames, out)):
+        _check_frame(f, "frame %d" % i)
+        _check_frame(o, "output %d" % i)
+        if f.device != dev or o.device != dev or f.shape != o.shape:
+            raise _lib.HpdError("render: frame %d and its output must have one size, on the records' device" % i)
+        setattr(arr[i], "in", f.data_ptr())
+        arr[i].out, arr[i].in_stride_row, arr[i].out_stride_row = o.data_ptr(), f.stride(0), o.stride(0)
+        arr[i].h, arr[i].w = f.shape[0], f.shape[1]
+    L = _lib.lib()
+    with torch.cuda.device(dev):
+        rc = L.hpd_render_poses(ctypes.byref(params), arr, n, records.data_ptr(),
+                                None if track_ids is None else track_ids.data_ptr(),
+                                None if coords is None else coords.data_ptr(), _stream_ptr(dev))
+    _lib.check(rc, "hpd_render_poses")
+    _count(L)
+    return out
+
+
 def _scales_from_lists(hm_lo, hm_hi, tag, hm_lo_f, hm_hi_f, tag_f):
     n = len(hm_lo)
     flip = len(hm_lo_f) > 0
@@ -822,6 +892,28 @@ def _(records, state, num_kpts, max_people, emb, max_age, min_keypoints, oks_thr
     n = records.shape[0]
     return (records.new_empty((n, max_people), dtype=torch.int32),
             records.new_empty((n, max_people, num_kpts, 2), dtype=torch.float64))
+
+
+@torch.library.custom_op("hpd::render_poses", mutates_args=())
+def render_poses_op(frames: Sequence[Tensor], records: Tensor, track_ids: Optional[Tensor], coords: Optional[Tensor],
+                    num_kpts: int, max_people: int, emb: int, limbs: Sequence[int], limb_colors: Sequence[int],
+                    joint_color: Sequence[int], track_colors: Sequence[int], untracked_color: Sequence[int],
+                    thickness: float, joint_radius: float, kpt_thr: float) -> List[Tensor]:
+    """Skeletons and joints of the persons of records[i] drawn into a new copy of frames[i] (hpd_render_poses; uint8
+    [h,w,3] CUDA frames, left unchanged): -> one new contiguous uint8 [h,w,3] tensor per frame.  ``limbs`` and the
+    colours are flat lists (pairs, RGB triples); ``track_ids`` int32 [n, max_people] and ``coords`` float64
+    [n, max_people, num_kpts, 2] are optional."""
+    params = render_params(num_kpts, max_people, emb, limbs, limb_colors, joint_color, track_colors, untracked_color,
+                           thickness, joint_radius, kpt_thr)
+    out = [torch.empty((f.shape[0], f.shape[1], 3), device=f.device, dtype=torch.uint8) for f in frames]
+    run_render(params, frames, out, records, track_ids, coords)
+    return out
+
+
+@render_poses_op.register_fake
+def _(frames, records, track_ids, coords, num_kpts, max_people, emb, limbs, limb_colors, joint_color, track_colors,
+      untracked_color, thickness, joint_radius, kpt_thr):
+    return [f.new_empty((f.shape[0], f.shape[1], 3), dtype=torch.uint8) for f in frames]
 
 
 @prepare_input_op.register_fake

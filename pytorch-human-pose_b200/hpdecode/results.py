@@ -11,7 +11,7 @@ evaluation consumers) are out of scope.
 the image's inverse affine matrix, so one device->host copy of the image's result record returns everything.
 """
 from dataclasses import dataclass
-from typing import List, Optional
+from typing import Any, List, Optional
 
 import numpy as np
 import torch
@@ -100,6 +100,8 @@ class InferenceKeypointsResult(BaseKeypointsResult):
     tag_thr: float
     track_ids: Optional[np.ndarray] = None   # int32 [P]: the persons' ids across frames (model.stream(track=True))
     smoothed_coords: Optional[np.ndarray] = None   # [P,K,2]: kpts_coords One-Euro filtered (model.stream(smooth=...))
+    rendered: Optional[Any] = None   # uint8 [h,w,3]: the frame with its persons drawn (model.stream(render=...)); a
+    #                                  NumPy array for a host frame, a CUDA tensor for a CUDA frame
 
     @classmethod
     def get_final_kpts_coords(cls, kpts_coords: np.ndarray, center, scale, hm_size) -> np.ndarray:
@@ -147,7 +149,7 @@ class InferenceKeypointsResult(BaseKeypointsResult):
 
     @classmethod
     def from_records(cls, rec: Records, b: int, raw_image, annot, model_input_image, limbs, det_thr, tag_thr,
-                     kpts_heatmaps=None, tags_heatmaps=None) -> "InferenceKeypointsResult":
+                     kpts_heatmaps=None, tags_heatmaps=None, rendered=None) -> "InferenceKeypointsResult":
         """Image b of a batch's host records -> the reference's result object (results.py:240-263).  The batched
         callers pass no maps (they stay on the device); ``from_preds`` passes them like the reference.  Records that
         carry track ids give the image's persons theirs, and smoothed coordinates, with ``kpts_coords``' dtype."""
@@ -157,7 +159,8 @@ class InferenceKeypointsResult(BaseKeypointsResult):
                    kpts_tags=grouped_joints[..., 3:], obj_scores=obj_scores, limbs=limbs, det_thr=det_thr,
                    tag_thr=tag_thr,
                    track_ids=None if rec.track_ids is None else rec.track_ids[b, :len(obj_scores)].copy(),
-                   smoothed_coords=None if rec.smoothed_coords is None else rec.smoothed_final_coords(b))
+                   smoothed_coords=None if rec.smoothed_coords is None else rec.smoothed_final_coords(b),
+                   rendered=rendered)
 
 
 class KeypointsResult(BaseKeypointsResult):

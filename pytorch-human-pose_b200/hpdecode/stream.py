@@ -15,10 +15,15 @@ frames instead and keeps ``depth`` batches in flight (``DecodePipeline`` lanes);
    runs ``PoseTracker.update`` on them in place (``hpd_track``) and copies the ids into the lane's pinned ids slot.  A
    change of frame size, which closes a batch, also resets the tracker (ids are not reused).  With ``smooth``, the
    tracker also filters the tracked joints (``PoseTracker.update_smoothed``, ``hpd_track_smooth``) and their coordinates
-   go to the lane's pinned coordinates slot in the same way; the size-change reset drops the filters with the tracks.
+   go to the lane's pinned coordinates slot in the same way; the size-change reset drops the filters with the tracks;
+7. with ``render=PoseStyle(...)``, the batch's frames are drawn with their persons (``hpd_render_poses``): on the
+   tracking stream after the tracker, with its ids and, with ``smooth``, the smoothed coordinates; without ``track``
+   on the lane's stream after the decode.  Host frames are drawn from the lane's staged copy into a per-lane device
+   buffer and copied into the lane's pinned rendered slot; CUDA frames are drawn into new CUDA tensors (the caller's
+   frames are not modified) and stay on the device.
 
 A lane and its staging slot are reused only after the host has waited for that lane's records copy and, when
-tracking, its ids (and coordinates) copy (events, not a device synchronise), so a lane's records are tracked before they are overwritten.  A batch closes when it is full or when the frame size changes, so frames of mixed sizes work;
+tracking, its ids (and coordinates) copy, and when rendering, its rendered copy (events, not a device synchronise), so a lane's records are tracked before they are overwritten.  A batch closes when it is full or when the frame size changes, so frames of mixed sizes work;
 results come back in submission order either way.  Geometry is computed once per distinct frame size.
 
 The stream decodes into the model decoder's buffer sets (slot = lane): do not call the model's other entry points
@@ -33,6 +38,7 @@ import torch
 from . import _lib, geometry, ops
 from .decoder import DecodePipeline, Records
 from .results import InferenceKeypointsResult
+from .render import PoseRenderer, PoseStyle
 from .track import OneEuro, PoseTracker
 
 
@@ -42,20 +48,24 @@ class FrameStream:
     ``records=True``, the frame's ``Records`` (one row).  Frames are uint8 [h,w,3] NumPy arrays or CUDA tensors.
     ``track=True``: the stream owns a ``PoseTracker`` (``tracker``, default settings) and every result carries its
     persons' ids across frames (``track_ids``).  ``smooth=OneEuro(fps)`` (needs ``track=True``): the tracker also
-    One-Euro filters the tracked joints, and every result carries ``smoothed_coords``."""
+    One-Euro filters the tracked joints, and every result carries ``smoothed_coords``.  ``render=PoseStyle(...)``: every
+    result carries ``rendered``, the frame with its persons drawn (coloured by track with ``track=True``): an owned
+    uint8 NumPy array for a host frame, a new CUDA tensor for a CUDA frame."""
 
     MAX_SIZES = 64    # distinct frame sizes whose geometry is kept
 
     def __init__(self, model, batch_size: int = 8, depth: int = 4, records: bool = False, track: bool = False,
-                 smooth: Optional[OneEuro] = None):
+                 smooth: Optional[OneEuro] = None, render: Optional[PoseStyle] = None):
         if batch_size < 1 or depth < 1:
             raise ValueError(f"batch_size and depth must be >= 1 (got {batch_size}, {depth})")
         if smooth is not None and not track:
             raise ValueError("smooth needs track=True: the filters follow the tracks")
         if smooth is not None and not isinstance(smooth, OneEuro):
             raise TypeError(f"smooth must be a hpdecode.OneEuro or None (got {type(smooth).__name__})")
+        if render is not None and not isinstance(render, PoseStyle):
+            raise TypeError(f"render must be a hpdecode.PoseStyle or None (got {type(render).__name__})")
         self.model, self.batch_size, self.depth, self.records = model, int(batch_size), int(depth), records
-        self.track, self.smooth = bool(track), smooth
+        self.track, self.smooth, self.render = bool(track), smooth, render
         self._open: list = []           # frames of the batch being filled
         self._open_hw = None
         self._inflight = deque()        # launched batches, oldest first
@@ -152,6 +162,11 @@ class FrameStream:
                 self._host_xy = torch.empty((self.depth, self.batch_size, M, K, 2), dtype=torch.float64,
                                             pin_memory=True)
             self._track_hw = None
+        self.renderer = None
+        if self.render is not None:
+            self.renderer = PoseRenderer(K, M, E, self.render, self.device)
+            self._rend_dev: List = [None] * self.depth    # per lane: host frames drawn, on the device
+            self._rend_host: List = [None] * self.depth   # per lane: their pinned copy
 
     def _stage(self, f, i):
         lane = self.pipe._next          # the lane the open batch will be submitted on
@@ -206,18 +221,46 @@ class FrameStream:
             return [m._net_outputs(x, xs_f[t] if m.use_flip else None) for t, x in enumerate(xs)]
 
         written = torch.cuda.Event()
+        outs = self._render_targets(lane, frames, hw) if self.render is not None else None
 
         def after_tail(ln, res):
             written.record()
             self._host_rec[lane][:n].copy_(res.records, non_blocking=True)
+            if outs is not None and not self.track:
+                self._draw(lane, imgs, frames, outs, res.records)
 
         ts = self._tag_scale
         res = self.pipe.submit(self._placeholders(n), (sizes_hw[2 * ts], sizes_hw[2 * ts + 1]), tag_scale=ts,
                                before_agg=before_agg, after_tail=after_tail, inv_affine=inv)
-        tracked = self._track(lane, hw, res, written) if self.track else None
-        return lane, frames, res, tracked     # res keeps the lane's buffer set alive until the batch is retired
+        tracked = self._track(lane, hw, res, written, imgs, frames, outs) if self.track else None
+        return lane, frames, res, tracked, outs     # res keeps the lane's buffer set alive until the batch is retired
 
-    def _track(self, lane, hw, res, written):
+    def _render_targets(self, lane, frames, hw):
+        """Where each frame is drawn: a slot of the lane's device buffer for a host frame, a new tensor (allocated on
+        the caller's stream) for a CUDA frame."""
+        h, w = hw
+        nb = h * w * 3
+        if any(not isinstance(f, torch.Tensor) for f in frames):
+            need = len(frames) * nb
+            if self._rend_dev[lane] is None or self._rend_dev[lane].numel() < need:
+                self._rend_dev[lane] = torch.empty((need,), dtype=torch.uint8, device=self.device)
+                self._rend_host[lane] = torch.empty((need,), dtype=torch.uint8, pin_memory=True)
+        return [torch.empty((h, w, 3), dtype=torch.uint8, device=self.device) if isinstance(f, torch.Tensor)
+                else self._rend_dev[lane][i * nb:(i + 1) * nb].view(h, w, 3) for i, f in enumerate(frames)]
+
+    def _draw(self, lane, imgs, frames, outs, records, ids=None, xy=None):
+        """Draws the batch on the current stream; host frames' drawings go on to the lane's pinned rendered slot."""
+        st = torch.cuda.current_stream(self.device)
+        for f, o in zip(frames, outs):
+            if isinstance(f, torch.Tensor):
+                f.record_stream(st)
+                o.record_stream(st)
+        ops.run_render(self.renderer.params, imgs, outs, records, ids, xy)
+        if any(not isinstance(f, torch.Tensor) for f in frames):
+            nb = len(frames) * outs[0].numel()
+            self._rend_host[lane][:nb].copy_(self._rend_dev[lane][:nb], non_blocking=True)
+
+    def _track(self, lane, hw, res, written, imgs, frames, outs):
         """Tracks the batch's records on the tracking stream once they are written; -> the event of the ids (and
         coordinates) copy."""
         st = self._track_stream
@@ -227,12 +270,15 @@ class FrameStream:
             if self._track_hw is not None and hw != self._track_hw:
                 self.tracker.reset()
             self._track_hw = hw
+            xy = None
             if self.smooth is None:
                 ids = self.tracker.update(res.records)
             else:
                 ids, xy = self.tracker.update_smoothed(res.records)
                 self._host_xy[lane][:xy.shape[0]].copy_(xy, non_blocking=True)
             self._host_ids[lane][:ids.shape[0]].copy_(ids, non_blocking=True)
+            if outs is not None:
+                self._draw(lane, imgs, frames, outs, res.records, ids, xy)
             done = torch.cuda.Event()
             done.record()
         return done
@@ -241,7 +287,7 @@ class FrameStream:
         return batch[2].ready.query() and (batch[3] is None or batch[3].query())
 
     def _finish(self, batch) -> list:
-        lane, frames, res, tracked = batch
+        lane, frames, res, tracked, outs = batch
         res.ready.synchronize()
         raw = self._host_rec[lane][:len(frames)].numpy().copy()
         ids = xy = None
@@ -250,10 +296,18 @@ class FrameStream:
             ids = self._host_ids[lane][:len(frames)].numpy().copy()
             if self.smooth is not None:
                 xy = self._host_xy[lane][:len(frames)].numpy().copy()
+        rendered = [None] * len(frames)
+        if outs is not None:
+            host = self._rend_host[lane]
+            for b, (f, o) in enumerate(zip(frames, outs)):
+                nb = o.numel()
+                rendered[b] = o if isinstance(f, torch.Tensor) else host[b * nb:(b + 1) * nb].numpy().reshape(o.shape).copy()
         M, K, E = self._rec_shape
         if self.records:
             return [Records(raw[b:b + 1], M, K, E, None if ids is None else ids[b:b + 1],
-                            None if xy is None else xy[b:b + 1]) for b in range(len(frames))]
+                            None if xy is None else xy[b:b + 1], None if r is None else r[None])
+                    for b, r in enumerate(rendered)]
         m, rec = self.model, Records(raw, M, K, E, ids, xy)
-        return [InferenceKeypointsResult.from_records(rec, b, f, None, None, m.limbs, m.det_thr, m.tag_thr)
+        return [InferenceKeypointsResult.from_records(rec, b, f, None, None, m.limbs, m.det_thr, m.tag_thr,
+                                                      rendered=rendered[b])
                 for b, f in enumerate(frames)]
